@@ -26,6 +26,14 @@ One "step" = one pass over the whole genome:
   secondary    BASELINE.json configs[1] (750 PWMs x 50,000 1 kb peaks per GPU, weak-scaled as in round 1),
                device-resident and end to end, in the `configs1` block of the same JSON line.
 Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` (rank 0) writes, after the timed steps, what the last timed step of each path returned, as
+float64 .npy files: `genome_counts` (per-motif site counts of the genome-wide scan, gathered over the ranks),
+`genome_sites_{motif,chrom,start,score,strand}` (a fixed, seeded sample of DUMP_SITES sites of rank 0's share,
+from the end-to-end leg, in site order), `configs1_counts` (rank 0's per-motif counts of the secondary block's
+device-resident leg) and `configs1_sites_{motif,region,start,score,strand}` (the same kind of sample of rank 0's
+sites from the secondary block's end-to-end leg; `start` is relative to the peak `region`).  The inputs are
+seeded, so two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import hashlib
@@ -56,6 +64,7 @@ MIN_UNIT_BP = 1 << 24             # last download (the only copies nothing hides
 # secondary block (configs[1])
 N_REGIONS = 50000
 REGION_BP = 1000
+DUMP_SITES = 1 << 19              # --dump-outputs: 2 samples of 5 float64 arrays of this many sites, 40 MB
 
 
 def genome_shape(scale=1.0):
@@ -466,6 +475,22 @@ def compare_window(res, ref_sites):
     return int(counts.sum()), bad
 
 
+def site_sample(prefix, offsets, arrays, n=DUMP_SITES, seed=0):
+    """A seeded sample of `n` sites of a motif-major result (all of them when there are fewer), in site order:
+    `<prefix>_motif` from the per-motif `offsets`, and `<prefix>_<name>` for every per-site array of `arrays`."""
+    total = int(offsets[-1])
+    idx = np.sort(np.random.default_rng(seed).choice(total, size=min(n, total), replace=False))
+    out = {prefix + "_motif": np.searchsorted(offsets, idx, side="right") - 1}
+    out.update({f"{prefix}_{name}": a[idx] for name, a in arrays.items()})
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args, rank, local_rank, world):
     import torch
     from motifscan_b200 import _lib, engine
@@ -622,11 +647,15 @@ def run_ours(args, rank, local_rank, world):
     if rank == 0:
         assert np.array_equal(total_b, total_counts) and np.array_equal(total_c, total_counts), "legs disagree on the per-motif counts"
     merge_ms = None
+    outputs = {"genome_counts": total_counts} if rank == 0 else {}
     if kept is not None:
         t0 = time.perf_counter()
         n_merged = len(kept.start)                            # the lazy host-side gather of the site arrays
         merge_ms = 1e3 * (time.perf_counter() - t0)
         assert n_merged == sites_here
+        if rank == 0 and args.dump_outputs:
+            outputs.update(site_sample("genome_sites", kept.offsets, {"chrom": kept.chrom_idx, "start": kept.start,
+                                                                     "score": kept.score, "strand": kept.strand}))
         kept.close()
     gs.close()
     h2d_all, d2h_all = sum_over_ranks(h2d_bytes), sum_over_ranks(d2h_sites)
@@ -634,6 +663,8 @@ def run_ours(args, rank, local_rank, world):
     # ---- secondary block: configs[1] -------------------------------------------------------------------------
     c1 = configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_over_ranks, rank, world, local_rank)
     launches += c1.pop("_launches")
+    outputs["configs1_counts"] = c1.pop("_counts")
+    outputs.update(c1.pop("_sample"))
     launches_all = sum_over_ranks(launches)
 
     if rank == 0:
@@ -721,6 +752,8 @@ def run_ours(args, rank, local_rank, world):
         if cpu is not None:
             line["cpu_baseline"] = cpu["all_cores"]
             line["cpu_baseline_1thread"] = cpu["one_thread"]
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     else:
         pass
@@ -771,6 +804,15 @@ def cpu_legs(engine, ctx, pg, pwms, cutoffs):
     return out
 
 
+def configs1_regions(pg, rank):
+    """A rank's configs[1] peaks: the largest chromosome and the sorted starts of its REGION_BP-base windows."""
+    chrom = max(pg.chroms, key=lambda c: pg.chrom_sizes[c])
+    size = pg.chrom_sizes[chrom]
+    rng = np.random.default_rng(50 + rank)
+    n_regions = min(N_REGIONS, max(size // (2 * REGION_BP), 1))
+    return chrom, np.sort(rng.integers(0, max(size - REGION_BP, 1), size=n_regions)).astype(np.int64)
+
+
 def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_over_ranks, rank, world, local_rank):
     """BASELINE.json configs[1] per GPU (weak-scaled, as in round 1): 50,000 peaks of 1 kb x 750 PWMs.
     `value`: the peaks' packed windows resident in HBM.  `e2e`: the product's resident-genome scanner path --
@@ -779,17 +821,15 @@ def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_ove
     k's sites overlaps step k + 1) and the timed region ends when the last step's sites are on the host."""
     import oracle  # noqa: F401  (CPU legs only, below)
     from motifscan_b200.genome import DeviceGenome
-    chrom = max(pg.chroms, key=lambda c: pg.chrom_sizes[c])
+    chrom, starts = configs1_regions(pg, rank)
     size = pg.chrom_sizes[chrom]
+    n_regions = len(starts)
 
     class One:                      # the largest chromosome, resident on this rank's GPU
         chroms, chrom_sizes = [chrom], {chrom: size}
     b0 = int(pg.block_off[pg.chrom_index[chrom]])
     nb = (size + 31) // 32
     resident = engine.SequenceSet.from_packed(ctx, [size], *pg.planes(b0, b0 + nb))
-    rng = np.random.default_rng(50 + rank)
-    n_regions = min(N_REGIONS, max(size // (2 * REGION_BP), 1))
-    starts = np.sort(rng.integers(0, max(size - REGION_BP, 1), size=n_regions)).astype(np.int64)
     idx = np.zeros(n_regions, dtype=np.int32)
     motifs = engine.MotifSet(ctx, pwms, cutoffs)
     units = N_MOTIFS * n_regions * REGION_BP
@@ -812,6 +852,7 @@ def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_ove
         launches += ctx.counters()["launches"]
     dev_ms = [phase["prefilter"][i] + phase["exact"][i] + phase["order"][i] for i in range(args.steps)]
     ms = max_over_ranks(sum(dev_ms) / len(dev_ms))
+    counts = ctx.site_counts(N_MOTIFS)
     windows.close()
 
     # end to end: two scanner workers on this GPU -- two host threads, each with its own context (stream), motif set
@@ -824,7 +865,7 @@ def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_ove
         c2 = engine.Context(local_rank)
         workers.append((c2, engine.MotifSet(c2, pwms, cutoffs), engine.SequenceSet.from_packed(c2, [size], *pg.planes(b0, b0 + nb))))
 
-    def run_worker(k, n_steps, out):
+    def run_worker(k, n_steps, out, keep):
         c, mo, res_genome = workers[k]
         prev, n_launch = None, 0
         for _ in range(n_steps):
@@ -837,13 +878,15 @@ def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_ove
                 prev.close()
             prev = res
         prev.wait()
-        out[k] = (prev.n_sites, n_launch)
-        prev.close()
+        out[k] = (prev.n_sites, n_launch, prev if keep else None)
+        if not keep:
+            prev.close()
 
-    def run_all(n_steps):
+    def run_all(n_steps, keep_last=False):
+        """`keep_last`: worker 0 returns its last result unclosed (for --dump-outputs)."""
         per = [n_steps // n_workers + (1 if k < n_steps % n_workers else 0) for k in range(n_workers)]
         out = [None] * n_workers
-        threads = [threading.Thread(target=run_worker, args=(k, per[k], out)) for k in range(n_workers) if per[k]]
+        threads = [threading.Thread(target=run_worker, args=(k, per[k], out, keep_last and k == 0)) for k in range(n_workers) if per[k]]
         for t in threads:
             t.start()
         for t in threads:
@@ -851,14 +894,19 @@ def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_ove
         return [o for o in out if o is not None]
     run_all(2 * min(args.warmup, 3))
     barrier()
-    e2e_steps = max(args.steps, 2 * n_workers)
+    e2e_steps = args.steps
     t0 = time.perf_counter()
-    done = run_all(e2e_steps)
+    done = run_all(e2e_steps, keep_last=bool(args.dump_outputs) and rank == 0)
     e2e_ms = 1e3 * (time.perf_counter() - t0) / e2e_steps
     sites = done[0][0]
     launches += sum(o[1] for o in done)
     barrier()
     e2e_ms = max_over_ranks(e2e_ms)
+    sample, last = {}, done[0][2]
+    if last is not None:
+        sample = site_sample("configs1_sites", last.offsets, {"region": last.seq_idx, "start": last.start,
+                                                              "score": last.score, "strand": last.strand})
+        last.close()
     for c2, mo2, rs2 in workers[1:]:
         mo2.close(), rs2.close(), c2.close()
     block = {
@@ -871,9 +919,10 @@ def configs1_block(args, engine, ctx, pg, pwms, cutoffs, torch, barrier, max_ove
                 "h2d_bytes_per_step": world * 20 * n_regions, "d2h_bytes_per_step": world * (12 * int(sites) + 8 * (N_MOTIFS + 1)),
                 "what": "region descriptors up, windows cut from the resident chromosome on the device, scan, all sites down (12 B each: "
                         "score + packed position and strand, MSB_SCAN_COMPACT); "
-                        f"{n_workers} scanner workers (host thread + context each) on the GPU, steps pipelined with MSB_SCAN_ASYNC; "
+                        f"{len(done)} scanner worker(s) (host thread + context each) on the GPU, a worker's consecutive steps "
+                        "pipelined with MSB_SCAN_ASYNC; "
                         "wall clock over all steps until the last sites are on the host", "steps": e2e_steps},
-        "_launches": launches,
+        "_launches": launches, "_counts": counts, "_sample": sample,
     }
     if world == 1 and not args.no_cpu:
         # Scanner-level CPU baseline (BASELINE.md section 3): the reference's Scanner.scan_motifs =
@@ -907,7 +956,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--scale", type=float, default=1.0, help="shrink every chromosome by this factor (development only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
