@@ -5,6 +5,8 @@
     python bench_configs.py build      configs[2]: motif --build, 750 motifs x 1e6 background samples
     python bench_configs.py genome     configs[3]: genome-wide scan, one GPU's share (1/8 of 3.1 Gbp)
     python bench_configs.py enrich     configs[4]: 200k target + 200k control 1 kb regions, 1900 motifs
+    python bench_configs.py whole-genome --genome-scale 1 --gpus 8
+                                       configs[3] genome with de-duplication (scan --whole-genome), tables and BED
 
 Each prints one JSON line: device-resident and end-to-end time, throughput, and a parity check of a
 bounded sample against the reference's CPU implementation (oracle/_ref when it compiled, else the
@@ -483,9 +485,80 @@ def bench_cli(args):
                        "first_difference": first_diff}}
 
 
+def bench_whole_genome(args):
+    """`scan --whole-genome` on the configs[3] genome and motif set (bench.py's: 750 motifs, cutoffs at p = 1e-4
+    floored at 1e-6) with the reference's de-duplication over whole chromosomes: the tables alone (no site array
+    leaves a device) and with every site gathered and written as BED, on one GPU and on `--gpus N` in the same
+    process.  The BED files go to a temporary directory (`--out-dir`) that is deleted afterwards."""
+    import shutil
+    import subprocess
+    import tempfile
+    import bench
+    from motifscan_b200 import _lib, engine
+    from motifscan_b200 import io as msio
+    from motifscan_b200.genome_scan import GenomeScanner
+    from motifscan_b200.region import GenomicRegion
+
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+    pg = bench.make_genome(0, args.genome_scale)
+    mats = bench.motif_workload()
+    ctx = engine.default_context(0)
+    cutoffs = bench.scan_cutoffs(bench.cutoffs_gpu(engine, ctx, mats))
+
+    class Pwm:
+        def __init__(self, k, m):
+            self.matrix_id, self.name, self.length = f"SYN{k:04d}.1", f"motif{k}", int(np.asarray(m).shape[1])
+    pwms = [Pwm(k, m) for k, m in enumerate(mats)]
+    regions = [GenomicRegion(c, 0, pg.chrom_sizes[c]) for c in pg.chroms]
+    total_bp = sum(pg.chrom_sizes.values())
+    out_root = tempfile.mkdtemp(prefix="msb_wg_", dir=args.out_dir)
+    legs = []
+    try:
+        for n in sorted({1, args.gpus}):
+            devices = list(range(n))
+            gs = GenomeScanner(pg, mats, cutoffs=cutoffs, devices=devices, unit_bp=bench.UNIT_BP)
+            raw = gs.scan(collect_sites=False)                  # sites before de-duplication (counts only)
+            n_raw = int(raw.counts.sum())
+            gs.close()
+            for site in (False, True):
+                gs = GenomeScanner(pg, mats, cutoffs=cutoffs, devices=devices, unit_bp=bench.UNIT_BP, remove_dup=True)
+                out_dir = os.path.join(out_root, f"{n}gpu_{int(site)}")
+                t0 = time.perf_counter()
+                res = gs.scan(collect_sites=site)
+                t_scan = time.perf_counter() - t0
+                msio.write_cell_tables(out_dir, pwms, regions, res.cell_counts.T, res.cell_best.T)
+                t_tables = time.perf_counter() - t0 - t_scan
+                leg = {"gpus": n, "site": site, "scan_s": t_scan, "tables_s": t_tables, "sites_raw": n_raw,
+                       "sites_dedup": int(res.counts.sum()), "stitch": gs.last_stitch,
+                       "device_ms": {k: sum(st.get(k, 0.0) for st in gs.last_stats) for k in ("prefilter", "exact", "order")},
+                       "note": "device_ms: summed over the GPUs; 'order' holds the sort, decode, de-duplication and boundary chains"}
+                if site:
+                    t1 = time.perf_counter()
+                    _ = res.chrom_idx                            # gather + corrections
+                    leg["gather_s"] = time.perf_counter() - t1
+                    t1 = time.perf_counter()
+                    msio.write_sites_bed(out_dir, pwms, regions, res)
+                    leg["bed_write_s"] = time.perf_counter() - t1
+                    leg["bed_bytes"] = sum(os.path.getsize(os.path.join(out_dir, "motif_sites", f))
+                                           for f in os.listdir(os.path.join(out_dir, "motif_sites")))
+                leg["wall_s"] = time.perf_counter() - t0
+                leg["motif_bp_per_s_scan"] = len(mats) * total_bp / t_scan
+                legs.append(leg)
+                gs.close()
+                shutil.rmtree(out_dir, ignore_errors=True)
+    finally:
+        shutil.rmtree(out_root, ignore_errors=True)
+    return {"config": f"whole-genome scan with de-duplication: {total_bp} bp synthetic hg19-shaped genome "
+                      f"(scale {args.genome_scale}) x {len(mats)} motifs, both strands, p=1e-4 cutoffs floored at 1e-6",
+            "card": smi.stdout.strip().splitlines(), "devices_visible": _lib.device_count(), "legs": legs,
+            "note": "wall_s = scan + tables (+ gather + BED write); the genome is generated and packed before the timed "
+                    "region; one pass per leg, no warm-up besides the counts-only pass"}
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("which", choices=["build", "genome", "enrich", "cli"])
+    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome"])
+    ap.add_argument("--out-dir", dest="out_dir", default=None)
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--genome-scale", dest="genome_scale", type=float, default=0.1)
     ap.add_argument("--steps", type=int, default=2)
@@ -502,7 +575,8 @@ def main():
     args = ap.parse_args()
     if args.motifs is None:
         args.motifs = 1900 if args.which in ("enrich", "cli") else 750
-    out = {"build": bench_build, "genome": bench_genome, "enrich": bench_enrich, "cli": bench_cli}[args.which](args)
+    out = {"build": bench_build, "genome": bench_genome, "enrich": bench_enrich, "cli": bench_cli,
+           "whole-genome": bench_whole_genome}[args.which](args)
     if out is not None:
         print(json.dumps(out))
 

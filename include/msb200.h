@@ -181,8 +181,10 @@ int msb_scan_ascii(msb_ctx *ctx, const msb_motifs *motifs, int64_t n_seqs, const
  * of its sequence, exactly as if the whole sequence had been scanned (cscore.c:336-340), so the
  * union over a partition of a chromosome into ranges equals the unchunked scan and no overlap has
  * to be shipped.  `end` is clipped at the sequence length; ranges must not overlap (MSB_EINVAL).
- * seq_idx / start of the sites refer to `seqs`.  MSB_SCAN_DEDUP is rejected (MSB_EINVAL): the reference
- * de-duplicates over a whole region's site list (scanner.py:171-193), which a range boundary would cut. */
+ * seq_idx / start of the sites refer to `seqs`.  MSB_SCAN_DEDUP de-duplicates per range when no sequence
+ * appears in more than one range of the call (MSB_EINVAL otherwise: the reference de-duplicates over a whole
+ * region's site list, scanner.py:171-193, which a second range of the sequence would cut); the chains of
+ * overlapping sites at the range edges are then kept for msb_scan_device_boundary_sites. */
 int msb_scan_ranges(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *seqs, int strand,
                     int flags, int64_t n_ranges, const int64_t *seq_idx, const int64_t *start,
                     const int64_t *end, msb_result **out);
@@ -199,6 +201,21 @@ int msb_scan_device_counts(msb_ctx *ctx, int64_t *counts, int32_t n_motifs);
  * msb_scan_ranges_device on this context: the only thing motif_enrichment needs from a scan
  * (stats.py:29-31 counts the regions whose site list is non-empty), reduced on the device. */
 int msb_scan_device_region_counts(msb_ctx *ctx, int64_t *counts, int32_t n_motifs);
+/* Boundary chains of the last msb_scan_ranges / msb_scan_ranges_device with MSB_SCAN_DEDUP on this context
+ * (MSB_EINVAL after any other scan).  A range is a piece of a longer sequence whose neighbours were scanned
+ * on their own; a dedup chain (same-strand sites with consecutive starts less than the motif length L apart)
+ * at a range edge may continue into a neighbour.  Per (motif, range, strand) the sites of the HEAD chain (the
+ * first chain, if its first site starts less than L - 1 bases after the range start) and of the TAIL chain
+ * (the last chain, if its last site starts after range end - L) come back raw, before de-duplication, in the
+ * order of the scan's sites: motif, seq_idx, start (relative to the sequence), score, strand and flags
+ * (bit 0: kept by the per-range de-duplication, bit 1: head chain, bit 2: tail chain; a chain that is both
+ * is listed once).  *n receives the number of such sites; the arrays are filled when cap >= *n. */
+int msb_scan_device_boundary_sites(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *motif, int32_t *seq_idx,
+                                   int32_t *start, double *score, int8_t *strand, int8_t *flags);
+/* Per (motif, sequence) cell of the last msb_scan_device / msb_scan_ranges_device on this context, reduced on
+ * the device: counts[m * n_seqs + s] = number of final sites, best[...] = their best score (NaN when empty).
+ * n_seqs must be the scanned set's sequence count.  Not after MSB_SCAN_COUNTS or a compact scan. */
+int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, int64_t *counts, double *best);
 int msb_result_wait(msb_result *res);
 int msb_result_total(const msb_result *res, int64_t *n_sites);
 int msb_result_counts(const msb_result *res, int64_t *counts /* n_motifs */);
@@ -244,6 +261,18 @@ int msb_merge_sites_compact(int32_t n_parts, int32_t n_motifs, const int64_t *co
 int msb_format_site_tables(int32_t n_motifs, const int64_t *offsets, const int32_t *seq_idx, const double *score,
                            int64_t r0, int64_t r1, const char *lead, const int64_t *lead_off, char **num_text,
                            int64_t *num_len, char **score_text, int64_t *score_len, int32_t n_threads);
+/* The same rows from dense cells: counts / best are n_rows x n_motifs row-major (best ignored where the count
+ * is 0); rows [0, n_rows) of lead / lead_off. */
+int msb_format_cell_tables(int64_t n_rows, int32_t n_motifs, const int64_t *counts, const double *best, const char *lead,
+                           const int64_t *lead_off, char **num_text, int64_t *num_len, char **score_text,
+                           int64_t *score_len, int32_t n_threads);
+/* One motif's motif_sites/<id>_<name>_sites.bed (io/__init__.py:41-55) written to `path`: per site, in the given
+ * order, "chrom<TAB>s<TAB>s + length<TAB>.<TAB>score<TAB>strand" with chrom = names[name_off[g] .. name_off[g + 1])
+ * of the site's group g, s = start + group_base[g] (group_base may be NULL), the score printed like Python's
+ * str() and strand 1 -> '+', else '-'.  Formatted in blocks on up to n_threads host threads, written in order. */
+int msb_write_sites_bed(const char *path, int64_t n, const int32_t *group, const int32_t *start, const int64_t *group_base,
+                        const double *score, const int8_t *strand, int32_t length, int64_t n_groups, const char *names,
+                        const int64_t *name_off, int32_t n_threads);
 int msb_text_free(char *text);
 
 /* ---- score (replaces motif_score_thread + motif_score, cscore.c:174-302) -------------------- */

@@ -69,6 +69,8 @@ SIGNATURES = {
     "msb_scan_device": (ctypes.c_int, [c_vp, c_vp, c_vp, ctypes.c_int, ctypes.c_int, c_i64p]),
     "msb_scan_device_counts": (ctypes.c_int, [c_vp, c_i64p, ctypes.c_int32]),
     "msb_scan_device_region_counts": (ctypes.c_int, [c_vp, c_i64p, ctypes.c_int32]),
+    "msb_scan_device_boundary_sites": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_f64p, c_i8p, c_i8p]),
+    "msb_scan_device_cell_stats": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int64, c_i64p, c_f64p]),
     "msb_result_wait": (ctypes.c_int, [c_vp]),
     "msb_merge_motif_major": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, c_i64p, ctypes.POINTER(c_vp), c_vp,
                                              ctypes.c_int32, c_i64p, ctypes.c_int32]),
@@ -80,6 +82,10 @@ SIGNATURES = {
                                           ctypes.POINTER(c_i64p), c_i64p]),
     "msb_format_site_tables": (ctypes.c_int, [ctypes.c_int32, c_i64p, c_i32p, c_f64p, ctypes.c_int64, ctypes.c_int64, ctypes.c_char_p,
                                               c_i64p, ctypes.POINTER(c_vp), c_i64p, ctypes.POINTER(c_vp), c_i64p, ctypes.c_int32]),
+    "msb_format_cell_tables": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32, c_i64p, c_f64p, ctypes.c_char_p, c_i64p,
+                                              ctypes.POINTER(c_vp), c_i64p, ctypes.POINTER(c_vp), c_i64p, ctypes.c_int32]),
+    "msb_write_sites_bed": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int64, c_i32p, c_i32p, c_i64p, c_f64p, c_i8p, ctypes.c_int32,
+                                           ctypes.c_int64, ctypes.c_char_p, c_i64p, ctypes.c_int32]),
     "msb_text_free": (ctypes.c_int, [c_vp]),
     "msb_result_total": (ctypes.c_int, [c_vp, c_i64p]),
     "msb_result_counts": (ctypes.c_int, [c_vp, c_i64p]),

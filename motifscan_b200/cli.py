@@ -12,7 +12,16 @@ Same flags as the reference's subcommands (cli/main.py:407-430, 504-579) and the
     the gene-distance-matched branch of cli/scan.py needs the annotation layer, which is out of
     scope -- when the genome directory holds an annotation file a warning says so;
 
+  * `scan --whole-genome` (instead of `-i`) scans every chromosome end to end and writes exactly what
+    `scan -i <one BED line "chrom 0 size" per chromosome> -w 0 --no-enrich` writes: one table row per
+    chromosome and, with `--site`, the de-duplicated sites.  The genome is always scanned through its packed
+    planes (`<name>.packed.*` cache, written when missing), cut into equal-work shares with `--gpus N`;
+    de-duplication runs per piece on the device and the chains of overlapping sites that cross a piece
+    boundary are joined on the host.  There is no control set, so no enrichment: `-c`, `--cf` and `--loc` are
+    errors; `-w`, `--n-random` and `--seed` are ignored;
+
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir
+    python -m motifscan_b200 scan --whole-genome -m <motif set> -g <genome> -o out_dir [--site]
     python -m motifscan_b200 motif --build <motif set> -g <genome>
 """
 import argparse
@@ -96,7 +105,51 @@ def load_built_pwms(name, genome_name):
     return pwms
 
 
+def run_whole_genome(args):
+    """`scan --whole-genome`: every chromosome as one region, through GenomeScanner with remove_dup."""
+    import time
+    from .genome_scan import GenomeScanner
+    from .region import GenomicRegion
+    logger.info("===== Loading data =====")
+    genome = load_genome(args.genome)
+    pwms = load_built_pwms(args.motif, genome.name)
+    try:
+        cutoffs = [pwm.cutoffs[args.p_value] for pwm in pwms]
+    except (TypeError, KeyError):
+        raise SystemExit(f"motifscan: error: PWMs have no motif score cutoff set for P-value {args.p_value!r}")
+    logger.info("===== Scanning motifs (whole genome) =====")
+    devices = _devices(args.n_gpus)
+    pg = packed_genome(genome, PACKED_MIN_BP, devices[0])
+    regions = [GenomicRegion(c, 0, genome.chrom_sizes[c]) for c in pg.chroms]
+    t0 = time.perf_counter()
+    gs = GenomeScanner(pg, pwms, cutoffs=cutoffs, strand=args.strand, devices=devices, remove_dup=True)
+    try:
+        sites = gs.scan(collect_sites=args.report_site)
+    finally:
+        gs.close()
+    seconds = time.perf_counter() - t0
+    total_bp = sum(genome.chrom_sizes[c] for c in pg.chroms)
+    logger.info(f"Scanned {len(pwms)} motifs x {total_bp} bp in {seconds:.3f} s: "
+                f"{len(pwms) * total_bp / max(seconds, 1e-12):.3e} motif*bp/s, {int(sites.counts.sum())} sites")
+    logger.info("Saving the result tables")
+    msio.write_cell_tables(args.output_dir, pwms, regions, sites.cell_counts.T, sites.cell_best.T)
+    if args.report_site:
+        msio.write_sites_bed(args.output_dir, pwms, regions, sites)
+    logger.info("===== MotifScan Finished =====")
+    return 0
+
+
 def run_scan(args):
+    if args.whole_genome == (args.input_file is not None):
+        raise SystemExit("motifscan scan: error: give exactly one of -i and --whole-genome")
+    if args.whole_genome:
+        for flag, given in (("-c", args.control_file is not None), ("--cf", args.control_format_given),
+                            ("--loc", args.location is not None)):
+            if given:
+                raise SystemExit(f"motifscan scan: error: {flag} has no meaning with --whole-genome (no enrichment)")
+        if args.plot_dist:
+            raise SystemExit("motifscan scan: --plot needs matplotlib, which is out of scope here")
+        return run_whole_genome(args)
     if args.location is not None:
         raise SystemExit("motifscan scan: --loc needs the gene annotation layer, which is out of scope here")
     if args.plot_dist:
@@ -190,7 +243,10 @@ def make_parser():
     sub = parser.add_subparsers(dest="command", required=True)
 
     scan = sub.add_parser("scan", help="Scan input regions to detect motif occurrences.")
-    scan.add_argument("-i", dest="input_file", required=True, metavar="FILE")
+    scan.add_argument("-i", dest="input_file", metavar="FILE")
+    scan.add_argument("--whole-genome", dest="whole_genome", action="store_true",
+                      help="scan every chromosome end to end instead of -i regions (implies --no-enrich; "
+                           "-w, --n-random and --seed are ignored)")
     scan.add_argument("-f", dest="input_format", choices=sorted(REGION_FORMATS), default="bed")
     scan.add_argument("-m", "--motif", dest="motif", required=True, metavar="NAME")
     scan.add_argument("-g", "--genome", dest="genome", required=True, metavar="GENOME")
@@ -204,7 +260,7 @@ def make_parser():
     scan.add_argument("--n-random", dest="n_random", type=_non_negative, default=5)
     scan.add_argument("--seed", dest="seed", type=int, default=None)
     scan.add_argument("-c", dest="control_file", metavar="FILE")
-    scan.add_argument("--cf", dest="control_format", choices=sorted(REGION_FORMATS), default="bed")
+    scan.add_argument("--cf", dest="control_format", choices=sorted(REGION_FORMATS), default=None)
     scan.add_argument("-t", "--threads", dest="n_threads", type=int, default=1)
     scan.add_argument("--gpus", dest="n_gpus", type=_positive, default=1, metavar="N",
                       help="GPUs of this box to scan on (regions are dealt to them in contiguous blocks)")
@@ -229,6 +285,10 @@ def make_parser():
 
 def main(argv=None):
     args = make_parser().parse_args(argv)
+    if args.command == "scan":
+        args.control_format_given = args.control_format is not None
+        if args.control_format is None:
+            args.control_format = "bed"
     logging.basicConfig(stream=sys.stderr, level=logging.DEBUG if args.verbose else logging.INFO,
                         format="%(message)s")
     return args.func(args)

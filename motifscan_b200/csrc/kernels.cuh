@@ -928,4 +928,102 @@ __global__ void __launch_bounds__(256) fill_i32_kernel(int32_t *__restrict__ p, 
     if (i < n) p[i] = v;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Boundary chains of a de-duplicated range scan.  A range [lo, hi) (packed positions) is a piece of a
+// longer sequence; the dedup chains of its edges may continue into the neighbouring pieces, which were
+// resolved on their own.  Per (motif, range) cell and strand, the HEAD chain (the first chain, when its
+// first site starts less than L - 1 bases into the range: a site of the preceding piece may sit less than
+// L before it) and the TAIL chain (the last chain, when its last site starts after hi - L) are emitted raw,
+// with their keep flags, so that the host can re-run the greedy rule over the joined chain.
+// One thread per cell; the walks never go further than the chains plus L positions.
+// Emitted flag bits: 1 kept by the device, 2 in the head chain, 4 in the tail chain.
+// mode 0: count[cell] = sites to emit; mode 1: write them at dst[cell] in site order.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+boundary_chains_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ seq_idx,
+                       const int32_t *__restrict__ start, const int8_t *__restrict__ strand,
+                       const double *__restrict__ score, const int32_t *__restrict__ keep, int64_t n,
+                       const int64_t *__restrict__ r_lo, const int64_t *__restrict__ r_hi, int64_t n_ranges,
+                       int32_t n_motifs, const int32_t *__restrict__ mlen, int key_shift, int mode,
+                       int64_t *__restrict__ count, const int64_t *__restrict__ dst, int32_t *__restrict__ o_motif,
+                       int32_t *__restrict__ o_seq, int32_t *__restrict__ o_start, double *__restrict__ o_score,
+                       int8_t *__restrict__ o_strand, int8_t *__restrict__ o_flags) {
+    const int64_t cell = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (cell >= (int64_t) n_motifs * n_ranges) return;
+    const uint32_t m = (uint32_t) (cell / n_ranges);
+    const int64_t r = cell % n_ranges, lo_p = r_lo[r], hi_p = r_hi[r];
+    const int32_t L = __ldg(mlen + m);
+    auto lower = [&](uint64_t k) {
+        int64_t a = 0, b = n;
+        while (a < b) { const int64_t mid = (a + b) >> 1; if (key[mid] < k) a = mid + 1; else b = mid; }
+        return a;
+    };
+    const int64_t a = lower(make_site_key(m, lo_p, 0, key_shift)), b = lower(make_site_key(m, hi_p, 0, key_shift));
+    int64_t emitted = 0;
+    if (b <= a) { if (mode == 0) count[cell] = 0; return; }
+    // head_end[x]: index of the last site of strand x's head chain (-1: none); tail_begin[x]: first site of its tail chain (n: none)
+    int64_t head_end[2] = {-1, -1}, tail_begin[2] = {n, n};
+    for (int x = 0; x < 2; x++) {
+        int64_t last = -1;
+        for (int64_t t = a; t < b; t++) {   // position tests first: they also end the walk on the other strand's sites
+            const int64_t p = site_pos(key[t], key_shift);
+            if (last < 0 ? p - lo_p >= L - 1 : p - site_pos(key[last], key_shift) >= L) break;
+            if ((int) key_rev(key[t]) == x) last = t;
+        }
+        head_end[x] = last;
+        int64_t first = n;
+        for (int64_t t = b - 1; t >= a; t--) {
+            const int64_t p = site_pos(key[t], key_shift);
+            if (first == n ? p <= hi_p - L : site_pos(key[first], key_shift) - p >= L) break;
+            if ((int) key_rev(key[t]) == x) first = t;
+        }
+        tail_begin[x] = first;
+    }
+    const int64_t h1 = max(head_end[0], head_end[1]);
+    const int64_t t0 = min(tail_begin[0], tail_begin[1]);
+    int64_t at = mode ? dst[cell] : 0;
+    for (int64_t t = a; t < b; t++) {
+        if (t > h1 && t < t0) { t = t0 - 1; continue; }   // the middle of the cell: nothing there to emit
+        const int x = (int) key_rev(key[t]);
+        const int fl = (t <= head_end[x] ? 2 : 0) | (t >= tail_begin[x] ? 4 : 0);
+        if (!fl) continue;
+        if (mode) {
+            o_motif[at] = (int32_t) m;
+            o_seq[at] = seq_idx[t];
+            o_start[at] = start[t];
+            o_score[at] = score[t];
+            o_strand[at] = strand[t];
+            o_flags[at] = (int8_t) (fl | (keep[t] ? 1 : 0));
+            at++;
+        }
+        emitted++;
+    }
+    if (mode == 0) count[cell] = emitted;
+}
+
+// Per (motif, sequence) cell of a scan's final (motif, sequence)-ordered sites: the number of sites and the best
+// score as an order_key (signed scores compare correctly as unsigned keys).  One thread per run of 32 sites, which
+// sums runs of one cell locally: the sites are sorted, so the atomics are one per cell boundary, not per site.
+__global__ void __launch_bounds__(256)
+cell_stats_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ seq_idx, const double *__restrict__ score,
+                  int64_t n, int key_shift, int64_t n_seqs, unsigned long long *__restrict__ count,
+                  unsigned long long *__restrict__ best) {
+    const int64_t i0 = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) * 32;
+    if (i0 >= n) return;
+    const int64_t i1 = min(i0 + 32, n);
+    int64_t cell = -1;
+    unsigned long long c = 0, k = 0;
+    for (int64_t i = i0; i < i1; i++) {
+        const int64_t ci = (int64_t) site_motif(key[i], key_shift) * n_seqs + seq_idx[i];
+        if (ci != cell) {
+            if (cell >= 0) { atomicAdd(count + cell, c); atomicMax(best + cell, k); }
+            cell = ci, c = 0, k = 0;
+        }
+        c++;
+        k = max(k, (unsigned long long) order_key(score[i]));
+    }
+    atomicAdd(count + cell, c);
+    atomicMax(best + cell, k);
+}
+
 }  // namespace msb

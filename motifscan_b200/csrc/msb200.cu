@@ -81,6 +81,9 @@ struct msb_ctx {
     DevBuf out_seq, out_start, out_strand, scores, scores_sorted, seg_off, ranks, sel;
     DevBuf keep, keep_pos, motif_counts, sel_aux, limit1;
     DevBuf lane_count;   // tensor-core prefilter: records per epilogue lane
+    // boundary chains of the last de-duplicated range scan (msb_scan_device_boundary_sites)
+    DevBuf bnd_range, bnd_cnt, bnd_dst, bnd_motif, bnd_seq, bnd_start, bnd_score, bnd_strand, bnd_flags;
+    int64_t last_boundary = -1;            // sites in the bnd_* arrays; -1: the last scan collected none
     // Final site arrays of a scan.  Two sets, used alternately: the device-to-host copy of scan k's
     // sites (on d2h_stream, MSB_SCAN_ASYNC) reads one set while scan k + 1 fills the other.
     struct FinSet {
@@ -108,6 +111,7 @@ struct msb_ctx {
     // results of the last msb_scan_device, still on the device
     int64_t last_sites = 0;
     int32_t last_n_motifs = 0;
+    int64_t last_n_seqs = 0;
     int last_key_shift = 0;
     // tuning / test knobs (msb_ctx_set_option): per context, so that contexts driven from different host
     // threads never see each other's settings
@@ -399,7 +403,9 @@ int msb_ctx_destroy(msb_ctx *ctx) {
                       &ctx->key_alt, &ctx->score_alt, &ctx->sort_tmp, &ctx->counters, &ctx->out_seq,
                       &ctx->out_start, &ctx->out_strand, &ctx->scores,
                       &ctx->scores_sorted, &ctx->seg_off, &ctx->ranks, &ctx->sel, &ctx->keep, &ctx->keep_pos,
-                      &ctx->motif_counts, &ctx->sel_aux, &ctx->limit1, &ctx->lane_count})
+                      &ctx->motif_counts, &ctx->sel_aux, &ctx->limit1, &ctx->lane_count, &ctx->bnd_range,
+                      &ctx->bnd_cnt, &ctx->bnd_dst, &ctx->bnd_motif, &ctx->bnd_seq, &ctx->bnd_start, &ctx->bnd_score,
+                      &ctx->bnd_strand, &ctx->bnd_flags})
         b->release();
     if (ctx->d2h_stream) cudaStreamSynchronize(ctx->d2h_stream);
     for (auto &f : ctx->fin) {
@@ -1327,9 +1333,10 @@ typedef std::function<int(size_t)> RangeHook;
 // `limit_override`: a device array of per-sequence start limits used instead of the set's own
 // (msb_score_select scans only the offset-0 window of every sample); `cand_scale`: the candidate buffers
 // are sized for that many times the usual candidate density.
+// `boundary`: with MSB_SCAN_DEDUP, also collect the boundary chains of every range (boundary_chains_kernel).
 static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int strand, int flags,
                        const RangeList *ranges = nullptr, const RangeHook *before_range = nullptr,
-                       const int32_t *limit_override = nullptr, int cand_scale = 1) {
+                       const int32_t *limit_override = nullptr, int cand_scale = 1, bool boundary = false) {
     if (!ctx || !M || !S) { set_error("msb_scan: null argument"); return MSB_EINVAL; }
     if (strand < 1 || strand > 3) { set_error("msb_scan: strand must be 1, 2 or 3"); return MSB_EINVAL; }
     if (M->ctx != ctx || S->ctx != ctx) { set_error("msb_scan: motifs/seqs belong to another context"); return MSB_EINVAL; }
@@ -1358,6 +1365,9 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
     std::fill(ctx->c, ctx->c + MSB_C_COUNT, 0);
     ctx->last_sites = 0;
     ctx->last_n_motifs = M->n;
+    ctx->last_n_seqs = S->n;
+    boundary = boundary && (flags & MSB_SCAN_DEDUP);
+    ctx->last_boundary = boundary ? 0 : -1;
     // this scan's final arrays go to the set the previous scan did not use; a copy that still reads it
     // (an asynchronous result two scans back) is waited for on the device, not on the host
     const int fin_set = ctx->fin_cur ^ 1;
@@ -1664,12 +1674,53 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
                                                       F.seq.as<int32_t>(), F.start.as<int32_t>(), F.strand.as<int8_t>());
             MSB_CUDA(cudaGetLastError());
             ctx->c[MSB_C_LAUNCHES] += 3;
+            // boundary chains, read from the raw sorted sites and their keep flags before anything reuses them
+            const int64_t n_ranges = (int64_t) ranges->size(), cells = (int64_t) M->n * n_ranges;
+            std::vector<int64_t> rr;
+            if (boundary && cells) {
+                rr.resize((size_t) 2 * n_ranges);
+                for (int64_t k = 0; k < n_ranges; k++) { rr[k] = (*ranges)[k].first; rr[n_ranges + k] = (*ranges)[k].second; }
+                MSB_TRY(ctx->bnd_range.ensure(rr.size() * 8));
+                MSB_TRY(ctx->bnd_cnt.ensure((size_t) (cells + 1) * 8));
+                MSB_TRY(ctx->bnd_dst.ensure((size_t) (cells + 1) * 8));
+                MSB_CUDA(cudaMemcpyAsync(ctx->bnd_range.p, rr.data(), rr.size() * 8, cudaMemcpyHostToDevice, st));
+                MSB_CUDA(cudaMemsetAsync(ctx->bnd_cnt.p, 0, (size_t) (cells + 1) * 8, st));
+            }
+            auto chains = [&](int mode) {
+                boundary_chains_kernel<<<(unsigned) ((cells + 255) / 256), 256, 0, st>>>(
+                    s_key.as<uint64_t>(), s_seq.as<int32_t>(), s_start.as<int32_t>(), s_strand.as<int8_t>(), s_score.as<double>(),
+                    ctx->keep.as<int32_t>(), n_hits, ctx->bnd_range.as<int64_t>(), ctx->bnd_range.as<int64_t>() + n_ranges, n_ranges,
+                    M->n, mv.len, key_shift, mode, ctx->bnd_cnt.as<int64_t>(), ctx->bnd_dst.as<int64_t>(), ctx->bnd_motif.as<int32_t>(),
+                    ctx->bnd_seq.as<int32_t>(), ctx->bnd_start.as<int32_t>(), ctx->bnd_score.as<double>(), ctx->bnd_strand.as<int8_t>(),
+                    ctx->bnd_flags.as<int8_t>());
+                ctx->c[MSB_C_LAUNCHES]++;
+                return cudaGetLastError();
+            };
+            int64_t n_boundary = 0;
+            if (boundary && cells) {
+                MSB_CUDA(chains(0));
+                size_t bs = 0;
+                MSB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bs, ctx->bnd_cnt.as<int64_t>(), ctx->bnd_dst.as<int64_t>(), cells + 1, st));
+                MSB_TRY(ctx->sort_tmp.ensure(std::max<size_t>(bs, 16)));
+                MSB_CUDA(cub::DeviceScan::ExclusiveSum(ctx->sort_tmp.p, bs, ctx->bnd_cnt.as<int64_t>(), ctx->bnd_dst.as<int64_t>(), cells + 1, st));
+                MSB_CUDA(cudaMemcpyAsync(&n_boundary, ctx->bnd_dst.as<int64_t>() + cells, 8, cudaMemcpyDeviceToHost, st));
+            }
             int32_t last_keep = 0;
             int64_t last_pos = 0;
             MSB_CUDA(cudaMemcpyAsync(&last_keep, ctx->keep.as<int32_t>() + (n_hits - 1), 4, cudaMemcpyDeviceToHost, st));
             MSB_CUDA(cudaMemcpyAsync(&last_pos, ctx->keep_pos.as<int64_t>() + (n_hits - 1), 8, cudaMemcpyDeviceToHost, st));
             MSB_CUDA(cudaStreamSynchronize(st));
             n_final = last_pos + last_keep;
+            if (n_boundary) {
+                MSB_TRY(ctx->bnd_motif.ensure((size_t) n_boundary * 4));
+                MSB_TRY(ctx->bnd_seq.ensure((size_t) n_boundary * 4));
+                MSB_TRY(ctx->bnd_start.ensure((size_t) n_boundary * 4));
+                MSB_TRY(ctx->bnd_score.ensure((size_t) n_boundary * 8));
+                MSB_TRY(ctx->bnd_strand.ensure((size_t) n_boundary));
+                MSB_TRY(ctx->bnd_flags.ensure((size_t) n_boundary));
+                MSB_CUDA(chains(1));
+                ctx->last_boundary = n_boundary;
+            }
         }
         ctx->fin_key = F.key.as<uint64_t>();
         ctx->fin_score = F.score.as<double>();
@@ -1750,19 +1801,79 @@ int msb_scan_device_region_counts(msb_ctx *ctx, int64_t *counts, int32_t n_motif
     return MSB_OK;
 }
 
+int msb_scan_device_boundary_sites(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *motif, int32_t *seq_idx, int32_t *start,
+                                   double *score, int8_t *strand, int8_t *flags) {
+    if (!ctx || !n) { set_error("msb_scan_device_boundary_sites: null"); return MSB_EINVAL; }
+    if (ctx->last_boundary < 0) {
+        set_error("msb_scan_device_boundary_sites: the last scan was not a de-duplicated range scan (MSB_SCAN_DEDUP)");
+        return MSB_EINVAL;
+    }
+    const int64_t nb = ctx->last_boundary;
+    *n = nb;
+    if (nb == 0 || cap < nb) return MSB_OK;
+    if (!motif || !seq_idx || !start || !score || !strand || !flags) { set_error("msb_scan_device_boundary_sites: null array"); return MSB_EINVAL; }
+    MSB_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    MSB_CUDA(cudaMemcpyAsync(motif, ctx->bnd_motif.p, (size_t) nb * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(seq_idx, ctx->bnd_seq.p, (size_t) nb * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(start, ctx->bnd_start.p, (size_t) nb * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(score, ctx->bnd_score.p, (size_t) nb * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(strand, ctx->bnd_strand.p, (size_t) nb, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(flags, ctx->bnd_flags.p, (size_t) nb, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    return MSB_OK;
+}
+
+int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, int64_t *counts, double *best) {
+    if (!ctx || n_seqs < 0 || ((!counts || !best) && n_motifs && n_seqs)) { set_error("msb_scan_device_cell_stats: null"); return MSB_EINVAL; }
+    if (n_motifs != ctx->last_n_motifs) { set_error("msb_scan_device_cell_stats: no scan with that many motifs"); return MSB_EINVAL; }
+    if (n_seqs != ctx->last_n_seqs) { set_error("msb_scan_device_cell_stats: n_seqs differs from the scanned set"); return MSB_EINVAL; }
+    const size_t cells = (size_t) n_motifs * (size_t) n_seqs;
+    if (cells == 0) return MSB_OK;
+    std::fill(counts, counts + cells, (int64_t) 0);
+    std::fill(best, best + cells, std::numeric_limits<double>::quiet_NaN());
+    if (ctx->last_counts_only) { set_error("msb_scan_device_cell_stats: the last scan kept per-motif counts only (MSB_SCAN_COUNTS)"); return MSB_EINVAL; }
+    if (ctx->last_compact) { set_error("msb_scan_device_cell_stats: the last scan kept compact sites (MSB_SCAN_COMPACT)"); return MSB_EINVAL; }
+    if (ctx->last_sites == 0) return MSB_OK;
+    MSB_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    MSB_TRY(ctx->sel.ensure(cells * 16));
+    MSB_CUDA(cudaMemsetAsync(ctx->sel.p, 0, cells * 16, st));
+    unsigned long long *d_count = ctx->sel.as<unsigned long long>(), *d_best = d_count + cells;
+    cell_stats_kernel<<<(unsigned) ((ctx->last_sites + 32 * 256 - 1) / (32 * 256)), 256, 0, st>>>(
+        ctx->fin_key, ctx->fin_seq, ctx->fin_score, ctx->last_sites, ctx->last_key_shift, n_seqs, d_count, d_best);
+    MSB_CUDA(cudaGetLastError());
+    std::vector<uint64_t> keys(cells);
+    MSB_CUDA(cudaMemcpyAsync(counts, d_count, cells * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(keys.data(), d_best, cells * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    for (size_t c = 0; c < cells; c++) {
+        if (!counts[c]) continue;
+        const uint64_t k = keys[c], b = (k >> 63) ? (k & 0x7fffffffffffffffull) : ~k;   // order_key_inv
+        std::memcpy(best + c, &b, 8);
+    }
+    return MSB_OK;
+}
+
 int msb_scan_ranges_device(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *S, int strand, int flags,
                            int64_t n_ranges, const int64_t *seq_idx, const int64_t *start, const int64_t *end,
                            int64_t *n_sites) {
     if (!S) { set_error("msb_scan_ranges: null seqs"); return MSB_EINVAL; }
-    if (flags & MSB_SCAN_DEDUP) {
-        // the reference de-duplicates over a whole region's site list (scanner.py:171-193); a range boundary
-        // would cut a chain of overlapping sites in two and the halves would be resolved independently
-        set_error("msb_scan_ranges: MSB_SCAN_DEDUP is not defined across range boundaries; scan whole sequences");
-        return MSB_EINVAL;
-    }
     RangeList ranges;
     MSB_TRY(make_ranges(S, n_ranges, seq_idx, start, end, &ranges));
-    MSB_TRY(scan_device(ctx, const_cast<msb_motifs *>(M), S, strand, flags, &ranges));
+    if (flags & MSB_SCAN_DEDUP) {
+        // the reference de-duplicates over a whole region's site list (scanner.py:171-193); two ranges of one
+        // sequence would cut a chain of overlapping sites in two and the halves would be resolved independently.
+        // With one range per sequence the per-sequence de-duplication is per range; the chains at the range edges
+        // are kept for the caller (msb_scan_device_boundary_sites), who knows what lies beyond them.
+        std::vector<int64_t> seqs(seq_idx, seq_idx + n_ranges);
+        std::sort(seqs.begin(), seqs.end());
+        if (std::adjacent_find(seqs.begin(), seqs.end()) != seqs.end()) {
+            set_error("msb_scan_ranges: MSB_SCAN_DEDUP is not defined across range boundaries; scan whole sequences");
+            return MSB_EINVAL;
+        }
+    }
+    MSB_TRY(scan_device(ctx, const_cast<msb_motifs *>(M), S, strand, flags, &ranges, nullptr, nullptr, 1, true));
     if (n_sites) *n_sites = ctx->last_sites;
     return MSB_OK;
 }
@@ -2222,6 +2333,85 @@ static inline int fmt_int(int64_t v, char *out) {
     return k;
 }
 
+template <typename Fn>
+static void run_threads(int nt, Fn &fn) {
+    std::vector<std::thread> pool;
+    for (int t = 1; t < nt; t++) pool.emplace_back(fn, t);
+    fn(0);
+    for (auto &th : pool) th.join();
+}
+
+// Rows of the two tables from dense [row][motif] cells (count, best score) as text, on `nt` host threads.
+template <typename Count>
+static int format_cell_tables(int64_t n_rows, int32_t n_motifs, const Count *counts, const double *best, const char *lead,
+                              const int64_t *lead_off, char **num_text, int64_t *num_len, char **score_text, int64_t *score_len,
+                              int nt) {
+    // a contiguous range of rows per thread, written with a bump pointer into a buffer sized for the worst case
+    // (a count has at most 11 characters as int32, 20 as int64, a double at most 24)
+    struct Part { char *num = nullptr, *score = nullptr; size_t n_num = 0, n_score = 0; };
+    std::vector<Part> parts((size_t) nt);
+    bool oom = false;
+    auto format = [&](int t) {
+        const int64_t a = n_rows * t / nt, b = n_rows * (t + 1) / nt;
+        if (b <= a) return;
+        const size_t lead_bytes = (size_t) (lead_off[b] - lead_off[a]);
+        Part &P = parts[t];
+        P.num = (char *) std::malloc(lead_bytes + (size_t) (b - a) * ((size_t) n_motifs * (sizeof(Count) == 4 ? 12 : 21) + 2));
+        P.score = (char *) std::malloc(lead_bytes + (size_t) (b - a) * ((size_t) n_motifs * 26 + 2));
+        if (!P.num || !P.score) { oom = true; return; }
+        char *pn = P.num, *ps = P.score;
+        for (int64_t r = a; r < b; r++) {
+            const char *l = lead + lead_off[r];
+            const size_t ln = (size_t) (lead_off[r + 1] - lead_off[r]);
+            std::memcpy(pn, l, ln); pn += ln;
+            std::memcpy(ps, l, ln); ps += ln;
+            const Count *c = counts + (size_t) r * n_motifs;
+            const double *s = best + (size_t) r * n_motifs;
+            for (int32_t m = 0; m < n_motifs; m++) {
+                if (m) { *pn++ = '\t'; *ps++ = '\t'; }
+                const int64_t cnt = (int64_t) c[m];
+                if (cnt == 0) {
+                    *pn++ = '0';
+                    *ps++ = 'N'; *ps++ = 'A';
+                } else {
+                    pn += fmt_int(cnt, pn);
+                    ps += py_float_str(s[m], ps);
+                }
+            }
+            *pn++ = '\n';
+            *ps++ = '\n';
+        }
+        P.n_num = (size_t) (pn - P.num);
+        P.n_score = (size_t) (ps - P.score);
+    };
+    run_threads(nt, format);
+    size_t total_num = 0, total_score = 0;
+    for (auto &P : parts) { total_num += P.n_num; total_score += P.n_score; }
+    char *out_num = oom ? nullptr : (char *) std::malloc(std::max<size_t>(total_num, 1));
+    char *out_score = oom ? nullptr : (char *) std::malloc(std::max<size_t>(total_score, 1));
+    if (!out_num || !out_score) {
+        for (auto &P : parts) { std::free(P.num); std::free(P.score); }
+        std::free(out_num); std::free(out_score);
+        set_error("out of host memory");
+        return MSB_ENOMEM;
+    }
+    std::vector<size_t> at_num((size_t) nt), at_score((size_t) nt);
+    size_t an = 0, as = 0;
+    for (int t = 0; t < nt; t++) { at_num[t] = an; at_score[t] = as; an += parts[t].n_num; as += parts[t].n_score; }
+    auto gather = [&](int t) {
+        if (parts[t].n_num) std::memcpy(out_num + at_num[t], parts[t].num, parts[t].n_num);
+        if (parts[t].n_score) std::memcpy(out_score + at_score[t], parts[t].score, parts[t].n_score);
+        std::free(parts[t].num);
+        std::free(parts[t].score);
+    };
+    run_threads(nt, gather);
+    *num_text = out_num;
+    *num_len = (int64_t) total_num;
+    *score_text = out_score;
+    *score_len = (int64_t) total_score;
+    return MSB_OK;
+}
+
 }  // namespace msb
 
 extern "C" {
@@ -2258,76 +2448,72 @@ int msb_format_site_tables(int32_t n_motifs, const int64_t *offsets, const int32
             }
         }
     };
-    // 2. rows -> text, a contiguous range of rows per thread, written with a bump pointer into a buffer sized for
-    //    the worst case (a count has at most 11 characters, a double at most 24)
-    struct Part { char *num = nullptr, *score = nullptr; size_t n_num = 0, n_score = 0; };
-    std::vector<Part> parts((size_t) nt);
-    bool oom = false;
-    auto format = [&](int t) {
-        const int64_t a = n_rows * t / nt, b = n_rows * (t + 1) / nt;
-        if (b <= a) return;
-        const size_t lead_bytes = (size_t) (lead_off[b] - lead_off[a]);
-        Part &P = parts[t];
-        P.num = (char *) std::malloc(lead_bytes + (size_t) (b - a) * ((size_t) n_motifs * 12 + 2));
-        P.score = (char *) std::malloc(lead_bytes + (size_t) (b - a) * ((size_t) n_motifs * 26 + 2));
-        if (!P.num || !P.score) { oom = true; return; }
-        char *pn = P.num, *ps = P.score;
-        for (int64_t r = a; r < b; r++) {
-            const char *l = lead + lead_off[r];
-            const size_t ln = (size_t) (lead_off[r + 1] - lead_off[r]);
-            std::memcpy(pn, l, ln); pn += ln;
-            std::memcpy(ps, l, ln); ps += ln;
-            const int32_t *c = counts.data() + (size_t) r * n_motifs;
-            const double *s = best.data() + (size_t) r * n_motifs;
-            for (int32_t m = 0; m < n_motifs; m++) {
-                if (m) { *pn++ = '\t'; *ps++ = '\t'; }
-                const int32_t cnt = c[m];
-                if (cnt == 0) {
-                    *pn++ = '0';
-                    *ps++ = 'N'; *ps++ = 'A';
-                } else {
-                    pn += fmt_int(cnt, pn);
-                    ps += py_float_str(s[m], ps);
-                }
-            }
-            *pn++ = '\n';
-            *ps++ = '\n';
-        }
-        P.n_num = (size_t) (pn - P.num);
-        P.n_score = (size_t) (ps - P.score);
-    };
-    auto run = [&](auto &fn) {
-        std::vector<std::thread> pool;
-        for (int t = 1; t < nt; t++) pool.emplace_back(fn, t);
-        fn(0);
-        for (auto &th : pool) th.join();
-    };
-    run(fill);
-    run(format);
-    size_t total_num = 0, total_score = 0;
-    for (auto &P : parts) { total_num += P.n_num; total_score += P.n_score; }
-    char *out_num = oom ? nullptr : (char *) std::malloc(std::max<size_t>(total_num, 1));
-    char *out_score = oom ? nullptr : (char *) std::malloc(std::max<size_t>(total_score, 1));
-    if (!out_num || !out_score) {
-        for (auto &P : parts) { std::free(P.num); std::free(P.score); }
-        std::free(out_num); std::free(out_score);
-        set_error("out of host memory");
-        return MSB_ENOMEM;
+    // 2. the rows as text
+    run_threads(nt, fill);
+    return format_cell_tables(n_rows, n_motifs, counts.data(), best.data(), lead, lead_off, num_text, num_len, score_text,
+                              score_len, nt);
+}
+
+int msb_format_cell_tables(int64_t n_rows, int32_t n_motifs, const int64_t *counts, const double *best, const char *lead,
+                           const int64_t *lead_off, char **num_text, int64_t *num_len, char **score_text, int64_t *score_len,
+                           int32_t n_threads) {
+    if (n_rows < 0 || n_motifs < 0 || !lead_off || !num_text || !num_len || !score_text || !score_len ||
+        (n_rows && n_motifs && (!counts || !best))) {
+        set_error("msb_format_cell_tables: bad argument");
+        return MSB_EINVAL;
     }
-    std::vector<size_t> at_num((size_t) nt), at_score((size_t) nt);
-    size_t an = 0, as = 0;
-    for (int t = 0; t < nt; t++) { at_num[t] = an; at_score[t] = as; an += parts[t].n_num; as += parts[t].n_score; }
-    auto gather = [&](int t) {
-        if (parts[t].n_num) std::memcpy(out_num + at_num[t], parts[t].num, parts[t].n_num);
-        if (parts[t].n_score) std::memcpy(out_score + at_score[t], parts[t].score, parts[t].n_score);
-        std::free(parts[t].num);
-        std::free(parts[t].score);
-    };
-    run(gather);
-    *num_text = out_num;
-    *num_len = (int64_t) total_num;
-    *score_text = out_score;
-    *score_len = (int64_t) total_score;
+    *num_text = *score_text = nullptr;
+    *num_len = *score_len = 0;
+    if (n_rows == 0) return MSB_OK;
+    return format_cell_tables(n_rows, n_motifs, counts, best, lead, lead_off, num_text, num_len, score_text, score_len,
+                              std::max(1, std::min<int>(n_threads, 64)));
+}
+
+int msb_write_sites_bed(const char *path, int64_t n, const int32_t *group, const int32_t *start, const int64_t *group_base,
+                        const double *score, const int8_t *strand, int32_t length, int64_t n_groups, const char *names,
+                        const int64_t *name_off, int32_t n_threads) {
+    if (!path || n < 0 || n_groups < 0 || !name_off || (n && (!group || !start || !score || !strand))) {
+        set_error("msb_write_sites_bed: bad argument");
+        return MSB_EINVAL;
+    }
+    size_t name_max = 0;
+    for (int64_t g = 0; g < n_groups; g++) name_max = std::max<size_t>(name_max, (size_t) (name_off[g + 1] - name_off[g]));
+    for (int64_t i = 0; i < n; i++)
+        if (group[i] < 0 || group[i] >= n_groups) { set_error("msb_write_sites_bed: group index out of range"); return MSB_EINVAL; }
+    FILE *f = std::fopen(path, "wb");
+    if (!f) { set_error(std::string("msb_write_sites_bed: cannot open ") + path); return MSB_EINVAL; }
+    // blocks of sites formatted on host threads, written in order: one round of `nt` blocks at a time
+    const int nt = std::max(1, std::min<int>(n_threads, 64));
+    const int64_t block = 1 << 18;
+    const size_t line_max = name_max + 2 * 21 + 3 + 25 + 4;
+    std::vector<std::vector<char>> buf((size_t) nt);
+    std::vector<size_t> used((size_t) nt);
+    try { for (auto &b : buf) b.resize((size_t) std::min(n, block) * line_max); }
+    catch (const std::bad_alloc &) { std::fclose(f); set_error("out of host memory"); return MSB_ENOMEM; }
+    bool io_ok = true;
+    for (int64_t r0 = 0; r0 < n && io_ok; r0 += block * nt) {
+        auto format = [&](int t) {
+            const int64_t a = std::min(n, r0 + block * t), b = std::min(n, a + block);
+            char *o = buf[t].data();
+            for (int64_t i = a; i < b; i++) {
+                const int32_t g = group[i];
+                const size_t ln = (size_t) (name_off[g + 1] - name_off[g]);
+                std::memcpy(o, names + name_off[g], ln); o += ln;
+                const int64_t s0 = (int64_t) start[i] + (group_base ? group_base[g] : 0);
+                *o++ = '\t'; o += fmt_int(s0, o);
+                *o++ = '\t'; o += fmt_int(s0 + length, o);
+                *o++ = '\t'; *o++ = '.'; *o++ = '\t';
+                o += py_float_str(score[i], o);
+                *o++ = '\t'; *o++ = strand[i] == 1 ? '+' : '-'; *o++ = '\n';
+            }
+            used[t] = (size_t) (o - buf[t].data());
+        };
+        run_threads(nt, format);
+        for (int t = 0; t < nt && io_ok; t++)
+            if (used[t] && std::fwrite(buf[t].data(), 1, used[t], f) != used[t]) io_ok = false;
+    }
+    if (std::fclose(f) != 0) io_ok = false;
+    if (!io_ok) { set_error(std::string("msb_write_sites_bed: write to ") + path + " failed"); return MSB_EINVAL; }
     return MSB_OK;
 }
 

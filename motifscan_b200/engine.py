@@ -67,6 +67,34 @@ class Context:
             check(self._lib.msb_scan_device_region_counts(self._h, ptr(out, ctypes.c_int64), int(n_motifs)))
         return out[:n_motifs]
 
+    def boundary_sites(self):
+        """Boundary chains of the last de-duplicated range scan on this context (msb_scan_device_boundary_sites):
+        a dict of equal-length arrays motif, seq_idx, start, score, strand, flags (bit 0 kept, bit 1 head chain,
+        bit 2 tail chain)."""
+        n = ctypes.c_int64(0)
+        with self._lock:
+            check(self._lib.msb_scan_device_boundary_sites(self._h, 0, ctypes.byref(n), None, None, None, None, None, None))
+            k = n.value
+            out = dict(motif=np.zeros(k, np.int32), seq_idx=np.zeros(k, np.int32), start=np.zeros(k, np.int32),
+                       score=np.zeros(k, np.float64), strand=np.zeros(k, np.int8), flags=np.zeros(k, np.int8))
+            if k:
+                check(self._lib.msb_scan_device_boundary_sites(
+                    self._h, k, ctypes.byref(n), ptr(out["motif"], ctypes.c_int32), ptr(out["seq_idx"], ctypes.c_int32),
+                    ptr(out["start"], ctypes.c_int32), ptr(out["score"], ctypes.c_double), ptr(out["strand"], ctypes.c_int8),
+                    ptr(out["flags"], ctypes.c_int8)))
+        return out
+
+    def cell_stats(self, n_motifs, n_seqs):
+        """(counts int64[n_motifs, n_seqs], best float64[n_motifs, n_seqs], NaN where empty) of the last scan on this
+        context, reduced on the device (msb_scan_device_cell_stats)."""
+        counts = np.zeros((n_motifs, n_seqs), dtype=np.int64)
+        best = np.full((n_motifs, n_seqs), np.nan)
+        if counts.size:
+            with self._lock:
+                check(self._lib.msb_scan_device_cell_stats(self._h, int(n_motifs), int(n_seqs), ptr(counts, ctypes.c_int64),
+                                                           ptr(best, ctypes.c_double)))
+        return counts, best
+
     def counters(self):
         a = np.zeros(len(_lib.C_NAMES), dtype=np.int64)
         check(self._lib.msb_ctx_counters(self._h, ptr(a, ctypes.c_int64), len(a)))
@@ -476,25 +504,25 @@ def _ranges(ranges):
     return (len(r), np.ascontiguousarray(r[:, 0]), np.ascontiguousarray(r[:, 1]), np.ascontiguousarray(r[:, 2]))
 
 
-def scan_ranges(ctx, motifs, seqs, strand, ranges, async_=False, compact=False):
+def scan_ranges(ctx, motifs, seqs, strand, ranges, async_=False, compact=False, remove_dup=False):
     """Scan only the windows that start in the given (sequence index, start, end) ranges of a
-    resident sequence set; sites refer to the sequences of `seqs` (msb_scan_ranges).  There is no
-    de-duplication here: it is defined over a whole region's site list (scanner.py:171-193), not
-    across range boundaries."""
+    resident sequence set; sites refer to the sequences of `seqs` (msb_scan_ranges).  `remove_dup`:
+    de-duplicate per range (scanner.py:171-193), which needs at most one range per sequence; the chains
+    at the range edges can then be read with `ctx.boundary_sites()`."""
     n, a, b, c = _ranges(ranges)
     h = ctypes.c_void_p()
-    flags = _flags(False, async_=async_, compact=compact)
+    flags = _flags(remove_dup, async_=async_, compact=compact)
     with ctx._lock:
         check(ctx._lib.msb_scan_ranges(ctx._h, motifs._h, seqs._h, int(strand), flags, n, ptr(a, ctypes.c_int64),
                                        ptr(b, ctypes.c_int64), ptr(c, ctypes.c_int64), ctypes.byref(h)))
     return ScanResult(ctx, h, motifs.n)
 
 
-def scan_ranges_device(ctx, motifs, seqs, strand, ranges, counts_only=False):
-    """The same, results left on the device (`ctx.site_counts`); returns the number of sites."""
+def scan_ranges_device(ctx, motifs, seqs, strand, ranges, counts_only=False, remove_dup=False):
+    """The same, results left on the device (`ctx.site_counts`, `ctx.cell_stats`); returns the number of sites."""
     n, a, b, c = _ranges(ranges)
     total = ctypes.c_int64(0)
-    flags = _flags(False, counts_only)
+    flags = _flags(remove_dup, counts_only)
     with ctx._lock:
         check(ctx._lib.msb_scan_ranges_device(ctx._h, motifs._h, seqs._h, int(strand), flags, n, ptr(a, ctypes.c_int64),
                                               ptr(b, ctypes.c_int64), ptr(c, ctypes.c_int64), ctypes.byref(total)))

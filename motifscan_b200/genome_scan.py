@@ -16,6 +16,7 @@ Ranks never exchange data -- the only cross-rank step is the caller's gather of 
 counts / site arrays.
 """
 import ctypes
+import time
 
 import numpy as np
 
@@ -249,10 +250,37 @@ class ShardedSites(GenomeSites):
                 self.chrom_idx, self.start, self.score, self.strand = engine.merge_sites(
                     cnt, [p[0].seq_idx for p in parts], [p[0].start for p in parts], [p[0].score for p in parts],
                     [p[0].strand for p in parts], seq_to_group=[p[1] for p in parts], seq_offset=[p[2] for p in parts])
+        fix = self.__dict__.get("_fix")
+        if fix is not None:
+            dev_counts = np.sum([p[0].counts for p in self._parts], axis=0)
+            self._apply_fix(fix, dev_counts)
         for p in self._parts:
             p[0].close()
         self._parts = []
         self._merged = True
+
+    def _apply_fix(self, fix, dev_counts):
+        """Sites that boundary stitching removed or restored (GenomeScanner with remove_dup): the arrays hold the
+        per-piece de-duplicated sites; entries are deleted and inserted at their (motif, chromosome, start, strand)
+        place."""
+        off = np.zeros(len(dev_counts) + 1, dtype=np.int64)
+        np.cumsum(dev_counts, out=off[1:])
+
+        def key(chrom, start, strand):
+            return (chrom.astype(np.int64) << 34) | (start.astype(np.int64) << 2) | strand.astype(np.int64)
+        pos = np.zeros(len(fix["motif"]), dtype=np.int64)
+        fkey = key(fix["chrom"], fix["start"], fix["strand"])
+        for m in np.unique(fix["motif"]):
+            a, b = off[m], off[m + 1]
+            sel = fix["motif"] == m
+            pos[sel] = a + np.searchsorted(key(self.chrom_idx[a:b], self.start[a:b], self.strand[a:b]), fkey[sel])
+        rm = np.sort(pos[~fix["add"]])
+        add = np.flatnonzero(fix["add"])
+        add = add[np.lexsort((fkey[add], fix["motif"][add]))]
+        at = pos[add] - np.searchsorted(rm, pos[add], side="left")
+        for name, val in (("chrom_idx", fix["chrom"]), ("start", fix["start"]), ("score", fix["score"]), ("strand", fix["strand"])):
+            arr = np.delete(getattr(self, name), rm)
+            setattr(self, name, np.insert(arr, at, val[add].astype(arr.dtype)))
 
     def __getattr__(self, name):
         if name in ("chrom_idx", "start", "score", "strand") and not self.__dict__.get("_merged", True):
@@ -266,6 +294,66 @@ class ShardedSites(GenomeSites):
         self._parts = []
 
 
+def _greedy_keep(start, score, length):
+    """Keep flags of the reference's greedy de-duplication (scanner.py:156-168) over one chain of one strand."""
+    keep = np.zeros(len(start), dtype=bool)
+    cur = -1
+    for i in range(len(start)):
+        if cur >= 0 and start[i] - start[cur] < length:
+            if score[cur] >= score[i]:
+                continue
+            keep[cur] = False
+        keep[i] = True
+        cur = i
+    return keep
+
+
+def stitch_boundaries(rec, piece_chrom, lengths):
+    """Chains of overlapping sites cut by piece boundaries, resolved as if the chromosome had been one sequence.
+
+    `rec`: the boundary sites of every piece (`Context.boundary_sites`), with `piece` (global piece index, pieces
+    in genome order) and `gstart` (start on the chromosome) added; `piece_chrom[p]`: chromosome of piece p, and
+    consecutive pieces of one chromosome are adjacent.  The tail chain of a piece is joined with the head chain of
+    the next piece when they are less than a motif length apart; a chain that is both the head and the tail of its
+    piece is carried on to the next boundary.  Every joined chain gets the greedy rule again.  Returns the indices
+    into `rec` whose keep flag changes, and the number of chains that crossed a boundary."""
+    changed, n_joined = [], 0
+    if not len(rec["motif"]):
+        return np.zeros(0, dtype=np.int64), 0
+    order = np.lexsort((rec["gstart"], rec["piece"], rec["strand"], rec["motif"]))
+    motif, strand, piece = rec["motif"][order], rec["strand"][order], rec["piece"][order]
+    gstart, score, flags = rec["gstart"][order], rec["score"][order], rec["flags"][order]
+    bounds = np.flatnonzero(np.diff(motif) | np.diff(strand) | np.diff(piece)) + 1
+    groups = np.split(np.arange(len(order)), bounds)       # one (motif, strand, piece) each, in genome order
+
+    def resolve(chain):
+        nonlocal n_joined
+        if len(chain) < 2 or piece[chain[0]] == piece[chain[-1]]:
+            return                                        # one piece: the device's flags are final
+        n_joined += 1
+        idx = np.asarray(chain)
+        keep = _greedy_keep(gstart[idx], score[idx], lengths[motif[idx[0]]])
+        changed.extend(order[idx[keep != ((flags[idx] & 1) == 1)]].tolist())
+
+    carry, key = [], None
+    for g in groups:
+        first = g[0]
+        head = [i for i in g if flags[i] & 2]
+        tail = [i for i in g if flags[i] & 4]
+        whole = bool(head) and bool(flags[head[0]] & 4)    # one chain from the piece's start to its end
+        this = (motif[first], strand[first], piece_chrom[piece[first]])
+        if carry and key == this and head and gstart[head[0]] - gstart[carry[-1]] < lengths[motif[first]]:
+            if whole:
+                carry = carry + head
+                continue
+            resolve(carry + head)
+        else:
+            resolve(carry)
+        carry, key = tail, this
+    resolve(carry)
+    return np.asarray(changed, dtype=np.int64), n_joined
+
+
 class GenomeScanner:
     """Genome-wide scan of a host `PackedGenome` on several GPUs: `devices` of THIS process (one host thread
     and one context per device; the C calls drop the GIL) times `world` processes (`rank` = this one).  The
@@ -277,8 +365,13 @@ class GenomeScanner:
     thread pool over motifs, cscore.c:323-328, 425-436)."""
 
     def __init__(self, pg, pwms, cutoffs=None, p_value="1e-4", strand="both", devices=None, world=1, rank=0,
-                 unit_bp=1 << 26, resident=False, contexts=None, compact=True):
+                 unit_bp=1 << 26, resident=False, contexts=None, compact=True, remove_dup=False):
+        if remove_dup and int(world) > 1:
+            raise ValueError("GenomeScanner: remove_dup=True needs the whole genome in one process (world = 1)")
         self.pg = pg
+        # the reference's adjacent-site de-duplication over whole chromosomes: per piece on the device, the chains
+        # that cross a unit or share boundary stitched on the host (stitch_boundaries)
+        self.remove_dup = bool(remove_dup)
         self.matrices = [getattr(pwm, "matrix", pwm) for pwm in pwms]
         if cutoffs is None:
             cutoffs = [pwm.cutoffs[p_value] for pwm in pwms]
@@ -311,7 +404,7 @@ class GenomeScanner:
             _lib.bind_thread_near(ctx.device)     # worker thread of one GPU: stay on that GPU's side of the host
         n_motifs = len(self.matrices)
         counts = np.zeros(n_motifs, dtype=np.int64)
-        parts, stats = [], {}
+        parts, stats, cells, bnd = [], {}, [], []
         kept = self.resident[k]
         nxt = None
         try:
@@ -326,13 +419,20 @@ class GenomeScanner:
                 ranges = [(j, 0, b - a) for j, (_, a, b, _) in enumerate(unit.pieces)]
                 with ctx._lock:   # the counts / timings read below belong to THIS scan even if the context is shared
                     if collect_sites:
-                        res = engine.scan_ranges(ctx, motifs, sset, self.strand, ranges, async_=True, compact=self.compact)
+                        res = engine.scan_ranges(ctx, motifs, sset, self.strand, ranges, async_=True, compact=self.compact,
+                                                 remove_dup=self.remove_dup)
                         parts.append((res, np.array([p[0] for p in unit.pieces]), np.array([p[1] for p in unit.pieces])))
                     else:
-                        engine.scan_ranges_device(ctx, motifs, sset, self.strand, ranges, counts_only=not order_sites)
+                        engine.scan_ranges_device(ctx, motifs, sset, self.strand, ranges, counts_only=not order_sites,
+                                                  remove_dup=self.remove_dup)
                         counts += ctx.site_counts(n_motifs)
                     t = ctx.timings()
                     c = ctx.counters()
+                    if self.remove_dup:
+                        t0 = time.perf_counter()
+                        cells.append(ctx.cell_stats(n_motifs, len(unit.pieces)))
+                        bnd.append(ctx.boundary_sites())
+                        stats["boundary_read_s"] = stats.get("boundary_read_s", 0.0) + time.perf_counter() - t0
                 for name in ("prefilter", "exact", "order"):
                     stats[name] = stats.get(name, 0.0) + t[name]
                 for name in ("launches", "prefilter_launches", "candidates", "hits"):
@@ -347,12 +447,17 @@ class GenomeScanner:
             if nxt is not None:
                 nxt.close()
         stats["units"] = len(units)
-        return counts, parts, stats
+        return counts, parts, stats, cells, bnd
 
     def scan(self, collect_sites=True, order_sites=False):
         """One pass over this process's shares.  Returns a `ShardedSites` (`collect_sites=False`: per-motif
         counts only -- MSB_SCAN_COUNTS, nothing but 8 bytes per motif and unit leaves a device;
-        `order_sites=True` then still orders the sites on the device, as a measurement of that stage)."""
+        `order_sites=True` then still orders the sites on the device, as a measurement of that stage).
+
+        With `remove_dup` the sites are the reference's de-duplicated ones over whole chromosomes, and the result
+        also carries `cell_counts` / `cell_best` (int64 / float64 [n_motifs, n_chroms], NaN where a cell is empty):
+        the sites and best score of every (motif, chromosome), which is all the two result tables need.  Without
+        `collect_sites` no site array leaves a device."""
         n = len(self.devices)
         if n == 1:
             outs = [self._scan_share(0, collect_sites, order_sites)]
@@ -363,7 +468,44 @@ class GenomeScanner:
         counts = np.sum([o[0] for o in outs], axis=0)
         parts = [p for o in outs for p in o[1]]
         self.last_stats = [o[2] for o in outs]
-        return ShardedSites(self.pg.chroms, len(self.matrices), counts, parts)
+        if not self.remove_dup:
+            return ShardedSites(self.pg.chroms, len(self.matrices), counts, parts)
+        units = [u for share in self.shares for u in share]
+        return self._stitched(units, [c for o in outs for c in o[3]], [b for o in outs for b in o[4]], parts)
+
+    def _stitched(self, units, cells, bnd, parts):
+        """Per-piece de-duplicated results of every unit (genome order) -> whole-chromosome results."""
+        t0 = time.perf_counter()
+        n_motifs, n_chroms = len(self.matrices), len(self.pg.chroms)
+        lengths = np.array([np.asarray(m).shape[1] for m in self.matrices], dtype=np.int64)
+        piece_chrom = np.array([p[0] for u in units for p in u.pieces], dtype=np.int64)
+        piece_a = np.array([p[1] for u in units for p in u.pieces], dtype=np.int64)
+        first = np.cumsum([0] + [len(u.pieces) for u in units])
+        rec = {name: np.concatenate([b[name] for b in bnd]) if bnd else np.zeros(0)
+               for name in ("motif", "seq_idx", "start", "score", "strand", "flags")}
+        rec["piece"] = np.concatenate([b["seq_idx"].astype(np.int64) + first[i] for i, b in enumerate(bnd)]) if bnd else np.zeros(0, np.int64)
+        rec["gstart"] = piece_a[rec["piece"]] + rec["start"] if len(rec["piece"]) else np.zeros(0, np.int64)
+        changed, n_joined = stitch_boundaries(rec, piece_chrom, lengths)
+        # per (motif, piece) -> per (motif, chromosome)
+        cell_counts = np.zeros((n_motifs, n_chroms), dtype=np.int64)
+        cell_best = np.full((n_motifs, n_chroms), np.nan)
+        for (cnt, best), u in zip(cells, units):
+            for j, p in enumerate(u.pieces):
+                cell_counts[:, p[0]] += cnt[:, j]
+                hit = cnt[:, j] > 0
+                cell_best[hit, p[0]] = np.fmax(cell_best[hit, p[0]], best[hit, j])
+        add = np.where((rec["flags"][changed] & 1) == 0, 1, -1) if len(changed) else np.zeros(0, np.int64)
+        np.add.at(cell_counts, (rec["motif"][changed], piece_chrom[rec["piece"][changed]]), add)
+        counts = cell_counts.sum(axis=1)
+        out = ShardedSites(self.pg.chroms, n_motifs, counts, parts)
+        out.cell_counts, out.cell_best = cell_counts, cell_best
+        if len(changed) and parts:
+            out._fix = dict(motif=rec["motif"][changed], chrom=piece_chrom[rec["piece"][changed]].astype(np.int32),
+                            start=rec["gstart"][changed].astype(np.int32), score=rec["score"][changed],
+                            strand=rec["strand"][changed], add=add > 0)
+        self.last_stitch = {"boundary_sites": int(len(rec["motif"])), "joined_chains": n_joined,
+                            "corrections": int(len(changed)), "removed": int((add < 0).sum()), "stitch_s": time.perf_counter() - t0}
+        return out
 
     def close(self):
         for kept in self.resident:
@@ -385,7 +527,7 @@ def plan_chunks(chrom_sizes, chunk_bp, halo, world=1, rank=0):
 
 
 def scan_genome(genome, pwms, p_value="1e-4", strand="both", chunk_bp=1 << 22, batch_bp=1 << 28,
-                ctx=None, world=1, rank=0, collect_sites=True, cutoffs=None, resident=True, devices=None):
+                ctx=None, world=1, rank=0, collect_sites=True, cutoffs=None, resident=True, devices=None, remove_dup=False):
     """Scan all chromosomes of `genome` (anything with `.chroms`, `.chrom_sizes`, `.fetch_bytes`).
 
     `devices=[...]`: use these GPUs of this process together (`GenomeScanner`; the genome is packed on
@@ -395,12 +537,21 @@ def scan_genome(genome, pwms, p_value="1e-4", strand="both", chunk_bp=1 << 22, b
     Returns a GenomeSites for this rank's chunks (`collect_sites=False`: counts only, the site
     arrays stay empty and nothing but the counts leaves the device).  A `genome.DeviceGenome` is
     scanned in place; a host genome is first made resident (`resident=True`, the default) or
-    streamed chunk by chunk with overlaps (`resident=False`)."""
+    streamed chunk by chunk with overlaps (`resident=False`).
+
+    `remove_dup=True`: the reference's de-duplication over whole chromosomes, always through `GenomeScanner`
+    (a host genome is packed first); a `genome.DeviceGenome` or `resident=False` is an error."""
     from .genome import PackedGenome
-    if devices is not None or isinstance(genome, PackedGenome):
+    if remove_dup:
+        if hasattr(genome, "chrom_index") and hasattr(genome, "seqs"):
+            raise ValueError("scan_genome: remove_dup=True scans a host or packed genome (GenomeScanner), not a DeviceGenome")
+        if not resident:
+            raise ValueError("scan_genome: remove_dup=True is not available on the streamed path (resident=False)")
+    if devices is not None or isinstance(genome, PackedGenome) or remove_dup:
         devices = list(devices) if devices is not None else [ctx.device if ctx is not None else 0]
         pg = genome if isinstance(genome, PackedGenome) else PackedGenome.from_genome(genome, engine.default_context(devices[0]))
-        gs = GenomeScanner(pg, pwms, cutoffs=cutoffs, p_value=p_value, strand=strand, devices=devices, world=world, rank=rank)
+        gs = GenomeScanner(pg, pwms, cutoffs=cutoffs, p_value=p_value, strand=strand, devices=devices, world=world, rank=rank,
+                           remove_dup=remove_dup)
         try:
             return gs.scan(collect_sites=collect_sites)
         finally:

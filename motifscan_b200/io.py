@@ -99,9 +99,80 @@ def write_sites_table(output_dir, pwms, regions, motif_sites):
             f_score.write(lead + "\t".join("NA" if c == 0 else str(v) for c, v in zip(counts[r].tolist(), row)) + "\n")
 
 
+def write_cell_tables(output_dir, pwms, regions, counts, best):
+    """The two tables from per-cell statistics: `counts` / `best` [n_regions, n_motifs] (a whole-genome scan's
+    per-(chromosome, motif) counts and best scores), formatted by the library (msb_format_cell_tables)."""
+    import ctypes
+    from . import _lib
+    lib = _lib.load()
+    os.makedirs(output_dir, exist_ok=True)
+    header = ("chr\tstart\tend\t" + "\t".join(_motif_names(pwms)) + "\n").encode()
+    counts = np.ascontiguousarray(counts, dtype=np.int64)
+    best = np.ascontiguousarray(best, dtype=np.float64)
+    leads = [f"{g.chrom}\t{g.start + 1}\t{g.end}\t".encode() for g in regions]
+    lead_off = np.zeros(len(leads) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in leads], out=lead_off[1:])
+    p_num, p_score = ctypes.c_void_p(), ctypes.c_void_p()
+    n_num, n_score = ctypes.c_int64(0), ctypes.c_int64(0)
+    _lib.check(lib.msb_format_cell_tables(len(leads), len(pwms), _lib.ptr(counts, ctypes.c_int64), _lib.ptr(best, ctypes.c_double),
+                                          b"".join(leads), _lib.ptr(lead_off, ctypes.c_int64), ctypes.byref(p_num),
+                                          ctypes.byref(n_num), ctypes.byref(p_score), ctypes.byref(n_score),
+                                          min(os.cpu_count() or 1, 32)))
+    try:
+        with open(os.path.join(output_dir, "motif_sites_number.xls"), "wb") as f_num, \
+                open(os.path.join(output_dir, "motif_sites_score.xls"), "wb") as f_score:
+            f_num.write(header)
+            f_score.write(header)
+            if n_num.value:
+                f_num.write((ctypes.c_char * n_num.value).from_address(p_num.value))
+                f_score.write((ctypes.c_char * n_score.value).from_address(p_score.value))
+    finally:
+        lib.msb_text_free(p_num)
+        lib.msb_text_free(p_score)
+
+
+def _site_arrays(motif_sites, regions):
+    """(offsets, group, start, group_base or None, score, strand, group names) of an array-backed result: the
+    `MotifSites` of a region scan (groups = regions, starts relative to the region's scan window) or the
+    `GenomeSites` of a whole-genome scan (groups = chromosomes, starts on the chromosome); None otherwise."""
+    if hasattr(motif_sites, "_off"):
+        base = np.asarray(motif_sites.seq_starts, dtype=np.int64)
+        return (motif_sites._off, motif_sites._seq_idx, motif_sites._start, base, motif_sites._score, motif_sites._strand,
+                [g.chrom for g in regions])
+    if hasattr(motif_sites, "chrom_idx"):
+        return (motif_sites.offsets, motif_sites.chrom_idx, motif_sites.start, None, motif_sites.score, motif_sites.strand,
+                list(motif_sites.chroms))
+    return None
+
+
 def write_sites_bed(output_dir, pwms, regions, motif_sites):
+    """One BED file per motif.  Array-backed results are formatted by the library on host threads and written in
+    blocks (msb_write_sites_bed, numbers like Python's str()); nested lists are written line by line."""
     out_dir = os.path.join(output_dir, "motif_sites")
     os.makedirs(out_dir, exist_ok=True)
+    arrays = _site_arrays(motif_sites, regions)
+    if arrays is not None:
+        import ctypes
+        from . import _lib
+        lib = _lib.load()
+        off, group, start, base, score, strand, names = arrays
+        group = np.ascontiguousarray(group, dtype=np.int32)
+        start = np.ascontiguousarray(start, dtype=np.int32)
+        score = np.ascontiguousarray(score, dtype=np.float64)
+        strand = np.ascontiguousarray(strand, dtype=np.int8)
+        enc = [x.encode() for x in names]
+        name_off = np.zeros(len(enc) + 1, dtype=np.int64)
+        np.cumsum([len(x) for x in enc], out=name_off[1:])
+        n_threads = min(os.cpu_count() or 1, 32)
+        for m, pwm in enumerate(pwms):
+            path = os.path.join(out_dir, replace_special_char(f"{pwm.matrix_id}_{pwm.name}") + "_sites.bed")
+            a, b = int(off[m]), int(off[m + 1])
+            _lib.check(lib.msb_write_sites_bed(
+                path.encode(), b - a, _lib.ptr(group[a:], ctypes.c_int32) if b > a else None,
+                _lib.ptr(start[a:], ctypes.c_int32) if b > a else None, _lib.ptr(base, ctypes.c_int64) if base is not None else None,
+                _lib.ptr(score[a:], ctypes.c_double) if b > a else None, _lib.ptr(strand[a:], ctypes.c_int8) if b > a else None,
+                int(pwm.length), len(enc), b"".join(enc), _lib.ptr(name_off, ctypes.c_int64), n_threads))
+        return
     for pwm, per_motif in zip(pwms, motif_sites):
         path = os.path.join(out_dir, replace_special_char(f"{pwm.matrix_id}_{pwm.name}") + "_sites.bed")
         with open(path, "w") as out:
