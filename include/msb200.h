@@ -71,9 +71,9 @@ enum { MSB_C_CANDIDATES = 0, MSB_C_DIRTY, MSB_C_HITS, MSB_C_LAUNCHES, MSB_C_RETR
        MSB_C_PREFILTER_LAUNCHES, MSB_C_COUNT };
 int msb_ctx_counters(const msb_ctx *ctx, int64_t *v, int n);
 
-/* Tuning / test knobs of ONE context (nothing is process-wide): "prefilter_tc" 1 = tensor-core prefilter
- * (default), 0 = shared-memory table prefilter; "prefilter_w" windows per thread of the table prefilter
- * (4 or 8); "ascii_slices" upload slices of msb_scan_ascii (1..7); "tc_first_lane_cap" records per lane
+/* Tuning / test knobs of ONE context (nothing is process-wide): "ascii_slices" upload slices of
+ * msb_scan_ascii (1..7); "tc_interleave" 0 = the prefilter's motif tiles in ascending length order instead
+ * of short and long alternating (default 1); "tc_first_lane_cap" records per lane
  * buffer on the first attempt (tests of the overflow retry; 0 = sized from the input); "poison_pool" 1 =
  * recycled device buffers are filled with 0xFF (tests: nothing may rely on stale contents); "tc_prof" 1
  * = per-role cycle counters of the tensor-core prefilter on stderr; "select_pilot" 0 = msb_score_select scores

@@ -10,26 +10,16 @@
 
 namespace msb {
 
-// ---- limits of the fast (table prefilter) path ------------------------------------------------
-constexpr int kMaxFastLen = 32;               // columns a prefilter looks at (the register window of the exact stage)
-constexpr int kMaxTcLen = 64;                 // longest motif the tensor-core path takes (prefiltered on kMaxFastLen columns)
-constexpr int kMaxGroups = kMaxFastLen / 2;   // 2-mer groups per motif (G = ceil(L/2))
-constexpr int kGroupWords = 16;               // 4^2 table entries per group, 32-bit each
-constexpr int kGroupBytes = kGroupWords * 4;  // 64 B: one group spans 16 banks, conflict-free
+// ---- limits of the prefilter path ------------------------------------------------------------
+constexpr int kMaxFastLen = 32;               // columns the prefilter looks at (the register window of the exact stage)
+constexpr int kMaxTcLen = 64;                 // longest motif the prefilter takes (prefiltered on kMaxFastLen columns)
 constexpr int kPadBases = 32;                 // every sequence is padded to a multiple of this
 
-// Site / candidate key: motif (or sorted-motif index) | packed position | strand bit.
+// Site key: motif | packed position | strand bit.
 // Sorting ascending by this key yields the reference's list order
 // (motif, sequence, start, forward before reverse; cscore.c:336-389).
 constexpr int kPosBits = 41;                  // packed positions < 2^41 (2.2e12 bases)
 constexpr int kMotifShift = kPosBits + 1;
-__host__ __device__ inline uint64_t make_key(uint32_t motif, int64_t pos, uint32_t rev) {
-    return ((uint64_t) motif << kMotifShift) | ((uint64_t) pos << 1) | rev;
-}
-__host__ __device__ inline uint32_t key_motif(uint64_t k) { return (uint32_t) (k >> kMotifShift); }
-__host__ __device__ inline int64_t key_pos(uint64_t k) {
-    return (int64_t) ((k >> 1) & ((1ull << kPosBits) - 1));
-}
 __host__ __device__ inline uint32_t key_rev(uint64_t k) { return (uint32_t) (k & 1); }
 // Site keys use the same layout with a per-scan motif shift = (bits of the largest packed position)
 // + 1, so the radix sort that orders the sites touches no empty bit range: 37 key bits = 5 passes
@@ -86,31 +76,6 @@ struct MotifView {
     const float *pwm32;      // the same matrices rounded to fp32, same layout (screening only)
     const float *floor32;    // [n_motifs] an fp32-accumulated raw score below this cannot be a site
     int32_t n_motifs;
-};
-
-// One launch of the prefilter kernel covers one batch of motifs whose tables fit in shared
-// memory.  Motifs are sorted by group count G so the kernel runs a fully unrolled loop per G.
-struct BatchDesc {
-    uint32_t tab_word_off;               // offset of this batch's tables in the table buffer
-    uint32_t tab_words;                  // multiple of 4
-    uint32_t first_sorted;               // sorted index of the batch's first motif
-    uint16_t g_count[kMaxGroups + 1];    // motifs with exactly g groups, g = 1..kMaxGroups
-};
-
-struct PrefilterParams {
-    SeqView seq;
-    const uint32_t *tab;       // all batches' tables
-    const int32_t *order;      // sorted index -> motif id
-    const int32_t *mlen;       // motif id -> length
-    BatchDesc batch;
-    int32_t lmax_all;          // longest motif of the whole set (dirty-window horizon)
-    int32_t emit_dirty;        // 1 on the first batch only
-    int32_t any_zero_hit;      // some motif's all-N score (0 / max_raw) passes its cutoff
-    uint64_t *cand;            // candidate keys (sorted-motif index in the motif field)
-    int64_t cand_cap;
-    int64_t *dirty;            // packed positions of windows that touch an N
-    int64_t dirty_cap;
-    unsigned long long *counters;  // [0] candidates, [1] dirty positions, [2] hits
 };
 
 }  // namespace msb

@@ -1,12 +1,10 @@
-// kernels.cuh -- device code of libmsb200 (sm_100a).
+// kernels.cuh -- device code of libmsb200 (sm_100a) except the prefilter (prefilter_tc.cuh).
 //
 //   encode_pack_kernel      ASCII -> 2-bit codes + N mask            (cscore.c:81-114)
-//   prefilter_kernel        every window x every motif x both strands, 16-bit fixed point,
-//                           conservative: emits a superset of the hits  (cscore.c:336-355)
-//   exact_candidates_kernel fp64 re-score of candidates in the reference's accumulation
-//                           order + the reference's hit predicate       (cscore.c:344-389)
+//   exact_records_kernel    fp64 re-score of the prefilter's candidates in the reference's
+//                           accumulation order + the reference's hit predicate (cscore.c:344-389)
 //   exact_dirty_kernel      the same for windows that touch a non-ACGT base
-//   exact_slow_kernel       the same for motifs the table path cannot take (L > 32, non-finite)
+//   exact_positions_kernel  the same for motifs the prefilter cannot take (L > 64, non-finite)
 //   decode_sites_kernel     sorted keys -> (seq_idx, start, strand); motif_offsets_kernel: CSR
 //   dedup_flags_kernel      adjacent-site de-duplication              (scanner.py:156-193)
 //   score0_kernel           offset-0 window score of every sequence     (cscore.c:191-223)
@@ -173,166 +171,6 @@ unpack_codes_kernel(SeqView S, const int64_t *__restrict__ seq_off, int8_t *__re
 }
 
 // ---------------------------------------------------------------------------------------------
-// prefilter.
-//
-// Work unit: a warp chunk of 32*W consecutive packed positions; lane l owns the W window
-// starts p0 .. p0+W-1 with p0 = chunk*32*W + l*W.  A thread keeps the pre-scaled 2-mer index of
-// every offset it can need (W + 2*(kMaxGroups-1) registers), so the per-motif inner loop is
-// one LDS [idx + motif_base + imm] plus a third of an IADD3 per 2 PWM columns of BOTH strands:
-// a table entry packs (forward sum << 16) + reverse sum of its two columns in 16-bit fixed
-// point, pre-biased so that bit 31 / bit 15 of the final sum is the "forward / reverse score
-// may reach the cutoff" flag.  Entries of one group are 16 consecutive words = 16 banks, lanes
-// that read the same word are broadcast: conflict-free by construction.
-// ---------------------------------------------------------------------------------------------
-template <int W> struct PF {
-    static constexpr int kIdx = W + 2 * (kMaxGroups - 1);  // 2-mer offsets a thread may use
-    static constexpr int kThreads = 512;
-    static constexpr int kChunk = 32 * W;
-};
-
-template <int G, int W>
-__device__ __forceinline__ uint32_t score_motif(const unsigned char *__restrict__ tab,
-                                                const uint32_t (&idx)[PF<W>::kIdx],
-                                                uint32_t (&acc)[W]) {
-    uint32_t any = 0;
-#pragma unroll
-    for (int w = 0; w < W; w++) {
-        uint32_t a = 0;
-#pragma unroll
-        for (int g = 0; g < G; g++)
-            a += *reinterpret_cast<const uint32_t *>(tab + g * kGroupBytes + idx[w + 2 * g]);
-        acc[w] = a;
-        any |= a;
-    }
-    return any & 0x80008000u;
-}
-
-template <int W>
-__device__ __forceinline__ void emit_candidates(const PrefilterParams &P,
-                                                const uint32_t (&acc)[W], uint32_t live,
-                                                uint32_t sorted_idx, int64_t p0, int32_t j0,
-                                                int32_t slen) {
-    int32_t L = __ldg(P.mlen + __ldg(P.order + sorted_idx));
-#pragma unroll
-    for (int w = 0; w < W; w++) {
-        uint32_t f = acc[w] & 0x80008000u;
-        if (f == 0 || !((live >> w) & 1u)) continue;
-        if (j0 + w + L > slen) continue;  // window runs past the sequence (cscore.c:340)
-        if (f & 0x80000000u) {
-            unsigned long long slot = atomicAdd(P.counters + 0, 1ull);
-            if ((int64_t) slot < P.cand_cap) P.cand[slot] = make_key(sorted_idx, p0 + w, 0);
-        }
-        if (f & 0x00008000u) {
-            unsigned long long slot = atomicAdd(P.counters + 0, 1ull);
-            if ((int64_t) slot < P.cand_cap) P.cand[slot] = make_key(sorted_idx, p0 + w, 1);
-        }
-    }
-}
-
-template <int G, int W>
-__device__ __forceinline__ void run_group(const PrefilterParams &P,
-                                          const unsigned char *__restrict__ &tab,
-                                          uint32_t &sorted_idx,
-                                          const uint32_t (&idx)[PF<W>::kIdx], uint32_t live,
-                                          int64_t p0, int32_t j0, int32_t slen) {
-    const int cnt = P.batch.g_count[G];
-    for (int i = 0; i < cnt; i++) {
-        uint32_t acc[W];
-        if (score_motif<G, W>(tab, idx, acc))
-            emit_candidates<W>(P, acc, live, sorted_idx, p0, j0, slen);
-        tab += G * kGroupBytes;
-        sorted_idx++;
-    }
-}
-
-template <int G, int W> struct GroupLoop {
-    static __device__ __forceinline__ void run(const PrefilterParams &P,
-                                               const unsigned char *__restrict__ &tab,
-                                               uint32_t &sorted_idx,
-                                               const uint32_t (&idx)[PF<W>::kIdx],
-                                               uint32_t live, int64_t p0, int32_t j0,
-                                               int32_t slen) {
-        GroupLoop<G - 1, W>::run(P, tab, sorted_idx, idx, live, p0, j0, slen);
-        run_group<G, W>(P, tab, sorted_idx, idx, live, p0, j0, slen);
-    }
-};
-template <int W> struct GroupLoop<0, W> {
-    static __device__ __forceinline__ void run(const PrefilterParams &, const unsigned char *__restrict__ &,
-                                               uint32_t &, const uint32_t (&)[PF<W>::kIdx],
-                                               uint32_t, int64_t, int32_t, int32_t) {}
-};
-
-template <int W>
-__global__ void __launch_bounds__(PF<W>::kThreads, 1)
-prefilter_kernel(const __grid_constant__ PrefilterParams P) {
-    extern __shared__ __align__(16) unsigned char s_tab[];
-    {
-        const uint4 *src = reinterpret_cast<const uint4 *>(P.tab + P.batch.tab_word_off);
-        uint4 *dst = reinterpret_cast<uint4 *>(s_tab);
-        const uint32_t n4 = P.batch.tab_words >> 2;
-        for (uint32_t i = threadIdx.x; i < n4; i += blockDim.x) dst[i] = __ldg(src + i);
-    }
-    __syncthreads();
-
-    const SeqView &S = P.seq;
-    const int lane = threadIdx.x & 31;
-    const int64_t warps_total = (int64_t) gridDim.x * (blockDim.x >> 5);
-    const int64_t warp_global = (int64_t) blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int64_t n_chunks = (S.total_packed + PF<W>::kChunk - 1) / PF<W>::kChunk;
-    const uint32_t horizon = P.lmax_all >= 32 ? 0xffffffffu : ((1u << P.lmax_all) - 1u);
-
-    for (int64_t chunk = warp_global; chunk < n_chunks; chunk += warps_total) {
-        const int64_t p0 = chunk * PF<W>::kChunk + (int64_t) lane * W;
-        if (p0 >= S.total_packed) continue;
-        const int64_t s = find_seq(S.poff, S.n_seqs, p0);
-        const int32_t j0 = (int32_t) (p0 - __ldg(S.poff + s));
-        const int32_t slen = __ldg(S.len + s);
-        if (j0 >= slen) continue;  // padding behind the sequence's last base
-
-        // N mask of [p0, p0 + W + 31): window w is "dirty" if any base in its horizon is N.
-        const uint32_t *mp = S.nmask + (p0 >> 5);
-        const uint64_t m64 = (((uint64_t) __ldg(mp + 1) << 32) | __ldg(mp)) >> (p0 & 31);
-        uint32_t live = 0;  // windows this thread scores with the table path
-#pragma unroll
-        for (int w = 0; w < W; w++) {
-            const uint32_t bits = (uint32_t) (m64 >> w) & horizon;
-            if (j0 + w < slen) {
-                if (bits == 0) {
-                    live |= 1u << w;
-                } else if (P.emit_dirty && !(bits == horizon && !P.any_zero_hit)) {
-                    // Touches an N: scored exactly by exact_dirty_kernel.  A window whose whole
-                    // horizon is N scores 0 for every motif and is dropped when no motif's
-                    // cutoff admits a zero score.
-                    unsigned long long slot = atomicAdd(P.counters + 1, 1ull);
-                    if ((int64_t) slot < P.dirty_cap) P.dirty[slot] = p0 + w;
-                }
-            }
-        }
-        if (live == 0) continue;
-
-        // 2-bit codes of [p0, p0 + 48 - (p0 & 15)) aligned to bit 0.
-        const uint32_t *cp = S.codes + (p0 >> 4);
-        const uint32_t sh = (uint32_t) (p0 & 15) * 2;
-        const uint32_t r0 = __ldg(cp), r1 = __ldg(cp + 1), r2 = __ldg(cp + 2);
-        uint32_t cw[4];
-        cw[0] = __funnelshift_r(r0, r1, sh);
-        cw[1] = __funnelshift_r(r1, r2, sh);
-        cw[2] = r2 >> sh;
-        cw[3] = 0;
-        uint32_t idx[PF<W>::kIdx];
-#pragma unroll
-        for (int k = 0; k < PF<W>::kIdx; k++) {
-            const uint32_t v = __funnelshift_r(cw[(2 * k) >> 5], cw[((2 * k) >> 5) + 1], (2 * k) & 31);
-            idx[k] = (v & 0xFu) << 2;
-        }
-
-        const unsigned char *tab = s_tab;
-        uint32_t sorted_idx = P.batch.first_sorted;
-        GroupLoop<kMaxGroups, W>::run(P, tab, sorted_idx, idx, live, p0, j0, slen);
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
 // exact stage: the reference's arithmetic, verbatim (cscore.c:341-389).
 // ---------------------------------------------------------------------------------------------
 struct ExactParams {
@@ -399,36 +237,6 @@ __device__ __forceinline__ double exact_raw_w(const Window32 &w, const double *_
         acc = __dadd_rn(acc, v);
     }
     return acc;
-}
-
-// `col_info` == nullptr: keys carry (sorted motif index, position, strand) and were validated by
-// the table prefilter.  Otherwise they are the tensor-core prefilter's raw keys (tile * 256 +
-// column, position): decode the column and drop windows that run past their sequence.
-__global__ void __launch_bounds__(256)
-exact_candidates_kernel(ExactParams E, const uint64_t *__restrict__ cand, int64_t n_cand,
-                        const int32_t *__restrict__ order, const uint32_t *__restrict__ col_info) {
-    int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_cand) return;
-    const uint64_t k = cand[i];
-    const int64_t p = key_pos(k);
-    uint32_t sorted = key_motif(k);
-    int rev = (int) key_rev(k);
-    if (col_info) {
-        const uint32_t info = __ldg(col_info + sorted);
-        if (info == 0xffffffffu) return;   // padding column of a tile
-        sorted = info >> 1;
-        rev = (int) (info & 1u);
-    }
-    const uint32_t m = (uint32_t) __ldg(order + sorted);
-    const int L = __ldg(E.mot.len + m);
-    if (col_info || E.seq.limit) {
-        const int64_t s = __ldg(E.seq.blk_seq + (p >> 5));
-        const int64_t j = p - __ldg(E.seq.poff + s);
-        if (j + L > (int64_t) __ldg(E.seq.len + s)) return;   // cscore.c:340
-        if (E.seq.limit && j >= (int64_t) __ldg(E.seq.limit + s)) return;   // the next chunk owns this start
-    }
-    const double *pw = E.mot.pwm + 4 * (int64_t) __ldg(E.mot.col_off + m);
-    test_and_emit(E, m, p, rev, exact_raw_w(load_window32(E.seq, p), pw, L, rev));   // prefilter motifs have L <= 32
 }
 
 // The tensor-core prefilter leaves its candidate records in one buffer per epilogue lane

@@ -70,7 +70,6 @@ struct msb_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     int sm_count = 0;
-    size_t smem_optin = 0;
     cudaEvent_t ev[8] = {};
     cudaStream_t copy_stream = nullptr;   // msb_scan_ascii: host-to-device slices overlap the scan (created on first use)
     cudaEvent_t slice_ev[8] = {};
@@ -115,27 +114,12 @@ struct msb_ctx {
     int last_key_shift = 0;
     // tuning / test knobs (msb_ctx_set_option): per context, so that contexts driven from different host
     // threads never see each other's settings
-    int opt_prefilter_tc = 1;        // 1: tensor-core prefilter (prefilter_tc.cuh), 0: shared-memory table prefilter
-    int opt_prefilter_w = 4;         // windows per thread of the table prefilter (4 or 8)
     int opt_tc_prof = 0;             // 1: print per-role cycle counters of the tensor-core prefilter to stderr
     int opt_ascii_slices = 4;        // msb_scan_ascii: upload slices (1..7)
     int opt_tc_first_lane_cap = 0;   // tests: records per lane buffer on the first attempt (0 = sized from the input)
     int opt_poison_pool = 0;         // tests: fill device buffers with 0xFF when they go back to the pool
     int opt_tc_interleave = 1;       // tensor-core prefilter: short and long motif tiles alternate (0: ascending by length)
     int opt_select_pilot = 1;        // msb_score_select: 0 = always score every sample for every motif (the plain form)
-};
-
-struct TableSet {
-    bool valid = false;
-    int strand = 0;
-    uint64_t cutoff_version = 0;
-    size_t smem_budget = 0;
-    std::vector<int32_t> order;       // sorted index -> motif id (fast motifs only)
-    std::vector<int32_t> slow;        // motif ids scored by the exact kernel everywhere
-    std::vector<BatchDesc> batches;
-    int32_t lmax_fast = 0;
-    int any_zero_hit = 0;
-    DevBuf d_tab, d_order, d_slow;
 };
 
 // Tensor-core prefilter tables (prefilter_tc.cuh).
@@ -160,7 +144,6 @@ struct msb_motifs {
     uint64_t cutoff_version = 1;
     int32_t lmax = 0;
     DevBuf d_pwm, d_col_off, d_len, d_cutoff, d_max_raw, d_pwm32, d_floor32;
-    TableSet tables[4];
     TcTableSet tc_tables[4];
     MotifView view() const {
         MotifView v;
@@ -363,7 +346,6 @@ int msb_ctx_create(int device, void *stream, msb_ctx **out) {
     if (!ctx) { set_error("out of host memory"); return MSB_ENOMEM; }
     ctx->device = device;
     ctx->sm_count = prop.multiProcessorCount;
-    ctx->smem_optin = prop.sharedMemPerBlockOptin;
     if (stream) {
         ctx->stream = (cudaStream_t) stream;
     } else {
@@ -385,8 +367,6 @@ int msb_ctx_create(int device, void *stream, msb_ctx **out) {
         if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
         ctx->aux_stream = nullptr;   // everything stays on the main stream
     }
-    cudaFuncSetAttribute(prefilter_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) ctx->smem_optin);
-    cudaFuncSetAttribute(prefilter_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) ctx->smem_optin);
     cudaFuncSetAttribute(prefilter_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemBytes);
     cudaFuncSetAttribute(prefilter_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemBytes);
     cudaFuncSetAttribute(select_ranks_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSelSmemKeys * 8);
@@ -583,7 +563,6 @@ int msb_motifs_destroy(msb_motifs *M) {
     cudaSetDevice(M->ctx->device);
     cudaStreamSynchronize(M->ctx->stream);
     for (DevBuf *b : {&M->d_pwm, &M->d_col_off, &M->d_len, &M->d_cutoff, &M->d_max_raw, &M->d_pwm32, &M->d_floor32}) b->release();
-    for (auto &t : M->tables) { t.d_tab.release(); t.d_order.release(); t.d_slow.release(); }
     for (auto &t : M->tc_tables) {
         t.d_btab.release(); t.d_col_info.release(); t.d_len.release(); t.d_order.release(); t.d_slow.release();
     }
@@ -923,180 +902,16 @@ int msb_seqs_destroy(msb_seqs *S) {
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------
-// Prefilter tables.
-//
-// For motif m (length L, G = ceil(L/2) groups) and 2-mer index i = b0 + 4*b1 of the bases at
-// window offsets 2g, 2g+1:
-//     f_g(i) = M[b0][2g] + M[b1][2g+1]                 forward   (cscore.c:348)
-//     r_g(i) = M[3-b0][L-1-2g] + M[3-b1][L-2-2g]       reverse   (cscore.c:351)
-// (second term dropped when 2g+1 == L).  With scale s, per-group minima and the real-valued
-// threshold T below, the stored 16-bit quantities are ceil((f_g - min f_g) * s), so that
-//     sum_g q_g  >=  s * (raw - sum_g min f_g)        for every window,
-// and a window is a candidate iff  sum_g q_g >= Qthr = floor(s * (T - sum_g min f_g)) - 1.
-// T is a strict under-estimate of the smallest exact raw score the reference could accept:
-//     score/max_raw - cutoff >= -1e-10  (evaluated in double, cscore.c:357-358)
-//     =>  raw >= max_raw * (cutoff - 1e-10) - 1e-12 * (max_raw * (|cutoff| + 1) + sum_c max_b |M[b][c]|)
-// (the 1e-12 term is > 1000x the worst-case rounding of the L-term double sum, the division
-// and the subtraction).  Hence candidates are a superset of the reference's hits; the exact
-// stage removes the rest.  Group 0 also carries the bias 32768 - Qthr, so bit 15 of the 16-bit
-// sum is the candidate flag; the forward quantity lives in bits 16..31 of the entry, the
-// reverse one in bits 0..15, and one 32-bit add accumulates both.
-// ------------------------------------------------------------------------------------------------
-namespace msb {
-
-// Motifs the prefilters can take.  The table prefilter holds at most kMaxFastLen columns; the tensor-core
-// prefilter takes up to kMaxTcLen columns: it looks at the first kMaxFastLen columns of a strand only
-// (tc_fill_column), the exact stage scores the whole window, and the producer's all-N test spans kMaxTcLen bases.
-static bool motif_is_fast(const msb_motifs *M, int32_t m, bool tensor = false) {
-    const int L = M->lens[m];
-    if (L < 1 || L > (tensor ? kMaxTcLen : kMaxFastLen)) return false;
-    const double *mat = M->mats.data() + M->mat_off[m];
-    for (int k = 0; k < 4 * L; k++)
-        if (!std::isfinite(mat[k])) return false;
-    return true;
-}
-
-static void build_motif_table(const msb_motifs *M, int32_t m, int strand, uint32_t *out /* G*16 words */) {
-    const int L = M->lens[m];
-    const int G = (L + 1) / 2;
-    const double *mat = M->mats.data() + M->mat_off[m];
-    auto at = [&](int row, int col) { return mat[(size_t) row * L + col]; };
-    const double max_raw = M->max_raw[m];
-    const double cutoff = M->cutoffs[m];
-    std::fill(out, out + (size_t) G * kGroupWords, 0u);
-    // Motifs that can never produce a site keep all-zero tables (flag bits never set):
-    // max_raw == 0 gives score = raw/0 = -inf or NaN; cutoff NaN / +inf fail the predicate.
-    if (!(max_raw > 0) || std::isnan(cutoff) || (std::isinf(cutoff) && cutoff > 0)) return;
-
-    double f[kMaxGroups][16], r[kMaxGroups][16];
-    double fmin_sum = 0, fmax_sum = 0, rmin_sum = 0, rmax_sum = 0, abs_sum = 0;
-    double fmin[kMaxGroups], rmin[kMaxGroups];
-    for (int c = 0; c < L; c++) {
-        double a = 0;
-        for (int row = 0; row < 4; row++) a = std::max(a, std::fabs(at(row, c)));
-        abs_sum += a;
-    }
-    for (int g = 0; g < G; g++) {
-        const int c0 = 2 * g, c1 = 2 * g + 1;
-        double fmn = INFINITY, fmx = -INFINITY, rmn = INFINITY, rmx = -INFINITY;
-        for (int i = 0; i < 16; i++) {
-            const int b0 = i & 3, b1 = i >> 2;
-            double fv = at(b0, c0), rv = at(3 - b0, L - 1 - c0);
-            if (c1 < L) { fv += at(b1, c1); rv += at(3 - b1, L - 1 - c1); }
-            f[g][i] = fv;
-            r[g][i] = rv;
-            fmn = std::min(fmn, fv); fmx = std::max(fmx, fv);
-            rmn = std::min(rmn, rv); rmx = std::max(rmx, rv);
-        }
-        fmin[g] = fmn; rmin[g] = rmn;
-        fmin_sum += fmn; fmax_sum += fmx; rmin_sum += rmn; rmax_sum += rmx;
-    }
-    double T;
-    if (std::isinf(cutoff)) {  // -inf: every window with a finite score is a site
-        T = std::min(fmin_sum, rmin_sum) - 1.0;
-    } else {
-        T = max_raw * (cutoff - 1e-10) - 1e-12 * (max_raw * (std::fabs(cutoff) + 1.0) + abs_sum);
-    }
-    const double lo = std::min(fmin_sum, rmin_sum), hi = std::max(fmax_sum, rmax_sum);
-    double range = std::max(std::max(hi - T, T - lo), 0.0);
-    double s = range > 0 ? 32000.0 / range : 1.0;
-    if (!(s < 1e9)) s = 1e9;
-    for (int dir = 0; dir < 2; dir++) {
-        if (!(strand & (dir ? 2 : 1))) continue;
-        const double (*v)[16] = dir ? r : f;
-        const double *vmin = dir ? rmin : fmin;
-        const double min_sum = dir ? rmin_sum : fmin_sum;
-        double qthr_d = std::floor(s * (T - min_sum)) - 1.0;
-        qthr_d = std::max(qthr_d, -32000.0 - 64.0);  // T below every score: all windows flagged
-        const int64_t bias = 32768 - (int64_t) qthr_d;
-        for (int g = 0; g < G; g++)
-            for (int i = 0; i < 16; i++) {
-                int64_t q = (int64_t) std::ceil((v[g][i] - vmin[g]) * s);
-                if (g == 0) q += bias;
-                // linear packing: sum of entries == (sum fwd) * 65536 + (sum rev)  (mod 2^32)
-                out[(size_t) g * kGroupWords + i] += dir ? (uint32_t) q : (uint32_t) (q << 16);
-            }
-    }
-}
-
-static int ensure_tables(msb_ctx *ctx, msb_motifs *M, int strand, TableSet **out) {
-    TableSet &T = M->tables[strand];
-    const size_t budget = ctx->smem_optin;
-    if (T.valid && T.cutoff_version == M->cutoff_version && T.smem_budget == budget) { *out = &T; return MSB_OK; }
-    T.valid = false;
-    T.order.clear();
-    T.slow.clear();
-    T.batches.clear();
-    T.lmax_fast = 0;
-    T.any_zero_hit = 0;
-    std::vector<int32_t> fast;
-    for (int32_t m = 0; m < M->n; m++) {
-        if (motif_is_fast(M, m)) fast.push_back(m);
-        else if (M->lens[m] >= 1) T.slow.push_back(m);  // L == 0: score is 0/0 = NaN, never a site
-    }
-    std::stable_sort(fast.begin(), fast.end(), [&](int32_t a, int32_t b) {
-        return (M->lens[a] + 1) / 2 < (M->lens[b] + 1) / 2;
-    });
-    T.order = fast;
-    std::vector<uint32_t> tab;
-    size_t total_words = 0;
-    for (int32_t m : fast) total_words += (size_t) ((M->lens[m] + 1) / 2) * kGroupWords;
-    tab.resize(total_words + 4);
-    size_t at = 0;
-    BatchDesc cur;
-    std::memset(&cur, 0, sizeof(cur));
-    auto flush = [&]() {
-        if (cur.tab_words) {
-            cur.tab_words = (cur.tab_words + 3) & ~3u;
-            T.batches.push_back(cur);
-        }
-    };
-    for (size_t k = 0; k < fast.size(); k++) {
-        const int32_t m = fast[k];
-        const int G = (M->lens[m] + 1) / 2;
-        const uint32_t words = (uint32_t) G * kGroupWords;
-        if (((size_t) cur.tab_words + words) * 4 > budget || cur.g_count[G] == 0xffff) {
-            flush();
-            std::memset(&cur, 0, sizeof(cur));
-        }
-        if (cur.tab_words == 0) {
-            cur.tab_word_off = (uint32_t) at;
-            cur.first_sorted = (uint32_t) k;
-        }
-        build_motif_table(M, m, strand, tab.data() + at);
-        at += words;
-        cur.tab_words += words;
-        cur.g_count[G]++;
-        T.lmax_fast = std::max(T.lmax_fast, M->lens[m]);
-        // all-N window: score = 0 / max_raw (cscore.c:342-357 with every base skipped)
-        const double z = 0.0 / M->max_raw[m];
-        if (z - M->cutoffs[m] >= -1e-10) T.any_zero_hit = 1;
-    }
-    flush();
-    MSB_TRY(T.d_tab.ensure(std::max<size_t>(tab.size() * 4, 16)));
-    MSB_TRY(T.d_order.ensure(std::max<size_t>(fast.size() * 4, 16)));
-    MSB_TRY(T.d_slow.ensure(std::max<size_t>(T.slow.size() * 4, 16)));
-    MSB_CUDA(cudaMemcpyAsync(T.d_tab.p, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    if (!fast.empty())
-        MSB_CUDA(cudaMemcpyAsync(T.d_order.p, fast.data(), fast.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    if (!T.slow.empty())
-        MSB_CUDA(cudaMemcpyAsync(T.d_slow.p, T.slow.data(), T.slow.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-    MSB_CUDA(cudaStreamSynchronize(ctx->stream));  // host vectors go out of scope
-    T.strand = strand;
-    T.cutoff_version = M->cutoff_version;
-    T.smem_budget = budget;
-    T.valid = true;
-    *out = &T;
-    return MSB_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// Tensor-core prefilter tables (prefilter_tc.cuh).
+// Prefilter tables (prefilter_tc.cuh).
 //
 // For one strand of motif m let V[b][c] be its PWM (forward: M[b][c], cscore.c:348; reverse:
 // M[3-b][L-1-c], cscore.c:351), colmax_c = max_b V[b][c] and d[b][c] = colmax_c - V[b][c] >= 0 the
-// "deficit" of base b at column c, so that  raw = sum_c colmax_c - sum_c d[b_c][c].  With the
-// conservative raw threshold T of build_motif_table, a window the reference can accept has
+// "deficit" of base b at column c, so that  raw = sum_c colmax_c - sum_c d[b_c][c].  The raw threshold
+// T is a strict under-estimate of the smallest exact raw score the reference could accept:
+//     score/max_raw - cutoff >= -1e-10  (evaluated in double, cscore.c:357-358)
+//     =>  raw >= T = max_raw * (cutoff - 1e-10) - 1e-12 * (max_raw * (|cutoff| + 1) + sum_c max_b |M[b][c]|)
+// (the 1e-12 term is > 1000x the worst-case rounding of the L-term double sum, the division
+// and the subtraction).  A window the reference can accept therefore has
 //     sum_c d[b_c][c]  <=  D = sum_c colmax_c - T (+ slack for the rounding of these host sums).
 // The stored e4m3 entries are  e[b][c] = RU( beta - s * d[b][c] )  (rounded towards +inf, floored
 // at -448), with beta an e4m3 value, C = L * beta and s = (C - C/64) / D.  Then for every window
@@ -1104,6 +919,20 @@ static int ensure_tables(msb_ctx *ctx, msb_motifs *M, int strand, TableSet **out
 // accumulation can lose (prefilter_tc.cuh), so the accumulator's sign bit is clear: the candidates
 // are a superset of the reference's hits.
 // ------------------------------------------------------------------------------------------------
+namespace msb {
+
+// Motifs the prefilter can take: up to kMaxTcLen columns.  It looks at the first kMaxFastLen columns of a
+// strand only (tc_fill_column), the exact stage scores the whole window, and the producer's all-N test spans
+// kMaxTcLen bases.
+static bool motif_is_fast(const msb_motifs *M, int32_t m) {
+    const int L = M->lens[m];
+    if (L < 1 || L > kMaxTcLen) return false;
+    const double *mat = M->mats.data() + M->mat_off[m];
+    for (int k = 0; k < 4 * L; k++)
+        if (!std::isfinite(mat[k])) return false;
+    return true;
+}
+
 static float e4m3_value(int v) {
     const int e = (v >> 3) & 15, m = v & 7;
     const float mag = e == 0 ? std::ldexp((float) m / 8.f, -6) : std::ldexp(1.f + (float) m / 8.f, e - 7);
@@ -1190,7 +1019,7 @@ static int ensure_tc_tables(msb_ctx *ctx, msb_motifs *M, int strand, TcTableSet 
     T.any_zero_hit = 0;
     std::vector<int32_t> fast;
     for (int32_t m = 0; m < M->n; m++) {
-        if (motif_is_fast(M, m, true)) fast.push_back(m);
+        if (motif_is_fast(M, m)) fast.push_back(m);
         else if (M->lens[m] >= 1) T.slow.push_back(m);
     }
     auto ksteps = [&](int32_t m) { return (std::min(M->lens[m], kMaxFastLen) + 7) / 8; };
@@ -1253,6 +1082,7 @@ static int ensure_tc_tables(msb_ctx *ctx, msb_motifs *M, int strand, TcTableSet 
             const int32_t m = fast[k];
             tc_len[k] = M->lens[m];
             T.lmax_fast = std::max(T.lmax_fast, M->lens[m]);
+            // all-N window: score = 0 / max_raw (cscore.c:342-357 with every base skipped)
             const double z = 0.0 / M->max_raw[m];
             if (z - M->cutoffs[m] >= -1e-10) T.any_zero_hit = 1;
         }
@@ -1342,8 +1172,6 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
     if (M->ctx != ctx || S->ctx != ctx) { set_error("msb_scan: motifs/seqs belong to another context"); return MSB_EINVAL; }
     MSB_CUDA(cudaSetDevice(ctx->device));
     MSB_TRY(seqs_ready(S));
-    const bool use_tc = ctx->opt_prefilter_tc != 0;
-    if (ranges && !use_tc) { set_error("msb_scan_ranges needs the tensor-core prefilter (prefilter_tc = 1)"); return MSB_EINVAL; }
     RangeList whole;
     if (!ranges) {
         if (S->total_packed) whole.push_back({0, S->total_packed});
@@ -1351,16 +1179,12 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
     }
     int64_t span = 0;
     for (auto &r : *ranges) span += r.second - r.first;
-    TableSet *T = nullptr;
     TcTableSet *TT = nullptr;
-    if (use_tc) MSB_TRY(ensure_tc_tables(ctx, M, strand, &TT));
-    else MSB_TRY(ensure_tables(ctx, M, strand, &T));
-    const int32_t n_fast = (int32_t) (use_tc ? TT->order.size() : T->order.size());
-    const int32_t n_slow = (int32_t) (use_tc ? TT->slow.size() : T->slow.size());
-    const int32_t *d_order = use_tc ? TT->d_order.as<int32_t>() : T->d_order.as<int32_t>();
-    const int32_t *d_slow = use_tc ? TT->d_slow.as<int32_t>() : T->d_slow.as<int32_t>();
-    const int32_t lmax_fast = use_tc ? TT->lmax_fast : T->lmax_fast;
-    const int any_zero_hit = use_tc ? TT->any_zero_hit : T->any_zero_hit;
+    MSB_TRY(ensure_tc_tables(ctx, M, strand, &TT));
+    const int32_t n_fast = (int32_t) TT->order.size();
+    const int32_t n_slow = (int32_t) TT->slow.size();
+    const int32_t *d_order = TT->d_order.as<int32_t>();
+    const int32_t *d_slow = TT->d_slow.as<int32_t>();
     cudaStream_t st = ctx->stream;
     std::fill(ctx->c, ctx->c + MSB_C_COUNT, 0);
     ctx->last_sites = 0;
@@ -1407,129 +1231,95 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
         tc_grid = std::max<int64_t>(tc_grid, std::min<int64_t>(ctx->sm_count, (r.second + kTcTileBases - 1) / kTcTileBases - r.first / kTcTileBases));
     const int32_t n_lanes = (int32_t) (tc_grid * kTcLanesPerCta);
     int64_t lane_cap = 0;
-    int64_t n_cand = 0, n_dirty = 0, n_rec = 0;
+    int64_t n_dirty = 0, n_rec = 0;
     MSB_CUDA(cudaEventRecord(ctx->ev[0], st));
     for (int attempt = 0;; attempt++) {
         MSB_TRY(ctx->cand.ensure((size_t) cand_cap * 8));
         MSB_TRY(ctx->dirty.ensure((size_t) dirty_cap * 8));
         MSB_CUDA(cudaMemsetAsync(ctx->counters.p, 0, 4 * sizeof(unsigned long long), st));
-        if (use_tc) {
-            TcParams P;
-            P.seq = sv;
-            P.btab = TT->d_btab.as<uint8_t>();
-            P.lmax_all = std::max(lmax_fast, 1);
-            P.any_zero_hit = any_zero_hit;
-            lane_cap = std::max<int64_t>(cand_cap / 2 / n_lanes, 1);   // 16-byte records per lane buffer
-            if (attempt == 0 && ctx->opt_tc_first_lane_cap > 0) lane_cap = std::min<int64_t>(lane_cap, ctx->opt_tc_first_lane_cap);
-            MSB_TRY(ctx->lane_count.ensure((size_t) n_lanes * 4));
-            MSB_CUDA(cudaMemsetAsync(ctx->lane_count.p, 0, (size_t) n_lanes * 4, st));
-            P.cand = ctx->cand.as<uint4>();
-            P.cand_cap = lane_cap;
-            P.lane_count = ctx->lane_count.as<uint32_t>();
-            P.dirty = ctx->dirty.as<int64_t>();
-            P.dirty_cap = dirty_cap;
-            P.counters = ctx->counters.as<unsigned long long>();
-            P.prof = nullptr;
-            DevBuf prof;
-            if (ctx->opt_tc_prof) {
-                MSB_TRY(prof.ensure((size_t) (ctx->sm_count + 16) * 16 * 8));
-                MSB_CUDA(cudaMemsetAsync(prof.p, 0, (size_t) (ctx->sm_count + 16) * 16 * 8, st));
-                P.prof = prof.as<long long>();
-            }
-            const size_t smem = kTcSmemBytes;  // > half an SM's shared memory: one CTA per SM, which owns the TMEM
-            unsigned grid = 1;
-            for (size_t ri = 0; ri < ranges->size(); ri++) {
-                const auto &r = (*ranges)[ri];
-                if (before_range) MSB_TRY((*before_range)(ri));
-                P.pos_lo = r.first;
-                P.pos_hi = r.second;
-                const int64_t n_ptiles = (r.second + kTcTileBases - 1) / kTcTileBases - r.first / kTcTileBases;
-                grid = (unsigned) std::min<int64_t>(ctx->sm_count, n_ptiles);
-                for (size_t b = 0; b < TT->batches.size(); b++) {
-                    P.batch = TT->batches[b];
-                    P.emit_dirty = (b == 0);
-                    if (ctx->opt_tc_prof) prefilter_tc_kernel<true><<<grid, kTcThreads, smem, st>>>(P);
-                    else prefilter_tc_kernel<false><<<grid, kTcThreads, smem, st>>>(P);
-                    MSB_CUDA(cudaGetLastError());
-                    ctx->c[MSB_C_LAUNCHES]++;
-                    ctx->c[MSB_C_PREFILTER_LAUNCHES]++;
-                }
-            }
-            lane_totals_kernel<<<(unsigned) std::min<int64_t>((n_lanes + 1023) / 1024, 128), 1024, 0, st>>>(ctx->lane_count.as<uint32_t>(), n_lanes, lane_cap,
-                                                   ctx->counters.as<unsigned long long>());
-            MSB_CUDA(cudaGetLastError());
-            ctx->c[MSB_C_LAUNCHES]++;
-            if (ctx->opt_tc_prof) {
-                std::vector<long long> h((size_t) (ctx->sm_count + 16) * 16);
-                MSB_CUDA(cudaMemcpyAsync(h.data(), prof.p, h.size() * 8, cudaMemcpyDeviceToHost, st));
-                MSB_CUDA(cudaStreamSynchronize(st));
-                const long long *o = h.data();   // CTA 0 of the last batch
-                const double un = (double) std::max<long long>(o[4], 1);
-                fprintf(stderr, "[tc_prof] cta0: %lld units, %.0f clk/unit | issuer: wait stream %.0f, wait tmem_empty %.0f, issue %.0f | "
-                        "epilogue warp 4: wait stream %.0f, wait tmem_full %.0f, ld %.0f, process %.0f (clk/unit); "
-                        "units with a candidate %.3f, process there %.0f clk, elsewhere %.0f clk\n",
-                        o[4], o[0] / un, o[1] / un, o[2] / un, o[3] / un, o[11] / un, o[8] / un, o[9] / un, o[10] / un,
-                        o[14] / un, (double) o[13] / std::max<long long>(o[14], 1),
-                        (double) (o[10] - o[13]) / std::max<long long>(o[12] - o[14], 1));
-                const long long *tl = h.data() + (size_t) grid * 16;
-                for (int i = 0; i < 12; i++)
-                    fprintf(stderr, "[tc_prof] unit %d: issuer woke %6lld issued %6lld | warp %lld wait_start %6lld woke %6lld ld_done %6lld proc_done %6lld\n",
-                            2000 + i, tl[i * 8 + 0] - tl[0], tl[i * 8 + 1] - tl[0], tl[i * 8 + 6], tl[i * 8 + 2] - tl[0], tl[i * 8 + 3] - tl[0],
-                            tl[i * 8 + 4] - tl[0], tl[i * 8 + 5] - tl[0]);
-                prof.release();
-            }
-        } else {
-        PrefilterParams P;
+        TcParams P;
         P.seq = sv;
-        P.tab = T->d_tab.as<uint32_t>();
-        P.order = T->d_order.as<int32_t>();
-        P.mlen = mv.len;
-        P.lmax_all = std::max(T->lmax_fast, 1);
-        P.any_zero_hit = T->any_zero_hit;
-        P.cand = ctx->cand.as<uint64_t>();
-        P.cand_cap = cand_cap;
+        P.btab = TT->d_btab.as<uint8_t>();
+        P.lmax_all = std::max(TT->lmax_fast, 1);
+        P.any_zero_hit = TT->any_zero_hit;
+        lane_cap = std::max<int64_t>(cand_cap / 2 / n_lanes, 1);   // 16-byte records per lane buffer
+        if (attempt == 0 && ctx->opt_tc_first_lane_cap > 0) lane_cap = std::min<int64_t>(lane_cap, ctx->opt_tc_first_lane_cap);
+        MSB_TRY(ctx->lane_count.ensure((size_t) n_lanes * 4));
+        MSB_CUDA(cudaMemsetAsync(ctx->lane_count.p, 0, (size_t) n_lanes * 4, st));
+        P.cand = ctx->cand.as<uint4>();
+        P.cand_cap = lane_cap;
+        P.lane_count = ctx->lane_count.as<uint32_t>();
         P.dirty = ctx->dirty.as<int64_t>();
         P.dirty_cap = dirty_cap;
         P.counters = ctx->counters.as<unsigned long long>();
-        for (size_t b = 0; b < T->batches.size(); b++) {
-            P.batch = T->batches[b];
-            P.emit_dirty = (b == 0);
-            const size_t smem = (size_t) P.batch.tab_words * 4;
-            if (ctx->opt_prefilter_w == 8)
-                prefilter_kernel<8><<<ctx->sm_count, PF<8>::kThreads, smem, st>>>(P);
-            else
-                prefilter_kernel<4><<<ctx->sm_count, PF<4>::kThreads, smem, st>>>(P);
-            MSB_CUDA(cudaGetLastError());
-            ctx->c[MSB_C_LAUNCHES]++;
-            ctx->c[MSB_C_PREFILTER_LAUNCHES]++;
+        P.prof = nullptr;
+        DevBuf prof;
+        if (ctx->opt_tc_prof) {
+            MSB_TRY(prof.ensure((size_t) (ctx->sm_count + 16) * 16 * 8));
+            MSB_CUDA(cudaMemsetAsync(prof.p, 0, (size_t) (ctx->sm_count + 16) * 16 * 8, st));
+            P.prof = prof.as<long long>();
         }
+        const size_t smem = kTcSmemBytes;  // > half an SM's shared memory: one CTA per SM, which owns the TMEM
+        unsigned grid = 1;
+        for (size_t ri = 0; ri < ranges->size(); ri++) {
+            const auto &r = (*ranges)[ri];
+            if (before_range) MSB_TRY((*before_range)(ri));
+            P.pos_lo = r.first;
+            P.pos_hi = r.second;
+            const int64_t n_ptiles = (r.second + kTcTileBases - 1) / kTcTileBases - r.first / kTcTileBases;
+            grid = (unsigned) std::min<int64_t>(ctx->sm_count, n_ptiles);
+            for (size_t b = 0; b < TT->batches.size(); b++) {
+                P.batch = TT->batches[b];
+                P.emit_dirty = (b == 0);
+                if (ctx->opt_tc_prof) prefilter_tc_kernel<true><<<grid, kTcThreads, smem, st>>>(P);
+                else prefilter_tc_kernel<false><<<grid, kTcThreads, smem, st>>>(P);
+                MSB_CUDA(cudaGetLastError());
+                ctx->c[MSB_C_LAUNCHES]++;
+                ctx->c[MSB_C_PREFILTER_LAUNCHES]++;
+            }
+        }
+        lane_totals_kernel<<<(unsigned) std::min<int64_t>((n_lanes + 1023) / 1024, 128), 1024, 0, st>>>(ctx->lane_count.as<uint32_t>(), n_lanes, lane_cap,
+                                               ctx->counters.as<unsigned long long>());
+        MSB_CUDA(cudaGetLastError());
+        ctx->c[MSB_C_LAUNCHES]++;
+        if (ctx->opt_tc_prof) {
+            std::vector<long long> h((size_t) (ctx->sm_count + 16) * 16);
+            MSB_CUDA(cudaMemcpyAsync(h.data(), prof.p, h.size() * 8, cudaMemcpyDeviceToHost, st));
+            MSB_CUDA(cudaStreamSynchronize(st));
+            const long long *o = h.data();   // CTA 0 of the last batch
+            const double un = (double) std::max<long long>(o[4], 1);
+            fprintf(stderr, "[tc_prof] cta0: %lld units, %.0f clk/unit | issuer: wait stream %.0f, wait tmem_empty %.0f, issue %.0f | "
+                    "epilogue warp 4: wait stream %.0f, wait tmem_full %.0f, ld %.0f, process %.0f (clk/unit); "
+                    "units with a candidate %.3f, process there %.0f clk, elsewhere %.0f clk\n",
+                    o[4], o[0] / un, o[1] / un, o[2] / un, o[3] / un, o[11] / un, o[8] / un, o[9] / un, o[10] / un,
+                    o[14] / un, (double) o[13] / std::max<long long>(o[14], 1),
+                    (double) (o[10] - o[13]) / std::max<long long>(o[12] - o[14], 1));
+            const long long *tl = h.data() + (size_t) grid * 16;
+            for (int i = 0; i < 12; i++)
+                fprintf(stderr, "[tc_prof] unit %d: issuer woke %6lld issued %6lld | warp %lld wait_start %6lld woke %6lld ld_done %6lld proc_done %6lld\n",
+                        2000 + i, tl[i * 8 + 0] - tl[0], tl[i * 8 + 1] - tl[0], tl[i * 8 + 6], tl[i * 8 + 2] - tl[0], tl[i * 8 + 3] - tl[0],
+                        tl[i * 8 + 4] - tl[0], tl[i * 8 + 5] - tl[0]);
+            prof.release();
         }
         MSB_CUDA(cudaEventRecord(ctx->ev[1], st));
         MSB_TRY(read_counters(ctx));
-        n_cand = (int64_t) ctx->h_counters[0];   // keys (table prefilter) or records (tensor-core prefilter)
+        n_rec = (int64_t) ctx->h_counters[0];   // records: (window, 64-column chunk) pairs with at least one flagged accumulator
         n_dirty = (int64_t) ctx->h_counters[1];
-        bool overflow = n_cand > cand_cap;
-        int64_t need = n_cand + n_cand / 16 + 1024;
-        if (use_tc) {
-            // a lane that ran out of room only counted: grow every lane buffer to the largest count seen
-            n_rec = n_cand;
-            const int64_t worst = (int64_t) ctx->h_counters[3];
-            overflow = worst > lane_cap;
-            need = (worst + worst / 8 + 16) * 2 * n_lanes;
-        }
+        // a lane that ran out of room only counted: grow every lane buffer to the largest count seen
+        const int64_t worst = (int64_t) ctx->h_counters[3];
+        const bool overflow = worst > lane_cap;
         if (!overflow && n_dirty <= dirty_cap) break;
         if (attempt >= 2) { set_error("msb_scan: candidate buffers kept overflowing"); return MSB_ENOMEM; }
         ctx->c[MSB_C_RETRIES]++;
-        if (overflow) cand_cap = std::max(cand_cap, need);
+        if (overflow) cand_cap = std::max(cand_cap, (worst + worst / 8 + 16) * 2 * n_lanes);
         dirty_cap = std::max(dirty_cap, n_dirty + n_dirty / 16 + 1024);
         MSB_CUDA(cudaEventRecord(ctx->ev[0], st));
     }
-    if (use_tc) n_cand = n_rec;   // records: (window, 64-column chunk) pairs with at least one flagged accumulator
-    ctx->c[MSB_C_CANDIDATES] = n_cand;
+    ctx->c[MSB_C_CANDIDATES] = n_rec;
     ctx->c[MSB_C_DIRTY] = n_dirty;
 
     // ---- stage 2: exact fp64 re-score ----------------------------------------------------------
-    int64_t hit_cap = std::max<int64_t>(n_cand + (use_tc ? n_cand / 4 : 0) + 1024, 1 << 16);   // a record can flag several columns
+    int64_t hit_cap = std::max<int64_t>(n_rec + n_rec / 4 + 1024, 1 << 16);   // a record can flag several columns
     if (n_dirty) hit_cap += std::min<int64_t>(n_dirty * 2 * std::max(n_fast, 1), 1 << 24);
     if (n_slow) hit_cap += 1 << 20;
     if (ctx->hit_key.cap / 8 > (size_t) hit_cap) hit_cap = (int64_t) (ctx->hit_key.cap / 8);
@@ -1569,15 +1359,10 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
             }
             ctx->c[MSB_C_LAUNCHES]++;
         }
-        if (use_tc && n_rec) {
+        if (n_rec) {
             exact_records_kernel<<<(unsigned) (((int64_t) n_lanes * 32 + 255) / 256), 256, 0, st>>>(
                 E, ctx->cand.as<uint4>(), lane_cap, ctx->lane_count.as<uint32_t>(), n_lanes, d_order,
                 TT->d_col_info.as<uint32_t>());
-            MSB_CUDA(cudaGetLastError());
-            ctx->c[MSB_C_LAUNCHES]++;
-        } else if (!use_tc && n_cand) {
-            exact_candidates_kernel<<<(unsigned) ((n_cand + 255) / 256), 256, 0, st>>>(
-                E, ctx->cand.as<uint64_t>(), n_cand, d_order, nullptr);
             MSB_CUDA(cudaGetLastError());
             ctx->c[MSB_C_LAUNCHES]++;
         }
@@ -1750,8 +1535,6 @@ extern "C" {
 
 int msb_ctx_set_option(msb_ctx *ctx, const char *name, int value) {
     if (!ctx) { set_error("msb_ctx_set_option: null ctx"); return MSB_EINVAL; }
-    if (name && !std::strcmp(name, "prefilter_w") && (value == 4 || value == 8)) { ctx->opt_prefilter_w = value; return MSB_OK; }
-    if (name && !std::strcmp(name, "prefilter_tc") && (value == 0 || value == 1)) { ctx->opt_prefilter_tc = value; return MSB_OK; }
     if (name && !std::strcmp(name, "tc_prof") && (value == 0 || value == 1)) { ctx->opt_tc_prof = value; return MSB_OK; }
     if (name && !std::strcmp(name, "tc_first_lane_cap") && value >= 0) { ctx->opt_tc_first_lane_cap = value; return MSB_OK; }
     if (name && !std::strcmp(name, "ascii_slices") && value >= 1 && value <= 7) { ctx->opt_ascii_slices = value; return MSB_OK; }
@@ -1907,9 +1690,9 @@ int msb_scan_ascii(msb_ctx *ctx, const msb_motifs *M, int64_t n_seqs, const char
     }
     MSB_CUDA(cudaSetDevice(ctx->device));
     const int64_t total_bp = seq_off[n_seqs];
-    // Small inputs, the table prefilter (no range launches) and an unusable copy stream take the plain path.
+    // Small inputs and an unusable copy stream take the plain path.
     const int kSlices = ctx->opt_ascii_slices;
-    bool sliced = ctx->opt_prefilter_tc != 0 && total_bp >= (8 << 20) && n_seqs >= kSlices;
+    bool sliced = total_bp >= (8 << 20) && n_seqs >= kSlices;
     if (sliced && ensure_copy_stream(ctx) != MSB_OK) sliced = false;
     if (sliced && !ctx->slice_ev[0]) {
         for (auto &evt : ctx->slice_ev)
@@ -2641,7 +2424,7 @@ int msb_score_select(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *S, int s
     MSB_CUDA(cudaMemcpyAsync(ctx->ranks.p, ranks, (size_t) n_ranks * 8, cudaMemcpyHostToDevice, st));
     double score_ms = 0, select_ms = 0;
     const int64_t kPilot = kSelSmemKeys;   // a pilot row fits the select kernel's shared-memory staging
-    const bool pilot = ctx->opt_select_pilot && ctx->opt_prefilter_tc && S->n >= 8 * kPilot && (deepest + 1) * 32 <= S->n;
+    const bool pilot = ctx->opt_select_pilot && S->n >= 8 * kPilot && (deepest + 1) * 32 <= S->n;
     ctx->c[MSB_C_RETRIES] = 0;
     if (!pilot) {
         MSB_TRY(score_select_direct(ctx, M, S, strand, 0, M->n, n_ranks, out, &score_ms, &select_ms));

@@ -1,6 +1,6 @@
 // prefilter_tc.cuh -- tensor-core prefilter (tcgen05.mma kind::f8f6f4, sm_100a).
 //
-// Same contract as prefilter_kernel (kernels.cuh): emit a SUPERSET of the windows the reference
+// The scan's first stage: emit a SUPERSET of the windows the reference
 // accepts (cscore.c:340-389); the fp64 exact stage decides.  Formulation:
 //
 //     D[128 windows x 256 motif-strands] = A[128 x K] * B[256 x K]^T,   K = 4 * Lpad  (e4m3 x e4m3 -> f16)
