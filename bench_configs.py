@@ -7,6 +7,8 @@
     python bench_configs.py enrich     configs[4]: 200k target + 200k control 1 kb regions, 1900 motifs
     python bench_configs.py whole-genome --genome-scale 1 --gpus 8
                                        configs[3] genome with de-duplication (scan --whole-genome), tables and BED
+    python bench_configs.py variants --genome-scale 0.1 --alleles 4000000
+                                       motifscan variant: SNVs / MNVs of a seeded VCF against the resident genome
 
 Each prints one JSON line: device-resident and end-to-end time, throughput, and a parity check of a
 bounded sample against the reference's CPU implementation (oracle/_ref when it compiled, else the
@@ -555,9 +557,222 @@ def bench_whole_genome(args):
                     "region; one pass per leg, no warm-up besides the counts-only pass"}
 
 
+def _oracle_variant_rows(pg, pwms, cutoffs, v, strand=3):
+    """The reference's arithmetic on host-built contexts (oracle.scan_arrays on each allele's ref and alt context,
+    windows that overlap the changed bases, the other allele's window scored with oracle.score_arrays): rows
+    (allele, motif, chromosome start, strand, ref_score, alt_score, effect) in the contract's order."""
+    import oracle
+    lens = [int(np.asarray(p).shape[1]) for p in pwms]
+    lmax = max(lens)
+    seqs, meta = [], []
+    for a in range(len(v)):
+        c, p, alt = v.chroms[v.chrom[a]], int(v.pos[a]), v.alt[a]
+        cs, ce = max(p - lmax + 1, 0), min(p + len(alt) + lmax - 1, pg.chrom_sizes[c])
+        ref_ctx = pg.decode_bytes(c, cs, ce).decode()
+        seqs += [ref_ctx, ref_ctx[:p - cs] + alt + ref_ctx[p - cs + len(alt):]]
+        meta.append((cs, p - cs, len(alt)))
+    mats = [np.asarray(p).tolist() for p in pwms]
+    counts, seq_idx, start, score, strd = oracle.scan_arrays(mats, list(cutoffs), seqs, strand, n_threads=os.cpu_count() or 1)
+    hits = {}
+    for m, q, s, sc, x in zip(np.repeat(np.arange(len(pwms)), counts).tolist(), seq_idx.tolist(), start.tolist(),
+                              score.tolist(), strd.tolist()):
+        a, side = divmod(q, 2)
+        if s + lens[m] > meta[a][1] and s < meta[a][1] + meta[a][2]:
+            hits.setdefault((a, m, s, x), [None, None])[side] = sc
+    todo = {}
+    for key, sides in hits.items():
+        for side in (0, 1):
+            if sides[side] is None:
+                todo.setdefault((key[1], key[3]), []).append((key, side, seqs[2 * key[0] + side][key[2]:key[2] + lens[key[1]]]))
+    for (m, x), items in todo.items():
+        for (key, side, _), val in zip(items, oracle.score_arrays([mats[m]], [w for _, _, w in items], x)[0].tolist()):
+            hits[key][side] = val
+    rows = []
+    for (a, m, s, x), (rs, al) in sorted(hits.items()):
+        rh, ah = rs - cutoffs[m] >= -1e-10, al - cutoffs[m] >= -1e-10
+        rows.append((a, m, meta[a][0] + s, x, rs, al, 3 if rh and ah else (1 if rh else 2)))
+    return rows
+
+
+def _synthetic_vcf(path, pg, n_alleles, seed=31):
+    """A seeded VCF of about `n_alleles` scanned alleles on `pg`: positions uniform over the non-N bases, REF from the
+    genome; ~90 % SNV records, ~8 % MNVs of 2-3 bases, ~2 % records with two ALTs, plus ~1 % records that are skipped
+    (indels, an unknown chromosome, a REF that does not match)."""
+    rng = np.random.default_rng(seed)
+    chroms = list(pg.chroms)
+    sizes = np.array([pg.chrom_sizes[c] for c in chroms], dtype=np.int64)
+    cum = np.concatenate([[0], np.cumsum(sizes)])
+    n_rec = int(n_alleles / 1.02)
+    kind = rng.random(n_rec)
+    r = np.where(kind < 0.90, 1, np.where(kind < 0.98, rng.integers(2, 4, n_rec), 1)).astype(np.int64)
+    two_alts = kind >= 0.98
+    pos = np.zeros(0, dtype=np.int64)
+    chrom = np.zeros(0, dtype=np.int64)
+    while len(pos) < n_rec:                      # uniform over the bases, rejecting N (and windows running off the end)
+        g = rng.integers(0, int(cum[-1]), 2 * n_rec)
+        c = np.searchsorted(cum, g, side="right") - 1
+        p = g - cum[c]
+        b = pg.block_off[c] + p // 32
+        ok = ((np.asarray(pg.nmask)[b] >> (p % 32).astype(np.uint32)) & 1) == 0
+        ok &= p + 3 <= sizes[c]
+        pos, chrom = np.concatenate([pos, p[ok]]), np.concatenate([chrom, c[ok]])
+    pos, chrom = pos[:n_rec], chrom[:n_rec]
+    acgt = np.frombuffer(b"ACGT", dtype=np.uint8)
+    k = np.arange(3)
+    q = pos[:, None] + k[None, :]
+    b = pg.block_off[chrom][:, None] + q // 32
+    word = np.asarray(pg.codes)[2 * b + (q % 32) // 16]
+    code = ((word >> (2 * (q % 16)).astype(np.uint32)) & 3).astype(np.int64)
+    isn = ((np.asarray(pg.nmask)[b] >> (q % 32).astype(np.uint32)) & 1) == 1
+    ref_bytes = np.where(isn, ord("N"), acgt[code]).astype(np.uint8)
+    alt_code = (code + rng.integers(1, 4, (n_rec, 3))) % 4
+    alt2_code = (alt_code + rng.integers(1, 3, (n_rec, 3))) % 4
+    alt2_code = np.where(alt2_code == code, (alt2_code + 1) % 4, alt2_code)
+    alt_bytes, alt2_bytes = acgt[alt_code], acgt[alt2_code]
+    skip = rng.random(n_rec) < 0.01
+    lines = []
+    refs = [bytes(row).decode() for row in ref_bytes]
+    alts = [bytes(row).decode() for row in alt_bytes]
+    alts2 = [bytes(row).decode() for row in alt2_bytes]
+    for i in range(n_rec):
+        ri = int(r[i])
+        ref, alt = refs[i][:ri], alts[i][:ri]
+        if two_alts[i]:
+            alt += "," + alts2[i][:ri]
+        chrom_name = chroms[chrom[i]]
+        if skip[i]:
+            which = i % 3
+            if which == 0:
+                alt = alt.split(",")[0] + "T"                          # insertion: unsupported
+            elif which == 1:
+                chrom_name = "chrUnknown"
+            else:
+                ref = alt.split(",")[0]                                # REF differs from the genome: ref_mismatch
+        lines.append(f"{chrom_name}\t{pos[i] + 1}\tv{i}\t{ref}\t{alt}\t.\tPASS\t.\n")
+    with open(path, "w") as fh:
+        fh.write("##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\n")
+        fh.writelines(lines)
+    return n_rec
+
+
+def bench_variants(args):
+    """`motifscan variant` on the configs[3]-shaped genome at `--genome-scale` with 750 motifs (cutoffs as `cli` makes
+    them) and a seeded VCF of `--alleles` alleles (default 4e6 x scale): VCF parsing, the device phases of
+    scan_variants, the native table writer, the whole command in a subprocess (wall time, peak RSS), and parity of a
+    seeded sample of alleles with the oracle.  Everything is written to a temporary directory that is deleted."""
+    import resource
+    import shutil
+    import subprocess
+    import tempfile
+    import bench
+    from motifscan_b200 import engine, synth
+    from motifscan_b200 import io as msio
+    from motifscan_b200.genome import DeviceGenome
+    from motifscan_b200.motif import MotifPwms, PositionWeightMatrix
+    from motifscan_b200.variants import Variants, read_vcf, scan_variants
+
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+    root = tempfile.mkdtemp(prefix="msb_var_", dir=args.out_dir)
+    try:
+        t0 = time.perf_counter()
+        pg = bench.make_genome(0, args.genome_scale)
+        gdir, mdir = os.path.join(root, "synth"), os.path.join(root, "jaspar_all")
+        os.makedirs(gdir), os.makedirs(mdir)
+        with open(os.path.join(gdir, "synth.fa"), "wb") as fh:
+            for c in pg.chroms:
+                fh.write(f">{c}\n".encode() + pg.decode_bytes(c, 0, pg.chrom_sizes[c]) + b"\n")
+        pg.save(os.path.join(gdir, "synth.packed"))
+        with open(os.path.join(gdir, "synth_bg_freq.txt"), "w") as fh:
+            fh.write("Base\tFrequency\n" + "".join(f"{b}\t{v}\n" for b, v in synth.BG.items()))
+        _, mats, ids = synth.motif_set(args.motifs, seed=2020)
+        ctx = engine.default_context(0)
+        mset = engine.MotifSet(ctx, mats)
+        bblob, boff = synth.background_samples(100000, 40, seed=1)
+        bg = engine.SequenceSet(ctx, blob=bblob, seq_off=boff)
+        cutoffs = np.maximum(np.around(engine.score_select(ctx, mset, bg, 3, [int(100000 * 1e-4) - 1])[:, 0], 8), 1e-6)
+        bg.close(), mset.close()
+        pwms = MotifPwms(name="jaspar_all", genome="synth")
+        for m, k, c in zip(mats, ids, cutoffs):
+            pwms.append(PositionWeightMatrix(m, name="TF" + k[2:6], matrix_id=k, cutoffs={"1e-4": float(c)}))
+        pwms.write_motifscan_pwms(os.path.join(mdir, "jaspar_all_synth_pwms.motifscan"))
+        n_alleles = args.alleles or int(4e6 * args.genome_scale)
+        vcf = os.path.join(root, "calls.vcf")
+        n_rec = _synthetic_vcf(vcf, pg, n_alleles)
+        setup_s = time.perf_counter() - t0
+
+        t0 = time.perf_counter()
+        v = read_vcf(vcf, pg)
+        parse_s = time.perf_counter() - t0
+        dg = DeviceGenome(pg, ctx)
+        runs = []
+        for _ in range(args.steps + 1):                                 # the first run warms up
+            sites = scan_variants(dg, mats, cutoffs, v)
+            runs.append((sites.seconds, sites.timings))
+        best = min(runs[1:], key=lambda x: x[0])
+        scan_s, dev = best
+        dev_total = sum(dev.values())
+        out = os.path.join(root, "tables")
+        t0 = time.perf_counter()
+        msio.write_variant_tables(out, pwms, v, sites)
+        write_s = time.perf_counter() - t0
+        out_bytes = {f: os.path.getsize(os.path.join(out, f)) for f in sorted(os.listdir(out))}
+        # parity: a seeded sample of alleles, scanned on their own and compared with the oracle and with the full run
+        rng = np.random.default_rng(5)
+        idx = np.sort(rng.choice(len(v), size=min(args.cpu_alleles, len(v)), replace=False))
+        sub = Variants(v.chroms, v.chrom[idx], v.pos[idx], [v.ref[i] for i in idx], [v.alt[i] for i in idx],
+                       [v.id[i] for i in idx], v.record[idx], v.skipped, v.n_records)
+        got = scan_variants(dg, mats, cutoffs, sub)
+        t0 = time.perf_counter()
+        want = _oracle_variant_rows(pg, mats, cutoffs, sub)
+        cpu_s = time.perf_counter() - t0
+        cols = list(zip(*want)) if want else [[]] * 7
+        same = (len(got) == len(want) and np.array_equal(got.allele, np.array(cols[0], np.int32))
+                and np.array_equal(got.motif, np.array(cols[1], np.int32)) and np.array_equal(got.start, np.array(cols[2], np.int64))
+                and np.array_equal(got.strand, np.array(cols[3], np.int8))
+                and np.array_equal(got.ref_score.view(np.uint64), np.array(cols[4], np.float64).view(np.uint64))
+                and np.array_equal(got.alt_score.view(np.uint64), np.array(cols[5], np.float64).view(np.uint64))
+                and np.array_equal(got.effect, np.array(cols[6], np.int8)))
+        in_full = np.isin(sites.allele, idx)
+        full_same = (np.array_equal(np.searchsorted(idx, sites.allele[in_full]), got.allele)
+                     and np.array_equal(sites.start[in_full], got.start) and np.array_equal(sites.motif[in_full], got.motif)
+                     and np.array_equal(sites.ref_score[in_full].view(np.uint64), got.ref_score.view(np.uint64))
+                     and np.array_equal(sites.alt_score[in_full].view(np.uint64), got.alt_score.view(np.uint64))
+                     and np.array_equal(sites.effect[in_full], got.effect))
+        dg.close()
+        # the whole command, as a user runs it (the packed cache next to the FASTA is used)
+        cmd = [sys.executable, "-m", "motifscan_b200", "variant", "-i", vcf, "-m", mdir, "-g", gdir, "-o",
+               os.path.join(root, "cli"), "-p", "1e-4"]
+        t0 = time.perf_counter()
+        proc = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True)
+        wall_s = time.perf_counter() - t0
+        if proc.returncode != 0:
+            raise SystemExit("motifscan variant failed:\n" + proc.stderr[-2000:])
+        rss_mb = resource.getrusage(resource.RUSAGE_CHILDREN).ru_maxrss / 1024.0
+        cli_same = all(open(os.path.join(root, "cli", f), "rb").read() == open(os.path.join(out, f), "rb").read()
+                       for f in out_bytes)
+        log = [line for line in proc.stderr.splitlines() if line.startswith("Scanned")]
+    finally:
+        shutil.rmtree(root, ignore_errors=True)
+    return {"config": f"motifscan variant: {n_rec} VCF records -> {len(v)} scanned alleles on a {sum(pg.chrom_sizes.values())} bp "
+                      f"synthetic genome (scale {args.genome_scale}) x {args.motifs} motifs, both strands, p=1e-4 cutoffs floored at 1e-6",
+            "card": smi.stdout.strip().splitlines(), "metric": "motif*bp/s over the context bases of both alleles",
+            "scan_s": scan_s, "value": sites.motif_bp / scan_s, "alleles_per_s": len(v) / scan_s,
+            "device_ms": dev, "device_ms_total": dev_total, "device_value": sites.motif_bp / max(dev_total / 1e3, 1e-12),
+            "motif_bp": sites.motif_bp, "context_bp_per_set": sites.context_bp, "rows": len(sites),
+            "rows_by_effect": sites.rows_by_effect(), "skipped": v.skipped, "vcf_parse_s": parse_s,
+            "writer": {"seconds": write_s, "bytes": out_bytes}, "setup_s": setup_s,
+            "cli": {"wall_s": wall_s, "peak_rss_mb": rss_mb, "tables_identical_to_the_library_run": bool(cli_same), "log": log},
+            "parity": {"sample_alleles": int(len(idx)), "rows": len(want), "identical_to_oracle": bool(same),
+                       "full_run_rows_of_the_sample_identical": bool(full_same), "oracle_s": cpu_s},
+            "note": "scan_s: scan_variants wall time (extract both context sets, two scans, rows, sort, copy back), best of "
+                    "--steps after one warm-up; device_ms per phase of that run"}
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome"])
+    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants"])
+    ap.add_argument("--alleles", type=int, default=None)
+    ap.add_argument("--cpu-alleles", dest="cpu_alleles", type=int, default=2000)
     ap.add_argument("--out-dir", dest="out_dir", default=None)
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--genome-scale", dest="genome_scale", type=float, default=0.1)
@@ -576,7 +791,7 @@ def main():
     if args.motifs is None:
         args.motifs = 1900 if args.which in ("enrich", "cli") else 750
     out = {"build": bench_build, "genome": bench_genome, "enrich": bench_enrich, "cli": bench_cli,
-           "whole-genome": bench_whole_genome}[args.which](args)
+           "whole-genome": bench_whole_genome, "variants": bench_variants}[args.which](args)
     if out is not None:
         print(json.dumps(out))
 

@@ -64,7 +64,7 @@ int msb_ctx_sync(msb_ctx *ctx);
 /* Per-phase device times (ms, CUDA events on the context's stream) of the last msb_scan /
  * msb_score / msb_seqs_from_ascii on this context.  Index by MSB_T_*. */
 enum { MSB_T_H2D = 0, MSB_T_ENCODE, MSB_T_PREFILTER, MSB_T_EXACT, MSB_T_ORDER, MSB_T_D2H,
-       MSB_T_SCORE, MSB_T_SELECT, MSB_T_COUNT };
+       MSB_T_SCORE, MSB_T_SELECT, MSB_T_ROWS, MSB_T_ROW_SORT, MSB_T_COUNT };
 int msb_ctx_timings(const msb_ctx *ctx, double *ms, int n);
 /* Counters of the last msb_scan: index by MSB_C_*. */
 enum { MSB_C_CANDIDATES = 0, MSB_C_DIRTY, MSB_C_HITS, MSB_C_LAUNCHES, MSB_C_RETRIES,
@@ -121,6 +121,13 @@ int msb_seqs_to_packed(msb_ctx *ctx, const msb_seqs *seqs, uint32_t *codes, uint
  * Only the 20 n bytes of the interval table cross PCIe. */
 int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx,
                      const int64_t *start, const int64_t *end, msb_seqs **out);
+/* msb_seqs_extract with bases substituted (the alternative alleles of a variant scan): after the cut, base
+ * sub_pos[k] of sequence i (relative to its clipped start), k in [sub_off[i], sub_off[i + 1]), becomes the A/C/G/T
+ * code sub_code[k] (0..3) and is no longer masked.  sub_off has n + 1 entries, sub_off[0] = 0; only the interval and
+ * substitution tables cross PCIe. */
+int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                           const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
+                           msb_seqs **out);
 /* Number of non-ACGT bases in each of n windows [start[i], start[i] + length) of sequence src_idx[i] of a
  * resident set (clipped at the sequence end): the device half of the background sampler's acceptance
  * test `seq.count('N') + seq.count('n') <= max_n` (genome/__init__.py:172-175) -- a window without
@@ -216,6 +223,21 @@ int msb_scan_device_boundary_sites(msb_ctx *ctx, int64_t cap, int64_t *n, int32_
  * the device: counts[m * n_seqs + s] = number of final sites, best[...] = their best score (NaN when empty).
  * n_seqs must be the scanned set's sequence count.  Not after MSB_SCAN_COUNTS or a compact scan. */
 int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, int64_t *counts, double *best);
+/* Variant-effect scan.  Sequence i of `ref` is allele i's context on the reference genome, sequence i of `alt` the
+ * same bases with the allele substituted (msb_seqs_extract / msb_seqs_extract_subst: equal lengths); the changed
+ * bases are [core_start[i], core_start[i] + core_len[i]) of it.  Both sets are scanned (msb_scan_device without
+ * flags); every final site whose window overlaps its core is re-scored on the other context with the reference's
+ * arithmetic and becomes a row when it is a site on at least one allele: effect 1 loss (site on ref only), 2 gain
+ * (alt only), 3 both -- one row per (allele, motif, start, strand), ordered by allele, motif, start, forward before
+ * reverse.  *n_rows receives the number of rows; read them with msb_scan_device_variant_rows.  Timings: prefilter /
+ * exact / order summed over the two scans, MSB_T_ROWS the row kernel, MSB_T_ROW_SORT the ordering of the rows. */
+int msb_scan_variants(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *ref, const msb_seqs *alt,
+                      const int32_t *core_start, const int32_t *core_len, int strand, int64_t *n_rows);
+/* The rows of the last msb_scan_variants (MSB_EINVAL after any other scan): *n receives their number, the arrays are
+ * filled when cap >= *n.  start is relative to the context; strand 1 / 2; ref_score / alt_score are the window's
+ * scores on the two alleles bit for bit; effect 1 / 2 / 3 as above.  MSB_T_D2H times the copies. */
+int msb_scan_device_variant_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *allele, int32_t *motif, int32_t *start,
+                                 int8_t *strand, double *ref_score, double *alt_score, int8_t *effect);
 int msb_result_wait(msb_result *res);
 int msb_result_total(const msb_result *res, int64_t *n_sites);
 int msb_result_counts(const msb_result *res, int64_t *counts /* n_motifs */);
@@ -273,6 +295,15 @@ int msb_format_cell_tables(int64_t n_rows, int32_t n_motifs, const int64_t *coun
 int msb_write_sites_bed(const char *path, int64_t n, const int32_t *group, const int32_t *start, const int64_t *group_base,
                         const double *score, const int8_t *strand, int32_t length, int64_t n_groups, const char *names,
                         const int64_t *name_off, int32_t n_threads);
+/* motif_variant_sites.xls written to `path`: `header` (may be NULL), then per row, in the given order,
+ * lead[lead_off[a] .. lead_off[a + 1]) of its allele a (the caller's "chrom<TAB>pos<TAB>id<TAB>ref<TAB>alt<TAB>"),
+ * motif_text[motif_off[m] .. motif_off[m + 1]) of its motif m ("id<TAB>name<TAB>"), then start, start + motif_len[m],
+ * '+' / '-', ref_score, alt_score (printed like Python's str()) and loss / gain / both for effect 1 / 2 / 3,
+ * tab-separated, "\n".  Formatted in blocks on up to n_threads host threads, written in order. */
+int msb_write_variant_table(const char *path, const char *header, int64_t n, const int32_t *allele, const int32_t *motif,
+                            const int32_t *start, const int8_t *strand, const double *ref_score, const double *alt_score,
+                            const int8_t *effect, int64_t n_alleles, const char *lead, const int64_t *lead_off, int32_t n_motifs,
+                            const char *motif_text, const int64_t *motif_off, const int32_t *motif_len, int32_t n_threads);
 int msb_text_free(char *text);
 
 /* ---- score (replaces motif_score_thread + motif_score, cscore.c:174-302) -------------------- */

@@ -18,7 +18,7 @@ MSB_SCAN_COUNTS = 2
 MSB_SCAN_ASYNC = 4
 MSB_SCAN_COMPACT = 8
 MSB_SEQS_ASYNC = 1
-T_NAMES = ("h2d", "encode", "prefilter", "exact", "order", "d2h", "score", "select")
+T_NAMES = ("h2d", "encode", "prefilter", "exact", "order", "d2h", "score", "select", "rows", "row_sort")
 C_NAMES = ("candidates", "dirty", "hits", "launches", "retries", "prefilter_launches")
 
 c_i32p = ctypes.POINTER(ctypes.c_int32)
@@ -52,6 +52,8 @@ SIGNATURES = {
     "msb_seqs_wait": (ctypes.c_int, [c_vp]),
     "msb_seqs_to_packed": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp]),
     "msb_seqs_extract": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, ctypes.POINTER(c_vp)]),
+    "msb_seqs_extract_subst": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, c_i64p, c_i32p, c_vp,
+                                              ctypes.POINTER(c_vp)]),
     "msb_seqs_lengths": (ctypes.c_int, [c_vp, c_i64p]),
     "msb_seqs_window_ncount": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, ctypes.c_int32, c_i32p]),
     "msb_seqs_set_start_limit": (ctypes.c_int, [c_vp, c_i32p]),
@@ -71,6 +73,9 @@ SIGNATURES = {
     "msb_scan_device_region_counts": (ctypes.c_int, [c_vp, c_i64p, ctypes.c_int32]),
     "msb_scan_device_boundary_sites": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_f64p, c_i8p, c_i8p]),
     "msb_scan_device_cell_stats": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int64, c_i64p, c_f64p]),
+    "msb_scan_variants": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
+    "msb_scan_device_variant_rows": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_i8p, c_f64p, c_f64p,
+                                                    c_i8p]),
     "msb_result_wait": (ctypes.c_int, [c_vp]),
     "msb_merge_motif_major": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, c_i64p, ctypes.POINTER(c_vp), c_vp,
                                              ctypes.c_int32, c_i64p, ctypes.c_int32]),
@@ -86,6 +91,9 @@ SIGNATURES = {
                                               ctypes.POINTER(c_vp), c_i64p, ctypes.POINTER(c_vp), c_i64p, ctypes.c_int32]),
     "msb_write_sites_bed": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int64, c_i32p, c_i32p, c_i64p, c_f64p, c_i8p, ctypes.c_int32,
                                            ctypes.c_int64, ctypes.c_char_p, c_i64p, ctypes.c_int32]),
+    "msb_write_variant_table": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int64, c_i32p, c_i32p, c_i32p, c_i8p,
+                                               c_f64p, c_f64p, c_i8p, ctypes.c_int64, ctypes.c_char_p, c_i64p, ctypes.c_int32,
+                                               ctypes.c_char_p, c_i64p, c_i32p, ctypes.c_int32]),
     "msb_text_free": (ctypes.c_int, [c_vp]),
     "msb_result_total": (ctypes.c_int, [c_vp, c_i64p]),
     "msb_result_counts": (ctypes.c_int, [c_vp, c_i64p]),

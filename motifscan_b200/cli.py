@@ -20,9 +20,13 @@ Same flags as the reference's subcommands (cli/main.py:407-430, 504-579) and the
     boundary are joined on the host.  There is no control set, so no enrichment: `-c`, `--cf` and `--loc` are
     errors; `-w`, `--n-random` and `--seed` are ignored;
 
+  * `variant` (not in the reference) scans the SNVs and MNVs of a VCF against the resident genome and reports the
+    motif sites each allele creates or destroys (motifscan_b200/variants.py; one GPU, `-t` ignored);
+
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir
     python -m motifscan_b200 scan --whole-genome -m <motif set> -g <genome> -o out_dir [--site]
     python -m motifscan_b200 motif --build <motif set> -g <genome>
+    python -m motifscan_b200 variant -i calls.vcf.gz -m <motif set> -g <genome> -o out_dir
 """
 import argparse
 import logging
@@ -184,6 +188,40 @@ def run_scan(args):
     return 0
 
 
+def run_variant(args):
+    """`variant`: sites gained / lost by the SNVs and MNVs of a VCF (variants.read_vcf / scan_variants)."""
+    from . import variants as msvar
+    from .genome import DeviceGenome
+    logger.info("===== Loading data =====")
+    genome = load_genome(args.genome)
+    pwms = load_built_pwms(args.motif, genome.name)
+    try:
+        cutoffs = [pwm.cutoffs[args.p_value] for pwm in pwms]
+    except (TypeError, KeyError):
+        raise SystemExit(f"motifscan: error: PWMs have no motif score cutoff set for P-value {args.p_value!r}")
+    pg = packed_genome(genome, PACKED_MIN_BP)
+    try:
+        vcf = msvar.read_vcf(args.input_file, pg)
+    except (OSError, UnicodeDecodeError, EOFError) as err:
+        raise SystemExit(f"motifscan variant: error: cannot read {args.input_file}: {err}")
+    except ValueError as err:
+        raise SystemExit(f"motifscan variant: error: {err}")
+    logger.info("===== Scanning variants =====")
+    dg = DeviceGenome(pg)
+    try:
+        sites = msvar.scan_variants(dg, pwms, cutoffs, vcf, strand=args.strand)
+    finally:
+        dg.close()
+    by = sites.rows_by_effect()
+    skipped = ", ".join(f"{k} {v}" for k, v in vcf.skipped.items())
+    logger.info(f"Scanned {len(vcf)} alleles (skipped: {skipped}) x {len(pwms)} motifs, {sites.motif_bp:.3e} motif*bp "
+                f"in {sites.seconds:.3f} s: {len(sites)} rows ({by['gain']} gain, {by['loss']} loss, {by['both']} both)")
+    logger.info("Saving the result tables")
+    msio.write_variant_tables(args.output_dir, pwms, vcf, sites)
+    logger.info("===== MotifScan Finished =====")
+    return 0
+
+
 def run_motif(args):
     if not args.build:
         raise SystemExit("motifscan motif: only --build is provided here (install / list need the remote databases)")
@@ -269,6 +307,17 @@ def make_parser():
     scan.add_argument("--plot", dest="plot_dist", action="store_true")
     scan.add_argument("--verbose", action="store_true")
     scan.set_defaults(func=run_scan)
+
+    variant = sub.add_parser("variant", help="Motif sites gained and lost by the SNVs / MNVs of a VCF.")
+    variant.add_argument("-i", dest="input_file", required=True, metavar="VCF")
+    variant.add_argument("-m", "--motif", dest="motif", required=True, metavar="NAME")
+    variant.add_argument("-g", "--genome", dest="genome", required=True, metavar="GENOME")
+    variant.add_argument("-p", dest="p_value", default="1e-4", choices=["1e-2", "1e-3", "1e-4", "1e-5", "1e-6"])
+    variant.add_argument("--strand", dest="strand", choices=["both", "+", "-"], default="both")
+    variant.add_argument("-t", "--threads", dest="n_threads", type=int, default=1)
+    variant.add_argument("-o", "--output-dir", dest="output_dir", required=True, metavar="DIR")
+    variant.add_argument("--verbose", action="store_true")
+    variant.set_defaults(func=run_variant)
 
     motif = sub.add_parser("motif", help="Motif set commands (only --build here).")
     motif.add_argument("--build", dest="build", metavar="NAME")

@@ -8,6 +8,8 @@
 //   decode_sites_kernel     sorted keys -> (seq_idx, start, strand); motif_offsets_kernel: CSR
 //   dedup_flags_kernel      adjacent-site de-duplication              (scanner.py:156-193)
 //   score0_kernel           offset-0 window score of every sequence     (cscore.c:191-223)
+//   extract_subst_kernel    resident-genome extraction with allele bases overlaid (variant contexts)
+//   variant_rows_kernel     sites of the ref / alt context scans -> gain / loss / both rows
 #pragma once
 #include "common.cuh"
 
@@ -74,18 +76,12 @@ encode_pack_kernel(const uint8_t *__restrict__ ascii, const int64_t *__restrict_
 // counterpart of Scanner._extract_seq's per-region fetch, scanner.py:71-87).  One thread per
 // 32-base block of the destination: 64 code bits + 32 mask bits funnel-shifted out of the source.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-extract_pack_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int64_t *__restrict__ src_start,
-                    const int64_t *__restrict__ poff, const int32_t *__restrict__ len, int64_t n_seqs,
-                    int64_t n_blocks, uint32_t *__restrict__ codes, uint32_t *__restrict__ nmask,
-                    int32_t *__restrict__ blk_seq) {
-    const int64_t b = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= n_blocks) return;
-    const int64_t p = b * kPadBases;
-    const int64_t s = find_seq(poff, n_seqs, p);
-    const int64_t j = p - __ldg(poff + s);
-    const int n = (int) min((int64_t) kPadBases, (int64_t) __ldg(len + s) - j);
-    uint32_t lo = 0, hi = 0, mask = 0;
+// The bases [j, j + n) (n <= 32) of destination sequence s, cut out of the source: returns the block's two code
+// words and its mask word, with every bit behind the n-th base cleared.
+__device__ __forceinline__ void extract_block(const SeqView &src, const int32_t *__restrict__ src_idx,
+                                              const int64_t *__restrict__ src_start, int64_t s, int64_t j, int n,
+                                              uint32_t &lo, uint32_t &hi, uint32_t &mask) {
+    lo = 0, hi = 0, mask = 0;
     if (n > 0) {
         const int64_t q = __ldg(src.poff + __ldg(src_idx + s)) + __ldg(src_start + s) + j;
         // the source buffers carry zero padding behind their last block (msb_seqs_from_ascii)
@@ -101,6 +97,53 @@ extract_pack_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int6
             if (n <= 16) { hi = 0; lo &= n == 16 ? 0xffffffffu : ((1u << (2 * n)) - 1u); }
             else hi &= (1u << (2 * (n - 16))) - 1u;
         }
+    }
+}
+
+__global__ void __launch_bounds__(256)
+extract_pack_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int64_t *__restrict__ src_start,
+                    const int64_t *__restrict__ poff, const int32_t *__restrict__ len, int64_t n_seqs,
+                    int64_t n_blocks, uint32_t *__restrict__ codes, uint32_t *__restrict__ nmask,
+                    int32_t *__restrict__ blk_seq) {
+    const int64_t b = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n_blocks) return;
+    const int64_t p = b * kPadBases;
+    const int64_t s = find_seq(poff, n_seqs, p);
+    const int64_t j = p - __ldg(poff + s);
+    const int n = (int) min((int64_t) kPadBases, (int64_t) __ldg(len + s) - j);
+    uint32_t lo, hi, mask;
+    extract_block(src, src_idx, src_start, s, j, n, lo, hi, mask);
+    codes[2 * b] = lo;
+    codes[2 * b + 1] = hi;
+    nmask[b] = mask;
+    blk_seq[b] = (int32_t) s;
+}
+
+// extract with substitutions (the alternative alleles of a variant scan): the same block extraction, then the
+// bases sub_pos[k] (relative to the destination sequence), k in [sub_off[s], sub_off[s + 1]), become the A/C/G/T
+// codes sub_code[k] and their N bits are cleared.  A sequence carries a handful of substituted bases (an SNV or
+// MNV), so every thread walks its sequence's list.
+__global__ void __launch_bounds__(256)
+extract_subst_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int64_t *__restrict__ src_start,
+                     const int64_t *__restrict__ sub_off, const int32_t *__restrict__ sub_pos,
+                     const uint8_t *__restrict__ sub_code, const int64_t *__restrict__ poff,
+                     const int32_t *__restrict__ len, int64_t n_seqs, int64_t n_blocks, uint32_t *__restrict__ codes,
+                     uint32_t *__restrict__ nmask, int32_t *__restrict__ blk_seq) {
+    const int64_t b = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n_blocks) return;
+    const int64_t p = b * kPadBases;
+    const int64_t s = find_seq(poff, n_seqs, p);
+    const int64_t j = p - __ldg(poff + s);
+    const int n = (int) min((int64_t) kPadBases, (int64_t) __ldg(len + s) - j);
+    uint32_t lo, hi, mask;
+    extract_block(src, src_idx, src_start, s, j, n, lo, hi, mask);
+    for (int64_t k = __ldg(sub_off + s), k1 = __ldg(sub_off + s + 1); k < k1; k++) {
+        const int64_t q = (int64_t) __ldg(sub_pos + k) - j;
+        if (q < 0 || q >= n) continue;
+        const uint32_t c = (uint32_t) __ldg(sub_code + k) & 3u;
+        mask &= ~(1u << q);
+        if (q < 16) lo = (lo & ~(3u << (2 * q))) | (c << (2 * q));
+        else hi = (hi & ~(3u << (2 * (q - 16)))) | (c << (2 * (q - 16)));
     }
     codes[2 * b] = lo;
     codes[2 * b + 1] = hi;
@@ -832,6 +875,81 @@ cell_stats_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ 
     }
     atomicAdd(count + cell, c);
     atomicMax(best + cell, k);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Variant rows (msb_scan_variants).  Sequence i of `ref` and of `alt` is allele i's context on the reference and
+// with the allele's bases substituted (same lengths, so the same packed layout); core [core_start[i], core_start[i] +
+// core_len[i]) holds the changed bases.  One thread per final site of either scan: a site whose window overlaps
+// the core is re-scored on the other context with the reference's arithmetic (exact_raw, cscore.c:341-389) and
+// becomes a row:
+//   ref-list site:  effect 1 (loss) or 3 (both, the alt window passes too);
+//   alt-list site:  effect 2 (gain) only when the ref window fails -- else the ref list already has the row.
+// Rows are appended (order restored by the sort on row_key = allele | motif | start | strand bit).
+// ---------------------------------------------------------------------------------------------
+struct VariantSide {
+    SeqView seq;                     // this list's contexts
+    const uint64_t *key;             // final sites of the scan of `seq` (motif in the key's motif field)
+    const int32_t *seq_idx, *start;
+    const int8_t *strand;
+    const double *score;
+    int64_t n;
+    int key_shift;
+};
+
+__device__ __forceinline__ bool site_predicate(const MotifView &M, uint32_t m, double raw, double &score) {
+    score = __ddiv_rn(raw, __ldg(M.max_raw + m));                        // cscore.c:357,374
+    return __dsub_rn(score, __ldg(M.cutoff + m)) >= -1e-10;              // cscore.c:358,375
+}
+
+__global__ void __launch_bounds__(256)
+variant_rows_kernel(VariantSide R, VariantSide A, MotifView M, const int32_t *__restrict__ core_start,
+                    const int32_t *__restrict__ core_len, int motif_bits, int start_bits,
+                    unsigned long long *__restrict__ n_rows, uint64_t *__restrict__ row_key,
+                    int32_t *__restrict__ row_idx, double *__restrict__ row_ref, double *__restrict__ row_alt,
+                    int8_t *__restrict__ row_eff) {
+    const int64_t t = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= R.n + A.n) return;
+    const bool from_ref = t < R.n;
+    const VariantSide &S = from_ref ? R : A;
+    const VariantSide &O = from_ref ? A : R;
+    const int64_t i = from_ref ? t : t - R.n;
+    const uint32_t m = site_motif(S.key[i], S.key_shift);
+    const int32_t s = S.seq_idx[i], st = S.start[i];
+    const int L = __ldg(M.len + m);
+    const int32_t c0 = __ldg(core_start + s), c1 = c0 + __ldg(core_len + s);
+    if (st >= c1 || st + L <= c0) return;                                // the window does not touch a changed base
+    const int rev = S.strand[i] == 2;
+    const double *pw = M.pwm + 4 * (int64_t) __ldg(M.col_off + m);
+    double other;
+    const bool other_hit = site_predicate(M, m, exact_raw(O.seq, pw, L, __ldg(O.seq.poff + s) + st, rev), other);
+    if (!from_ref && other_hit) return;                                  // a site on both alleles: the ref list's row
+    const unsigned long long slot = atomicAdd(n_rows, 1ull);
+    row_key[slot] = ((((uint64_t) s << motif_bits | m) << start_bits | (uint64_t) st) << 1) | (uint64_t) rev;
+    row_idx[slot] = (int32_t) slot;
+    row_ref[slot] = from_ref ? S.score[i] : other;
+    row_alt[slot] = from_ref ? other : S.score[i];
+    row_eff[slot] = (int8_t) (from_ref ? (other_hit ? 3 : 1) : 2);
+}
+
+// Sorted row keys + the permutation -> the row arrays in order.
+__global__ void __launch_bounds__(256)
+variant_gather_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ idx, int64_t n, int motif_bits,
+                      int start_bits, const double *__restrict__ ref_in, const double *__restrict__ alt_in,
+                      const int8_t *__restrict__ eff_in, int32_t *__restrict__ allele, int32_t *__restrict__ motif,
+                      int32_t *__restrict__ start, int8_t *__restrict__ strand, double *__restrict__ ref_out,
+                      double *__restrict__ alt_out, int8_t *__restrict__ eff_out) {
+    const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t k = key[i];
+    const int32_t j = idx[i];
+    allele[i] = (int32_t) (k >> (motif_bits + start_bits + 1));
+    motif[i] = (int32_t) ((k >> (start_bits + 1)) & ((1ull << motif_bits) - 1ull));
+    start[i] = (int32_t) ((k >> 1) & ((1ull << start_bits) - 1ull));
+    strand[i] = (int8_t) ((k & 1ull) + 1);
+    ref_out[i] = ref_in[j];
+    alt_out[i] = alt_in[j];
+    eff_out[i] = eff_in[j];
 }
 
 }  // namespace msb

@@ -83,6 +83,10 @@ struct msb_ctx {
     // boundary chains of the last de-duplicated range scan (msb_scan_device_boundary_sites)
     DevBuf bnd_range, bnd_cnt, bnd_dst, bnd_motif, bnd_seq, bnd_start, bnd_score, bnd_strand, bnd_flags;
     int64_t last_boundary = -1;            // sites in the bnd_* arrays; -1: the last scan collected none
+    // rows of the last msb_scan_variants (msb_scan_device_variant_rows): unsorted, sort keys, then in row order
+    DevBuf vr_key, vr_idx, vr_ref, vr_alt, vr_eff, vr_key_sorted, vr_idx_sorted, vr_core;
+    DevBuf vo_allele, vo_motif, vo_start, vo_strand, vo_ref, vo_alt, vo_eff;
+    int64_t last_variant_rows = -1;        // -1: the last scan was not a variant scan
     // Final site arrays of a scan.  Two sets, used alternately: the device-to-host copy of scan k's
     // sites (on d2h_stream, MSB_SCAN_ASYNC) reads one set while scan k + 1 fills the other.
     struct FinSet {
@@ -91,6 +95,8 @@ struct msb_ctx {
         bool pending = false;
     } fin[2];
     int fin_cur = 0;
+    bool fin_hold = false;                 // msb_scan_variants: the other set holds the ref scan's sites, which the alt scan
+                                           // must neither reuse nor release
     bool last_counts_only = false;
     bool last_compact = false;             // MSB_SCAN_COMPACT: fin[].start holds (packed position << 1 | strand) as uint32
     const msb_seqs *last_seqs = nullptr;   // the sequence set of the last scan (its layout decodes compact sites)
@@ -385,7 +391,9 @@ int msb_ctx_destroy(msb_ctx *ctx) {
                       &ctx->scores_sorted, &ctx->seg_off, &ctx->ranks, &ctx->sel, &ctx->keep, &ctx->keep_pos,
                       &ctx->motif_counts, &ctx->sel_aux, &ctx->limit1, &ctx->lane_count, &ctx->bnd_range,
                       &ctx->bnd_cnt, &ctx->bnd_dst, &ctx->bnd_motif, &ctx->bnd_seq, &ctx->bnd_start, &ctx->bnd_score,
-                      &ctx->bnd_strand, &ctx->bnd_flags})
+                      &ctx->bnd_strand, &ctx->bnd_flags, &ctx->vr_key, &ctx->vr_idx, &ctx->vr_ref, &ctx->vr_alt,
+                      &ctx->vr_eff, &ctx->vr_key_sorted, &ctx->vr_idx_sorted, &ctx->vr_core, &ctx->vo_allele,
+                      &ctx->vo_motif, &ctx->vo_start, &ctx->vo_strand, &ctx->vo_ref, &ctx->vo_alt, &ctx->vo_eff})
         b->release();
     if (ctx->d2h_stream) cudaStreamSynchronize(ctx->d2h_stream);
     for (auto &f : ctx->fin) {
@@ -760,25 +768,41 @@ int msb_seqs_to_packed(msb_ctx *ctx, const msb_seqs *S, uint32_t *codes, uint32_
     return MSB_OK;
 }
 
-int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx,
-                     const int64_t *start, const int64_t *end, msb_seqs **out) {
+}  // extern "C"
+
+// msb_seqs_extract, and with a substitution table (sub_off != nullptr) msb_seqs_extract_subst.
+static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                        const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
+                        msb_seqs **out, const char *what) {
     if (!ctx || !src || !out || n < 0 || (n > 0 && (!src_idx || !start || !end))) {
-        set_error("msb_seqs_extract: bad argument");
+        set_error(std::string(what) + ": bad argument");
         return MSB_EINVAL;
     }
     *out = nullptr;
-    if (src->ctx != ctx) { set_error("msb_seqs_extract: source belongs to another context"); return MSB_EINVAL; }
+    if (src->ctx != ctx) { set_error(std::string(what) + ": source belongs to another context"); return MSB_EINVAL; }
     MSB_TRY(seqs_ready(src));
     // pysam's fetch (genome/__init__.py:135) clips `end` at the sequence length; an interval that
     // starts behind it, or is reversed, is empty.
     std::vector<int64_t> seq_off((size_t) n + 1, 0), clipped_start((size_t) std::max<int64_t>(n, 1), 0);
     for (int64_t i = 0; i < n; i++) {
-        if (src_idx[i] < 0 || src_idx[i] >= src->n) { set_error("msb_seqs_extract: source index out of range"); return MSB_EINVAL; }
-        if (start[i] < 0) { set_error("msb_seqs_extract: negative start"); return MSB_EINVAL; }
+        if (src_idx[i] < 0 || src_idx[i] >= src->n) { set_error(std::string(what) + ": source index out of range"); return MSB_EINVAL; }
+        if (start[i] < 0) { set_error(std::string(what) + ": negative start"); return MSB_EINVAL; }
         const int64_t slen = src->seq_off[src_idx[i] + 1] - src->seq_off[src_idx[i]];
         const int64_t a = std::min(start[i], slen), b = std::min(end[i], slen);
         clipped_start[i] = a;
         seq_off[i + 1] = seq_off[i] + std::max<int64_t>(b - a, 0);
+    }
+    const int64_t n_sub = sub_off ? sub_off[n] : 0;
+    if (sub_off) {
+        if (sub_off[0] != 0 || (n_sub > 0 && (!sub_pos || !sub_code))) { set_error(std::string(what) + ": bad substitution table"); return MSB_EINVAL; }
+        for (int64_t i = 0; i < n; i++) {
+            if (sub_off[i + 1] < sub_off[i]) { set_error(std::string(what) + ": substitution offsets not ascending"); return MSB_EINVAL; }
+            for (int64_t k = sub_off[i]; k < sub_off[i + 1]; k++)
+                if (sub_pos[k] < 0 || sub_pos[k] >= seq_off[i + 1] - seq_off[i] || sub_code[k] > 3) {
+                    set_error(std::string(what) + ": substitution outside its sequence or not an A/C/G/T code");
+                    return MSB_EINVAL;
+                }
+        }
     }
     MSB_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
@@ -786,36 +810,69 @@ int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t
     msb_seqs *S = nullptr;
     std::vector<int32_t> lens;
     MSB_TRY(seqs_prepare(ctx, n, seq_off.data(), &S, lens));
-    // the interval table rides in the (otherwise unused here) ASCII scratch: src_idx (4n) | start (8n)
-    const size_t idx_bytes = ((size_t) n * 4 + 15) & ~(size_t) 15;
-    int rc = ctx->ascii.ensure(std::max<size_t>(idx_bytes + (size_t) n * 8, 16));
+    // the tables ride in the (otherwise unused here) ASCII scratch:
+    // src_idx (4n) | start (8n) [| sub_off (8 (n + 1)) | sub_pos (4 n_sub) | sub_code (n_sub)]
+    auto al = [](size_t x) { return (x + 15) & ~(size_t) 15; };
+    const size_t o_start = al((size_t) n * 4), o_soff = o_start + al((size_t) n * 8);
+    const size_t o_spos = o_soff + al((size_t) (n + 1) * 8), o_scode = o_spos + al((size_t) n_sub * 4);
+    const size_t bytes = sub_off ? o_scode + (size_t) n_sub : o_start + (size_t) n * 8;
+    int rc = ctx->ascii.ensure(std::max<size_t>(bytes, 16));
     if (rc != MSB_OK) { msb_seqs_destroy(S); return rc; }
+    char *base = (char *) ctx->ascii.p;
     const int64_t n_blocks = S->total_packed / kPadBases;
     cudaError_t e = cudaSuccess;
     auto step = [&](cudaError_t x) { if (e == cudaSuccess) e = x; };
     if (n) {
-        step(cudaMemcpyAsync(ctx->ascii.p, src_idx, (size_t) n * 4, cudaMemcpyHostToDevice, st));
-        step(cudaMemcpyAsync((char *) ctx->ascii.p + idx_bytes, clipped_start.data(), (size_t) n * 8, cudaMemcpyHostToDevice, st));
+        step(cudaMemcpyAsync(base, src_idx, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+        step(cudaMemcpyAsync(base + o_start, clipped_start.data(), (size_t) n * 8, cudaMemcpyHostToDevice, st));
+    }
+    if (sub_off) {
+        step(cudaMemcpyAsync(base + o_soff, sub_off, (size_t) (n + 1) * 8, cudaMemcpyHostToDevice, st));
+        if (n_sub) {
+            step(cudaMemcpyAsync(base + o_spos, sub_pos, (size_t) n_sub * 4, cudaMemcpyHostToDevice, st));
+            step(cudaMemcpyAsync(base + o_scode, sub_code, (size_t) n_sub, cudaMemcpyHostToDevice, st));
+        }
     }
     step(cudaEventRecord(ctx->ev[1], st));
     if (e == cudaSuccess && n_blocks > 0) {
         const int64_t grid = (n_blocks + 255) / 256;
-        extract_pack_kernel<<<(unsigned) grid, 256, 0, st>>>(
-            src->view(), ctx->ascii.as<int32_t>(), (const int64_t *) ((char *) ctx->ascii.p + idx_bytes),
-            S->d_poff.as<int64_t>(), S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(),
-            S->d_nmask.as<uint32_t>(), S->d_blk_seq.as<int32_t>());
+        if (sub_off)
+            extract_subst_kernel<<<(unsigned) grid, 256, 0, st>>>(
+                src->view(), (const int32_t *) base, (const int64_t *) (base + o_start), (const int64_t *) (base + o_soff),
+                (const int32_t *) (base + o_spos), (const uint8_t *) (base + o_scode), S->d_poff.as<int64_t>(),
+                S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(), S->d_nmask.as<uint32_t>(),
+                S->d_blk_seq.as<int32_t>());
+        else
+            extract_pack_kernel<<<(unsigned) grid, 256, 0, st>>>(
+                src->view(), (const int32_t *) base, (const int64_t *) (base + o_start), S->d_poff.as<int64_t>(),
+                S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(), S->d_nmask.as<uint32_t>(),
+                S->d_blk_seq.as<int32_t>());
         step(cudaGetLastError());
     }
     step(cudaEventRecord(ctx->ev[2], st));
     step(cudaStreamSynchronize(st));  // host tables go out of scope
     if (e != cudaSuccess) {
         msb_seqs_destroy(S);
-        return cuda_fail(e, "msb_seqs_extract", __FILE__, __LINE__);
+        return cuda_fail(e, what, __FILE__, __LINE__);
     }
     ctx->t[MSB_T_H2D] = ev_ms(ctx->ev[0], ctx->ev[1]);
     ctx->t[MSB_T_ENCODE] = ev_ms(ctx->ev[1], ctx->ev[2]);
     *out = S;
     return MSB_OK;
+}
+
+extern "C" {
+
+int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx,
+                     const int64_t *start, const int64_t *end, msb_seqs **out) {
+    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, out, "msb_seqs_extract");
+}
+
+int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                           const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
+                           msb_seqs **out) {
+    if (!sub_off) { set_error("msb_seqs_extract_subst: null substitution offsets"); return MSB_EINVAL; }
+    return seqs_extract(ctx, src, n, src_idx, start, end, sub_off, sub_pos, sub_code, out, "msb_seqs_extract_subst");
 }
 
 int msb_seqs_window_ncount(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
@@ -1192,6 +1249,7 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
     ctx->last_n_seqs = S->n;
     boundary = boundary && (flags & MSB_SCAN_DEDUP);
     ctx->last_boundary = boundary ? 0 : -1;
+    ctx->last_variant_rows = -1;
     // this scan's final arrays go to the set the previous scan did not use; a copy that still reads it
     // (an asynchronous result two scans back) is waited for on the device, not on the host
     const int fin_set = ctx->fin_cur ^ 1;
@@ -1401,7 +1459,7 @@ static int scan_device(msb_ctx *ctx, msb_motifs *M, const msb_seqs *S, int stran
         MSB_CUDA(cub::DeviceScan::ExclusiveSum(ctx->sort_tmp.p, scan_bytes, ctx->motif_counts.as<int64_t>(), F.offsets.as<int64_t>(), M->n + 1, st));
     } else if (n_hits) {
         const bool dedup = (flags & MSB_SCAN_DEDUP) != 0;
-        if ((size_t) n_hits * 25 > ((size_t) 4 << 30)) {
+        if ((size_t) n_hits * 25 > ((size_t) 4 << 30) && !ctx->fin_hold) {
             // a very large result (billions of sites): the other set of final arrays, which only exists so that a
             // copy can overlap the next scan, gives its memory back first
             msb_ctx::FinSet &O = ctx->fin[fin_set ^ 1];
@@ -1635,6 +1693,148 @@ int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, i
         const uint64_t k = keys[c], b = (k >> 63) ? (k & 0x7fffffffffffffffull) : ~k;   // order_key_inv
         std::memcpy(best + c, &b, 8);
     }
+    return MSB_OK;
+}
+
+int msb_scan_variants(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int32_t *core_start,
+                      const int32_t *core_len, int strand, int64_t *n_rows) {
+    if (!ctx || !M || !ref || !alt) { set_error("msb_scan_variants: null argument"); return MSB_EINVAL; }
+    if (ref->n != alt->n || ref->seq_off != alt->seq_off) {
+        set_error("msb_scan_variants: the ref and alt sets must hold sequences of the same lengths");
+        return MSB_EINVAL;
+    }
+    const int64_t n = ref->n;
+    if (n > 0 && (!core_start || !core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
+    int32_t max_len = 0;
+    for (int64_t i = 0; i < n; i++) {
+        const int64_t len = ref->seq_off[i + 1] - ref->seq_off[i];
+        max_len = std::max<int32_t>(max_len, (int32_t) len);
+        if (core_start[i] < 0 || core_len[i] < 1 || (int64_t) core_start[i] + core_len[i] > len) {
+            set_error("msb_scan_variants: core outside its context");
+            return MSB_EINVAL;
+        }
+    }
+    int seq_bits = 0, motif_bits = 0, start_bits = 0;
+    while ((1ll << seq_bits) < n) seq_bits++;
+    while ((1ll << motif_bits) < (int64_t) M->n) motif_bits++;
+    while ((1ll << start_bits) < (int64_t) max_len) start_bits++;
+    if (seq_bits + motif_bits + start_bits + 1 > 64) { set_error("msb_scan_variants: too many alleles x motifs x context bases for a 64-bit row key"); return MSB_EINVAL; }
+    // the two scans: the ref sites stay in their final set while the alt scan fills the other one
+    double t_pre = 0, t_exact = 0, t_order = 0;
+    MSB_TRY(scan_device(ctx, const_cast<msb_motifs *>(M), ref, strand, 0));
+    const msb_ctx::FinSet &FR = ctx->fin[ctx->fin_cur];
+    VariantSide R;
+    R.seq = ref->view();
+    R.key = FR.key.as<uint64_t>(); R.seq_idx = FR.seq.as<int32_t>(); R.start = FR.start.as<int32_t>();
+    R.strand = FR.strand.as<int8_t>(); R.score = FR.score.as<double>();
+    R.n = ctx->last_sites;
+    R.key_shift = ctx->last_key_shift;
+    t_pre += ctx->t[MSB_T_PREFILTER]; t_exact += ctx->t[MSB_T_EXACT]; t_order += ctx->t[MSB_T_ORDER];
+    const int64_t c_retries = ctx->c[MSB_C_RETRIES];
+    ctx->fin_hold = true;
+    const int rc_alt = scan_device(ctx, const_cast<msb_motifs *>(M), alt, strand, 0);
+    ctx->fin_hold = false;
+    MSB_TRY(rc_alt);
+    ctx->c[MSB_C_RETRIES] += c_retries;
+    const msb_ctx::FinSet &FA = ctx->fin[ctx->fin_cur];
+    VariantSide A;
+    A.seq = alt->view();
+    A.key = FA.key.as<uint64_t>(); A.seq_idx = FA.seq.as<int32_t>(); A.start = FA.start.as<int32_t>();
+    A.strand = FA.strand.as<int8_t>(); A.score = FA.score.as<double>();
+    A.n = ctx->last_sites;
+    A.key_shift = ctx->last_key_shift;
+    t_pre += ctx->t[MSB_T_PREFILTER]; t_exact += ctx->t[MSB_T_EXACT]; t_order += ctx->t[MSB_T_ORDER];
+    if (R.n == 0) R.key = nullptr;   // empty lists: nothing is read
+    if (A.n == 0) A.key = nullptr;
+    // rows: at most one per site of either list
+    cudaStream_t st = ctx->stream;
+    const int64_t cap = std::max<int64_t>(R.n + A.n, 1);
+    MSB_TRY(ctx->vr_key.ensure((size_t) cap * 8));
+    MSB_TRY(ctx->vr_idx.ensure((size_t) cap * 4));
+    MSB_TRY(ctx->vr_ref.ensure((size_t) cap * 8));
+    MSB_TRY(ctx->vr_alt.ensure((size_t) cap * 8));
+    MSB_TRY(ctx->vr_eff.ensure((size_t) cap));
+    MSB_TRY(ctx->vr_core.ensure((size_t) std::max<int64_t>(2 * n, 1) * 4));
+    if (n) {
+        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.p, core_start, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.as<int32_t>() + n, core_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+    }
+    MSB_CUDA(cudaMemsetAsync(ctx->counters.p, 0, sizeof(unsigned long long), st));
+    MSB_CUDA(cudaEventRecord(ctx->ev[4], st));
+    if (R.n + A.n) {
+        variant_rows_kernel<<<(unsigned) ((R.n + A.n + 255) / 256), 256, 0, st>>>(
+            R, A, M->view(), ctx->vr_core.as<int32_t>(), ctx->vr_core.as<int32_t>() + n, motif_bits, start_bits,
+            ctx->counters.as<unsigned long long>(), ctx->vr_key.as<uint64_t>(), ctx->vr_idx.as<int32_t>(),
+            ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>());
+        MSB_CUDA(cudaGetLastError());
+        ctx->c[MSB_C_LAUNCHES]++;
+    }
+    MSB_CUDA(cudaEventRecord(ctx->ev[5], st));
+    MSB_TRY(read_counters(ctx));
+    const int64_t rows = (int64_t) ctx->h_counters[0];
+    if (rows) {
+        // (allele, motif, start, strand) order: one radix sort of the row keys with the row index as the value
+        MSB_TRY(ctx->vr_key_sorted.ensure((size_t) rows * 8));
+        MSB_TRY(ctx->vr_idx_sorted.ensure((size_t) rows * 4));
+        MSB_TRY(ctx->vo_allele.ensure((size_t) rows * 4));
+        MSB_TRY(ctx->vo_motif.ensure((size_t) rows * 4));
+        MSB_TRY(ctx->vo_start.ensure((size_t) rows * 4));
+        MSB_TRY(ctx->vo_strand.ensure((size_t) rows));
+        MSB_TRY(ctx->vo_ref.ensure((size_t) rows * 8));
+        MSB_TRY(ctx->vo_alt.ensure((size_t) rows * 8));
+        MSB_TRY(ctx->vo_eff.ensure((size_t) rows));
+        const int end_bit = seq_bits + motif_bits + start_bits + 1;
+        size_t tmp_bytes = 0;
+        MSB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, ctx->vr_key.as<uint64_t>(), ctx->vr_key_sorted.as<uint64_t>(),
+                                                 ctx->vr_idx.as<int32_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, 0, end_bit, st));
+        MSB_TRY(ctx->sort_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        MSB_CUDA(cub::DeviceRadixSort::SortPairs(ctx->sort_tmp.p, tmp_bytes, ctx->vr_key.as<uint64_t>(), ctx->vr_key_sorted.as<uint64_t>(),
+                                                 ctx->vr_idx.as<int32_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, 0, end_bit, st));
+        variant_gather_kernel<<<(unsigned) ((rows + 255) / 256), 256, 0, st>>>(
+            ctx->vr_key_sorted.as<uint64_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, motif_bits, start_bits,
+            ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>(), ctx->vo_allele.as<int32_t>(),
+            ctx->vo_motif.as<int32_t>(), ctx->vo_start.as<int32_t>(), ctx->vo_strand.as<int8_t>(), ctx->vo_ref.as<double>(),
+            ctx->vo_alt.as<double>(), ctx->vo_eff.as<int8_t>());
+        MSB_CUDA(cudaGetLastError());
+        ctx->c[MSB_C_LAUNCHES] += 2;
+    }
+    MSB_CUDA(cudaEventRecord(ctx->ev[6], st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    ctx->t[MSB_T_PREFILTER] = t_pre;
+    ctx->t[MSB_T_EXACT] = t_exact;
+    ctx->t[MSB_T_ORDER] = t_order;
+    ctx->t[MSB_T_ROWS] = ev_ms(ctx->ev[4], ctx->ev[5]);
+    ctx->t[MSB_T_ROW_SORT] = ev_ms(ctx->ev[5], ctx->ev[6]);
+    ctx->t[MSB_T_D2H] = 0;
+    ctx->last_variant_rows = rows;
+    if (n_rows) *n_rows = rows;
+    return MSB_OK;
+}
+
+int msb_scan_device_variant_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *allele, int32_t *motif, int32_t *start,
+                                 int8_t *strand, double *ref_score, double *alt_score, int8_t *effect) {
+    if (!ctx || !n) { set_error("msb_scan_device_variant_rows: null"); return MSB_EINVAL; }
+    if (ctx->last_variant_rows < 0) { set_error("msb_scan_device_variant_rows: the last scan was not msb_scan_variants"); return MSB_EINVAL; }
+    const int64_t rows = ctx->last_variant_rows;
+    *n = rows;
+    if (rows == 0 || cap < rows) return MSB_OK;
+    if (!allele || !motif || !start || !strand || !ref_score || !alt_score || !effect) {
+        set_error("msb_scan_device_variant_rows: null array");
+        return MSB_EINVAL;
+    }
+    MSB_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    MSB_CUDA(cudaEventRecord(ctx->ev[0], st));
+    MSB_CUDA(cudaMemcpyAsync(allele, ctx->vo_allele.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(motif, ctx->vo_motif.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(start, ctx->vo_start.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(strand, ctx->vo_strand.p, (size_t) rows, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(ref_score, ctx->vo_ref.p, (size_t) rows * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(alt_score, ctx->vo_alt.p, (size_t) rows * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(effect, ctx->vo_eff.p, (size_t) rows, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaEventRecord(ctx->ev[1], st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    ctx->t[MSB_T_D2H] = ev_ms(ctx->ev[0], ctx->ev[1]);
     return MSB_OK;
 }
 
@@ -2297,6 +2497,69 @@ int msb_write_sites_bed(const char *path, int64_t n, const int32_t *group, const
     }
     if (std::fclose(f) != 0) io_ok = false;
     if (!io_ok) { set_error(std::string("msb_write_sites_bed: write to ") + path + " failed"); return MSB_EINVAL; }
+    return MSB_OK;
+}
+
+int msb_write_variant_table(const char *path, const char *header, int64_t n, const int32_t *allele, const int32_t *motif,
+                            const int32_t *start, const int8_t *strand, const double *ref_score, const double *alt_score,
+                            const int8_t *effect, int64_t n_alleles, const char *lead, const int64_t *lead_off, int32_t n_motifs,
+                            const char *motif_text, const int64_t *motif_off, const int32_t *motif_len, int32_t n_threads) {
+    if (!path || n < 0 || n_alleles < 0 || n_motifs < 0 || !lead_off || !motif_off || (n_motifs && !motif_len) ||
+        (n && (!allele || !motif || !start || !strand || !ref_score || !alt_score || !effect))) {
+        set_error("msb_write_variant_table: bad argument");
+        return MSB_EINVAL;
+    }
+    size_t lead_max = 0, motif_max = 0;
+    for (int64_t a = 0; a < n_alleles; a++) lead_max = std::max<size_t>(lead_max, (size_t) (lead_off[a + 1] - lead_off[a]));
+    for (int32_t m = 0; m < n_motifs; m++) motif_max = std::max<size_t>(motif_max, (size_t) (motif_off[m + 1] - motif_off[m]));
+    for (int64_t i = 0; i < n; i++)
+        if (allele[i] < 0 || allele[i] >= n_alleles || motif[i] < 0 || motif[i] >= n_motifs || effect[i] < 1 || effect[i] > 3) {
+            set_error("msb_write_variant_table: row refers to an unknown allele, motif or effect");
+            return MSB_EINVAL;
+        }
+    FILE *f = std::fopen(path, "wb");
+    if (!f) { set_error(std::string("msb_write_variant_table: cannot open ") + path); return MSB_EINVAL; }
+    bool io_ok = true;
+    if (header) {
+        const size_t hn = std::strlen(header);
+        io_ok = std::fwrite(header, 1, hn, f) == hn;
+    }
+    // blocks of rows formatted on host threads, written in order (msb_write_sites_bed's scheme)
+    const int nt = std::max(1, std::min<int>(n_threads, 64));
+    const int64_t block = 1 << 17;
+    const size_t line_max = lead_max + motif_max + 2 * 21 + 2 * 25 + 16;
+    std::vector<std::vector<char>> buf((size_t) nt);
+    std::vector<size_t> used((size_t) nt);
+    try { for (auto &b : buf) b.resize((size_t) std::min(n, block) * line_max); }
+    catch (const std::bad_alloc &) { std::fclose(f); set_error("out of host memory"); return MSB_ENOMEM; }
+    static const char *const kEffect[4] = {"", "loss", "gain", "both"};
+    for (int64_t r0 = 0; r0 < n && io_ok; r0 += block * nt) {
+        auto format = [&](int t) {
+            const int64_t a = std::min(n, r0 + block * t), b = std::min(n, a + block);
+            char *o = buf[t].data();
+            for (int64_t i = a; i < b; i++) {
+                const int32_t al = allele[i], m = motif[i];
+                const size_t ln = (size_t) (lead_off[al + 1] - lead_off[al]), mn = (size_t) (motif_off[m + 1] - motif_off[m]);
+                std::memcpy(o, lead + lead_off[al], ln); o += ln;
+                std::memcpy(o, motif_text + motif_off[m], mn); o += mn;
+                o += fmt_int(start[i], o);
+                *o++ = '\t'; o += fmt_int((int64_t) start[i] + motif_len[m], o);
+                *o++ = '\t'; *o++ = strand[i] == 1 ? '+' : '-';
+                *o++ = '\t'; o += py_float_str(ref_score[i], o);
+                *o++ = '\t'; o += py_float_str(alt_score[i], o);
+                *o++ = '\t';
+                const char *e = kEffect[effect[i]];
+                std::memcpy(o, e, 4); o += 4;
+                *o++ = '\n';
+            }
+            used[t] = (size_t) (o - buf[t].data());
+        };
+        run_threads(nt, format);
+        for (int t = 0; t < nt && io_ok; t++)
+            if (used[t] && std::fwrite(buf[t].data(), 1, used[t], f) != used[t]) io_ok = false;
+    }
+    if (std::fclose(f) != 0) io_ok = false;
+    if (!io_ok) { set_error(std::string("msb_write_variant_table: write to ") + path + " failed"); return MSB_EINVAL; }
     return MSB_OK;
 }
 

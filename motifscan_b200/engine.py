@@ -227,6 +227,28 @@ class SequenceSet:
                                              ptr(start, ctypes.c_int64), ptr(end, ctypes.c_int64), ctypes.byref(h)))
         return SequenceSet(self.ctx, _handle=h)
 
+    def extract_subst(self, src_idx, start, end, sub_off, sub_pos, sub_code):
+        """`extract` with bases substituted (msb_seqs_extract_subst): base sub_pos[k] of sequence i (relative to
+        its start), k in [sub_off[i], sub_off[i + 1]), becomes the A/C/G/T code sub_code[k] (0..3).  Only the
+        interval and substitution tables cross PCIe."""
+        src_idx = np.ascontiguousarray(np.asarray(src_idx, dtype=np.int32))
+        start = np.ascontiguousarray(np.asarray(start, dtype=np.int64))
+        end = np.ascontiguousarray(np.asarray(end, dtype=np.int64))
+        sub_off = np.ascontiguousarray(np.asarray(sub_off, dtype=np.int64))
+        sub_pos = np.ascontiguousarray(np.asarray(sub_pos, dtype=np.int32))
+        sub_code = np.ascontiguousarray(np.asarray(sub_code, dtype=np.uint8))
+        if not (src_idx.shape == start.shape == end.shape and src_idx.ndim == 1):
+            raise ValueError("src_idx, start and end must be 1-d arrays of one length")
+        if sub_off.shape != (len(src_idx) + 1,) or sub_pos.shape != sub_code.shape or len(sub_pos) != int(sub_off[-1]):
+            raise ValueError("sub_off must have n + 1 entries and sub_pos / sub_code sub_off[-1]")
+        h = ctypes.c_void_p()
+        with self.ctx._lock:
+            check(self._lib.msb_seqs_extract_subst(self.ctx._h, self._h, len(src_idx), ptr(src_idx, ctypes.c_int32),
+                                                   ptr(start, ctypes.c_int64), ptr(end, ctypes.c_int64),
+                                                   ptr(sub_off, ctypes.c_int64), ptr(sub_pos, ctypes.c_int32),
+                                                   ctypes.c_void_p(sub_code.ctypes.data), ctypes.byref(h)))
+        return SequenceSet(self.ctx, _handle=h)
+
     def window_ncount(self, src_idx, start, length):
         """Non-ACGT bases in each window [start[i], start[i] + length) of sequence src_idx[i]."""
         src_idx = np.ascontiguousarray(np.asarray(src_idx, dtype=np.int32))
@@ -527,6 +549,31 @@ def scan_ranges_device(ctx, motifs, seqs, strand, ranges, counts_only=False, rem
         check(ctx._lib.msb_scan_ranges_device(ctx._h, motifs._h, seqs._h, int(strand), flags, n, ptr(a, ctypes.c_int64),
                                               ptr(b, ctypes.c_int64), ptr(c, ctypes.c_int64), ctypes.byref(total)))
     return total.value
+
+
+def scan_variants(ctx, motifs, ref, alt, core_start, core_len, strand):
+    """Variant-effect scan (msb_scan_variants): sequence i of `ref` / `alt` is allele i's context without / with the
+    allele, its changed bases [core_start[i], core_start[i] + core_len[i]).  Returns a dict of row arrays in (allele,
+    motif, start, strand) order: allele int32, motif int32, start int32 (relative to the context), strand int8 (1 / 2),
+    ref_score / alt_score float64 (the window's exact score on each allele) and effect int8 (1 loss, 2 gain, 3 both)."""
+    core_start = np.ascontiguousarray(np.asarray(core_start, dtype=np.int32))
+    core_len = np.ascontiguousarray(np.asarray(core_len, dtype=np.int32))
+    if core_start.shape != (ref.n,) or core_len.shape != (ref.n,):
+        raise ValueError("one core per context is required")
+    n = ctypes.c_int64(0)
+    with ctx._lock:
+        check(ctx._lib.msb_scan_variants(ctx._h, motifs._h, ref._h, alt._h, ptr(core_start, ctypes.c_int32),
+                                         ptr(core_len, ctypes.c_int32), int(strand), ctypes.byref(n)))
+        k = n.value
+        out = dict(allele=np.zeros(k, np.int32), motif=np.zeros(k, np.int32), start=np.zeros(k, np.int32),
+                   strand=np.zeros(k, np.int8), ref_score=np.zeros(k, np.float64), alt_score=np.zeros(k, np.float64),
+                   effect=np.zeros(k, np.int8))
+        if k:
+            check(ctx._lib.msb_scan_device_variant_rows(
+                ctx._h, k, ctypes.byref(n), ptr(out["allele"], ctypes.c_int32), ptr(out["motif"], ctypes.c_int32),
+                ptr(out["start"], ctypes.c_int32), ptr(out["strand"], ctypes.c_int8), ptr(out["ref_score"], ctypes.c_double),
+                ptr(out["alt_score"], ctypes.c_double), ptr(out["effect"], ctypes.c_int8)))
+    return out
 
 
 def score(ctx, motifs, seqs, strand):

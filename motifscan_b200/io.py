@@ -5,6 +5,7 @@ columns and number formatting (`str()` of ints and Python floats), fed from the 
     motif_sites_score.xls    same header, the best score per motif or `NA`
     motif_sites/<id>_<name>_sites.bed   chrom, site start, start + L, '.', score, strand
     motif_enrichment.xls     sorted by (enriched p-value, -fold change)
+    motif_variant_sites.xls / motif_variant_summary.xls   `motifscan variant` (write_variant_tables)
 """
 import os
 import re
@@ -179,6 +180,58 @@ def write_sites_bed(output_dir, pwms, regions, motif_sites):
             for region, cell in zip(regions, per_motif):
                 for site in cell:
                     out.write(f"{region.chrom}\t{site.start}\t{site.start + pwm.length}\t.\t{site.score}\t{site.strand}\n")
+
+
+VARIANT_SITES_HEADER = ("chrom\tpos\tid\tref\talt\tmotif_id\tmotif_name\tstart\tend\tstrand\tref_score\talt_score\t"
+                        "effect\n")
+VARIANT_SUMMARY_HEADER = "motif_id\tmotif_name\tn_gain\tn_loss\tn_both\n"
+
+
+def write_variant_tables(output_dir, pwms, variants, sites):
+    """The two tables of `motifscan variant` (variants.scan_variants):
+
+        motif_variant_sites.xls    one row per (allele, motif, window, strand) that is a site on at least one allele:
+                                   chrom, pos, id, ref and alt as in the VCF (alt = the allele), motif id and name,
+                                   the window [start, end) 0-based half-open, strand, both scores and the effect
+        motif_variant_summary.xls  per motif, the alleles with at least one gain / loss / both row
+
+    The site rows are formatted by the library on host threads (msb_write_variant_table; scores like Python's
+    str()), so tens of millions of rows never become Python objects."""
+    import ctypes
+    from . import _lib
+    lib = _lib.load()
+    os.makedirs(output_dir, exist_ok=True)
+    allele = np.ascontiguousarray(sites.allele, dtype=np.int32)
+    used, row_allele = np.unique(allele, return_inverse=True)          # leads only for alleles with a row
+    row_allele = np.ascontiguousarray(row_allele, dtype=np.int32)
+    leads = [f"{variants.chroms[variants.chrom[a]]}\t{int(variants.pos[a]) + 1}\t{variants.id[a]}\t{variants.ref[a]}\t"
+             f"{variants.alt[a]}\t".encode() for a in used.tolist()]
+    lead_off = np.zeros(len(leads) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in leads], out=lead_off[1:])
+    mtext = [f"{pwm.matrix_id}\t{pwm.name}\t".encode() for pwm in pwms]
+    motif_off = np.zeros(len(mtext) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in mtext], out=motif_off[1:])
+    motif_len = np.array([int(pwm.length) for pwm in pwms] or [0], dtype=np.int32)
+    n = len(allele)
+    motif = np.ascontiguousarray(sites.motif, dtype=np.int32)
+    start = np.ascontiguousarray(sites.start, dtype=np.int32)
+    strand = np.ascontiguousarray(sites.strand, dtype=np.int8)
+    ref_score = np.ascontiguousarray(sites.ref_score, dtype=np.float64)
+    alt_score = np.ascontiguousarray(sites.alt_score, dtype=np.float64)
+    effect = np.ascontiguousarray(sites.effect, dtype=np.int8)
+    arrays = [(row_allele, ctypes.c_int32), (motif, ctypes.c_int32), (start, ctypes.c_int32), (strand, ctypes.c_int8),
+              (ref_score, ctypes.c_double), (alt_score, ctypes.c_double), (effect, ctypes.c_int8)]
+    _lib.check(lib.msb_write_variant_table(
+        os.path.join(output_dir, "motif_variant_sites.xls").encode(), VARIANT_SITES_HEADER.encode(), n,
+        *[_lib.ptr(a, ct) if n else None for a, ct in arrays], len(leads), b"".join(leads),
+        _lib.ptr(lead_off, ctypes.c_int64), len(pwms), b"".join(mtext), _lib.ptr(motif_off, ctypes.c_int64),
+        _lib.ptr(motif_len, ctypes.c_int32), min(os.cpu_count() or 1, 32)))
+    summary = sites.summary()
+    with open(os.path.join(output_dir, "motif_variant_summary.xls"), "w") as out:
+        out.write(VARIANT_SUMMARY_HEADER)
+        for m, pwm in enumerate(pwms):
+            out.write(f"{pwm.matrix_id}\t{pwm.name}\t{int(summary['n_gain'][m])}\t{int(summary['n_loss'][m])}\t"
+                      f"{int(summary['n_both'][m])}\n")
 
 
 def write_enrich_table(output_dir, enrichment_results):
