@@ -970,6 +970,8 @@ int msb_seqs_destroy(msb_seqs *S) {
 // (the 1e-12 term is > 1000x the worst-case rounding of the L-term double sum, the division
 // and the subtraction).  A window the reference can accept therefore has
 //     sum_c d[b_c][c]  <=  D = sum_c colmax_c - T (+ slack for the rounding of these host sums).
+// (For a motif longer than kMaxFastLen, colmax_c of a column behind the first kMaxFastLen is replaced by
+// max(colmax_c, 0): an N there adds 0; see tc_fill_column.)
 // The stored e4m3 entries are  e[b][c] = RU( beta - s * d[b][c] )  (rounded towards +inf, floored
 // at -448), with beta an e4m3 value, C = L * beta and s = (C - C/64) / D.  Then for every window
 // with sum d <= D:   sum_c e >= C - s * sum d >= C/64 > 5,  more than the tensor core's f16
@@ -1029,9 +1031,11 @@ static void tc_fill_column(const msb_motifs *M, int32_t m, int rev, uint8_t *til
     const double cutoff = M->cutoffs[m];
     if (!(max_raw > 0) || std::isnan(cutoff) || (std::isinf(cutoff) && cutoff > 0)) { tc_fill_never(tile, col); return; }
     // A motif longer than kMaxFastLen columns is prefiltered on its first kMaxFastLen columns (of this strand)
-    // alone: the columns behind them are taken at their best (deficit 0), which can only admit more
-    // windows -- the budget D below still comes from the whole motif, and sum over the kept columns of d <=
-    // sum over all columns of d <= D for every window the reference accepts.
+    // alone.  An N anywhere in those columns makes the window dirty (the producer's horizon), so on this path
+    // they hold A/C/G/T.  A column behind them may hold an N, which adds 0 (cscore.c:346): such a column
+    // contributes at most max(colmax_c, 0), more than colmax_c when all four entries are negative.  So the
+    // budget below takes colmax_c for the kept columns and max(colmax_c, 0) for the others; then the sum over
+    // the kept columns of d <= D for every window the reference accepts, whatever sits behind them.
     const int kept = std::min(L, kMaxFastLen);
     double cms = 0, abs_sum = 0;
     std::vector<double> colmax((size_t) L);
@@ -1039,7 +1043,7 @@ static void tc_fill_column(const msb_motifs *M, int32_t m, int rev, uint8_t *til
         double mx = -INFINITY, a = 0;
         for (int b = 0; b < 4; b++) { mx = std::max(mx, V(b, c)); a = std::max(a, std::fabs(V(b, c))); }
         colmax[c] = mx;
-        cms += mx;
+        cms += c < kept ? mx : std::max(mx, 0.0);
         abs_sum += a;
     }
     double D;
