@@ -7,8 +7,10 @@
     python bench_configs.py enrich     configs[4]: 200k target + 200k control 1 kb regions, 1900 motifs
     python bench_configs.py whole-genome --genome-scale 1 --gpus 8
                                        configs[3] genome with de-duplication (scan --whole-genome), tables and BED
-    python bench_configs.py variants --genome-scale 0.1 --alleles 4000000
-                                       motifscan variant: SNVs / MNVs of a seeded VCF against the resident genome
+    python bench_configs.py variants --genome-scale 0.1 --alleles 4000000 [--indel-fraction 0.15]
+                                       motifscan variant: SNVs / MNVs (and with --indel-fraction that share of
+                                       deletions and insertions, scanned with --indels) of a seeded VCF against
+                                       the resident genome
 
 Each prints one JSON line: device-resident and end-to-end time, throughput, and a parity check of a
 bounded sample against the reference's CPU implementation (oracle/_ref when it compiled, else the
@@ -557,47 +559,74 @@ def bench_whole_genome(args):
                     "region; one pass per leg, no warm-up besides the counts-only pass"}
 
 
+def _oracle_trim(ref, alt):
+    """(offset of the change in REF, r', inserted bases): an indel without its longest common prefix and then suffix
+    (bases compared as scoring sees them); SNVs / MNVs as they are."""
+    if len(ref) == len(alt):
+        return 0, len(ref), alt
+    code = lambda b: "ACGT".find(b.upper()) if b.upper() in "ACGT" else 4   # noqa: E731
+    m, pre, suf = min(len(ref), len(alt)), 0, 0
+    while pre < m and code(ref[pre]) == code(alt[pre]):
+        pre += 1
+    while suf < m - pre and code(ref[-1 - suf]) == code(alt[-1 - suf]):
+        suf += 1
+    return pre, len(ref) - pre - suf, alt[pre:len(alt) - suf]
+
+
 def _oracle_variant_rows(pg, pwms, cutoffs, v, strand=3):
     """The reference's arithmetic on host-built contexts (oracle.scan_arrays on each allele's ref and alt context,
     windows that overlap the changed bases, the other allele's window scored with oracle.score_arrays): rows
-    (allele, motif, chromosome start, strand, ref_score, alt_score, effect) in the contract's order."""
+    (allele, motif, chromosome start, strand, ref_score, alt_score, effect, paired) in the contract's order.  An indel's
+    window with no counterpart on the other allele is unpaired, its other score NaN."""
     import oracle
     lens = [int(np.asarray(p).shape[1]) for p in pwms]
     lmax = max(lens)
     seqs, meta = [], []
     for a in range(len(v)):
-        c, p, alt = v.chroms[v.chrom[a]], int(v.pos[a]), v.alt[a]
-        cs, ce = max(p - lmax + 1, 0), min(p + len(alt) + lmax - 1, pg.chrom_sizes[c])
+        c = v.chroms[v.chrom[a]]
+        pre, r, ins = _oracle_trim(v.ref[a], v.alt[a])
+        p = int(v.pos[a]) + pre
+        cs, ce = max(p - lmax + 1, 0), min(p + r + lmax - 1, pg.chrom_sizes[c])
         ref_ctx = pg.decode_bytes(c, cs, ce).decode()
-        seqs += [ref_ctx, ref_ctx[:p - cs] + alt + ref_ctx[p - cs + len(alt):]]
-        meta.append((cs, p - cs, len(alt)))
+        seqs += [ref_ctx, ref_ctx[:p - cs] + ins + ref_ctx[p - cs + r:]]
+        meta.append((cs, p - cs, r, len(ins)))
     mats = [np.asarray(p).tolist() for p in pwms]
     counts, seq_idx, start, score, strd = oracle.scan_arrays(mats, list(cutoffs), seqs, strand, n_threads=os.cpu_count() or 1)
     hits = {}
     for m, q, s, sc, x in zip(np.repeat(np.arange(len(pwms)), counts).tolist(), seq_idx.tolist(), start.tolist(),
                               score.tolist(), strd.tolist()):
         a, side = divmod(q, 2)
-        if s + lens[m] > meta[a][1] and s < meta[a][1] + meta[a][2]:
-            hits.setdefault((a, m, s, x), [None, None])[side] = sc
+        cs, c0, r, k_alt = meta[a]
+        if s + lens[m] > c0 and s < c0 + (k_alt if side else r):
+            paired = s < c0 + min(r, k_alt) and s + lens[m] <= len(seqs[2 * a + 1 - side])
+            hits.setdefault((a, m, s, x) if paired else (a, m, s, x, side), [None, None])[side] = sc
     todo = {}
     for key, sides in hits.items():
         for side in (0, 1):
-            if sides[side] is None:
+            if len(key) == 4 and sides[side] is None:
                 todo.setdefault((key[1], key[3]), []).append((key, side, seqs[2 * key[0] + side][key[2]:key[2] + lens[key[1]]]))
     for (m, x), items in todo.items():
         for (key, side, _), val in zip(items, oracle.score_arrays([mats[m]], [w for _, _, w in items], x)[0].tolist()):
             hits[key][side] = val
     rows = []
-    for (a, m, s, x), (rs, al) in sorted(hits.items()):
+    for key, (rs, al) in hits.items():
+        a, m, s, x = key[:4]
+        if len(key) == 5:
+            rows.append((a, m, meta[a][0] + s, x, np.nan if rs is None else rs, np.nan if al is None else al,
+                         1 if key[4] == 0 else 2, False))
+            continue
         rh, ah = rs - cutoffs[m] >= -1e-10, al - cutoffs[m] >= -1e-10
-        rows.append((a, m, meta[a][0] + s, x, rs, al, 3 if rh and ah else (1 if rh else 2)))
+        rows.append((a, m, meta[a][0] + s, x, rs, al, 3 if rh and ah else (1 if rh else 2), True))
+    rows.sort(key=lambda t: t[:4])
     return rows
 
 
-def _synthetic_vcf(path, pg, n_alleles, seed=31):
+def _synthetic_vcf(path, pg, n_alleles, seed=31, indel_fraction=0.0):
     """A seeded VCF of about `n_alleles` scanned alleles on `pg`: positions uniform over the non-N bases, REF from the
     genome; ~90 % SNV records, ~8 % MNVs of 2-3 bases, ~2 % records with two ALTs, plus ~1 % records that are skipped
-    (indels, an unknown chromosome, a REF that does not match)."""
+    (indels, an unknown chromosome, a REF that does not match).  `indel_fraction` of the other records become
+    deletions or insertions (half each) of 1-50 bases, 1 % of them of 80-150 bases, longer than every motif (drawn
+    from their own seeded stream, so 0 leaves the file as it is)."""
     rng = np.random.default_rng(seed)
     chroms = list(pg.chroms)
     sizes = np.array([pg.chrom_sizes[c] for c in chroms], dtype=np.int64)
@@ -630,6 +659,13 @@ def _synthetic_vcf(path, pg, n_alleles, seed=31):
     alt2_code = np.where(alt2_code == code, (alt2_code + 1) % 4, alt2_code)
     alt_bytes, alt2_bytes = acgt[alt_code], acgt[alt2_code]
     skip = rng.random(n_rec) < 0.01
+    indel = np.zeros(n_rec, dtype=bool)
+    if indel_fraction > 0:
+        irng = np.random.default_rng(seed + 1)
+        indel = (irng.random(n_rec) < indel_fraction) & ~skip
+        ilen = np.where(irng.random(n_rec) < 0.01, irng.integers(80, 151, n_rec), irng.integers(1, 51, n_rec))
+        is_del = irng.random(n_rec) < 0.5
+        ins_bases = acgt[irng.integers(0, 4, (n_rec, 150))]
     lines = []
     refs = [bytes(row).decode() for row in ref_bytes]
     alts = [bytes(row).decode() for row in alt_bytes]
@@ -640,6 +676,14 @@ def _synthetic_vcf(path, pg, n_alleles, seed=31):
         if two_alts[i]:
             alt += "," + alts2[i][:ri]
         chrom_name = chroms[chrom[i]]
+        if indel[i]:
+            k = int(ilen[i])
+            if is_del[i]:
+                ref = pg.decode_bytes(chrom_name, int(pos[i]), min(int(pos[i]) + 1 + k, int(sizes[chrom[i]]))).decode()
+                alt = ref[0]
+            else:
+                ref = refs[i][0]
+                alt = ref + bytes(ins_bases[i, :k]).decode()
         if skip[i]:
             which = i % 3
             if which == 0:
@@ -697,11 +741,12 @@ def bench_variants(args):
         pwms.write_motifscan_pwms(os.path.join(mdir, "jaspar_all_synth_pwms.motifscan"))
         n_alleles = args.alleles or int(4e6 * args.genome_scale)
         vcf = os.path.join(root, "calls.vcf")
-        n_rec = _synthetic_vcf(vcf, pg, n_alleles)
+        indels = args.indel_fraction > 0
+        n_rec = _synthetic_vcf(vcf, pg, n_alleles, indel_fraction=args.indel_fraction)
         setup_s = time.perf_counter() - t0
 
         t0 = time.perf_counter()
-        v = read_vcf(vcf, pg)
+        v = read_vcf(vcf, pg, indels=indels)
         parse_s = time.perf_counter() - t0
         dg = DeviceGenome(pg, ctx)
         runs = []
@@ -720,28 +765,28 @@ def bench_variants(args):
         rng = np.random.default_rng(5)
         idx = np.sort(rng.choice(len(v), size=min(args.cpu_alleles, len(v)), replace=False))
         sub = Variants(v.chroms, v.chrom[idx], v.pos[idx], [v.ref[i] for i in idx], [v.alt[i] for i in idx],
-                       [v.id[i] for i in idx], v.record[idx], v.skipped, v.n_records)
+                       [v.id[i] for i in idx], v.record[idx], v.skipped, v.n_records, indels=v.indels)
         got = scan_variants(dg, mats, cutoffs, sub)
         t0 = time.perf_counter()
         want = _oracle_variant_rows(pg, mats, cutoffs, sub)
         cpu_s = time.perf_counter() - t0
-        cols = list(zip(*want)) if want else [[]] * 7
+        cols = list(zip(*want)) if want else [[]] * 8
         same = (len(got) == len(want) and np.array_equal(got.allele, np.array(cols[0], np.int32))
                 and np.array_equal(got.motif, np.array(cols[1], np.int32)) and np.array_equal(got.start, np.array(cols[2], np.int64))
                 and np.array_equal(got.strand, np.array(cols[3], np.int8))
                 and np.array_equal(got.ref_score.view(np.uint64), np.array(cols[4], np.float64).view(np.uint64))
                 and np.array_equal(got.alt_score.view(np.uint64), np.array(cols[5], np.float64).view(np.uint64))
-                and np.array_equal(got.effect, np.array(cols[6], np.int8)))
+                and np.array_equal(got.effect, np.array(cols[6], np.int8)) and np.array_equal(got.paired, np.array(cols[7], bool)))
         in_full = np.isin(sites.allele, idx)
         full_same = (np.array_equal(np.searchsorted(idx, sites.allele[in_full]), got.allele)
                      and np.array_equal(sites.start[in_full], got.start) and np.array_equal(sites.motif[in_full], got.motif)
                      and np.array_equal(sites.ref_score[in_full].view(np.uint64), got.ref_score.view(np.uint64))
                      and np.array_equal(sites.alt_score[in_full].view(np.uint64), got.alt_score.view(np.uint64))
-                     and np.array_equal(sites.effect[in_full], got.effect))
+                     and np.array_equal(sites.effect[in_full], got.effect) and np.array_equal(sites.paired[in_full], got.paired))
         dg.close()
         # the whole command, as a user runs it (the packed cache next to the FASTA is used)
         cmd = [sys.executable, "-m", "motifscan_b200", "variant", "-i", vcf, "-m", mdir, "-g", gdir, "-o",
-               os.path.join(root, "cli"), "-p", "1e-4"]
+               os.path.join(root, "cli"), "-p", "1e-4"] + (["--indels"] if indels else [])
         t0 = time.perf_counter()
         proc = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True)
         wall_s = time.perf_counter() - t0
@@ -753,7 +798,15 @@ def bench_variants(args):
         log = [line for line in proc.stderr.splitlines() if line.startswith("Scanned")]
     finally:
         shutil.rmtree(root, ignore_errors=True)
-    return {"config": f"motifscan variant: {n_rec} VCF records -> {len(v)} scanned alleles on a {sum(pg.chrom_sizes.values())} bp "
+    extra = {}
+    if indels:
+        is_indel = np.fromiter((len(a) != len(r) for a, r in zip(v.alt, v.ref)), dtype=bool, count=len(v))
+        extra = {"indel_fraction": args.indel_fraction, "indel_alleles": int(is_indel.sum()),
+                 "sample_indel_alleles": int(is_indel[idx].sum()),
+                 "rows_by_pairing": {"paired": int(sites.paired.sum()),
+                                     "unpaired_loss": int((~sites.paired & (sites.effect == 1)).sum()),
+                                     "unpaired_gain": int((~sites.paired & (sites.effect == 2)).sum())}}
+    return {**extra, "config": f"motifscan variant: {n_rec} VCF records -> {len(v)} scanned alleles on a {sum(pg.chrom_sizes.values())} bp "
                       f"synthetic genome (scale {args.genome_scale}) x {args.motifs} motifs, both strands, p=1e-4 cutoffs floored at 1e-6",
             "card": smi.stdout.strip().splitlines(), "metric": "motif*bp/s over the context bases of both alleles",
             "scan_s": scan_s, "value": sites.motif_bp / scan_s, "alleles_per_s": len(v) / scan_s,
@@ -773,6 +826,7 @@ def main():
     ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants"])
     ap.add_argument("--alleles", type=int, default=None)
     ap.add_argument("--cpu-alleles", dest="cpu_alleles", type=int, default=2000)
+    ap.add_argument("--indel-fraction", dest="indel_fraction", type=float, default=0.0)
     ap.add_argument("--out-dir", dest="out_dir", default=None)
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--genome-scale", dest="genome_scale", type=float, default=0.1)

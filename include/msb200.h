@@ -128,6 +128,14 @@ int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t
 int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
                            const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
                            msb_seqs **out);
+/* msb_seqs_extract with a splice (the alternative alleles of a variant scan with indels): sequence i is the cut
+ * interval (clipped like msb_seqs_extract) with its bases [splice_at[i], splice_at[i] + del_len[i]) replaced by the
+ * A/C/G/T codes ins_code[ins_off[i] .. ins_off[i + 1]) (0..3), either side possibly empty, so it is
+ * del_len[i] - (ins_off[i + 1] - ins_off[i]) bases shorter than the interval.  ins_off has n + 1 entries, ins_off[0] =
+ * 0; a splice outside its interval or a code above 3 is MSB_EINVAL.  Only the tables cross PCIe. */
+int msb_seqs_extract_splice(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                            const int64_t *end, const int32_t *splice_at, const int32_t *del_len, const int64_t *ins_off,
+                            const uint8_t *ins_code, msb_seqs **out);
 /* Number of non-ACGT bases in each of n windows [start[i], start[i] + length) of sequence src_idx[i] of a
  * resident set (clipped at the sequence end): the device half of the background sampler's acceptance
  * test `seq.count('N') + seq.count('n') <= max_n` (genome/__init__.py:172-175) -- a window without
@@ -233,9 +241,20 @@ int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, i
  * exact / order summed over the two scans, MSB_T_ROWS the row kernel, MSB_T_ROW_SORT the ordering of the rows. */
 int msb_scan_variants(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *ref, const msb_seqs *alt,
                       const int32_t *core_start, const int32_t *core_len, int strand, int64_t *n_rows);
-/* The rows of the last msb_scan_variants (MSB_EINVAL after any other scan): *n receives their number, the arrays are
+/* msb_scan_variants with a core length per side (indels): the changed bases are [core_start[i], core_start[i] +
+ * ref_core_len[i]) of ref context i and [core_start[i], core_start[i] + alt_core_len[i]) of alt context i (one of the two
+ * may be 0, not both); the contexts must differ in length by exactly alt_core_len[i] - ref_core_len[i].  A site of length L
+ * at s touches the change when s < core_start + its own side's core length and s + L > core_start (a 0-length core: the
+ * window straddles the junction).  It is paired with the other context's window at s when s < core_start + the shorter
+ * core length and that window fits in the other context; paired sites make rows exactly as above.  An unpaired ref site
+ * is a row with effect 5 (loss, alt_score NaN), an unpaired alt site one with effect 6 (gain, ref_score NaN).  With
+ * equal core lengths this is msb_scan_variants. */
+int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *ref, const msb_seqs *alt,
+                         const int32_t *core_start, const int32_t *ref_core_len, const int32_t *alt_core_len, int strand,
+                         int64_t *n_rows);
+/* The rows of the last msb_scan_variants / msb_scan_variants_ex (MSB_EINVAL after any other scan): *n receives their number, the arrays are
  * filled when cap >= *n.  start is relative to the context; strand 1 / 2; ref_score / alt_score are the window's
- * scores on the two alleles bit for bit; effect 1 / 2 / 3 as above.  MSB_T_D2H times the copies. */
+ * scores on the two alleles bit for bit; effect 1 / 2 / 3 (or 5 / 6) as above.  MSB_T_D2H times the copies. */
 int msb_scan_device_variant_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *allele, int32_t *motif, int32_t *start,
                                  int8_t *strand, double *ref_score, double *alt_score, int8_t *effect);
 int msb_result_wait(msb_result *res);
@@ -299,7 +318,8 @@ int msb_write_sites_bed(const char *path, int64_t n, const int32_t *group, const
  * lead[lead_off[a] .. lead_off[a + 1]) of its allele a (the caller's "chrom<TAB>pos<TAB>id<TAB>ref<TAB>alt<TAB>"),
  * motif_text[motif_off[m] .. motif_off[m + 1]) of its motif m ("id<TAB>name<TAB>"), then start, start + motif_len[m],
  * '+' / '-', ref_score, alt_score (printed like Python's str()) and loss / gain / both for effect 1 / 2 / 3,
- * tab-separated, "\n".  Formatted in blocks on up to n_threads host threads, written in order. */
+ * tab-separated, "\n".  Effect 5 is a loss and 6 a gain whose other allele has no window (msb_scan_variants_ex): the
+ * missing score is written as NA.  Any other effect is MSB_EINVAL.  Formatted in blocks on up to n_threads host threads, written in order. */
 int msb_write_variant_table(const char *path, const char *header, int64_t n, const int32_t *allele, const int32_t *motif,
                             const int32_t *start, const int8_t *strand, const double *ref_score, const double *alt_score,
                             const int8_t *effect, int64_t n_alleles, const char *lead, const int64_t *lead_off, int32_t n_motifs,

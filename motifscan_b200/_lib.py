@@ -54,6 +54,8 @@ SIGNATURES = {
     "msb_seqs_extract": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, ctypes.POINTER(c_vp)]),
     "msb_seqs_extract_subst": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, c_i64p, c_i32p, c_vp,
                                               ctypes.POINTER(c_vp)]),
+    "msb_seqs_extract_splice": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, c_i32p, c_i32p, c_i64p, c_vp,
+                                               ctypes.POINTER(c_vp)]),
     "msb_seqs_lengths": (ctypes.c_int, [c_vp, c_i64p]),
     "msb_seqs_window_ncount": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, ctypes.c_int32, c_i32p]),
     "msb_seqs_set_start_limit": (ctypes.c_int, [c_vp, c_i32p]),
@@ -74,6 +76,7 @@ SIGNATURES = {
     "msb_scan_device_boundary_sites": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_f64p, c_i8p, c_i8p]),
     "msb_scan_device_cell_stats": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int64, c_i64p, c_f64p]),
     "msb_scan_variants": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
+    "msb_scan_variants_ex": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32p, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
     "msb_scan_device_variant_rows": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_i8p, c_f64p, c_f64p,
                                                     c_i8p]),
     "msb_result_wait": (ctypes.c_int, [c_vp]),

@@ -21,12 +21,13 @@ Same flags as the reference's subcommands (cli/main.py:407-430, 504-579) and the
     errors; `-w`, `--n-random` and `--seed` are ignored;
 
   * `variant` (not in the reference) scans the SNVs and MNVs of a VCF against the resident genome and reports the
-    motif sites each allele creates or destroys (motifscan_b200/variants.py; one GPU, `-t` ignored);
+    motif sites each allele creates or destroys (motifscan_b200/variants.py; one GPU, `-t` ignored); `--indels` scans
+    insertions and deletions too, as the VCF places them (normalise it first);
 
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir
     python -m motifscan_b200 scan --whole-genome -m <motif set> -g <genome> -o out_dir [--site]
     python -m motifscan_b200 motif --build <motif set> -g <genome>
-    python -m motifscan_b200 variant -i calls.vcf.gz -m <motif set> -g <genome> -o out_dir
+    python -m motifscan_b200 variant -i calls.vcf.gz -m <motif set> -g <genome> -o out_dir [--indels]
 """
 import argparse
 import logging
@@ -189,7 +190,8 @@ def run_scan(args):
 
 
 def run_variant(args):
-    """`variant`: sites gained / lost by the SNVs and MNVs of a VCF (variants.read_vcf / scan_variants)."""
+    """`variant`: sites gained / lost by the SNVs and MNVs (and with --indels the indels) of a VCF
+    (variants.read_vcf / scan_variants)."""
     from . import variants as msvar
     from .genome import DeviceGenome
     logger.info("===== Loading data =====")
@@ -201,7 +203,7 @@ def run_variant(args):
         raise SystemExit(f"motifscan: error: PWMs have no motif score cutoff set for P-value {args.p_value!r}")
     pg = packed_genome(genome, PACKED_MIN_BP)
     try:
-        vcf = msvar.read_vcf(args.input_file, pg)
+        vcf = msvar.read_vcf(args.input_file, pg, indels=args.indels)
     except (OSError, UnicodeDecodeError, EOFError) as err:
         raise SystemExit(f"motifscan variant: error: cannot read {args.input_file}: {err}")
     except ValueError as err:
@@ -214,7 +216,8 @@ def run_variant(args):
         dg.close()
     by = sites.rows_by_effect()
     skipped = ", ".join(f"{k} {v}" for k, v in vcf.skipped.items())
-    logger.info(f"Scanned {len(vcf)} alleles (skipped: {skipped}) x {len(pwms)} motifs, {sites.motif_bp:.3e} motif*bp "
+    n_indels = f", {sum(len(r) != len(a) for r, a in zip(vcf.ref, vcf.alt))} of them indels" if args.indels else ""
+    logger.info(f"Scanned {len(vcf)} alleles{n_indels} (skipped: {skipped}) x {len(pwms)} motifs, {sites.motif_bp:.3e} motif*bp "
                 f"in {sites.seconds:.3f} s: {len(sites)} rows ({by['gain']} gain, {by['loss']} loss, {by['both']} both)")
     logger.info("Saving the result tables")
     msio.write_variant_tables(args.output_dir, pwms, vcf, sites)
@@ -308,13 +311,15 @@ def make_parser():
     scan.add_argument("--verbose", action="store_true")
     scan.set_defaults(func=run_scan)
 
-    variant = sub.add_parser("variant", help="Motif sites gained and lost by the SNVs / MNVs of a VCF.")
+    variant = sub.add_parser("variant", help="Motif sites gained and lost by the SNVs / MNVs (and indels) of a VCF.")
     variant.add_argument("-i", dest="input_file", required=True, metavar="VCF")
     variant.add_argument("-m", "--motif", dest="motif", required=True, metavar="NAME")
     variant.add_argument("-g", "--genome", dest="genome", required=True, metavar="GENOME")
     variant.add_argument("-p", dest="p_value", default="1e-4", choices=["1e-2", "1e-3", "1e-4", "1e-5", "1e-6"])
     variant.add_argument("--strand", dest="strand", choices=["both", "+", "-"], default="both")
     variant.add_argument("-t", "--threads", dest="n_threads", type=int, default=1)
+    variant.add_argument("--indels", action="store_true",
+                         help="Also scan insertions and deletions (not left-aligned: normalise the VCF first).")
     variant.add_argument("-o", "--output-dir", dest="output_dir", required=True, metavar="DIR")
     variant.add_argument("--verbose", action="store_true")
     variant.set_defaults(func=run_variant)

@@ -9,6 +9,7 @@
 //   dedup_flags_kernel      adjacent-site de-duplication              (scanner.py:156-193)
 //   score0_kernel           offset-0 window score of every sequence     (cscore.c:191-223)
 //   extract_subst_kernel    resident-genome extraction with allele bases overlaid (variant contexts)
+//   extract_splice_kernel   resident-genome extraction with bases deleted and inserted (indel contexts)
 //   variant_rows_kernel     sites of the ref / alt context scans -> gain / loss / both rows
 #pragma once
 #include "common.cuh"
@@ -147,6 +148,49 @@ extract_subst_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int
     }
     codes[2 * b] = lo;
     codes[2 * b + 1] = hi;
+    nmask[b] = mask;
+    blk_seq[b] = (int32_t) s;
+}
+
+// extract with a splice (the alternative alleles of a variant scan with indels): destination sequence s = source
+// [start, start + c) + the A/C/G/T codes ins_code[ins_off[s] .. ins_off[s + 1]) + source [start + c + r, end), with
+// c = splice_at[s] and r = del_len[s].  A 32-base block may hold pieces of all three: each flank is cut by
+// extract_block at its own source offset and shifted into place; the inserted bases are set one by one.
+__global__ void __launch_bounds__(256)
+extract_splice_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int64_t *__restrict__ src_start,
+                      const int32_t *__restrict__ splice_at, const int32_t *__restrict__ del_len,
+                      const int64_t *__restrict__ ins_off, const uint8_t *__restrict__ ins_code,
+                      const int64_t *__restrict__ poff, const int32_t *__restrict__ len, int64_t n_seqs,
+                      int64_t n_blocks, uint32_t *__restrict__ codes, uint32_t *__restrict__ nmask,
+                      int32_t *__restrict__ blk_seq) {
+    const int64_t b = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n_blocks) return;
+    const int64_t p = b * kPadBases;
+    const int64_t s = find_seq(poff, n_seqs, p);
+    const int64_t j = p - __ldg(poff + s);
+    const int n = (int) min((int64_t) kPadBases, (int64_t) __ldg(len + s) - j);
+    const int64_t c = __ldg(splice_at + s), i0 = __ldg(ins_off + s);
+    const int64_t a = __ldg(ins_off + s + 1) - i0, r = __ldg(del_len + s);
+    uint32_t lo, hi, mask;
+    // left flank: destination [j, min(j + n, c)) = source [j, ...)
+    extract_block(src, src_idx, src_start, s, j, (int) max(min((int64_t) n, c - j), (int64_t) 0), lo, hi, mask);
+    uint64_t code = (uint64_t) hi << 32 | lo;
+    // right flank: destination [d0, j + n) = source [d0 + r - a, ...), d0 = max(j, c + a)
+    const int64_t d0 = max(j, c + a);
+    if (d0 < j + n) {
+        uint32_t rl, rh, rm;
+        extract_block(src, src_idx, src_start, s, d0 + r - a, (int) (j + n - d0), rl, rh, rm);
+        const int k = (int) (d0 - j);                                    // 0 <= k < n <= 32
+        code |= ((uint64_t) rh << 32 | rl) << (2 * k);
+        mask |= rm << k;
+    }
+    // inserted bases: destination [max(j, c), min(j + n, c + a)) (their mask bits are already clear)
+    for (int64_t q = max(j, c), q1 = min(j + n, c + a); q < q1; q++) {
+        const int k = (int) (q - j);
+        code |= (uint64_t) (__ldg(ins_code + i0 + (q - c)) & 3u) << (2 * k);
+    }
+    codes[2 * b] = (uint32_t) code;
+    codes[2 * b + 1] = (uint32_t) (code >> 32);
     nmask[b] = mask;
     blk_seq[b] = (int32_t) s;
 }
@@ -878,14 +922,18 @@ cell_stats_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Variant rows (msb_scan_variants).  Sequence i of `ref` and of `alt` is allele i's context on the reference and
-// with the allele's bases substituted (same lengths, so the same packed layout); core [core_start[i], core_start[i] +
-// core_len[i]) holds the changed bases.  One thread per final site of either scan: a site whose window overlaps
-// the core is re-scored on the other context with the reference's arithmetic (exact_raw, cscore.c:341-389) and
-// becomes a row:
+// Variant rows (msb_scan_variants_ex).  Sequence i of `ref` and of `alt` is allele i's context on the reference and
+// with the allele applied; both start at the same base, and the changed bases are [c, c + ref_len[i]) of the ref
+// context and [c, c + alt_len[i]) of the alt context, c = core_start[i] (equal lengths for an SNV / MNV, one of them
+// possibly 0 for an indel).  One thread per final site of either scan.  A site of length L at s is affected when
+// s < c + k and s + L > c, k = its own side's changed length (for k = 0: the window straddles the junction).  It is
+// paired with the other context's window at s when s < c + min(ref_len, alt_len) and that window fits in the other
+// context; a paired window is re-scored there with the reference's arithmetic (exact_raw, cscore.c:341-389):
 //   ref-list site:  effect 1 (loss) or 3 (both, the alt window passes too);
 //   alt-list site:  effect 2 (gain) only when the ref window fails -- else the ref list already has the row.
-// Rows are appended (order restored by the sort on row_key = allele | motif | start | strand bit).
+// An unpaired site has no window on the other allele: effect 5 (loss) or 6 (gain), the other score NaN.  Rows are
+// appended (order restored by the sort on row_key = allele | motif | start | strand bit); no two rows share a key,
+// as at most one side has unpaired windows.
 // ---------------------------------------------------------------------------------------------
 struct VariantSide {
     SeqView seq;                     // this list's contexts
@@ -904,7 +952,7 @@ __device__ __forceinline__ bool site_predicate(const MotifView &M, uint32_t m, d
 
 __global__ void __launch_bounds__(256)
 variant_rows_kernel(VariantSide R, VariantSide A, MotifView M, const int32_t *__restrict__ core_start,
-                    const int32_t *__restrict__ core_len, int motif_bits, int start_bits,
+                    const int32_t *__restrict__ ref_len, const int32_t *__restrict__ alt_len, int motif_bits, int start_bits,
                     unsigned long long *__restrict__ n_rows, uint64_t *__restrict__ row_key,
                     int32_t *__restrict__ row_idx, double *__restrict__ row_ref, double *__restrict__ row_alt,
                     int8_t *__restrict__ row_eff) {
@@ -917,19 +965,23 @@ variant_rows_kernel(VariantSide R, VariantSide A, MotifView M, const int32_t *__
     const uint32_t m = site_motif(S.key[i], S.key_shift);
     const int32_t s = S.seq_idx[i], st = S.start[i];
     const int L = __ldg(M.len + m);
-    const int32_t c0 = __ldg(core_start + s), c1 = c0 + __ldg(core_len + s);
-    if (st >= c1 || st + L <= c0) return;                                // the window does not touch a changed base
+    const int32_t c0 = __ldg(core_start + s), kr = __ldg(ref_len + s), ka = __ldg(alt_len + s);
+    if (st >= c0 + (from_ref ? kr : ka) || st + L <= c0) return;        // the window does not touch a changed base
+    const bool paired = st < c0 + min(kr, ka) && st + L <= __ldg(O.seq.len + s);
     const int rev = S.strand[i] == 2;
-    const double *pw = M.pwm + 4 * (int64_t) __ldg(M.col_off + m);
-    double other;
-    const bool other_hit = site_predicate(M, m, exact_raw(O.seq, pw, L, __ldg(O.seq.poff + s) + st, rev), other);
-    if (!from_ref && other_hit) return;                                  // a site on both alleles: the ref list's row
+    double other = __longlong_as_double(0x7ff8000000000000ll);           // NaN: no window on the other allele
+    bool other_hit = false;
+    if (paired) {
+        const double *pw = M.pwm + 4 * (int64_t) __ldg(M.col_off + m);
+        other_hit = site_predicate(M, m, exact_raw(O.seq, pw, L, __ldg(O.seq.poff + s) + st, rev), other);
+        if (!from_ref && other_hit) return;                              // a site on both alleles: the ref list's row
+    }
     const unsigned long long slot = atomicAdd(n_rows, 1ull);
     row_key[slot] = ((((uint64_t) s << motif_bits | m) << start_bits | (uint64_t) st) << 1) | (uint64_t) rev;
     row_idx[slot] = (int32_t) slot;
     row_ref[slot] = from_ref ? S.score[i] : other;
     row_alt[slot] = from_ref ? other : S.score[i];
-    row_eff[slot] = (int8_t) (from_ref ? (other_hit ? 3 : 1) : 2);
+    row_eff[slot] = (int8_t) ((from_ref ? (other_hit ? 3 : 1) : 2) | (paired ? 0 : 4));
 }
 
 // Sorted row keys + the permutation -> the row arrays in order.

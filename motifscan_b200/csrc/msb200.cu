@@ -770,9 +770,11 @@ int msb_seqs_to_packed(msb_ctx *ctx, const msb_seqs *S, uint32_t *codes, uint32_
 
 }  // extern "C"
 
-// msb_seqs_extract, and with a substitution table (sub_off != nullptr) msb_seqs_extract_subst.
+// msb_seqs_extract; with a substitution table (sub_off != nullptr) msb_seqs_extract_subst; with a splice table
+// (ins_off != nullptr) msb_seqs_extract_splice.
 static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
                         const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
+                        const int32_t *splice_at, const int32_t *del_len, const int64_t *ins_off, const uint8_t *ins_code,
                         msb_seqs **out, const char *what) {
     if (!ctx || !src || !out || n < 0 || (n > 0 && (!src_idx || !start || !end))) {
         set_error(std::string(what) + ": bad argument");
@@ -784,14 +786,32 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
     // pysam's fetch (genome/__init__.py:135) clips `end` at the sequence length; an interval that
     // starts behind it, or is reversed, is empty.
     std::vector<int64_t> seq_off((size_t) n + 1, 0), clipped_start((size_t) std::max<int64_t>(n, 1), 0);
+    const int64_t n_ins = ins_off ? ins_off[n] : 0;
+    if (ins_off && (ins_off[0] != 0 || (n > 0 && (!splice_at || !del_len)) || (n_ins > 0 && !ins_code))) {
+        set_error(std::string(what) + ": bad splice table");
+        return MSB_EINVAL;
+    }
     for (int64_t i = 0; i < n; i++) {
         if (src_idx[i] < 0 || src_idx[i] >= src->n) { set_error(std::string(what) + ": source index out of range"); return MSB_EINVAL; }
         if (start[i] < 0) { set_error(std::string(what) + ": negative start"); return MSB_EINVAL; }
         const int64_t slen = src->seq_off[src_idx[i] + 1] - src->seq_off[src_idx[i]];
         const int64_t a = std::min(start[i], slen), b = std::min(end[i], slen);
+        int64_t len = std::max<int64_t>(b - a, 0);
+        if (ins_off) {
+            // the cut interval loses [splice_at, splice_at + del_len) and gains the inserted bases there
+            if (ins_off[i + 1] < ins_off[i]) { set_error(std::string(what) + ": insertion offsets not ascending"); return MSB_EINVAL; }
+            if (splice_at[i] < 0 || del_len[i] < 0 || (int64_t) splice_at[i] + del_len[i] > len) {
+                set_error(std::string(what) + ": splice outside its interval");
+                return MSB_EINVAL;
+            }
+            len += ins_off[i + 1] - ins_off[i] - del_len[i];
+            if (len > (int64_t) 0x7fffffff - 64) { set_error(std::string(what) + ": spliced sequence >= 2^31 bases"); return MSB_EINVAL; }
+        }
         clipped_start[i] = a;
-        seq_off[i + 1] = seq_off[i] + std::max<int64_t>(b - a, 0);
+        seq_off[i + 1] = seq_off[i] + len;
     }
+    for (int64_t k = 0; k < n_ins; k++)
+        if (ins_code[k] > 3) { set_error(std::string(what) + ": inserted base not an A/C/G/T code"); return MSB_EINVAL; }
     const int64_t n_sub = sub_off ? sub_off[n] : 0;
     if (sub_off) {
         if (sub_off[0] != 0 || (n_sub > 0 && (!sub_pos || !sub_code))) { set_error(std::string(what) + ": bad substitution table"); return MSB_EINVAL; }
@@ -812,10 +832,13 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
     MSB_TRY(seqs_prepare(ctx, n, seq_off.data(), &S, lens));
     // the tables ride in the (otherwise unused here) ASCII scratch:
     // src_idx (4n) | start (8n) [| sub_off (8 (n + 1)) | sub_pos (4 n_sub) | sub_code (n_sub)]
+    //                           [| splice_at (4n) | del_len (4n) | ins_off (8 (n + 1)) | ins_code (n_ins)]
     auto al = [](size_t x) { return (x + 15) & ~(size_t) 15; };
     const size_t o_start = al((size_t) n * 4), o_soff = o_start + al((size_t) n * 8);
     const size_t o_spos = o_soff + al((size_t) (n + 1) * 8), o_scode = o_spos + al((size_t) n_sub * 4);
-    const size_t bytes = sub_off ? o_scode + (size_t) n_sub : o_start + (size_t) n * 8;
+    const size_t o_at = o_soff, o_del = o_at + al((size_t) n * 4), o_ioff = o_del + al((size_t) n * 4);
+    const size_t o_icode = o_ioff + al((size_t) (n + 1) * 8);
+    const size_t bytes = sub_off ? o_scode + (size_t) n_sub : ins_off ? o_icode + (size_t) n_ins : o_start + (size_t) n * 8;
     int rc = ctx->ascii.ensure(std::max<size_t>(bytes, 16));
     if (rc != MSB_OK) { msb_seqs_destroy(S); return rc; }
     char *base = (char *) ctx->ascii.p;
@@ -833,6 +856,14 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
             step(cudaMemcpyAsync(base + o_scode, sub_code, (size_t) n_sub, cudaMemcpyHostToDevice, st));
         }
     }
+    if (ins_off) {
+        if (n) {
+            step(cudaMemcpyAsync(base + o_at, splice_at, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+            step(cudaMemcpyAsync(base + o_del, del_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+        }
+        step(cudaMemcpyAsync(base + o_ioff, ins_off, (size_t) (n + 1) * 8, cudaMemcpyHostToDevice, st));
+        if (n_ins) step(cudaMemcpyAsync(base + o_icode, ins_code, (size_t) n_ins, cudaMemcpyHostToDevice, st));
+    }
     step(cudaEventRecord(ctx->ev[1], st));
     if (e == cudaSuccess && n_blocks > 0) {
         const int64_t grid = (n_blocks + 255) / 256;
@@ -842,6 +873,12 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
                 (const int32_t *) (base + o_spos), (const uint8_t *) (base + o_scode), S->d_poff.as<int64_t>(),
                 S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(), S->d_nmask.as<uint32_t>(),
                 S->d_blk_seq.as<int32_t>());
+        else if (ins_off)
+            extract_splice_kernel<<<(unsigned) grid, 256, 0, st>>>(
+                src->view(), (const int32_t *) base, (const int64_t *) (base + o_start), (const int32_t *) (base + o_at),
+                (const int32_t *) (base + o_del), (const int64_t *) (base + o_ioff), (const uint8_t *) (base + o_icode),
+                S->d_poff.as<int64_t>(), S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(),
+                S->d_nmask.as<uint32_t>(), S->d_blk_seq.as<int32_t>());
         else
             extract_pack_kernel<<<(unsigned) grid, 256, 0, st>>>(
                 src->view(), (const int32_t *) base, (const int64_t *) (base + o_start), S->d_poff.as<int64_t>(),
@@ -865,14 +902,24 @@ extern "C" {
 
 int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx,
                      const int64_t *start, const int64_t *end, msb_seqs **out) {
-    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, out, "msb_seqs_extract");
+    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                        out, "msb_seqs_extract");
 }
 
 int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
                            const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
                            msb_seqs **out) {
     if (!sub_off) { set_error("msb_seqs_extract_subst: null substitution offsets"); return MSB_EINVAL; }
-    return seqs_extract(ctx, src, n, src_idx, start, end, sub_off, sub_pos, sub_code, out, "msb_seqs_extract_subst");
+    return seqs_extract(ctx, src, n, src_idx, start, end, sub_off, sub_pos, sub_code, nullptr, nullptr, nullptr, nullptr,
+                        out, "msb_seqs_extract_subst");
+}
+
+int msb_seqs_extract_splice(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                            const int64_t *end, const int32_t *splice_at, const int32_t *del_len, const int64_t *ins_off,
+                            const uint8_t *ins_code, msb_seqs **out) {
+    if (!ins_off) { set_error("msb_seqs_extract_splice: null insertion offsets"); return MSB_EINVAL; }
+    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, splice_at, del_len, ins_off, ins_code,
+                        out, "msb_seqs_extract_splice");
 }
 
 int msb_seqs_window_ncount(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
@@ -1709,11 +1756,27 @@ int msb_scan_variants(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, co
     }
     const int64_t n = ref->n;
     if (n > 0 && (!core_start || !core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
+    for (int64_t i = 0; i < n; i++)
+        if (core_len[i] < 1) { set_error("msb_scan_variants: core outside its context"); return MSB_EINVAL; }
+    return msb_scan_variants_ex(ctx, M, ref, alt, core_start, core_len, core_len, strand, n_rows);
+}
+
+int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int32_t *core_start,
+                         const int32_t *ref_core_len, const int32_t *alt_core_len, int strand, int64_t *n_rows) {
+    if (!ctx || !M || !ref || !alt) { set_error("msb_scan_variants: null argument"); return MSB_EINVAL; }
+    if (ref->n != alt->n) { set_error("msb_scan_variants: the ref and alt sets must hold the same number of contexts"); return MSB_EINVAL; }
+    const int64_t n = ref->n;
+    if (n > 0 && (!core_start || !ref_core_len || !alt_core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
     int32_t max_len = 0;
     for (int64_t i = 0; i < n; i++) {
-        const int64_t len = ref->seq_off[i + 1] - ref->seq_off[i];
-        max_len = std::max<int32_t>(max_len, (int32_t) len);
-        if (core_start[i] < 0 || core_len[i] < 1 || (int64_t) core_start[i] + core_len[i] > len) {
+        const int64_t len_r = ref->seq_off[i + 1] - ref->seq_off[i], len_a = alt->seq_off[i + 1] - alt->seq_off[i];
+        max_len = std::max<int32_t>(max_len, (int32_t) std::max(len_r, len_a));
+        if (len_a - len_r != (int64_t) alt_core_len[i] - ref_core_len[i]) {
+            set_error("msb_scan_variants: a context's length change differs from its core's");
+            return MSB_EINVAL;
+        }
+        if (core_start[i] < 0 || ref_core_len[i] < 0 || alt_core_len[i] < 0 || std::max(ref_core_len[i], alt_core_len[i]) < 1 ||
+            (int64_t) core_start[i] + ref_core_len[i] > len_r || (int64_t) core_start[i] + alt_core_len[i] > len_a) {
             set_error("msb_scan_variants: core outside its context");
             return MSB_EINVAL;
         }
@@ -1758,16 +1821,18 @@ int msb_scan_variants(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, co
     MSB_TRY(ctx->vr_ref.ensure((size_t) cap * 8));
     MSB_TRY(ctx->vr_alt.ensure((size_t) cap * 8));
     MSB_TRY(ctx->vr_eff.ensure((size_t) cap));
-    MSB_TRY(ctx->vr_core.ensure((size_t) std::max<int64_t>(2 * n, 1) * 4));
+    MSB_TRY(ctx->vr_core.ensure((size_t) std::max<int64_t>(3 * n, 1) * 4));
     if (n) {
         MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.p, core_start, (size_t) n * 4, cudaMemcpyHostToDevice, st));
-        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.as<int32_t>() + n, core_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.as<int32_t>() + n, ref_core_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.as<int32_t>() + 2 * n, alt_core_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
     }
     MSB_CUDA(cudaMemsetAsync(ctx->counters.p, 0, sizeof(unsigned long long), st));
     MSB_CUDA(cudaEventRecord(ctx->ev[4], st));
     if (R.n + A.n) {
         variant_rows_kernel<<<(unsigned) ((R.n + A.n + 255) / 256), 256, 0, st>>>(
-            R, A, M->view(), ctx->vr_core.as<int32_t>(), ctx->vr_core.as<int32_t>() + n, motif_bits, start_bits,
+            R, A, M->view(), ctx->vr_core.as<int32_t>(), ctx->vr_core.as<int32_t>() + n, ctx->vr_core.as<int32_t>() + 2 * n,
+            motif_bits, start_bits,
             ctx->counters.as<unsigned long long>(), ctx->vr_key.as<uint64_t>(), ctx->vr_idx.as<int32_t>(),
             ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>());
         MSB_CUDA(cudaGetLastError());
@@ -2517,7 +2582,7 @@ int msb_write_variant_table(const char *path, const char *header, int64_t n, con
     for (int64_t a = 0; a < n_alleles; a++) lead_max = std::max<size_t>(lead_max, (size_t) (lead_off[a + 1] - lead_off[a]));
     for (int32_t m = 0; m < n_motifs; m++) motif_max = std::max<size_t>(motif_max, (size_t) (motif_off[m + 1] - motif_off[m]));
     for (int64_t i = 0; i < n; i++)
-        if (allele[i] < 0 || allele[i] >= n_alleles || motif[i] < 0 || motif[i] >= n_motifs || effect[i] < 1 || effect[i] > 3) {
+        if (allele[i] < 0 || allele[i] >= n_alleles || motif[i] < 0 || motif[i] >= n_motifs || effect[i] < 1 || effect[i] > 6 || effect[i] == 4) {
             set_error("msb_write_variant_table: row refers to an unknown allele, motif or effect");
             return MSB_EINVAL;
         }
@@ -2536,6 +2601,7 @@ int msb_write_variant_table(const char *path, const char *header, int64_t n, con
     std::vector<size_t> used((size_t) nt);
     try { for (auto &b : buf) b.resize((size_t) std::min(n, block) * line_max); }
     catch (const std::bad_alloc &) { std::fclose(f); set_error("out of host memory"); return MSB_ENOMEM; }
+    // effect 5 / 6: a loss / gain with no window on the other allele (an indel), its score written as NA
     static const char *const kEffect[4] = {"", "loss", "gain", "both"};
     for (int64_t r0 = 0; r0 < n && io_ok; r0 += block * nt) {
         auto format = [&](int t) {
@@ -2549,10 +2615,13 @@ int msb_write_variant_table(const char *path, const char *header, int64_t n, con
                 o += fmt_int(start[i], o);
                 *o++ = '\t'; o += fmt_int((int64_t) start[i] + motif_len[m], o);
                 *o++ = '\t'; *o++ = strand[i] == 1 ? '+' : '-';
-                *o++ = '\t'; o += py_float_str(ref_score[i], o);
-                *o++ = '\t'; o += py_float_str(alt_score[i], o);
+                const int eff = effect[i];
                 *o++ = '\t';
-                const char *e = kEffect[effect[i]];
+                if (eff == 6) { std::memcpy(o, "NA", 2); o += 2; } else o += py_float_str(ref_score[i], o);
+                *o++ = '\t';
+                if (eff == 5) { std::memcpy(o, "NA", 2); o += 2; } else o += py_float_str(alt_score[i], o);
+                *o++ = '\t';
+                const char *e = kEffect[eff & 3];
                 std::memcpy(o, e, 4); o += 4;
                 *o++ = '\n';
             }

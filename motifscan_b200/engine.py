@@ -249,6 +249,30 @@ class SequenceSet:
                                                    ctypes.c_void_p(sub_code.ctypes.data), ctypes.byref(h)))
         return SequenceSet(self.ctx, _handle=h)
 
+    def extract_splice(self, src_idx, start, end, splice_at, del_len, ins_off, ins_code):
+        """`extract` with a splice (msb_seqs_extract_splice): bases [splice_at[i], splice_at[i] + del_len[i]) of
+        sequence i (relative to its start) are replaced by the A/C/G/T codes ins_code[ins_off[i] .. ins_off[i + 1])
+        (0..3); either side may be empty.  Only the interval and splice tables cross PCIe."""
+        src_idx = np.ascontiguousarray(np.asarray(src_idx, dtype=np.int32))
+        start = np.ascontiguousarray(np.asarray(start, dtype=np.int64))
+        end = np.ascontiguousarray(np.asarray(end, dtype=np.int64))
+        splice_at = np.ascontiguousarray(np.asarray(splice_at, dtype=np.int32))
+        del_len = np.ascontiguousarray(np.asarray(del_len, dtype=np.int32))
+        ins_off = np.ascontiguousarray(np.asarray(ins_off, dtype=np.int64))
+        ins_code = np.ascontiguousarray(np.asarray(ins_code, dtype=np.uint8))
+        if not (src_idx.shape == start.shape == end.shape == splice_at.shape == del_len.shape and src_idx.ndim == 1):
+            raise ValueError("src_idx, start, end, splice_at and del_len must be 1-d arrays of one length")
+        if ins_off.shape != (len(src_idx) + 1,) or ins_code.ndim != 1 or len(ins_code) != int(ins_off[-1]):
+            raise ValueError("ins_off must have n + 1 entries and ins_code ins_off[-1]")
+        h = ctypes.c_void_p()
+        with self.ctx._lock:
+            check(self._lib.msb_seqs_extract_splice(self.ctx._h, self._h, len(src_idx), ptr(src_idx, ctypes.c_int32),
+                                                    ptr(start, ctypes.c_int64), ptr(end, ctypes.c_int64),
+                                                    ptr(splice_at, ctypes.c_int32), ptr(del_len, ctypes.c_int32),
+                                                    ptr(ins_off, ctypes.c_int64), ctypes.c_void_p(ins_code.ctypes.data),
+                                                    ctypes.byref(h)))
+        return SequenceSet(self.ctx, _handle=h)
+
     def window_ncount(self, src_idx, start, length):
         """Non-ACGT bases in each window [start[i], start[i] + length) of sequence src_idx[i]."""
         src_idx = np.ascontiguousarray(np.asarray(src_idx, dtype=np.int32))
@@ -560,19 +584,42 @@ def scan_variants(ctx, motifs, ref, alt, core_start, core_len, strand):
     core_len = np.ascontiguousarray(np.asarray(core_len, dtype=np.int32))
     if core_start.shape != (ref.n,) or core_len.shape != (ref.n,):
         raise ValueError("one core per context is required")
-    n = ctypes.c_int64(0)
     with ctx._lock:
+        n = ctypes.c_int64(0)
         check(ctx._lib.msb_scan_variants(ctx._h, motifs._h, ref._h, alt._h, ptr(core_start, ctypes.c_int32),
                                          ptr(core_len, ctypes.c_int32), int(strand), ctypes.byref(n)))
-        k = n.value
-        out = dict(allele=np.zeros(k, np.int32), motif=np.zeros(k, np.int32), start=np.zeros(k, np.int32),
-                   strand=np.zeros(k, np.int8), ref_score=np.zeros(k, np.float64), alt_score=np.zeros(k, np.float64),
-                   effect=np.zeros(k, np.int8))
-        if k:
-            check(ctx._lib.msb_scan_device_variant_rows(
-                ctx._h, k, ctypes.byref(n), ptr(out["allele"], ctypes.c_int32), ptr(out["motif"], ctypes.c_int32),
-                ptr(out["start"], ctypes.c_int32), ptr(out["strand"], ctypes.c_int8), ptr(out["ref_score"], ctypes.c_double),
-                ptr(out["alt_score"], ctypes.c_double), ptr(out["effect"], ctypes.c_int8)))
+        return _variant_rows(ctx, n.value)
+
+
+def scan_variants_ex(ctx, motifs, ref, alt, core_start, ref_core_len, alt_core_len, strand):
+    """scan_variants with a changed length per side (msb_scan_variants_ex, indels): the changed bases are
+    [core_start[i], core_start[i] + ref_core_len[i]) of ref context i and [core_start[i], core_start[i] +
+    alt_core_len[i]) of alt context i.  The same row arrays; effect 5 is a loss and 6 a gain whose window does not
+    exist on the other allele (its score NaN)."""
+    core_start = np.ascontiguousarray(np.asarray(core_start, dtype=np.int32))
+    ref_core_len = np.ascontiguousarray(np.asarray(ref_core_len, dtype=np.int32))
+    alt_core_len = np.ascontiguousarray(np.asarray(alt_core_len, dtype=np.int32))
+    if not core_start.shape == ref_core_len.shape == alt_core_len.shape == (ref.n,):
+        raise ValueError("one core per context is required")
+    with ctx._lock:
+        n = ctypes.c_int64(0)
+        check(ctx._lib.msb_scan_variants_ex(ctx._h, motifs._h, ref._h, alt._h, ptr(core_start, ctypes.c_int32),
+                                            ptr(ref_core_len, ctypes.c_int32), ptr(alt_core_len, ctypes.c_int32),
+                                            int(strand), ctypes.byref(n)))
+        return _variant_rows(ctx, n.value)
+
+
+def _variant_rows(ctx, k):
+    """The k rows of the last variant scan on `ctx` (caller holds its lock)."""
+    n = ctypes.c_int64(0)
+    out = dict(allele=np.zeros(k, np.int32), motif=np.zeros(k, np.int32), start=np.zeros(k, np.int32),
+               strand=np.zeros(k, np.int8), ref_score=np.zeros(k, np.float64), alt_score=np.zeros(k, np.float64),
+               effect=np.zeros(k, np.int8))
+    if k:
+        check(ctx._lib.msb_scan_device_variant_rows(
+            ctx._h, k, ctypes.byref(n), ptr(out["allele"], ctypes.c_int32), ptr(out["motif"], ctypes.c_int32),
+            ptr(out["start"], ctypes.c_int32), ptr(out["strand"], ctypes.c_int8), ptr(out["ref_score"], ctypes.c_double),
+            ptr(out["alt_score"], ctypes.c_double), ptr(out["effect"], ctypes.c_int8)))
     return out
 
 

@@ -192,7 +192,8 @@ def write_variant_tables(output_dir, pwms, variants, sites):
 
         motif_variant_sites.xls    one row per (allele, motif, window, strand) that is a site on at least one allele:
                                    chrom, pos, id, ref and alt as in the VCF (alt = the allele), motif id and name,
-                                   the window [start, end) 0-based half-open, strand, both scores and the effect
+                                   the window [start, end) 0-based half-open on the allele's haplotype, strand,
+                                   both scores (NA where an indel leaves no window on that allele) and the effect
         motif_variant_summary.xls  per motif, the alleles with at least one gain / loss / both row
 
     The site rows are formatted by the library on host threads (msb_write_variant_table; scores like Python's
@@ -218,7 +219,7 @@ def write_variant_tables(output_dir, pwms, variants, sites):
     strand = np.ascontiguousarray(sites.strand, dtype=np.int8)
     ref_score = np.ascontiguousarray(sites.ref_score, dtype=np.float64)
     alt_score = np.ascontiguousarray(sites.alt_score, dtype=np.float64)
-    effect = np.ascontiguousarray(sites.effect, dtype=np.int8)
+    effect = np.ascontiguousarray(np.where(sites.paired, sites.effect, sites.effect | 4), dtype=np.int8)
     arrays = [(row_allele, ctypes.c_int32), (motif, ctypes.c_int32), (start, ctypes.c_int32), (strand, ctypes.c_int8),
               (ref_score, ctypes.c_double), (alt_score, ctypes.c_double), (effect, ctypes.c_int8)]
     _lib.check(lib.msb_write_variant_table(
