@@ -8,6 +8,7 @@
     python bench_configs.py whole-genome --genome-scale 1 --gpus 8
                                        configs[3] genome with de-duplication (scan --whole-genome), tables and BED
     python bench_configs.py variants --genome-scale 0.1 --alleles 4000000 [--indel-fraction 0.15]
+    python bench_configs.py haplotypes --genome-scale 0.1 --alleles 400000 --samples 16 [--indel-fraction 0.15]
                                        motifscan variant: SNVs / MNVs (and with --indel-fraction that share of
                                        deletions and insertions, scanned with --indels) of a seeded VCF against
                                        the resident genome
@@ -821,10 +822,197 @@ def bench_variants(args):
                     "--steps after one warm-up; device_ms per phase of that run"}
 
 
+def _synthetic_phased_vcf(path, pg, n_alleles, n_samples, seed=37, indel_fraction=0.0):
+    """A seeded phased VCF of about `n_alleles` alleles on `pg` and `n_samples` samples whose allele spacing makes
+    multi-allele clusters: alleles come in bursts of 1-8 (positions uniform over the non-N bases), 1-20 bases apart;
+    SNVs, and with `indel_fraction` deletions / insertions (half each) of 1-20 bases.  Each allele has a frequency
+    drawn from Beta(0.5, 2) and each haplotype carries it with that probability, so haplotypes carry different subsets
+    of a burst.  Returns (records, alleles)."""
+    rng = np.random.default_rng(seed)
+    chroms = list(pg.chroms)
+    sizes = np.array([pg.chrom_sizes[c] for c in chroms], dtype=np.int64)
+    cum = np.concatenate([[0], np.cumsum(sizes)])
+    n_bursts = max(n_alleles // 4, 1)
+    burst = rng.integers(1, 9, n_bursts)
+    g = rng.integers(0, int(cum[-1]), n_bursts)
+    c = np.searchsorted(cum, g, side="right") - 1
+    start = g - cum[c]
+    cs = np.cumsum(rng.integers(1, 21, int(burst.sum())))
+    pos = np.repeat(start, burst) + cs - np.repeat(cs[np.cumsum(burst) - burst], burst)
+    chrom = np.repeat(c, burst)
+    ok = pos + 25 < sizes[chrom]
+    pos, chrom = pos[ok], chrom[ok]
+    order = np.lexsort((pos, chrom))
+    pos, chrom = pos[order], chrom[order]
+    keep = np.ones(len(pos), dtype=bool)
+    keep[1:] = (pos[1:] != pos[:-1]) | (chrom[1:] != chrom[:-1])
+    pos, chrom = pos[keep], chrom[keep]
+    n = len(pos)
+    b = pg.block_off[chrom] + pos // 32
+    isn = ((np.asarray(pg.nmask)[b] >> (pos % 32).astype(np.uint32)) & 1) == 1
+    pos, chrom, n = pos[~isn], chrom[~isn], int((~isn).sum())
+    kind = rng.random(n)
+    is_del = kind < indel_fraction / 2
+    is_ins = (kind >= indel_fraction / 2) & (kind < indel_fraction)
+    ilen = rng.integers(1, 21, n)
+    acgt = "ACGT"
+    af = rng.beta(0.5, 2.0, n)
+    carry = rng.random((n, 2 * n_samples)) < af[:, None]
+    lines = []
+    for i in range(n):
+        cn, p = chroms[chrom[i]], int(pos[i])
+        if is_del[i]:
+            ref = pg.decode_bytes(cn, p, p + 1 + int(ilen[i])).decode()
+            alt = ref[0]
+        else:
+            ref = pg.decode_bytes(cn, p, p + 1).decode()
+            alt = ref + "".join(rng.choice(list(acgt), int(ilen[i]))) if is_ins[i] else \
+                acgt[(acgt.find(ref.upper()) + int(rng.integers(1, 4))) % 4]
+        row = carry[i]
+        gts = "\t".join(f"{int(row[2 * k])}|{int(row[2 * k + 1])}" for k in range(n_samples))
+        lines.append(f"{cn}\t{p + 1}\th{i}\t{ref}\t{alt}\t.\tPASS\t.\tGT\t{gts}\n")
+    with open(path, "w") as fh:
+        fh.write("##fileformat=VCFv4.2\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t" +
+                 "\t".join(f"S{k}" for k in range(n_samples)) + "\n")
+        fh.writelines(lines)
+    return n
+
+
+def bench_haplotypes(args):
+    """`motifscan variant --haplotypes` on the configs[3]-shaped genome at `--genome-scale` with 750 motifs and a
+    seeded phased VCF of `--alleles` alleles x `--samples` samples (_synthetic_phased_vcf): VCF + GT parsing, the
+    clustering, the device phases of scan_haplotypes, rows by effect, the whole command in a subprocess (wall time,
+    peak RSS) and parity of a seeded sample of clusters with the oracle of tests/test_gpu_haplotypes.py."""
+    import resource
+    import shutil
+    import subprocess
+    import tempfile
+    import bench
+    from motifscan_b200 import engine, synth
+    from motifscan_b200.genome import DeviceGenome
+    from motifscan_b200.motif import MotifPwms, PositionWeightMatrix
+    from motifscan_b200.variants import Haplotypes, haplotype_clusters, read_vcf, scan_haplotypes
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_gpu_haplotypes import oracle_rows
+
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+    root = tempfile.mkdtemp(prefix="msb_hap_", dir=args.out_dir)
+    try:
+        t0 = time.perf_counter()
+        pg = bench.make_genome(0, args.genome_scale)
+        gdir, mdir = os.path.join(root, "synth"), os.path.join(root, "jaspar_all")
+        os.makedirs(gdir), os.makedirs(mdir)
+        with open(os.path.join(gdir, "synth.fa"), "wb") as fh:
+            for c in pg.chroms:
+                fh.write(f">{c}\n".encode() + pg.decode_bytes(c, 0, pg.chrom_sizes[c]) + b"\n")
+        pg.save(os.path.join(gdir, "synth.packed"))
+        with open(os.path.join(gdir, "synth_bg_freq.txt"), "w") as fh:
+            fh.write("Base\tFrequency\n" + "".join(f"{b}\t{v}\n" for b, v in synth.BG.items()))
+        _, mats, ids = synth.motif_set(args.motifs, seed=2020)
+        ctx = engine.default_context(0)
+        mset = engine.MotifSet(ctx, mats)
+        bblob, boff = synth.background_samples(100000, 40, seed=1)
+        bg = engine.SequenceSet(ctx, blob=bblob, seq_off=boff)
+        cutoffs = np.maximum(np.around(engine.score_select(ctx, mset, bg, 3, [int(100000 * 1e-4) - 1])[:, 0], 8), 1e-6)
+        bg.close(), mset.close()
+        pwms = MotifPwms(name="jaspar_all", genome="synth")
+        for m, k, c in zip(mats, ids, cutoffs):
+            pwms.append(PositionWeightMatrix(m, name="TF" + k[2:6], matrix_id=k, cutoffs={"1e-4": float(c)}))
+        pwms.write_motifscan_pwms(os.path.join(mdir, "jaspar_all_synth_pwms.motifscan"))
+        n_alleles = args.alleles or int(1e6 * args.genome_scale)
+        vcf = os.path.join(root, "phased.vcf")
+        indels = args.indel_fraction > 0
+        n_rec = _synthetic_phased_vcf(vcf, pg, n_alleles, args.samples, indel_fraction=args.indel_fraction)
+        setup_s = time.perf_counter() - t0
+        lmax = max(m.shape[1] for m in mats)
+        t0 = time.perf_counter()
+        v = read_vcf(vcf, pg, indels=indels, samples="all")
+        parse_s = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        h = haplotype_clusters(v, lmax)
+        cluster_s = time.perf_counter() - t0
+        dg = DeviceGenome(pg, ctx)
+        runs = []
+        for _ in range(args.steps + 1):                                 # the first run warms up
+            sites = scan_haplotypes(dg, mats, cutoffs, h)
+            runs.append((sites.seconds, sites.timings))
+        scan_s, dev = min(runs[1:], key=lambda x: x[0])
+        # parity: a seeded sample of clusters, scanned on their own and compared with the oracle and the full run
+        rng = np.random.default_rng(5)
+        sel = np.sort(rng.choice(len(h), size=min(args.cpu_clusters, len(h)), replace=False))
+        cnt = h.sizes()[sel]
+        aoff = np.concatenate([[0], np.cumsum(cnt)])
+        alle = h.allele[np.repeat(h.allele_off[sel], cnt) + np.arange(int(cnt.sum())) - np.repeat(aoff[:-1], cnt)]
+        sub = Haplotypes(v, lmax, h.chrom[sel], aoff, alle, np.zeros(len(sel) + 1, np.int64), [], [], 0)
+        got = scan_haplotypes(dg, mats, cutoffs, sub)
+        dg.close()
+
+        class _Chrom:
+            def __init__(self, c):
+                self.c = c
+
+            def __len__(self):
+                return int(pg.chrom_sizes[self.c])
+
+            def __getitem__(self, sl):
+                return pg.decode_bytes(self.c, sl.start, min(sl.stop, len(self))).decode()
+
+        texts = {c: _Chrom(c) for c in pg.chroms}
+        t0 = time.perf_counter()
+        want = oracle_rows(texts, sub, mats, cutoffs, "both")
+        cpu_s = time.perf_counter() - t0
+        cols = list(zip(*want)) if want else [[]] * 9
+        same = len(got) == len(want)
+        for name, k, dt in (("cluster", 0, np.int32), ("motif", 1, np.int32), ("strand", 2, np.int8), ("ref_start", 3, np.int64),
+                            ("alt_start", 4, np.int64), ("effect", 7, np.int8), ("paired", 8, bool)):
+            same = same and np.array_equal(getattr(got, name), np.array(cols[k], dt))
+        for name, k in (("ref_score", 5), ("alt_score", 6)):
+            w = np.array(cols[k], np.float64)
+            same = same and np.array_equal(np.isnan(getattr(got, name)), np.isnan(w)) and np.array_equal(
+                getattr(got, name)[~np.isnan(w)].view(np.uint64), w[~np.isnan(w)].view(np.uint64))
+        in_full = np.isin(sites.cluster, sel)
+        full_same = (np.array_equal(np.searchsorted(sel, sites.cluster[in_full]), got.cluster)
+                     and np.array_equal(sites.ref_start[in_full], got.ref_start)
+                     and np.array_equal(sites.alt_start[in_full], got.alt_start)
+                     and np.array_equal(sites.ref_score[in_full].view(np.uint64), got.ref_score.view(np.uint64)))
+        cmd = [sys.executable, "-m", "motifscan_b200", "variant", "-i", vcf, "-m", mdir, "-g", gdir, "-o",
+               os.path.join(root, "cli"), "-p", "1e-4", "--haplotypes"] + (["--indels"] if indels else [])
+        t0 = time.perf_counter()
+        proc = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True)
+        wall_s = time.perf_counter() - t0
+        if proc.returncode != 0:
+            raise SystemExit("motifscan variant --haplotypes failed:\n" + proc.stderr[-2000:])
+        rss_mb = resource.getrusage(resource.RUSAGE_CHILDREN).ru_maxrss / 1024.0
+        out_bytes = {f: os.path.getsize(os.path.join(root, "cli", f)) for f in sorted(os.listdir(os.path.join(root, "cli")))}
+        log = [line for line in proc.stderr.splitlines() if line.startswith(("Read", "Scanned"))]
+    finally:
+        shutil.rmtree(root, ignore_errors=True)
+    sizes = h.sizes()
+    hist = np.bincount(np.minimum(sizes, 16))
+    return {"config": f"motifscan variant --haplotypes: {n_rec} VCF records x {args.samples} samples -> {len(v)} alleles, "
+                      f"{len(v.call_allele)} haplotype calls, {len(h)} distinct clusters on a {sum(pg.chrom_sizes.values())} bp "
+                      f"synthetic genome (scale {args.genome_scale}) x {args.motifs} motifs, both strands, p=1e-4 cutoffs "
+                      f"floored at 1e-6, indel fraction {args.indel_fraction}",
+            "card": smi.stdout.strip().splitlines(), "clusters": len(h),
+            "cluster_size_hist": {(str(k) if k < 16 else "16+"): int(x) for k, x in enumerate(hist) if x},
+            "max_cluster_size": int(sizes.max()), "call_skipped": {**v.call_skipped, "overlap": h.overlap},
+            "context_bp_per_set": sites.context_bp, "motif_bp": sites.motif_bp, "scan_s": scan_s,
+            "value": sites.motif_bp / scan_s, "device_ms": dev, "rows": len(sites), "rows_by_effect": sites.rows_by_effect(),
+            "vcf_parse_s": parse_s, "cluster_s": cluster_s, "setup_s": setup_s,
+            "cli": {"wall_s": wall_s, "peak_rss_mb": rss_mb, "bytes": out_bytes, "log": log},
+            "parity": {"sample_clusters": int(len(sel)), "rows": len(want), "identical_to_oracle": bool(same),
+                       "full_run_rows_of_the_sample_identical": bool(full_same), "oracle_s": cpu_s},
+            "note": "scan_s: scan_haplotypes wall time (extract both context sets, two scans, rows, sort, copy back), best "
+                    "of --steps after one warm-up; device_ms per phase of that run; value in motif*bp/s over the context "
+                    "bases of both sides"}
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants"])
+    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants", "haplotypes"])
     ap.add_argument("--alleles", type=int, default=None)
+    ap.add_argument("--samples", type=int, default=16)
+    ap.add_argument("--cpu-clusters", dest="cpu_clusters", type=int, default=500)
     ap.add_argument("--cpu-alleles", dest="cpu_alleles", type=int, default=2000)
     ap.add_argument("--indel-fraction", dest="indel_fraction", type=float, default=0.0)
     ap.add_argument("--out-dir", dest="out_dir", default=None)
@@ -845,7 +1033,7 @@ def main():
     if args.motifs is None:
         args.motifs = 1900 if args.which in ("enrich", "cli") else 750
     out = {"build": bench_build, "genome": bench_genome, "enrich": bench_enrich, "cli": bench_cli,
-           "whole-genome": bench_whole_genome, "variants": bench_variants}[args.which](args)
+           "whole-genome": bench_whole_genome, "variants": bench_variants, "haplotypes": bench_haplotypes}[args.which](args)
     if out is not None:
         print(json.dumps(out))
 

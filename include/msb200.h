@@ -136,6 +136,16 @@ int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const i
 int msb_seqs_extract_splice(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
                             const int64_t *end, const int32_t *splice_at, const int32_t *del_len, const int64_t *ins_off,
                             const uint8_t *ins_code, msb_seqs **out);
+/* msb_seqs_extract with several edits per sequence (the haplotypes of a cluster of alleles): sequence i is the cut
+ * interval (clipped like msb_seqs_extract) with each edit k in [edit_off[i], edit_off[i + 1]) -- its bases
+ * [edit_at[k], edit_at[k] + edit_del[k]), relative to the interval -- replaced by the A/C/G/T codes
+ * ins_code[ins_off[k] .. ins_off[k + 1]) (0..3).  edit_off has n + 1 entries and ins_off n_edits + 1, both starting at
+ * 0.  Edits out of order, overlapping (an insertion occupies its junction: the next edit starts at or behind
+ * edit_at + max(edit_del, 1)), outside their interval, or a code above 3 are MSB_EINVAL.  Only the tables cross PCIe.
+ * msb_seqs_extract_splice is this call with one edit per sequence. */
+int msb_seqs_extract_edits(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                           const int64_t *end, const int64_t *edit_off, const int32_t *edit_at, const int32_t *edit_del,
+                           const int64_t *ins_off, const uint8_t *ins_code, msb_seqs **out);
 /* Number of non-ACGT bases in each of n windows [start[i], start[i] + length) of sequence src_idx[i] of a
  * resident set (clipped at the sequence end): the device half of the background sampler's acceptance
  * test `seq.count('N') + seq.count('n') <= max_n` (genome/__init__.py:172-175) -- a window without
@@ -252,11 +262,31 @@ int msb_scan_variants(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *re
 int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *ref, const msb_seqs *alt,
                          const int32_t *core_start, const int32_t *ref_core_len, const int32_t *alt_core_len, int strand,
                          int64_t *n_rows);
-/* The rows of the last msb_scan_variants / msb_scan_variants_ex (MSB_EINVAL after any other scan): *n receives their number, the arrays are
- * filled when cap >= *n.  start is relative to the context; strand 1 / 2; ref_score / alt_score are the window's
- * scores on the two alleles bit for bit; effect 1 / 2 / 3 (or 5 / 6) as above.  MSB_T_D2H times the copies. */
+/* msb_scan_variants_ex with several edits per context (the haplotypes of a cluster of alleles): context i carries the
+ * edits k in [edit_off[i], edit_off[i + 1]) (edit_off has n + 1 entries, edit_off[0] = 0), edit k replacing the ref
+ * bases [edit_at[k], edit_at[k] + edit_ref_len[k]) by edit_alt_len[k] alt bases (not both 0).  The edits of a context
+ * are ordered and do not overlap (the next starts at or behind edit_at + max(edit_ref_len, 1)); on the alt context
+ * edit k starts at edit_at[k] + the net length change of the edits before it.  A site of length L at s on one side is
+ * affected when s < start + len and s + L > start for some edit's core on that side (a 0-length core: the window
+ * straddles the junction).  Inside edit k's core at offset o < min(ref len, alt len) it maps to the other side's core
+ * start + o, behind that offset it has no partner; in a stretch between cores it maps by the net shift of the edits
+ * before it.  A mapped window that fits in the other context is paired.  Rows are made as by msb_scan_variants_ex and
+ * ordered by context, motif, own-side start (the ref start for effect 1 / 3 / 5, the alt start for 2 / 6), strand, ref
+ * before alt. */
+int msb_scan_haplotypes(msb_ctx *ctx, const msb_motifs *motifs, const msb_seqs *ref, const msb_seqs *alt,
+                        const int64_t *edit_off, const int32_t *edit_at, const int32_t *edit_ref_len,
+                        const int32_t *edit_alt_len, int strand, int64_t *n_rows);
+/* The rows of the last msb_scan_variants / msb_scan_variants_ex / msb_scan_haplotypes (MSB_EINVAL after any other
+ * scan): *n receives their number, the arrays are filled when cap >= *n.  start is relative to the context (for
+ * msb_scan_haplotypes the own-side start); strand 1 / 2; ref_score / alt_score are the window's scores on the two
+ * alleles bit for bit; effect 1 / 2 / 3 (or 5 / 6) as above.  MSB_T_D2H times the copies. */
 int msb_scan_device_variant_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *allele, int32_t *motif, int32_t *start,
                                  int8_t *strand, double *ref_score, double *alt_score, int8_t *effect);
+/* msb_scan_device_variant_rows plus other_start: the window's start on the other side, relative to that context, or -1
+ * when it has no partner there. */
+int msb_scan_device_haplotype_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *context, int32_t *motif, int32_t *start,
+                                   int8_t *strand, double *ref_score, double *alt_score, int8_t *effect,
+                                   int32_t *other_start);
 int msb_result_wait(msb_result *res);
 int msb_result_total(const msb_result *res, int64_t *n_sites);
 int msb_result_counts(const msb_result *res, int64_t *counts /* n_motifs */);
@@ -324,6 +354,15 @@ int msb_write_variant_table(const char *path, const char *header, int64_t n, con
                             const int32_t *start, const int8_t *strand, const double *ref_score, const double *alt_score,
                             const int8_t *effect, int64_t n_alleles, const char *lead, const int64_t *lead_off, int32_t n_motifs,
                             const char *motif_text, const int64_t *motif_off, const int32_t *motif_len, int32_t n_threads);
+/* motif_haplotype_sites.xls, formatted like msb_write_variant_table: per row lead[lead_off[c] .. lead_off[c + 1]) of its
+ * cluster c (the caller's "chrom<TAB>cluster<TAB>ids<TAB>"), the motif text, ref_start, ref_start + motif_len[m],
+ * alt_start, alt_start + motif_len[m] (NA<TAB>NA for a start below 0: no window on that side), then strand, scores and
+ * effect exactly as there (effects 1 / 2 / 3 / 5 / 6, the missing score of 5 / 6 as NA). */
+int msb_write_haplotype_table(const char *path, const char *header, int64_t n, const int32_t *cluster, const int32_t *motif,
+                              const int64_t *ref_start, const int64_t *alt_start, const int8_t *strand, const double *ref_score,
+                              const double *alt_score, const int8_t *effect, int64_t n_clusters, const char *lead,
+                              const int64_t *lead_off, int32_t n_motifs, const char *motif_text, const int64_t *motif_off,
+                              const int32_t *motif_len, int32_t n_threads);
 int msb_text_free(char *text);
 
 /* ---- score (replaces motif_score_thread + motif_score, cscore.c:174-302) -------------------- */

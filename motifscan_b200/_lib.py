@@ -56,6 +56,8 @@ SIGNATURES = {
                                               ctypes.POINTER(c_vp)]),
     "msb_seqs_extract_splice": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, c_i32p, c_i32p, c_i64p, c_vp,
                                                ctypes.POINTER(c_vp)]),
+    "msb_seqs_extract_edits": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, c_i64p, c_i64p, c_i32p, c_i32p, c_i64p,
+                                              c_vp, ctypes.POINTER(c_vp)]),
     "msb_seqs_lengths": (ctypes.c_int, [c_vp, c_i64p]),
     "msb_seqs_window_ncount": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, c_i64p, ctypes.c_int32, c_i32p]),
     "msb_seqs_set_start_limit": (ctypes.c_int, [c_vp, c_i32p]),
@@ -79,6 +81,9 @@ SIGNATURES = {
     "msb_scan_variants_ex": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32p, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
     "msb_scan_device_variant_rows": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_i8p, c_f64p, c_f64p,
                                                     c_i8p]),
+    "msb_scan_haplotypes": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i64p, c_i32p, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
+    "msb_scan_device_haplotype_rows": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_i8p, c_f64p,
+                                                      c_f64p, c_i8p, c_i32p]),
     "msb_result_wait": (ctypes.c_int, [c_vp]),
     "msb_merge_motif_major": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, c_i64p, ctypes.POINTER(c_vp), c_vp,
                                              ctypes.c_int32, c_i64p, ctypes.c_int32]),
@@ -97,6 +102,9 @@ SIGNATURES = {
     "msb_write_variant_table": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int64, c_i32p, c_i32p, c_i32p, c_i8p,
                                                c_f64p, c_f64p, c_i8p, ctypes.c_int64, ctypes.c_char_p, c_i64p, ctypes.c_int32,
                                                ctypes.c_char_p, c_i64p, c_i32p, ctypes.c_int32]),
+    "msb_write_haplotype_table": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int64, c_i32p, c_i32p, c_i64p,
+                                                 c_i64p, c_i8p, c_f64p, c_f64p, c_i8p, ctypes.c_int64, ctypes.c_char_p, c_i64p,
+                                                 ctypes.c_int32, ctypes.c_char_p, c_i64p, c_i32p, ctypes.c_int32]),
     "msb_text_free": (ctypes.c_int, [c_vp]),
     "msb_result_total": (ctypes.c_int, [c_vp, c_i64p]),
     "msb_result_counts": (ctypes.c_int, [c_vp, c_i64p]),

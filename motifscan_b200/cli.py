@@ -22,12 +22,14 @@ Same flags as the reference's subcommands (cli/main.py:407-430, 504-579) and the
 
   * `variant` (not in the reference) scans the SNVs and MNVs of a VCF against the resident genome and reports the
     motif sites each allele creates or destroys (motifscan_b200/variants.py; one GPU, `-t` ignored); `--indels` scans
-    insertions and deletions too, as the VCF places them (normalise it first);
+    insertions and deletions too, as the VCF places them (normalise it first); `--haplotypes` reads the phased
+    genotypes and scans the alleles each haplotype carries within a motif width of each other together;
 
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir
     python -m motifscan_b200 scan --whole-genome -m <motif set> -g <genome> -o out_dir [--site]
     python -m motifscan_b200 motif --build <motif set> -g <genome>
     python -m motifscan_b200 variant -i calls.vcf.gz -m <motif set> -g <genome> -o out_dir [--indels]
+    python -m motifscan_b200 variant -i phased.vcf.gz -m <motif set> -g <genome> -o out_dir --haplotypes [--samples A,B]
 """
 import argparse
 import logging
@@ -201,13 +203,20 @@ def run_variant(args):
         cutoffs = [pwm.cutoffs[args.p_value] for pwm in pwms]
     except (TypeError, KeyError):
         raise SystemExit(f"motifscan: error: PWMs have no motif score cutoff set for P-value {args.p_value!r}")
+    if args.samples and not args.haplotypes:
+        raise SystemExit("motifscan variant: error: --samples needs --haplotypes")
+    samples = None
+    if args.haplotypes:
+        samples = [x for x in args.samples.split(",") if x] if args.samples else "all"
     pg = packed_genome(genome, PACKED_MIN_BP)
     try:
-        vcf = msvar.read_vcf(args.input_file, pg, indels=args.indels)
+        vcf = msvar.read_vcf(args.input_file, pg, indels=args.indels, samples=samples)
     except (OSError, UnicodeDecodeError, EOFError) as err:
         raise SystemExit(f"motifscan variant: error: cannot read {args.input_file}: {err}")
     except ValueError as err:
         raise SystemExit(f"motifscan variant: error: {err}")
+    if args.haplotypes:
+        return _run_haplotypes(args, msvar, pg, pwms, cutoffs, vcf)
     logger.info("===== Scanning variants =====")
     dg = DeviceGenome(pg)
     try:
@@ -221,6 +230,31 @@ def run_variant(args):
                 f"in {sites.seconds:.3f} s: {len(sites)} rows ({by['gain']} gain, {by['loss']} loss, {by['both']} both)")
     logger.info("Saving the result tables")
     msio.write_variant_tables(args.output_dir, pwms, vcf, sites)
+    logger.info("===== MotifScan Finished =====")
+    return 0
+
+
+def _run_haplotypes(args, msvar, pg, pwms, cutoffs, vcf):
+    """`variant --haplotypes`: sites gained / lost by each phased haplotype's clusters of alleles
+    (variants.haplotype_clusters / scan_haplotypes)."""
+    from .genome import DeviceGenome
+    lmax = max((int(p.length) for p in pwms), default=1)
+    haps = msvar.haplotype_clusters(vcf, lmax)
+    skipped = ", ".join(f"{k} {v}" for k, v in vcf.skipped.items())
+    calls = ", ".join(f"{k} {v}" for k, v in {**vcf.call_skipped, "overlap": haps.overlap}.items())
+    logger.info(f"Read {len(vcf)} alleles (skipped: {skipped}) and {len(vcf.call_allele)} haplotype calls of "
+                f"{len(vcf.samples)} samples (skipped: {calls}): {len(haps)} distinct clusters")
+    logger.info("===== Scanning haplotypes =====")
+    dg = DeviceGenome(pg)
+    try:
+        sites = msvar.scan_haplotypes(dg, pwms, cutoffs, haps, strand=args.strand)
+    finally:
+        dg.close()
+    by = sites.rows_by_effect()
+    logger.info(f"Scanned {len(haps)} clusters x {len(pwms)} motifs, {sites.motif_bp:.3e} motif*bp in {sites.seconds:.3f} s: "
+                f"{len(sites)} rows ({by['gain']} gain, {by['loss']} loss, {by['both']} both)")
+    logger.info("Saving the result tables")
+    msio.write_haplotype_tables(args.output_dir, pwms, haps, sites)
     logger.info("===== MotifScan Finished =====")
     return 0
 
@@ -320,6 +354,11 @@ def make_parser():
     variant.add_argument("-t", "--threads", dest="n_threads", type=int, default=1)
     variant.add_argument("--indels", action="store_true",
                          help="Also scan insertions and deletions (not left-aligned: normalise the VCF first).")
+    variant.add_argument("--haplotypes", action="store_true",
+                         help="Scan each sample's phased haplotypes: alleles in cis within a motif width are scanned "
+                              "together (writes the motif_haplotype_* tables instead).")
+    variant.add_argument("--samples", dest="samples", default=None, metavar="A,B,...",
+                         help="With --haplotypes: read only these samples (default: all).")
     variant.add_argument("-o", "--output-dir", dest="output_dir", required=True, metavar="DIR")
     variant.add_argument("--verbose", action="store_true")
     variant.set_defaults(func=run_variant)

@@ -9,7 +9,7 @@
 //   dedup_flags_kernel      adjacent-site de-duplication              (scanner.py:156-193)
 //   score0_kernel           offset-0 window score of every sequence     (cscore.c:191-223)
 //   extract_subst_kernel    resident-genome extraction with allele bases overlaid (variant contexts)
-//   extract_splice_kernel   resident-genome extraction with bases deleted and inserted (indel contexts)
+//   extract_edits_kernel    resident-genome extraction with bases deleted and inserted (indel and haplotype contexts)
 //   variant_rows_kernel     sites of the ref / alt context scans -> gain / loss / both rows
 #pragma once
 #include "common.cuh"
@@ -152,42 +152,59 @@ extract_subst_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int
     blk_seq[b] = (int32_t) s;
 }
 
-// extract with a splice (the alternative alleles of a variant scan with indels): destination sequence s = source
-// [start, start + c) + the A/C/G/T codes ins_code[ins_off[s] .. ins_off[s + 1]) + source [start + c + r, end), with
-// c = splice_at[s] and r = del_len[s].  A 32-base block may hold pieces of all three: each flank is cut by
-// extract_block at its own source offset and shifted into place; the inserted bases are set one by one.
+// extract with edits (the alternative alleles of a variant scan with indels, and the haplotypes of a cluster of
+// alleles): destination sequence s is its source interval with each edit k in [edit_off[s], edit_off[s + 1]) --
+// bases [at_k, at_k + del_k) of the interval, in order and not overlapping -- replaced by the A/C/G/T codes
+// ins_code[ins_off[k] .. ins_off[k + 1]); edit_off == nullptr: one edit per sequence, edit s.  edit_dst[k] is where
+// edit k's inserted bases start in the destination (at_k + the net length change of the edits before it).  The destination alternates flanks (source bases) and
+// inserted pieces; a block finds its first piece by a binary search over its sequence's edits and walks pieces until
+// it is full -- any number of them (ten adjacent SNVs put twenty pieces into one block).  A flank is cut by
+// extract_block at its source offset and shifted into place; inserted bases are set directly (their mask bits stay
+// clear).
 __global__ void __launch_bounds__(256)
-extract_splice_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int64_t *__restrict__ src_start,
-                      const int32_t *__restrict__ splice_at, const int32_t *__restrict__ del_len,
-                      const int64_t *__restrict__ ins_off, const uint8_t *__restrict__ ins_code,
-                      const int64_t *__restrict__ poff, const int32_t *__restrict__ len, int64_t n_seqs,
-                      int64_t n_blocks, uint32_t *__restrict__ codes, uint32_t *__restrict__ nmask,
-                      int32_t *__restrict__ blk_seq) {
+extract_edits_kernel(SeqView src, const int32_t *__restrict__ src_idx, const int64_t *__restrict__ src_start,
+                     const int64_t *__restrict__ edit_off, const int32_t *__restrict__ edit_at,
+                     const int32_t *__restrict__ edit_del, const int32_t *__restrict__ edit_dst,
+                     const int64_t *__restrict__ ins_off, const uint8_t *__restrict__ ins_code,
+                     const int64_t *__restrict__ poff, const int32_t *__restrict__ len, int64_t n_seqs,
+                     int64_t n_blocks, uint32_t *__restrict__ codes, uint32_t *__restrict__ nmask,
+                     int32_t *__restrict__ blk_seq) {
     const int64_t b = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= n_blocks) return;
     const int64_t p = b * kPadBases;
     const int64_t s = find_seq(poff, n_seqs, p);
     const int64_t j = p - __ldg(poff + s);
-    const int n = (int) min((int64_t) kPadBases, (int64_t) __ldg(len + s) - j);
-    const int64_t c = __ldg(splice_at + s), i0 = __ldg(ins_off + s);
-    const int64_t a = __ldg(ins_off + s + 1) - i0, r = __ldg(del_len + s);
-    uint32_t lo, hi, mask;
-    // left flank: destination [j, min(j + n, c)) = source [j, ...)
-    extract_block(src, src_idx, src_start, s, j, (int) max(min((int64_t) n, c - j), (int64_t) 0), lo, hi, mask);
-    uint64_t code = (uint64_t) hi << 32 | lo;
-    // right flank: destination [d0, j + n) = source [d0 + r - a, ...), d0 = max(j, c + a)
-    const int64_t d0 = max(j, c + a);
-    if (d0 < j + n) {
-        uint32_t rl, rh, rm;
-        extract_block(src, src_idx, src_start, s, d0 + r - a, (int) (j + n - d0), rl, rh, rm);
-        const int k = (int) (d0 - j);                                    // 0 <= k < n <= 32
-        code |= ((uint64_t) rh << 32 | rl) << (2 * k);
-        mask |= rm << k;
+    const int64_t dlen = __ldg(len + s), jn = j + min((int64_t) kPadBases, dlen - j);
+    const int64_t e0 = edit_off ? __ldg(edit_off + s) : s, e1 = edit_off ? __ldg(edit_off + s + 1) : s + 1;
+    // the first edit whose inserted piece ends behind j (these ends never decrease): the block starts in the flank
+    // before it or inside its inserted piece
+    int64_t lo = e0, hi = e1;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(edit_dst + mid) + (__ldg(ins_off + mid + 1) - __ldg(ins_off + mid)) > j) hi = mid; else lo = mid + 1;
     }
-    // inserted bases: destination [max(j, c), min(j + n, c + a)) (their mask bits are already clear)
-    for (int64_t q = max(j, c), q1 = min(j + n, c + a); q < q1; q++) {
-        const int k = (int) (q - j);
-        code |= (uint64_t) (__ldg(ins_code + i0 + (q - c)) & 3u) << (2 * k);
+    uint64_t code = 0;
+    uint32_t mask = 0;
+    int64_t d = j;
+    for (int64_t k = lo; d < jn; k++) {
+        // flank before edit k: destination [d, fe) = source [d - shift, ...), shift = the net change of edits < k
+        const int64_t fe = k < e1 ? __ldg(edit_dst + k) : dlen;
+        if (d < fe) {
+            const int64_t shift = k > e0 ? __ldg(edit_dst + k - 1) + (__ldg(ins_off + k) - __ldg(ins_off + k - 1)) -
+                                               (__ldg(edit_at + k - 1) + __ldg(edit_del + k - 1)) : 0;
+            const int64_t d1 = min(fe, jn);
+            uint32_t rl, rh, rm;
+            extract_block(src, src_idx, src_start, s, d - shift, (int) (d1 - d), rl, rh, rm);
+            const int q = (int) (d - j);                                 // 0 <= q < 32
+            code |= ((uint64_t) rh << 32 | rl) << (2 * q);
+            mask |= rm << q;
+            d = d1;
+        }
+        if (d >= jn) break;
+        // inserted bases of edit k: destination [edit_dst[k], + its length), d inside it
+        const int64_t i0 = __ldg(ins_off + k), ds = __ldg(edit_dst + k);
+        const int64_t d1 = min(ds + (__ldg(ins_off + k + 1) - i0), jn);
+        for (; d < d1; d++) code |= (uint64_t) (__ldg(ins_code + i0 + (d - ds)) & 3u) << (2 * (d - j));
     }
     codes[2 * b] = (uint32_t) code;
     codes[2 * b + 1] = (uint32_t) (code >> 32);
@@ -922,18 +939,30 @@ cell_stats_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Variant rows (msb_scan_variants_ex).  Sequence i of `ref` and of `alt` is allele i's context on the reference and
-// with the allele applied; both start at the same base, and the changed bases are [c, c + ref_len[i]) of the ref
-// context and [c, c + alt_len[i]) of the alt context, c = core_start[i] (equal lengths for an SNV / MNV, one of them
-// possibly 0 for an indel).  One thread per final site of either scan.  A site of length L at s is affected when
-// s < c + k and s + L > c, k = its own side's changed length (for k = 0: the window straddles the junction).  It is
-// paired with the other context's window at s when s < c + min(ref_len, alt_len) and that window fits in the other
-// context; a paired window is re-scored there with the reference's arithmetic (exact_raw, cscore.c:341-389):
+// Variant rows (msb_scan_variants_ex, msb_scan_haplotypes).  Sequence i of `ref` and of `alt` is context i on the
+// reference and with its edits applied; both start at the same base.  Edit k in [edit_off[i], edit_off[i + 1])
+// replaces the ref bases [R.at[k], R.at[k] + R.len[k]) by the alt bases [A.at[k], A.at[k] + A.len[k]); A.at is R.at
+// shifted by the net length change of the edits before k (edit_off == nullptr: one edit per context, edit i, and
+// A.at == R.at).  The edits are ordered and do not overlap, so on each side
+// both their starts and their ends never decrease.  One thread per final site of either scan.  A site of length L at
+// s is affected when it touches some edit's core on its own side: s < at + len and s + L > at (a 0-length core: the
+// window straddles the junction) -- the first edit k whose core ends behind s decides, found by binary search (dense
+// clusters have many edits).  Its window maps to the other side: inside core k at offset o, to the other core's
+// start + o when o < min(ref len, alt len) (else it has no partner); before core k, by the net shift of the edits
+// before k.  It is paired when the mapped window fits in the other context; a paired window is re-scored there with
+// the reference's arithmetic (exact_raw, cscore.c:341-389):
 //   ref-list site:  effect 1 (loss) or 3 (both, the alt window passes too);
 //   alt-list site:  effect 2 (gain) only when the ref window fails -- else the ref list already has the row.
-// An unpaired site has no window on the other allele: effect 5 (loss) or 6 (gain), the other score NaN.  Rows are
-// appended (order restored by the sort on row_key = allele | motif | start | strand bit); no two rows share a key,
-// as at most one side has unpaired windows.
+// The alt list may leave a passing pair to the ref list only because a paired pair of windows is affected on both
+// sides or on neither: both windows are placed by the same edit k (the map keeps a start in the same stretch or at the
+// same core offset), and both reach core k exactly when s + L passes its start on that side.  The tests' oracle
+// derives the rows without this invariant.
+// An unpaired site has no window on the other allele: effect 5 (loss) or 6 (gain), the other score NaN, other start
+// -1 (row_other == nullptr: not recorded).  Rows are appended (order restored by the sort on row_key = context | motif | own-side start | strand bit
+// [| side bit]).  With several edits per context the two sides' coordinates diverge and a ref row and an alt row can
+// share (start, strand); the side bit (side_bits = 1) then keeps their keys apart.  With one edit at most one side
+// has unpaired windows and no two rows share (start, strand), so side_bits = 0 leaves the single-allele keys as they
+// were.
 // ---------------------------------------------------------------------------------------------
 struct VariantSide {
     SeqView seq;                     // this list's contexts
@@ -941,6 +970,7 @@ struct VariantSide {
     const int32_t *seq_idx, *start;
     const int8_t *strand;
     const double *score;
+    const int32_t *at, *len;         // this side's edit cores
     int64_t n;
     int key_shift;
 };
@@ -951,11 +981,10 @@ __device__ __forceinline__ bool site_predicate(const MotifView &M, uint32_t m, d
 }
 
 __global__ void __launch_bounds__(256)
-variant_rows_kernel(VariantSide R, VariantSide A, MotifView M, const int32_t *__restrict__ core_start,
-                    const int32_t *__restrict__ ref_len, const int32_t *__restrict__ alt_len, int motif_bits, int start_bits,
-                    unsigned long long *__restrict__ n_rows, uint64_t *__restrict__ row_key,
+variant_rows_kernel(VariantSide R, VariantSide A, MotifView M, const int64_t *__restrict__ edit_off, int motif_bits,
+                    int start_bits, int side_bits, unsigned long long *__restrict__ n_rows, uint64_t *__restrict__ row_key,
                     int32_t *__restrict__ row_idx, double *__restrict__ row_ref, double *__restrict__ row_alt,
-                    int8_t *__restrict__ row_eff) {
+                    int8_t *__restrict__ row_eff, int32_t *__restrict__ row_other) {
     const int64_t t = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= R.n + A.n) return;
     const bool from_ref = t < R.n;
@@ -965,35 +994,53 @@ variant_rows_kernel(VariantSide R, VariantSide A, MotifView M, const int32_t *__
     const uint32_t m = site_motif(S.key[i], S.key_shift);
     const int32_t s = S.seq_idx[i], st = S.start[i];
     const int L = __ldg(M.len + m);
-    const int32_t c0 = __ldg(core_start + s), kr = __ldg(ref_len + s), ka = __ldg(alt_len + s);
-    if (st >= c0 + (from_ref ? kr : ka) || st + L <= c0) return;        // the window does not touch a changed base
-    const bool paired = st < c0 + min(kr, ka) && st + L <= __ldg(O.seq.len + s);
+    int64_t lo = edit_off ? __ldg(edit_off + s) : s, hi = edit_off ? __ldg(edit_off + s + 1) : s + 1;
+    const int64_t e1 = hi;
+    while (lo < hi) {                                                    // the first edit whose core ends behind st
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(S.at + mid) + __ldg(S.len + mid) > st) hi = mid; else lo = mid + 1;
+    }
+    if (lo == e1) return;                                                // behind every core
+    const int32_t at = __ldg(S.at + lo), oat = __ldg(O.at + lo);
+    if (at >= st + L) return;                                            // the window does not touch a changed base
+    int32_t ost;                                                         // the window's start on the other side
+    bool paired = true;
+    if (st >= at) {                                                      // inside core lo
+        paired = st - at < min(__ldg(S.len + lo), __ldg(O.len + lo));
+        ost = oat + (st - at);
+    } else {                                                             // in the shared stretch before core lo
+        ost = st + (oat - at);
+    }
+    paired = paired && ost + L <= __ldg(O.seq.len + s);
     const int rev = S.strand[i] == 2;
     double other = __longlong_as_double(0x7ff8000000000000ll);           // NaN: no window on the other allele
     bool other_hit = false;
     if (paired) {
         const double *pw = M.pwm + 4 * (int64_t) __ldg(M.col_off + m);
-        other_hit = site_predicate(M, m, exact_raw(O.seq, pw, L, __ldg(O.seq.poff + s) + st, rev), other);
+        other_hit = site_predicate(M, m, exact_raw(O.seq, pw, L, __ldg(O.seq.poff + s) + ost, rev), other);
         if (!from_ref && other_hit) return;                              // a site on both alleles: the ref list's row
     }
     const unsigned long long slot = atomicAdd(n_rows, 1ull);
-    row_key[slot] = ((((uint64_t) s << motif_bits | m) << start_bits | (uint64_t) st) << 1) | (uint64_t) rev;
+    row_key[slot] = (((((uint64_t) s << motif_bits | m) << start_bits | (uint64_t) st) << 1 | (uint64_t) rev)
+                     << side_bits) | (uint64_t) (from_ref ? 0 : side_bits);
     row_idx[slot] = (int32_t) slot;
     row_ref[slot] = from_ref ? S.score[i] : other;
     row_alt[slot] = from_ref ? other : S.score[i];
     row_eff[slot] = (int8_t) ((from_ref ? (other_hit ? 3 : 1) : 2) | (paired ? 0 : 4));
+    if (row_other) row_other[slot] = paired ? ost : -1;
 }
 
 // Sorted row keys + the permutation -> the row arrays in order.
 __global__ void __launch_bounds__(256)
 variant_gather_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ idx, int64_t n, int motif_bits,
-                      int start_bits, const double *__restrict__ ref_in, const double *__restrict__ alt_in,
-                      const int8_t *__restrict__ eff_in, int32_t *__restrict__ allele, int32_t *__restrict__ motif,
-                      int32_t *__restrict__ start, int8_t *__restrict__ strand, double *__restrict__ ref_out,
-                      double *__restrict__ alt_out, int8_t *__restrict__ eff_out) {
+                      int start_bits, int side_bits, const double *__restrict__ ref_in, const double *__restrict__ alt_in,
+                      const int8_t *__restrict__ eff_in, const int32_t *__restrict__ other_in, int32_t *__restrict__ allele,
+                      int32_t *__restrict__ motif, int32_t *__restrict__ start, int8_t *__restrict__ strand,
+                      double *__restrict__ ref_out, double *__restrict__ alt_out, int8_t *__restrict__ eff_out,
+                      int32_t *__restrict__ other_out) {
     const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint64_t k = key[i];
+    const uint64_t k = key[i] >> side_bits;
     const int32_t j = idx[i];
     allele[i] = (int32_t) (k >> (motif_bits + start_bits + 1));
     motif[i] = (int32_t) ((k >> (start_bits + 1)) & ((1ull << motif_bits) - 1ull));
@@ -1002,6 +1049,7 @@ variant_gather_kernel(const uint64_t *__restrict__ key, const int32_t *__restric
     ref_out[i] = ref_in[j];
     alt_out[i] = alt_in[j];
     eff_out[i] = eff_in[j];
+    if (other_out) other_out[i] = other_in[j];
 }
 
 }  // namespace msb

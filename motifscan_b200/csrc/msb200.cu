@@ -83,10 +83,12 @@ struct msb_ctx {
     // boundary chains of the last de-duplicated range scan (msb_scan_device_boundary_sites)
     DevBuf bnd_range, bnd_cnt, bnd_dst, bnd_motif, bnd_seq, bnd_start, bnd_score, bnd_strand, bnd_flags;
     int64_t last_boundary = -1;            // sites in the bnd_* arrays; -1: the last scan collected none
-    // rows of the last msb_scan_variants (msb_scan_device_variant_rows): unsorted, sort keys, then in row order
-    DevBuf vr_key, vr_idx, vr_ref, vr_alt, vr_eff, vr_key_sorted, vr_idx_sorted, vr_core;
-    DevBuf vo_allele, vo_motif, vo_start, vo_strand, vo_ref, vo_alt, vo_eff;
+    // rows of the last variant / haplotype scan (msb_scan_device_variant_rows): unsorted, sort keys, then in row
+    // order; vr_core holds the edit tables (ref at | alt at | ref len | alt len), vr_eoff the edit offsets
+    DevBuf vr_key, vr_idx, vr_ref, vr_alt, vr_eff, vr_other, vr_key_sorted, vr_idx_sorted, vr_core, vr_eoff;
+    DevBuf vo_allele, vo_motif, vo_start, vo_strand, vo_ref, vo_alt, vo_eff, vo_other;
     int64_t last_variant_rows = -1;        // -1: the last scan was not a variant scan
+    bool last_rows_other = false;          // the last variant scan recorded other-side starts (msb_scan_haplotypes)
     // Final site arrays of a scan.  Two sets, used alternately: the device-to-host copy of scan k's
     // sites (on d2h_stream, MSB_SCAN_ASYNC) reads one set while scan k + 1 fills the other.
     struct FinSet {
@@ -392,8 +394,9 @@ int msb_ctx_destroy(msb_ctx *ctx) {
                       &ctx->motif_counts, &ctx->sel_aux, &ctx->limit1, &ctx->lane_count, &ctx->bnd_range,
                       &ctx->bnd_cnt, &ctx->bnd_dst, &ctx->bnd_motif, &ctx->bnd_seq, &ctx->bnd_start, &ctx->bnd_score,
                       &ctx->bnd_strand, &ctx->bnd_flags, &ctx->vr_key, &ctx->vr_idx, &ctx->vr_ref, &ctx->vr_alt,
-                      &ctx->vr_eff, &ctx->vr_key_sorted, &ctx->vr_idx_sorted, &ctx->vr_core, &ctx->vo_allele,
-                      &ctx->vo_motif, &ctx->vo_start, &ctx->vo_strand, &ctx->vo_ref, &ctx->vo_alt, &ctx->vo_eff})
+                      &ctx->vr_eff, &ctx->vr_other, &ctx->vr_key_sorted, &ctx->vr_idx_sorted, &ctx->vr_core,
+                      &ctx->vr_eoff, &ctx->vo_allele, &ctx->vo_motif, &ctx->vo_start, &ctx->vo_strand, &ctx->vo_ref,
+                      &ctx->vo_alt, &ctx->vo_eff, &ctx->vo_other})
         b->release();
     if (ctx->d2h_stream) cudaStreamSynchronize(ctx->d2h_stream);
     for (auto &f : ctx->fin) {
@@ -770,12 +773,13 @@ int msb_seqs_to_packed(msb_ctx *ctx, const msb_seqs *S, uint32_t *codes, uint32_
 
 }  // extern "C"
 
-// msb_seqs_extract; with a substitution table (sub_off != nullptr) msb_seqs_extract_subst; with a splice table
-// (ins_off != nullptr) msb_seqs_extract_splice.
+// msb_seqs_extract; with a substitution table (sub_off != nullptr) msb_seqs_extract_subst; with an edit table
+// (ins_off != nullptr) msb_seqs_extract_edits, or with edit_off == nullptr (one edit per sequence)
+// msb_seqs_extract_splice.
 static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
                         const int64_t *end, const int64_t *sub_off, const int32_t *sub_pos, const uint8_t *sub_code,
-                        const int32_t *splice_at, const int32_t *del_len, const int64_t *ins_off, const uint8_t *ins_code,
-                        msb_seqs **out, const char *what) {
+                        const int64_t *edit_off, const int32_t *edit_at, const int32_t *edit_del, const int64_t *ins_off,
+                        const uint8_t *ins_code, msb_seqs **out, const char *what) {
     if (!ctx || !src || !out || n < 0 || (n > 0 && (!src_idx || !start || !end))) {
         set_error(std::string(what) + ": bad argument");
         return MSB_EINVAL;
@@ -786,26 +790,44 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
     // pysam's fetch (genome/__init__.py:135) clips `end` at the sequence length; an interval that
     // starts behind it, or is reversed, is empty.
     std::vector<int64_t> seq_off((size_t) n + 1, 0), clipped_start((size_t) std::max<int64_t>(n, 1), 0);
-    const int64_t n_ins = ins_off ? ins_off[n] : 0;
-    if (ins_off && (ins_off[0] != 0 || (n > 0 && (!splice_at || !del_len)) || (n_ins > 0 && !ins_code))) {
-        set_error(std::string(what) + ": bad splice table");
+    const bool edits = ins_off != nullptr, one_each = edits && !edit_off;
+    const int64_t n_edits = !edits ? 0 : one_each ? n : edit_off[n], n_ins = edits ? ins_off[n_edits] : 0;
+    if (edits && ((edit_off && edit_off[0] != 0) || ins_off[0] != 0 || (n_edits > 0 && (!edit_at || !edit_del)) ||
+                  (n_ins > 0 && !ins_code))) {
+        set_error(std::string(what) + ": bad edit table");
         return MSB_EINVAL;
     }
+    // where each edit's bases land (one edit per sequence: at its own start, edit_at)
+    std::vector<int32_t> edit_dst((size_t) (one_each ? 0 : std::max<int64_t>(n_edits, 1)));
     for (int64_t i = 0; i < n; i++) {
         if (src_idx[i] < 0 || src_idx[i] >= src->n) { set_error(std::string(what) + ": source index out of range"); return MSB_EINVAL; }
         if (start[i] < 0) { set_error(std::string(what) + ": negative start"); return MSB_EINVAL; }
         const int64_t slen = src->seq_off[src_idx[i] + 1] - src->seq_off[src_idx[i]];
         const int64_t a = std::min(start[i], slen), b = std::min(end[i], slen);
         int64_t len = std::max<int64_t>(b - a, 0);
-        if (ins_off) {
-            // the cut interval loses [splice_at, splice_at + del_len) and gains the inserted bases there
-            if (ins_off[i + 1] < ins_off[i]) { set_error(std::string(what) + ": insertion offsets not ascending"); return MSB_EINVAL; }
-            if (splice_at[i] < 0 || del_len[i] < 0 || (int64_t) splice_at[i] + del_len[i] > len) {
-                set_error(std::string(what) + ": splice outside its interval");
-                return MSB_EINVAL;
+        if (edits) {
+            // the cut interval loses each edit's [at, at + del) and gains its inserted bases there
+            const int64_t e0 = one_each ? i : edit_off[i], e1 = one_each ? i + 1 : edit_off[i + 1];
+            if (e1 < e0) { set_error(std::string(what) + ": edit offsets not ascending"); return MSB_EINVAL; }
+            const int64_t ilen = len;
+            for (int64_t k = e0; k < e1; k++) {
+                if (ins_off[k + 1] < ins_off[k]) { set_error(std::string(what) + ": insertion offsets not ascending"); return MSB_EINVAL; }
+                if (edit_at[k] < 0 || edit_del[k] < 0 || (int64_t) edit_at[k] + edit_del[k] > ilen) {
+                    set_error(std::string(what) + ": edit outside its interval");
+                    return MSB_EINVAL;
+                }
+                if (k > e0) {
+                    // an insertion occupies its junction: the next edit starts behind at + max(del, 1)
+                    if (edit_at[k] < edit_at[k - 1]) { set_error(std::string(what) + ": edits out of order"); return MSB_EINVAL; }
+                    if (edit_at[k] < edit_at[k - 1] + std::max(edit_del[k - 1], 1)) {
+                        set_error(std::string(what) + ": edits overlap");
+                        return MSB_EINVAL;
+                    }
+                }
+                if (!one_each) edit_dst[(size_t) k] = (int32_t) (edit_at[k] + (len - ilen));
+                len += ins_off[k + 1] - ins_off[k] - edit_del[k];
+                if (len > (int64_t) 0x7fffffff - 64) { set_error(std::string(what) + ": edited sequence >= 2^31 bases"); return MSB_EINVAL; }
             }
-            len += ins_off[i + 1] - ins_off[i] - del_len[i];
-            if (len > (int64_t) 0x7fffffff - 64) { set_error(std::string(what) + ": spliced sequence >= 2^31 bases"); return MSB_EINVAL; }
         }
         clipped_start[i] = a;
         seq_off[i + 1] = seq_off[i] + len;
@@ -832,13 +854,16 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
     MSB_TRY(seqs_prepare(ctx, n, seq_off.data(), &S, lens));
     // the tables ride in the (otherwise unused here) ASCII scratch:
     // src_idx (4n) | start (8n) [| sub_off (8 (n + 1)) | sub_pos (4 n_sub) | sub_code (n_sub)]
-    //                           [| splice_at (4n) | del_len (4n) | ins_off (8 (n + 1)) | ins_code (n_ins)]
+    //                           [| edit_off (8 (n + 1)) | edit_at, edit_del, edit_dst (4 n_edits each)
+    //                            | ins_off (8 (n_edits + 1)) | ins_code (n_ins)]; one edit per sequence: no
+    //                            edit_off, and edit_dst is edit_at
     auto al = [](size_t x) { return (x + 15) & ~(size_t) 15; };
     const size_t o_start = al((size_t) n * 4), o_soff = o_start + al((size_t) n * 8);
     const size_t o_spos = o_soff + al((size_t) (n + 1) * 8), o_scode = o_spos + al((size_t) n_sub * 4);
-    const size_t o_at = o_soff, o_del = o_at + al((size_t) n * 4), o_ioff = o_del + al((size_t) n * 4);
-    const size_t o_icode = o_ioff + al((size_t) (n + 1) * 8);
-    const size_t bytes = sub_off ? o_scode + (size_t) n_sub : ins_off ? o_icode + (size_t) n_ins : o_start + (size_t) n * 8;
+    const size_t o_eoff = o_soff, o_at = o_eoff + al((size_t) (n + 1) * 8), o_del = o_at + al((size_t) n_edits * 4);
+    const size_t o_dst = o_del + al((size_t) n_edits * 4), o_ioff = o_dst + al((size_t) n_edits * 4);
+    const size_t o_icode = o_ioff + al((size_t) (n_edits + 1) * 8);
+    const size_t bytes = sub_off ? o_scode + (size_t) n_sub : edits ? o_icode + (size_t) n_ins : o_start + (size_t) n * 8;
     int rc = ctx->ascii.ensure(std::max<size_t>(bytes, 16));
     if (rc != MSB_OK) { msb_seqs_destroy(S); return rc; }
     char *base = (char *) ctx->ascii.p;
@@ -856,12 +881,15 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
             step(cudaMemcpyAsync(base + o_scode, sub_code, (size_t) n_sub, cudaMemcpyHostToDevice, st));
         }
     }
-    if (ins_off) {
-        if (n) {
-            step(cudaMemcpyAsync(base + o_at, splice_at, (size_t) n * 4, cudaMemcpyHostToDevice, st));
-            step(cudaMemcpyAsync(base + o_del, del_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+    if (edits) {
+        if (!one_each) step(cudaMemcpyAsync(base + o_eoff, edit_off, (size_t) (n + 1) * 8, cudaMemcpyHostToDevice, st));
+        if (n_edits) {
+            step(cudaMemcpyAsync(base + o_at, edit_at, (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
+            step(cudaMemcpyAsync(base + o_del, edit_del, (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
+            if (!one_each)
+                step(cudaMemcpyAsync(base + o_dst, edit_dst.data(), (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
         }
-        step(cudaMemcpyAsync(base + o_ioff, ins_off, (size_t) (n + 1) * 8, cudaMemcpyHostToDevice, st));
+        step(cudaMemcpyAsync(base + o_ioff, ins_off, (size_t) (n_edits + 1) * 8, cudaMemcpyHostToDevice, st));
         if (n_ins) step(cudaMemcpyAsync(base + o_icode, ins_code, (size_t) n_ins, cudaMemcpyHostToDevice, st));
     }
     step(cudaEventRecord(ctx->ev[1], st));
@@ -873,12 +901,14 @@ static int seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int3
                 (const int32_t *) (base + o_spos), (const uint8_t *) (base + o_scode), S->d_poff.as<int64_t>(),
                 S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(), S->d_nmask.as<uint32_t>(),
                 S->d_blk_seq.as<int32_t>());
-        else if (ins_off)
-            extract_splice_kernel<<<(unsigned) grid, 256, 0, st>>>(
-                src->view(), (const int32_t *) base, (const int64_t *) (base + o_start), (const int32_t *) (base + o_at),
-                (const int32_t *) (base + o_del), (const int64_t *) (base + o_ioff), (const uint8_t *) (base + o_icode),
-                S->d_poff.as<int64_t>(), S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(),
-                S->d_nmask.as<uint32_t>(), S->d_blk_seq.as<int32_t>());
+        else if (edits)
+            extract_edits_kernel<<<(unsigned) grid, 256, 0, st>>>(
+                src->view(), (const int32_t *) base, (const int64_t *) (base + o_start),
+                one_each ? nullptr : (const int64_t *) (base + o_eoff), (const int32_t *) (base + o_at),
+                (const int32_t *) (base + o_del), (const int32_t *) (base + (one_each ? o_at : o_dst)),
+                (const int64_t *) (base + o_ioff), (const uint8_t *) (base + o_icode), S->d_poff.as<int64_t>(),
+                S->d_len.as<int32_t>(), n, n_blocks, S->d_codes.as<uint32_t>(), S->d_nmask.as<uint32_t>(),
+                S->d_blk_seq.as<int32_t>());
         else
             extract_pack_kernel<<<(unsigned) grid, 256, 0, st>>>(
                 src->view(), (const int32_t *) base, (const int64_t *) (base + o_start), S->d_poff.as<int64_t>(),
@@ -903,7 +933,7 @@ extern "C" {
 int msb_seqs_extract(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx,
                      const int64_t *start, const int64_t *end, msb_seqs **out) {
     return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
-                        out, "msb_seqs_extract");
+                        nullptr, out, "msb_seqs_extract");
 }
 
 int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
@@ -911,15 +941,24 @@ int msb_seqs_extract_subst(msb_ctx *ctx, const msb_seqs *src, int64_t n, const i
                            msb_seqs **out) {
     if (!sub_off) { set_error("msb_seqs_extract_subst: null substitution offsets"); return MSB_EINVAL; }
     return seqs_extract(ctx, src, n, src_idx, start, end, sub_off, sub_pos, sub_code, nullptr, nullptr, nullptr, nullptr,
-                        out, "msb_seqs_extract_subst");
+                        nullptr, out, "msb_seqs_extract_subst");
 }
 
 int msb_seqs_extract_splice(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
                             const int64_t *end, const int32_t *splice_at, const int32_t *del_len, const int64_t *ins_off,
                             const uint8_t *ins_code, msb_seqs **out) {
     if (!ins_off) { set_error("msb_seqs_extract_splice: null insertion offsets"); return MSB_EINVAL; }
-    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, splice_at, del_len, ins_off, ins_code,
-                        out, "msb_seqs_extract_splice");
+    // one edit per sequence (edit_off == nullptr)
+    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, nullptr, splice_at, del_len,
+                        ins_off, ins_code, out, "msb_seqs_extract_splice");
+}
+
+int msb_seqs_extract_edits(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
+                           const int64_t *end, const int64_t *edit_off, const int32_t *edit_at, const int32_t *edit_del,
+                           const int64_t *ins_off, const uint8_t *ins_code, msb_seqs **out) {
+    if (!edit_off || !ins_off) { set_error("msb_seqs_extract_edits: null edit offsets"); return MSB_EINVAL; }
+    return seqs_extract(ctx, src, n, src_idx, start, end, nullptr, nullptr, nullptr, edit_off, edit_at, edit_del, ins_off,
+                        ins_code, out, "msb_seqs_extract_edits");
 }
 
 int msb_seqs_window_ncount(msb_ctx *ctx, const msb_seqs *src, int64_t n, const int32_t *src_idx, const int64_t *start,
@@ -1747,45 +1786,47 @@ int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, i
     return MSB_OK;
 }
 
-int msb_scan_variants(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int32_t *core_start,
-                      const int32_t *core_len, int strand, int64_t *n_rows) {
-    if (!ctx || !M || !ref || !alt) { set_error("msb_scan_variants: null argument"); return MSB_EINVAL; }
-    if (ref->n != alt->n || ref->seq_off != alt->seq_off) {
-        set_error("msb_scan_variants: the ref and alt sets must hold sequences of the same lengths");
-        return MSB_EINVAL;
-    }
-    const int64_t n = ref->n;
-    if (n > 0 && (!core_start || !core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
-    for (int64_t i = 0; i < n; i++)
-        if (core_len[i] < 1) { set_error("msb_scan_variants: core outside its context"); return MSB_EINVAL; }
-    return msb_scan_variants_ex(ctx, M, ref, alt, core_start, core_len, core_len, strand, n_rows);
-}
+}  // extern "C"
 
-int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int32_t *core_start,
-                         const int32_t *ref_core_len, const int32_t *alt_core_len, int strand, int64_t *n_rows) {
-    if (!ctx || !M || !ref || !alt) { set_error("msb_scan_variants: null argument"); return MSB_EINVAL; }
-    if (ref->n != alt->n) { set_error("msb_scan_variants: the ref and alt sets must hold the same number of contexts"); return MSB_EINVAL; }
+// msb_scan_variants_ex / msb_scan_haplotypes: context i carries the edits [edit_off[i], edit_off[i + 1]), edit k
+// replacing the ref bases [at[k], at[k] + ref_len[k]) by alt_len[k] bases; edit_off == nullptr: one edit per context,
+// edit i (msb_scan_variants_ex: no offset table, no alt starts and no other-side starts on the device).  Checks the tables, runs the two scans and
+// the row kernel, and leaves the rows in order on the device.
+static int scan_edit_rows(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int64_t *edit_off,
+                          const int32_t *at, const int32_t *ref_len, const int32_t *alt_len, int strand, int64_t *n_rows,
+                          const char *what) {
     const int64_t n = ref->n;
-    if (n > 0 && (!core_start || !ref_core_len || !alt_core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
+    auto fail = [&](const char *msg) { set_error(std::string(what) + ": " + msg); return MSB_EINVAL; };
+    const bool one_each = edit_off == nullptr;
+    if (!one_each && edit_off[0] != 0) return fail("edit offsets must start at 0");
+    const int64_t n_edits = one_each ? n : edit_off[n];
+    std::vector<int32_t> alt_at((size_t) (one_each ? 0 : std::max<int64_t>(n_edits, 1)));
     int32_t max_len = 0;
     for (int64_t i = 0; i < n; i++) {
+        const int64_t e0 = one_each ? i : edit_off[i], e1 = one_each ? i + 1 : edit_off[i + 1];
+        if (e1 < e0) return fail("edit offsets not ascending");
         const int64_t len_r = ref->seq_off[i + 1] - ref->seq_off[i], len_a = alt->seq_off[i + 1] - alt->seq_off[i];
         max_len = std::max<int32_t>(max_len, (int32_t) std::max(len_r, len_a));
-        if (len_a - len_r != (int64_t) alt_core_len[i] - ref_core_len[i]) {
-            set_error("msb_scan_variants: a context's length change differs from its core's");
-            return MSB_EINVAL;
+        int64_t shift = 0, prev_end = 0;
+        for (int64_t k = e0; k < e1; k++) {
+            if (at[k] < 0 || ref_len[k] < 0 || alt_len[k] < 0 || std::max(ref_len[k], alt_len[k]) < 1 ||
+                (int64_t) at[k] + ref_len[k] > len_r || (int64_t) at[k] + shift + alt_len[k] > len_a)
+                return fail("core outside its context");
+            // an insertion occupies its junction: the next edit starts behind at + max(ref_len, 1)
+            if (k > e0 && at[k] < prev_end) return fail("edits out of order or overlapping");
+            if (!one_each) alt_at[(size_t) k] = (int32_t) (at[k] + shift);
+            shift += alt_len[k] - ref_len[k];
+            prev_end = (int64_t) at[k] + std::max(ref_len[k], 1);
         }
-        if (core_start[i] < 0 || ref_core_len[i] < 0 || alt_core_len[i] < 0 || std::max(ref_core_len[i], alt_core_len[i]) < 1 ||
-            (int64_t) core_start[i] + ref_core_len[i] > len_r || (int64_t) core_start[i] + alt_core_len[i] > len_a) {
-            set_error("msb_scan_variants: core outside its context");
-            return MSB_EINVAL;
-        }
+        if (len_a - len_r != shift) return fail("a context's length change differs from its edits'");
     }
     int seq_bits = 0, motif_bits = 0, start_bits = 0;
+    const int side_bits = n_edits > n ? 1 : 0;      // several edits in a context: ref and alt rows may share a start
     while ((1ll << seq_bits) < n) seq_bits++;
     while ((1ll << motif_bits) < (int64_t) M->n) motif_bits++;
     while ((1ll << start_bits) < (int64_t) max_len) start_bits++;
-    if (seq_bits + motif_bits + start_bits + 1 > 64) { set_error("msb_scan_variants: too many alleles x motifs x context bases for a 64-bit row key"); return MSB_EINVAL; }
+    if (seq_bits + motif_bits + start_bits + 1 + side_bits > 64)
+        return fail("too many contexts x motifs x context bases for a 64-bit row key");
     // the two scans: the ref sites stay in their final set while the alt scan fills the other one
     double t_pre = 0, t_exact = 0, t_order = 0;
     MSB_TRY(scan_device(ctx, const_cast<msb_motifs *>(M), ref, strand, 0));
@@ -1821,20 +1862,31 @@ int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref,
     MSB_TRY(ctx->vr_ref.ensure((size_t) cap * 8));
     MSB_TRY(ctx->vr_alt.ensure((size_t) cap * 8));
     MSB_TRY(ctx->vr_eff.ensure((size_t) cap));
-    MSB_TRY(ctx->vr_core.ensure((size_t) std::max<int64_t>(3 * n, 1) * 4));
-    if (n) {
-        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.p, core_start, (size_t) n * 4, cudaMemcpyHostToDevice, st));
-        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.as<int32_t>() + n, ref_core_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
-        MSB_CUDA(cudaMemcpyAsync(ctx->vr_core.as<int32_t>() + 2 * n, alt_core_len, (size_t) n * 4, cudaMemcpyHostToDevice, st));
+    if (!one_each) MSB_TRY(ctx->vr_other.ensure((size_t) cap * 4));
+    // device edit table: at | ref len | alt len [| alt at]
+    MSB_TRY(ctx->vr_core.ensure((size_t) std::max<int64_t>((one_each ? 3 : 4) * n_edits, 1) * 4));
+    int32_t *d_core = ctx->vr_core.as<int32_t>();
+    if (!one_each) {
+        MSB_TRY(ctx->vr_eoff.ensure((size_t) (n + 1) * 8));
+        MSB_CUDA(cudaMemcpyAsync(ctx->vr_eoff.p, edit_off, (size_t) (n + 1) * 8, cudaMemcpyHostToDevice, st));
     }
+    if (n_edits) {
+        MSB_CUDA(cudaMemcpyAsync(d_core, at, (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
+        MSB_CUDA(cudaMemcpyAsync(d_core + n_edits, ref_len, (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
+        MSB_CUDA(cudaMemcpyAsync(d_core + 2 * n_edits, alt_len, (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
+        if (!one_each)
+            MSB_CUDA(cudaMemcpyAsync(d_core + 3 * n_edits, alt_at.data(), (size_t) n_edits * 4, cudaMemcpyHostToDevice, st));
+    }
+    R.at = d_core; R.len = d_core + n_edits; A.len = d_core + 2 * n_edits; A.at = one_each ? d_core : d_core + 3 * n_edits;
+    const int64_t *d_eoff = one_each ? nullptr : ctx->vr_eoff.as<int64_t>();
+    int32_t *d_other = one_each ? nullptr : ctx->vr_other.as<int32_t>();
     MSB_CUDA(cudaMemsetAsync(ctx->counters.p, 0, sizeof(unsigned long long), st));
     MSB_CUDA(cudaEventRecord(ctx->ev[4], st));
     if (R.n + A.n) {
         variant_rows_kernel<<<(unsigned) ((R.n + A.n + 255) / 256), 256, 0, st>>>(
-            R, A, M->view(), ctx->vr_core.as<int32_t>(), ctx->vr_core.as<int32_t>() + n, ctx->vr_core.as<int32_t>() + 2 * n,
-            motif_bits, start_bits,
+            R, A, M->view(), d_eoff, motif_bits, start_bits, side_bits,
             ctx->counters.as<unsigned long long>(), ctx->vr_key.as<uint64_t>(), ctx->vr_idx.as<int32_t>(),
-            ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>());
+            ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>(), d_other);
         MSB_CUDA(cudaGetLastError());
         ctx->c[MSB_C_LAUNCHES]++;
     }
@@ -1842,7 +1894,7 @@ int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref,
     MSB_TRY(read_counters(ctx));
     const int64_t rows = (int64_t) ctx->h_counters[0];
     if (rows) {
-        // (allele, motif, start, strand) order: one radix sort of the row keys with the row index as the value
+        // (context, motif, start, strand, side) order: one radix sort of the row keys with the row index as the value
         MSB_TRY(ctx->vr_key_sorted.ensure((size_t) rows * 8));
         MSB_TRY(ctx->vr_idx_sorted.ensure((size_t) rows * 4));
         MSB_TRY(ctx->vo_allele.ensure((size_t) rows * 4));
@@ -1852,7 +1904,8 @@ int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref,
         MSB_TRY(ctx->vo_ref.ensure((size_t) rows * 8));
         MSB_TRY(ctx->vo_alt.ensure((size_t) rows * 8));
         MSB_TRY(ctx->vo_eff.ensure((size_t) rows));
-        const int end_bit = seq_bits + motif_bits + start_bits + 1;
+        if (!one_each) MSB_TRY(ctx->vo_other.ensure((size_t) rows * 4));
+        const int end_bit = seq_bits + motif_bits + start_bits + 1 + side_bits;
         size_t tmp_bytes = 0;
         MSB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, ctx->vr_key.as<uint64_t>(), ctx->vr_key_sorted.as<uint64_t>(),
                                                  ctx->vr_idx.as<int32_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, 0, end_bit, st));
@@ -1860,10 +1913,11 @@ int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref,
         MSB_CUDA(cub::DeviceRadixSort::SortPairs(ctx->sort_tmp.p, tmp_bytes, ctx->vr_key.as<uint64_t>(), ctx->vr_key_sorted.as<uint64_t>(),
                                                  ctx->vr_idx.as<int32_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, 0, end_bit, st));
         variant_gather_kernel<<<(unsigned) ((rows + 255) / 256), 256, 0, st>>>(
-            ctx->vr_key_sorted.as<uint64_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, motif_bits, start_bits,
-            ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>(), ctx->vo_allele.as<int32_t>(),
-            ctx->vo_motif.as<int32_t>(), ctx->vo_start.as<int32_t>(), ctx->vo_strand.as<int8_t>(), ctx->vo_ref.as<double>(),
-            ctx->vo_alt.as<double>(), ctx->vo_eff.as<int8_t>());
+            ctx->vr_key_sorted.as<uint64_t>(), ctx->vr_idx_sorted.as<int32_t>(), rows, motif_bits, start_bits, side_bits,
+            ctx->vr_ref.as<double>(), ctx->vr_alt.as<double>(), ctx->vr_eff.as<int8_t>(), d_other,
+            ctx->vo_allele.as<int32_t>(), ctx->vo_motif.as<int32_t>(), ctx->vo_start.as<int32_t>(), ctx->vo_strand.as<int8_t>(),
+            ctx->vo_ref.as<double>(), ctx->vo_alt.as<double>(), ctx->vo_eff.as<int8_t>(),
+            one_each ? nullptr : ctx->vo_other.as<int32_t>());
         MSB_CUDA(cudaGetLastError());
         ctx->c[MSB_C_LAUNCHES] += 2;
     }
@@ -1876,35 +1930,97 @@ int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref,
     ctx->t[MSB_T_ROW_SORT] = ev_ms(ctx->ev[5], ctx->ev[6]);
     ctx->t[MSB_T_D2H] = 0;
     ctx->last_variant_rows = rows;
+    ctx->last_rows_other = !one_each;
     if (n_rows) *n_rows = rows;
     return MSB_OK;
 }
 
-int msb_scan_device_variant_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *allele, int32_t *motif, int32_t *start,
-                                 int8_t *strand, double *ref_score, double *alt_score, int8_t *effect) {
-    if (!ctx || !n) { set_error("msb_scan_device_variant_rows: null"); return MSB_EINVAL; }
-    if (ctx->last_variant_rows < 0) { set_error("msb_scan_device_variant_rows: the last scan was not msb_scan_variants"); return MSB_EINVAL; }
+extern "C" {
+
+int msb_scan_variants(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int32_t *core_start,
+                      const int32_t *core_len, int strand, int64_t *n_rows) {
+    if (!ctx || !M || !ref || !alt) { set_error("msb_scan_variants: null argument"); return MSB_EINVAL; }
+    if (ref->n != alt->n || ref->seq_off != alt->seq_off) {
+        set_error("msb_scan_variants: the ref and alt sets must hold sequences of the same lengths");
+        return MSB_EINVAL;
+    }
+    const int64_t n = ref->n;
+    if (n > 0 && (!core_start || !core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
+    for (int64_t i = 0; i < n; i++)
+        if (core_len[i] < 1) { set_error("msb_scan_variants: core outside its context"); return MSB_EINVAL; }
+    return msb_scan_variants_ex(ctx, M, ref, alt, core_start, core_len, core_len, strand, n_rows);
+}
+
+int msb_scan_variants_ex(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int32_t *core_start,
+                         const int32_t *ref_core_len, const int32_t *alt_core_len, int strand, int64_t *n_rows) {
+    if (!ctx || !M || !ref || !alt) { set_error("msb_scan_variants: null argument"); return MSB_EINVAL; }
+    if (ref->n != alt->n) { set_error("msb_scan_variants: the ref and alt sets must hold the same number of contexts"); return MSB_EINVAL; }
+    const int64_t n = ref->n;
+    if (n > 0 && (!core_start || !ref_core_len || !alt_core_len)) { set_error("msb_scan_variants: null core table"); return MSB_EINVAL; }
+    // one edit per context (edit_off == nullptr)
+    return scan_edit_rows(ctx, M, ref, alt, nullptr, core_start, ref_core_len, alt_core_len, strand, n_rows,
+                          "msb_scan_variants");
+}
+
+int msb_scan_haplotypes(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *ref, const msb_seqs *alt, const int64_t *edit_off,
+                        const int32_t *edit_at, const int32_t *edit_ref_len, const int32_t *edit_alt_len, int strand,
+                        int64_t *n_rows) {
+    if (!ctx || !M || !ref || !alt || !edit_off) { set_error("msb_scan_haplotypes: null argument"); return MSB_EINVAL; }
+    if (ref->n != alt->n) { set_error("msb_scan_haplotypes: the ref and alt sets must hold the same number of contexts"); return MSB_EINVAL; }
+    if (edit_off[ref->n] > 0 && (!edit_at || !edit_ref_len || !edit_alt_len)) {
+        set_error("msb_scan_haplotypes: null edit table");
+        return MSB_EINVAL;
+    }
+    return scan_edit_rows(ctx, M, ref, alt, edit_off, edit_at, edit_ref_len, edit_alt_len, strand, n_rows, "msb_scan_haplotypes");
+}
+
+static int device_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *context, int32_t *motif, int32_t *start,
+                       int8_t *strand, double *ref_score, double *alt_score, int8_t *effect, int32_t *other_start,
+                       const char *what) {
+    if (!ctx || !n) { set_error(std::string(what) + ": null"); return MSB_EINVAL; }
+    if (ctx->last_variant_rows < 0) { set_error(std::string(what) + ": the last scan was not a variant scan"); return MSB_EINVAL; }
     const int64_t rows = ctx->last_variant_rows;
     *n = rows;
     if (rows == 0 || cap < rows) return MSB_OK;
-    if (!allele || !motif || !start || !strand || !ref_score || !alt_score || !effect) {
-        set_error("msb_scan_device_variant_rows: null array");
+    if (!context || !motif || !start || !strand || !ref_score || !alt_score || !effect) {
+        set_error(std::string(what) + ": null array");
         return MSB_EINVAL;
     }
     MSB_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     MSB_CUDA(cudaEventRecord(ctx->ev[0], st));
-    MSB_CUDA(cudaMemcpyAsync(allele, ctx->vo_allele.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(context, ctx->vo_allele.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaMemcpyAsync(motif, ctx->vo_motif.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaMemcpyAsync(start, ctx->vo_start.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaMemcpyAsync(strand, ctx->vo_strand.p, (size_t) rows, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaMemcpyAsync(ref_score, ctx->vo_ref.p, (size_t) rows * 8, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaMemcpyAsync(alt_score, ctx->vo_alt.p, (size_t) rows * 8, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaMemcpyAsync(effect, ctx->vo_eff.p, (size_t) rows, cudaMemcpyDeviceToHost, st));
+    if (other_start) MSB_CUDA(cudaMemcpyAsync(other_start, ctx->vo_other.p, (size_t) rows * 4, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaEventRecord(ctx->ev[1], st));
     MSB_CUDA(cudaStreamSynchronize(st));
     ctx->t[MSB_T_D2H] = ev_ms(ctx->ev[0], ctx->ev[1]);
     return MSB_OK;
+}
+
+int msb_scan_device_variant_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *allele, int32_t *motif, int32_t *start,
+                                 int8_t *strand, double *ref_score, double *alt_score, int8_t *effect) {
+    return device_rows(ctx, cap, n, allele, motif, start, strand, ref_score, alt_score, effect, nullptr,
+                       "msb_scan_device_variant_rows");
+}
+
+int msb_scan_device_haplotype_rows(msb_ctx *ctx, int64_t cap, int64_t *n, int32_t *context, int32_t *motif, int32_t *start,
+                                   int8_t *strand, double *ref_score, double *alt_score, int8_t *effect, int32_t *other_start) {
+    if (ctx && ctx->last_variant_rows >= 0 && !ctx->last_rows_other) {
+        set_error("msb_scan_device_haplotype_rows: the last scan was not msb_scan_haplotypes");
+        return MSB_EINVAL;
+    }
+    if (ctx && ctx->last_variant_rows > 0 && cap >= ctx->last_variant_rows && !other_start) {
+        set_error("msb_scan_device_haplotype_rows: null array");
+        return MSB_EINVAL;
+    }
+    return device_rows(ctx, cap, n, context, motif, start, strand, ref_score, alt_score, effect, other_start,
+                       "msb_scan_device_haplotype_rows");
 }
 
 int msb_scan_ranges_device(msb_ctx *ctx, const msb_motifs *M, const msb_seqs *S, int strand, int flags,
@@ -2569,6 +2685,62 @@ int msb_write_sites_bed(const char *path, int64_t n, const int32_t *group, const
     return MSB_OK;
 }
 
+}  // extern "C"
+
+// The end of a variant / haplotype table row: strand, ref_score, alt_score (printed like Python's str(); effect 6 has
+// no ref window and 5 no alt window, the missing score is NA) and the effect name.
+static const size_t kRowTailMax = 64;            // 2 + 2 x (1 + 25) + 6 bytes at most
+static char *fmt_row_tail(char *o, int8_t strand, double ref_score, double alt_score, int eff) {
+    static const char *const kEffect[4] = {"", "loss", "gain", "both"};
+    *o++ = '\t'; *o++ = strand == 1 ? '+' : '-';
+    *o++ = '\t';
+    if (eff == 6) { std::memcpy(o, "NA", 2); o += 2; } else o += py_float_str(ref_score, o);
+    *o++ = '\t';
+    if (eff == 5) { std::memcpy(o, "NA", 2); o += 2; } else o += py_float_str(alt_score, o);
+    *o++ = '\t';
+    std::memcpy(o, kEffect[eff & 3], 4); o += 4;
+    *o++ = '\n';
+    return o;
+}
+
+static bool row_effect_ok(int8_t eff) { return eff >= 1 && eff <= 6 && eff != 4; }
+
+// Writes `header` then n rows, row i formatted by row(i, o) (returns the end; at most line_max bytes) in blocks on up
+// to n_threads host threads, written in order (msb_write_sites_bed's scheme).
+template <class Row>
+static int write_table_rows(const char *path, const char *header, int64_t n, size_t line_max, int32_t n_threads, Row row,
+                            const char *what) {
+    FILE *f = std::fopen(path, "wb");
+    if (!f) { set_error(std::string(what) + ": cannot open " + path); return MSB_EINVAL; }
+    bool io_ok = true;
+    if (header) {
+        const size_t hn = std::strlen(header);
+        io_ok = std::fwrite(header, 1, hn, f) == hn;
+    }
+    const int nt = std::max(1, std::min<int>(n_threads, 64));
+    const int64_t block = 1 << 17;
+    std::vector<std::vector<char>> buf((size_t) nt);
+    std::vector<size_t> used((size_t) nt);
+    try { for (auto &b : buf) b.resize((size_t) std::min(n, block) * line_max); }
+    catch (const std::bad_alloc &) { std::fclose(f); set_error("out of host memory"); return MSB_ENOMEM; }
+    for (int64_t r0 = 0; r0 < n && io_ok; r0 += block * nt) {
+        auto format = [&](int t) {
+            const int64_t a = std::min(n, r0 + block * t), b = std::min(n, a + block);
+            char *o = buf[t].data();
+            for (int64_t i = a; i < b; i++) o = row(i, o);
+            used[t] = (size_t) (o - buf[t].data());
+        };
+        run_threads(nt, format);
+        for (int t = 0; t < nt && io_ok; t++)
+            if (used[t] && std::fwrite(buf[t].data(), 1, used[t], f) != used[t]) io_ok = false;
+    }
+    if (std::fclose(f) != 0) io_ok = false;
+    if (!io_ok) { set_error(std::string(what) + ": write to " + path + " failed"); return MSB_EINVAL; }
+    return MSB_OK;
+}
+
+extern "C" {
+
 int msb_write_variant_table(const char *path, const char *header, int64_t n, const int32_t *allele, const int32_t *motif,
                             const int32_t *start, const int8_t *strand, const double *ref_score, const double *alt_score,
                             const int8_t *effect, int64_t n_alleles, const char *lead, const int64_t *lead_off, int32_t n_motifs,
@@ -2582,58 +2754,59 @@ int msb_write_variant_table(const char *path, const char *header, int64_t n, con
     for (int64_t a = 0; a < n_alleles; a++) lead_max = std::max<size_t>(lead_max, (size_t) (lead_off[a + 1] - lead_off[a]));
     for (int32_t m = 0; m < n_motifs; m++) motif_max = std::max<size_t>(motif_max, (size_t) (motif_off[m + 1] - motif_off[m]));
     for (int64_t i = 0; i < n; i++)
-        if (allele[i] < 0 || allele[i] >= n_alleles || motif[i] < 0 || motif[i] >= n_motifs || effect[i] < 1 || effect[i] > 6 || effect[i] == 4) {
+        if (allele[i] < 0 || allele[i] >= n_alleles || motif[i] < 0 || motif[i] >= n_motifs || !row_effect_ok(effect[i])) {
             set_error("msb_write_variant_table: row refers to an unknown allele, motif or effect");
             return MSB_EINVAL;
         }
-    FILE *f = std::fopen(path, "wb");
-    if (!f) { set_error(std::string("msb_write_variant_table: cannot open ") + path); return MSB_EINVAL; }
-    bool io_ok = true;
-    if (header) {
-        const size_t hn = std::strlen(header);
-        io_ok = std::fwrite(header, 1, hn, f) == hn;
+    auto row = [&](int64_t i, char *o) {
+        const int32_t al = allele[i], m = motif[i];
+        const size_t ln = (size_t) (lead_off[al + 1] - lead_off[al]), mn = (size_t) (motif_off[m + 1] - motif_off[m]);
+        std::memcpy(o, lead + lead_off[al], ln); o += ln;
+        std::memcpy(o, motif_text + motif_off[m], mn); o += mn;
+        o += fmt_int(start[i], o);
+        *o++ = '\t'; o += fmt_int((int64_t) start[i] + motif_len[m], o);
+        return fmt_row_tail(o, strand[i], ref_score[i], alt_score[i], effect[i]);
+    };
+    return write_table_rows(path, header, n, lead_max + motif_max + 2 * 22 + kRowTailMax, n_threads, row,
+                            "msb_write_variant_table");
+}
+
+int msb_write_haplotype_table(const char *path, const char *header, int64_t n, const int32_t *cluster, const int32_t *motif,
+                              const int64_t *ref_start, const int64_t *alt_start, const int8_t *strand, const double *ref_score,
+                              const double *alt_score, const int8_t *effect, int64_t n_clusters, const char *lead,
+                              const int64_t *lead_off, int32_t n_motifs, const char *motif_text, const int64_t *motif_off,
+                              const int32_t *motif_len, int32_t n_threads) {
+    if (!path || n < 0 || n_clusters < 0 || n_motifs < 0 || !lead_off || !motif_off || (n_motifs && !motif_len) ||
+        (n && (!cluster || !motif || !ref_start || !alt_start || !strand || !ref_score || !alt_score || !effect))) {
+        set_error("msb_write_haplotype_table: bad argument");
+        return MSB_EINVAL;
     }
-    // blocks of rows formatted on host threads, written in order (msb_write_sites_bed's scheme)
-    const int nt = std::max(1, std::min<int>(n_threads, 64));
-    const int64_t block = 1 << 17;
-    const size_t line_max = lead_max + motif_max + 2 * 21 + 2 * 25 + 16;
-    std::vector<std::vector<char>> buf((size_t) nt);
-    std::vector<size_t> used((size_t) nt);
-    try { for (auto &b : buf) b.resize((size_t) std::min(n, block) * line_max); }
-    catch (const std::bad_alloc &) { std::fclose(f); set_error("out of host memory"); return MSB_ENOMEM; }
-    // effect 5 / 6: a loss / gain with no window on the other allele (an indel), its score written as NA
-    static const char *const kEffect[4] = {"", "loss", "gain", "both"};
-    for (int64_t r0 = 0; r0 < n && io_ok; r0 += block * nt) {
-        auto format = [&](int t) {
-            const int64_t a = std::min(n, r0 + block * t), b = std::min(n, a + block);
-            char *o = buf[t].data();
-            for (int64_t i = a; i < b; i++) {
-                const int32_t al = allele[i], m = motif[i];
-                const size_t ln = (size_t) (lead_off[al + 1] - lead_off[al]), mn = (size_t) (motif_off[m + 1] - motif_off[m]);
-                std::memcpy(o, lead + lead_off[al], ln); o += ln;
-                std::memcpy(o, motif_text + motif_off[m], mn); o += mn;
-                o += fmt_int(start[i], o);
-                *o++ = '\t'; o += fmt_int((int64_t) start[i] + motif_len[m], o);
-                *o++ = '\t'; *o++ = strand[i] == 1 ? '+' : '-';
-                const int eff = effect[i];
-                *o++ = '\t';
-                if (eff == 6) { std::memcpy(o, "NA", 2); o += 2; } else o += py_float_str(ref_score[i], o);
-                *o++ = '\t';
-                if (eff == 5) { std::memcpy(o, "NA", 2); o += 2; } else o += py_float_str(alt_score[i], o);
-                *o++ = '\t';
-                const char *e = kEffect[eff & 3];
-                std::memcpy(o, e, 4); o += 4;
-                *o++ = '\n';
-            }
-            used[t] = (size_t) (o - buf[t].data());
-        };
-        run_threads(nt, format);
-        for (int t = 0; t < nt && io_ok; t++)
-            if (used[t] && std::fwrite(buf[t].data(), 1, used[t], f) != used[t]) io_ok = false;
-    }
-    if (std::fclose(f) != 0) io_ok = false;
-    if (!io_ok) { set_error(std::string("msb_write_variant_table: write to ") + path + " failed"); return MSB_EINVAL; }
-    return MSB_OK;
+    size_t lead_max = 0, motif_max = 0;
+    for (int64_t c = 0; c < n_clusters; c++) lead_max = std::max<size_t>(lead_max, (size_t) (lead_off[c + 1] - lead_off[c]));
+    for (int32_t m = 0; m < n_motifs; m++) motif_max = std::max<size_t>(motif_max, (size_t) (motif_off[m + 1] - motif_off[m]));
+    for (int64_t i = 0; i < n; i++)
+        if (cluster[i] < 0 || cluster[i] >= n_clusters || motif[i] < 0 || motif[i] >= n_motifs || !row_effect_ok(effect[i])) {
+            set_error("msb_write_haplotype_table: row refers to an unknown cluster, motif or effect");
+            return MSB_EINVAL;
+        }
+    auto window = [](int64_t s, int32_t len, char *o) {                 // [s, s + len), or NA NA when s < 0
+        if (s < 0) { std::memcpy(o, "NA\tNA", 5); return o + 5; }
+        o += fmt_int(s, o);
+        *o++ = '\t';
+        return o + fmt_int(s + len, o);
+    };
+    auto row = [&](int64_t i, char *o) {
+        const int32_t c = cluster[i], m = motif[i];
+        const size_t ln = (size_t) (lead_off[c + 1] - lead_off[c]), mn = (size_t) (motif_off[m + 1] - motif_off[m]);
+        std::memcpy(o, lead + lead_off[c], ln); o += ln;
+        std::memcpy(o, motif_text + motif_off[m], mn); o += mn;
+        o = window(ref_start[i], motif_len[m], o);
+        *o++ = '\t';
+        o = window(alt_start[i], motif_len[m], o);
+        return fmt_row_tail(o, strand[i], ref_score[i], alt_score[i], effect[i]);
+    };
+    return write_table_rows(path, header, n, lead_max + motif_max + 4 * 22 + kRowTailMax, n_threads, row,
+                            "msb_write_haplotype_table");
 }
 
 int msb_text_free(char *text) {

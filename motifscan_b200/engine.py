@@ -273,6 +273,34 @@ class SequenceSet:
                                                     ctypes.byref(h)))
         return SequenceSet(self.ctx, _handle=h)
 
+    def extract_edits(self, src_idx, start, end, edit_off, edit_at, edit_del, ins_off, ins_code):
+        """`extract` with several edits per sequence (msb_seqs_extract_edits): edit k in [edit_off[i], edit_off[i + 1])
+        of sequence i replaces its bases [edit_at[k], edit_at[k] + edit_del[k]) (relative to the interval) by the A/C/G/T
+        codes ins_code[ins_off[k] .. ins_off[k + 1]) (0..3).  The edits of a sequence are ordered and do not overlap.
+        Only the interval and edit tables cross PCIe."""
+        src_idx = np.ascontiguousarray(np.asarray(src_idx, dtype=np.int32))
+        start = np.ascontiguousarray(np.asarray(start, dtype=np.int64))
+        end = np.ascontiguousarray(np.asarray(end, dtype=np.int64))
+        edit_off = np.ascontiguousarray(np.asarray(edit_off, dtype=np.int64))
+        edit_at = np.ascontiguousarray(np.asarray(edit_at, dtype=np.int32))
+        edit_del = np.ascontiguousarray(np.asarray(edit_del, dtype=np.int32))
+        ins_off = np.ascontiguousarray(np.asarray(ins_off, dtype=np.int64))
+        ins_code = np.ascontiguousarray(np.asarray(ins_code, dtype=np.uint8))
+        if not (src_idx.shape == start.shape == end.shape and src_idx.ndim == 1):
+            raise ValueError("src_idx, start and end must be 1-d arrays of one length")
+        if edit_off.shape != (len(src_idx) + 1,) or edit_at.shape != edit_del.shape or edit_at.shape != (int(edit_off[-1]),):
+            raise ValueError("edit_off must have n + 1 entries and edit_at / edit_del edit_off[-1]")
+        if ins_off.shape != (len(edit_at) + 1,) or ins_code.ndim != 1 or len(ins_code) != int(ins_off[-1]):
+            raise ValueError("ins_off must have one entry per edit + 1 and ins_code ins_off[-1]")
+        h = ctypes.c_void_p()
+        with self.ctx._lock:
+            check(self._lib.msb_seqs_extract_edits(self.ctx._h, self._h, len(src_idx), ptr(src_idx, ctypes.c_int32),
+                                                   ptr(start, ctypes.c_int64), ptr(end, ctypes.c_int64),
+                                                   ptr(edit_off, ctypes.c_int64), ptr(edit_at, ctypes.c_int32),
+                                                   ptr(edit_del, ctypes.c_int32), ptr(ins_off, ctypes.c_int64),
+                                                   ctypes.c_void_p(ins_code.ctypes.data), ctypes.byref(h)))
+        return SequenceSet(self.ctx, _handle=h)
+
     def window_ncount(self, src_idx, start, length):
         """Non-ACGT bases in each window [start[i], start[i] + length) of sequence src_idx[i]."""
         src_idx = np.ascontiguousarray(np.asarray(src_idx, dtype=np.int32))
@@ -609,17 +637,46 @@ def scan_variants_ex(ctx, motifs, ref, alt, core_start, ref_core_len, alt_core_l
         return _variant_rows(ctx, n.value)
 
 
-def _variant_rows(ctx, k):
-    """The k rows of the last variant scan on `ctx` (caller holds its lock)."""
+def scan_haplotypes(ctx, motifs, ref, alt, edit_off, edit_at, edit_ref_len, edit_alt_len, strand):
+    """scan_variants_ex with several edits per context (msb_scan_haplotypes): edit k in [edit_off[i], edit_off[i + 1])
+    of context i replaces the ref bases [edit_at[k], edit_at[k] + edit_ref_len[k]) by edit_alt_len[k] alt bases.  The
+    same row arrays with `context` for `allele`, `start` on the row's own side (alt for effect 2 / 6, else ref) and
+    `other_start`, the window's start on the other side (-1: none); rows in (context, motif, start, strand, ref before
+    alt) order."""
+    edit_off = np.ascontiguousarray(np.asarray(edit_off, dtype=np.int64))
+    edit_at = np.ascontiguousarray(np.asarray(edit_at, dtype=np.int32))
+    edit_ref_len = np.ascontiguousarray(np.asarray(edit_ref_len, dtype=np.int32))
+    edit_alt_len = np.ascontiguousarray(np.asarray(edit_alt_len, dtype=np.int32))
+    if edit_off.shape != (ref.n + 1,):
+        raise ValueError("edit_off must have one entry per context + 1")
+    if not edit_at.shape == edit_ref_len.shape == edit_alt_len.shape == (int(edit_off[-1]),):
+        raise ValueError("edit_at / edit_ref_len / edit_alt_len must have edit_off[-1] entries")
+    with ctx._lock:
+        n = ctypes.c_int64(0)
+        check(ctx._lib.msb_scan_haplotypes(ctx._h, motifs._h, ref._h, alt._h, ptr(edit_off, ctypes.c_int64),
+                                           ptr(edit_at, ctypes.c_int32), ptr(edit_ref_len, ctypes.c_int32),
+                                           ptr(edit_alt_len, ctypes.c_int32), int(strand), ctypes.byref(n)))
+        out = _variant_rows(ctx, n.value, other=True)
+    out["context"] = out.pop("allele")
+    return out
+
+
+def _variant_rows(ctx, k, other=False):
+    """The k rows of the last variant scan on `ctx` (caller holds its lock); `other`: with other_start."""
     n = ctypes.c_int64(0)
     out = dict(allele=np.zeros(k, np.int32), motif=np.zeros(k, np.int32), start=np.zeros(k, np.int32),
                strand=np.zeros(k, np.int8), ref_score=np.zeros(k, np.float64), alt_score=np.zeros(k, np.float64),
                effect=np.zeros(k, np.int8))
+    if other:
+        out["other_start"] = np.zeros(k, np.int32)
     if k:
-        check(ctx._lib.msb_scan_device_variant_rows(
-            ctx._h, k, ctypes.byref(n), ptr(out["allele"], ctypes.c_int32), ptr(out["motif"], ctypes.c_int32),
-            ptr(out["start"], ctypes.c_int32), ptr(out["strand"], ctypes.c_int8), ptr(out["ref_score"], ctypes.c_double),
-            ptr(out["alt_score"], ctypes.c_double), ptr(out["effect"], ctypes.c_int8)))
+        args = [ctx._h, k, ctypes.byref(n), ptr(out["allele"], ctypes.c_int32), ptr(out["motif"], ctypes.c_int32),
+                ptr(out["start"], ctypes.c_int32), ptr(out["strand"], ctypes.c_int8), ptr(out["ref_score"], ctypes.c_double),
+                ptr(out["alt_score"], ctypes.c_double), ptr(out["effect"], ctypes.c_int8)]
+        if other:
+            check(ctx._lib.msb_scan_device_haplotype_rows(*args, ptr(out["other_start"], ctypes.c_int32)))
+        else:
+            check(ctx._lib.msb_scan_device_variant_rows(*args))
     return out
 
 

@@ -235,6 +235,73 @@ def write_variant_tables(output_dir, pwms, variants, sites):
                       f"{int(summary['n_both'][m])}\n")
 
 
+HAPLOTYPE_SITES_HEADER = ("chrom\tcluster\tids\tmotif_id\tmotif_name\tref_start\tref_end\talt_start\talt_end\tstrand\t"
+                          "ref_score\talt_score\teffect\n")
+HAPLOTYPE_CLUSTERS_HEADER = "cluster\tchrom\talleles\tids\tcarriers\n"
+HAPLOTYPE_SUMMARY_HEADER = "motif_id\tmotif_name\tn_gain\tn_loss\tn_both\thap_gain\thap_loss\thap_both\n"
+
+
+def write_haplotype_tables(output_dir, pwms, haplotypes, sites):
+    """The three tables of `motifscan variant --haplotypes` (variants.scan_haplotypes):
+
+        motif_haplotype_sites.xls     one row per (cluster, motif, window pair, strand) that is a site on at least one
+                                      side: chrom, cluster, the alleles' IDs (comma-separated), motif id and name, the
+                                      window on the chromosome [ref_start, ref_end) and on the haplotype [alt_start,
+                                      alt_end) (0-based half-open; NA NA where it has none), strand, both scores (NA
+                                      where there is no window) and the effect
+        motif_haplotype_clusters.xls  per cluster: chrom, its alleles as POS:REF>ALT and their IDs (comma-separated),
+                                      and its carriers as sample:1 / sample:2 (first / second haplotype)
+        motif_haplotype_summary.xls   per motif, the clusters with at least one gain / loss / both row and the
+                                      haplotypes that carry such a cluster
+
+    The site rows are formatted by the library on host threads (msb_write_haplotype_table, shared with
+    msb_write_variant_table)."""
+    import ctypes
+    from . import _lib
+    lib = _lib.load()
+    os.makedirs(output_dir, exist_ok=True)
+    v, h = haplotypes.variants, haplotypes
+    ids = [",".join(v.id[a] for a in h.allele[h.allele_off[c]:h.allele_off[c + 1]].tolist()) for c in range(len(h))]
+    cluster = np.ascontiguousarray(sites.cluster, dtype=np.int32)
+    used, row_cluster = np.unique(cluster, return_inverse=True)        # leads only for clusters with a row
+    row_cluster = np.ascontiguousarray(row_cluster.reshape(-1), dtype=np.int32)
+    leads = [f"{v.chroms[h.chrom[c]]}\t{c}\t{ids[c]}\t".encode() for c in used.tolist()]
+    lead_off = np.zeros(len(leads) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in leads], out=lead_off[1:])
+    mtext = [f"{pwm.matrix_id}\t{pwm.name}\t".encode() for pwm in pwms]
+    motif_off = np.zeros(len(mtext) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in mtext], out=motif_off[1:])
+    motif_len = np.array([int(pwm.length) for pwm in pwms] or [0], dtype=np.int32)
+    n = len(cluster)
+    arrays = [(row_cluster, ctypes.c_int32), (np.ascontiguousarray(sites.motif, dtype=np.int32), ctypes.c_int32),
+              (np.ascontiguousarray(sites.ref_start, dtype=np.int64), ctypes.c_int64),
+              (np.ascontiguousarray(sites.alt_start, dtype=np.int64), ctypes.c_int64),
+              (np.ascontiguousarray(sites.strand, dtype=np.int8), ctypes.c_int8),
+              (np.ascontiguousarray(sites.ref_score, dtype=np.float64), ctypes.c_double),
+              (np.ascontiguousarray(sites.alt_score, dtype=np.float64), ctypes.c_double),
+              (np.ascontiguousarray(np.where(sites.paired, sites.effect, sites.effect | 4), dtype=np.int8), ctypes.c_int8)]
+    _lib.check(lib.msb_write_haplotype_table(
+        os.path.join(output_dir, "motif_haplotype_sites.xls").encode(), HAPLOTYPE_SITES_HEADER.encode(), n,
+        *[_lib.ptr(a, ct) if n else None for a, ct in arrays], len(leads), b"".join(leads),
+        _lib.ptr(lead_off, ctypes.c_int64), len(pwms), b"".join(mtext), _lib.ptr(motif_off, ctypes.c_int64),
+        _lib.ptr(motif_len, ctypes.c_int32), min(os.cpu_count() or 1, 32)))
+    with open(os.path.join(output_dir, "motif_haplotype_clusters.xls"), "w") as out:
+        out.write(HAPLOTYPE_CLUSTERS_HEADER)
+        for c in range(len(h)):
+            alleles = ",".join(f"{int(v.pos[a]) + 1}:{v.ref[a]}>{v.alt[a]}"
+                               for a in h.allele[h.allele_off[c]:h.allele_off[c + 1]].tolist())
+            k0, k1 = int(h.carrier_off[c]), int(h.carrier_off[c + 1])
+            carriers = ",".join(f"{v.samples[s]}:{x + 1}" for s, x in zip(h.carrier_sample[k0:k1].tolist(),
+                                                                           h.carrier_hap[k0:k1].tolist()))
+            out.write(f"{c}\t{v.chroms[h.chrom[c]]}\t{alleles}\t{ids[c]}\t{carriers}\n")
+    summary = sites.summary()
+    with open(os.path.join(output_dir, "motif_haplotype_summary.xls"), "w") as out:
+        out.write(HAPLOTYPE_SUMMARY_HEADER)
+        for m, pwm in enumerate(pwms):
+            out.write(f"{pwm.matrix_id}\t{pwm.name}\t" + "\t".join(
+                str(int(summary[k][m])) for k in ("n_gain", "n_loss", "n_both", "hap_gain", "hap_loss", "hap_both")) + "\n")
+
+
 def write_enrich_table(output_dir, enrichment_results):
     os.makedirs(output_dir, exist_ok=True)
     enrichment_results.sort(key=lambda res: (res.p_enriched, -res.fold_change))   # io/__init__.py:63
