@@ -378,12 +378,14 @@ def bench_enrich(args):
             "parity": {"regions_with_site_counts_identical_on_sample": bool(np.array_equal(got, want))}}
 
 
-def bench_cli(args):
+def bench_cli(args, pair_flags=False):
     """configs[4] through the command line: `python -m motifscan_b200 scan` on 200k target + 200k control 1 kb regions x
     1,900 motifs (20 of them 33-40 columns long), a synthetic genome directory with a packed-genome cache next to
     the FASTA; wall time and peak RSS of the whole process (region parsing, scans, both site tables -- 1,900 columns
     x 200,000 rows each -- and the enrichment table).  The first `--cpu-regions` rows of the tables are compared with
-    the reference pipeline (its extension on the CPU, its regrouping, de-duplication and writers restated)."""
+    the reference pipeline (its extension on the CPU, its regrouping, de-duplication and writers restated).
+    `pair_flags`: the same command with `--cooccur --spacing-anchor <first --anchors motifs> --spacing-max D` is run
+    alternately with the plain one; its other output files must be byte-identical to the plain run's."""
     import resource
     import shutil
     import subprocess
@@ -432,16 +434,31 @@ def bench_cli(args):
     cmd = [sys.executable, "-m", "motifscan_b200", "scan", "-i", os.path.join(root, "targets.bed"), "-c", os.path.join(root, "controls.bed"),
            "-m", mdir, "-g", gdir, "-o", out, "-w", "0", "-p", "1e-4", "--gpus", str(args.gpus)]
     runs = []
+    pair_out = os.path.join(root, "out_pairs")
+    pair_cmd = cmd[:cmd.index("-o")] + ["-o", pair_out] + cmd[cmd.index("-o") + 2:] + [
+        "--cooccur", "--spacing-anchor", ",".join(ids[:args.anchors]), "--spacing-max", str(args.spacing_max)]
+    pair_runs = []
     for _ in range(2):
-        shutil.rmtree(out, ignore_errors=True)
-        before = resource.getrusage(resource.RUSAGE_CHILDREN).ru_maxrss
-        t0 = time.perf_counter()
-        proc = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True)
-        dt = time.perf_counter() - t0
-        if proc.returncode != 0:
-            raise SystemExit("motifscan scan failed:\n" + proc.stderr[-2000:])
-        runs.append((dt, max(resource.getrusage(resource.RUSAGE_CHILDREN).ru_maxrss, before) / 1024.0))
+        for c, o, into in ((cmd, out, runs),) + (((pair_cmd, pair_out, pair_runs),) if pair_flags else ()):
+            shutil.rmtree(o, ignore_errors=True)
+            before = resource.getrusage(resource.RUSAGE_CHILDREN).ru_maxrss
+            t0 = time.perf_counter()
+            proc = subprocess.run(c, cwd=ROOT, capture_output=True, text=True)
+            dt = time.perf_counter() - t0
+            if proc.returncode != 0:
+                raise SystemExit("motifscan scan failed:\n" + proc.stderr[-2000:])
+            into.append((dt, max(resource.getrusage(resource.RUSAGE_CHILDREN).ru_maxrss, before) / 1024.0))
     wall_s, rss_mb = min(r[0] for r in runs), runs[-1][1]
+    pairs = None
+    if pair_flags:
+        import filecmp
+        common = sorted(os.listdir(out))
+        pairs = {"wall_s": min(r[0] for r in pair_runs), "runs_s": [r[0] for r in pair_runs],
+                 "plain_runs_s": [r[0] for r in runs], "command_extra": pair_cmd[len(cmd):],
+                 "new_files_bytes": {k: os.path.getsize(os.path.join(pair_out, k)) for k in sorted(os.listdir(pair_out))
+                                     if k not in common},
+                 "other_files_identical": all(filecmp.cmp(os.path.join(out, k), os.path.join(pair_out, k), shallow=False)
+                                              for k in common)}
     # parity sample: the first rows of the two tables vs the reference pipeline
     n = args.cpu_regions
     kind, ext = cpu_ext()
@@ -479,6 +496,8 @@ def bench_cli(args):
                                       "motif_lengths": [int(mats[k - 3].shape[1]) for k in cols[:8] if k >= 3]}
     sizes_out = {name: os.path.getsize(os.path.join(out, name)) for name in sorted(os.listdir(out))}
     shutil.rmtree(root, ignore_errors=True)
+    if pairs is not None:
+        return pairs
     return {"config": f"configs[4] through the CLI: motifscan scan, {args.regions} target + {args.regions} control 1 kb regions x {args.motifs} motifs "
                       f"(20 of 33-40 columns), genome {sum(pg.chrom_sizes.values())} bp with a packed cache, --gpus {args.gpus}",
             "metric": "wall seconds of the whole command (parse, scan, 2 site tables, enrichment table)", "wall_s": wall_s,
@@ -1007,9 +1026,142 @@ def bench_haplotypes(args):
                     "bases of both sides"}
 
 
+def _popc_peak():
+    """bench_micro/popc_peak.cu compiled into a temporary directory and run: the POPC issue rate of this GPU."""
+    import subprocess
+    import tempfile
+    with tempfile.TemporaryDirectory() as tmp:
+        exe = os.path.join(tmp, "popc_peak")
+        subprocess.run([os.environ.get("NVCC", "nvcc"), "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
+                        "-o", exe, os.path.join(ROOT, "bench_micro", "popc_peak.cu")], check=True)
+        return json.loads(subprocess.run([exe], check=True, capture_output=True, text=True).stdout.strip().splitlines()[-1])
+
+
+def bench_cooccur(args):
+    """`scan --cooccur --spacing-anchor` at the configs[4] size: target and control regions scanned in blocks, pair
+    counts and spacing histograms reduced on the device after each block's scan and summed, then the host statistics
+    and the native table writer.  Parity: the first --cpu-regions regions against the oracle, as integers."""
+    import subprocess
+    import tempfile
+    import oracle
+    from motifscan_b200 import engine, synth
+    from motifscan_b200 import io as msio
+    from motifscan_b200.cooccur import cooccur_table, spacing_rows
+    from motifscan_b200.motif import PositionWeightMatrix
+    ctx = engine.default_context(0)
+    _, pwms, ids = synth.motif_set(args.motifs, seed=2020, n_long=20)
+    motifs = engine.MotifSet(ctx, pwms)
+    lmax = max(p.shape[1] for p in pwms)
+    bblob, boff = synth.background_samples(100000, lmax, seed=1)
+    bg = engine.SequenceSet(ctx, blob=bblob, seq_off=boff)
+    cutoffs = np.around(engine.score_select(ctx, motifs, bg, 3, [int(100000 * 1e-4) - 1])[:, 0], 8)
+    bg.close()
+    motifs.set_cutoffs(cutoffs)
+    lengths = [p.shape[1] for p in pwms]
+    anchors = list(range(args.anchors))
+    D = args.spacing_max
+    sets = [synth.peak_set(args.regions, 1000, seed=seed) for seed in (200, 201)]
+    phases = ("prefilter", "exact", "order", "pairs", "spacing")
+
+    def scan_pairs(blob, off, spacing):
+        counts = np.zeros((args.motifs, args.motifs), dtype=np.int64)
+        hist = np.zeros((len(anchors), args.motifs, 2, 2 * D + 1), dtype=np.int64) if spacing else None
+        ms = dict.fromkeys(phases, 0.0)
+        word_pairs = 0
+        for a in range(0, args.regions, args.region_block):
+            b = min(args.regions, a + args.region_block)
+            sset = engine.SequenceSet(ctx, blob=blob[off[a]:off[b]], seq_off=off[a:b + 1] - off[a])
+            engine.scan_device(ctx, motifs, sset, 3, remove_dup=True)
+            counts += ctx.pair_counts(args.motifs, b - a)
+            if spacing:
+                hist += ctx.spacing(motifs, anchors, D)
+            t = ctx.timings()
+            for k in phases:
+                ms[k] += t[k] if (k != "spacing" or spacing) else 0.0
+            word_pairs += args.motifs * (args.motifs + 1) // 2 * ((b - a + 31) // 32)
+            sset.close()
+        return counts, hist, ms, word_pairs
+
+    runs = []
+    for _ in range(args.steps + 1):
+        t0 = time.perf_counter()
+        c_in, h_in, ms_in, wp = scan_pairs(*sets[0], True)
+        c_ctl, _, ms_ctl, _ = scan_pairs(*sets[1], False)
+        runs.append((time.perf_counter() - t0, ms_in, ms_ctl))
+    scan_s, ms_in, ms_ctl = min(runs[1:], key=lambda r: r[0])
+    t0 = time.perf_counter()
+    table = cooccur_table(c_in, args.regions, c_ctl, args.regions, n_threads=min(os.cpu_count() or 1, 16))
+    stats_s = time.perf_counter() - t0
+    t0 = time.perf_counter()
+    table1 = cooccur_table(c_in, args.regions, c_ctl, args.regions, n_threads=1)
+    stats_1t_s = time.perf_counter() - t0
+    same = all(np.array_equal(np.asarray(x).view(np.uint8), np.asarray(y).view(np.uint8)) for x, y in zip(table, table1))
+    objs = []
+    for k, p in enumerate(pwms):
+        objs.append(PositionWeightMatrix(p, name=f"TF{k}", matrix_id=ids[k]))
+    with tempfile.TemporaryDirectory() as tmp:
+        t0 = time.perf_counter()
+        msio.write_cooccur_table(tmp, objs, table)
+        write_s = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        rows = spacing_rows(h_in, anchors, lengths)
+        msio.write_spacing_table(tmp, objs, anchors, rows)
+        spacing_host_s = time.perf_counter() - t0
+        table_mb = os.path.getsize(os.path.join(tmp, "motif_cooccurrence.xls")) / 1e6
+    # parity: the first cpu_regions target regions, device vs oracle, as integers
+    n = args.cpu_regions
+    blob, off = sets[0]
+    seqs = strs(blob, off, range(n))
+    sset = engine.SequenceSet(ctx, blob=blob[:off[n]], seq_off=off[:n + 1])
+    engine.scan_device(ctx, motifs, sset, 3, remove_dup=True)
+    got_c = ctx.pair_counts(args.motifs, n)
+    got_h = ctx.spacing(motifs, anchors, D)
+    sset.close()
+    flat = oracle.c_scan_motif([p.tolist() for p in pwms], cutoffs.tolist(), seqs, 3, os.cpu_count() or 1)
+    nested = oracle.deduplicate_motif_sites(oracle.make_motif_sites(flat, [0] * n), lengths)
+    hit = [{r for r, cell in enumerate(per) if cell} for per in nested]
+    want_c = np.zeros_like(got_c)
+    for a_ in range(args.motifs):
+        for b_ in range(a_, args.motifs):
+            want_c[a_, b_] = want_c[b_, a_] = len(hit[a_] & hit[b_])
+    want_h = np.zeros_like(got_h)
+    for k, A in enumerate(anchors):
+        for r, cell in enumerate(nested[A]):
+            for sa in cell:
+                for B in range(args.motifs):
+                    for sb in nested[B][r]:
+                        if B == A and sb.start == sa.start and sb.strand == sa.strand:
+                            continue
+                        d = sb.start - sa.start if sa.strand == "+" else (sa.start + lengths[A]) - (sb.start + lengths[B])
+                        if -D <= d <= D:
+                            want_h[k, B, int(sa.strand != sb.strand), d + D] += 1
+    cli = bench_cli(args, pair_flags=True)
+    peak = _popc_peak()
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                          text=True).stdout.strip().splitlines()[0]
+    popc_rate = wp / (ms_in["pairs"] * 1e-3) if ms_in["pairs"] > 0 else None   # one POPC per word pair
+    return {"config": f"cooccur: {args.regions} target + {args.regions} control 1 kb regions x {args.motifs} motifs "
+                      f"(20 of 33-40 columns), blocks of {args.region_block} regions, --anchors {args.anchors} "
+                      f"--spacing-max {D}",
+            "card": card,
+            "device_ms_target": ms_in, "device_ms_control": ms_ctl,
+            "pairs_word_pairs_per_set": wp, "pairs_popc_per_s": popc_rate,
+            "popc_peak": peak,
+            "pairs_share_of_popc_peak": popc_rate and popc_rate / peak["popc_per_s"],
+            "scan_and_reduce_wall_s": scan_s,
+            "host_stats_s": stats_s, "host_stats_1thread_s": stats_1t_s, "threaded_stats_identical": bool(same),
+            "cooccur_writer_s": write_s, "cooccur_table_mb": table_mb, "spacing_rows_and_writer_s": spacing_host_s,
+            "spacing_rows": len(rows), "pair_rows": int(len(table.a)),
+            "cli_wall_s": {"plain": min(cli["plain_runs_s"]), "with_cooccur_and_spacing": cli["wall_s"], "runs": cli},
+            "parity": {"regions": n, "pair_counts_equal": bool(np.array_equal(got_c, want_c)),
+                       "spacing_equal": bool(np.array_equal(got_h, want_h)), "pairs_in_hist": int(want_h.sum()),
+                       "cells_with_both": int((want_c > 0).sum())}}
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants", "haplotypes"])
+    ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants", "haplotypes",
+                                          "cooccur"])
     ap.add_argument("--alleles", type=int, default=None)
     ap.add_argument("--samples", type=int, default=16)
     ap.add_argument("--cpu-clusters", dest="cpu_clusters", type=int, default=500)
@@ -1028,12 +1180,17 @@ def main():
     ap.add_argument("--cpu-bp", dest="cpu_bp", type=int, default=2000000)
     ap.add_argument("--regions", type=int, default=200000)
     ap.add_argument("--region-block", dest="region_block", type=int, default=50000)
-    ap.add_argument("--cpu-regions", dest="cpu_regions", type=int, default=4000)
+    ap.add_argument("--cpu-regions", dest="cpu_regions", type=int, default=None)
+    ap.add_argument("--anchors", type=int, default=4)
+    ap.add_argument("--spacing-max", dest="spacing_max", type=int, default=50)
     args = ap.parse_args()
     if args.motifs is None:
-        args.motifs = 1900 if args.which in ("enrich", "cli") else 750
+        args.motifs = 1900 if args.which in ("enrich", "cli", "cooccur") else 750
+    if args.cpu_regions is None:
+        args.cpu_regions = 2000 if args.which == "cooccur" else 4000
     out = {"build": bench_build, "genome": bench_genome, "enrich": bench_enrich, "cli": bench_cli,
-           "whole-genome": bench_whole_genome, "variants": bench_variants, "haplotypes": bench_haplotypes}[args.which](args)
+           "whole-genome": bench_whole_genome, "variants": bench_variants, "haplotypes": bench_haplotypes,
+           "cooccur": bench_cooccur}[args.which](args)
     if out is not None:
         print(json.dumps(out))
 

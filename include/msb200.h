@@ -62,9 +62,10 @@ int msb_ctx_create(int device, void *stream, msb_ctx **ctx);
 int msb_ctx_destroy(msb_ctx *ctx);
 int msb_ctx_sync(msb_ctx *ctx);
 /* Per-phase device times (ms, CUDA events on the context's stream) of the last msb_scan /
- * msb_score / msb_seqs_from_ascii on this context.  Index by MSB_T_*. */
+ * msb_score / msb_seqs_from_ascii on this context.  Index by MSB_T_*.  MSB_T_PAIRS and MSB_T_SPACING hold the
+ * last msb_scan_device_pair_counts / msb_scan_device_spacing. */
 enum { MSB_T_H2D = 0, MSB_T_ENCODE, MSB_T_PREFILTER, MSB_T_EXACT, MSB_T_ORDER, MSB_T_D2H,
-       MSB_T_SCORE, MSB_T_SELECT, MSB_T_ROWS, MSB_T_ROW_SORT, MSB_T_COUNT };
+       MSB_T_SCORE, MSB_T_SELECT, MSB_T_ROWS, MSB_T_ROW_SORT, MSB_T_PAIRS, MSB_T_SPACING, MSB_T_COUNT };
 int msb_ctx_timings(const msb_ctx *ctx, double *ms, int n);
 /* Counters of the last msb_scan: index by MSB_C_*. */
 enum { MSB_C_CANDIDATES = 0, MSB_C_DIRTY, MSB_C_HITS, MSB_C_LAUNCHES, MSB_C_RETRIES,
@@ -77,7 +78,10 @@ int msb_ctx_counters(const msb_ctx *ctx, int64_t *v, int n);
  * buffer on the first attempt (tests of the overflow retry; 0 = sized from the input); "poison_pool" 1 =
  * recycled device buffers are filled with 0xFF (tests: nothing may rely on stale contents); "tc_prof" 1
  * = per-role cycle counters of the tensor-core prefilter on stderr; "select_pilot" 0 = msb_score_select scores
- * every sample for every motif instead of the pilot + scan scheme (A/B tests). */
+ * every sample for every motif instead of the pilot + scan scheme (A/B tests); "pair_pass_words" words of each motif's
+ * sequence bits per pass of msb_scan_device_pair_counts (tests of the word-range passes; 0 = sized from a 256 MB
+ * budget); "pair_split_words" words each CTA of the pair-count kernel covers, rounded up to whole 32-word chunks (tests
+ * of CTAs that loop over several chunks; 0 = sized to fill every SM). */
 int msb_ctx_set_option(msb_ctx *ctx, const char *name, int value);
 
 /* Pinned host memory for callers that want full-speed H2D (cudaHostAlloc / cudaFreeHost). */
@@ -241,6 +245,21 @@ int msb_scan_device_boundary_sites(msb_ctx *ctx, int64_t cap, int64_t *n, int32_
  * the device: counts[m * n_seqs + s] = number of final sites, best[...] = their best score (NaN when empty).
  * n_seqs must be the scanned set's sequence count.  Not after MSB_SCAN_COUNTS or a compact scan. */
 int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, int64_t *counts, double *best);
+/* Motif co-occurrence of the last msb_scan_device / msb_scan_ranges_device / msb_scan / msb_scan_ascii on this context:
+ * counts[a * n_motifs + b] = number of sequences with at least one final site of motif a and one of motif b (the full
+ * symmetric matrix; the diagonal is msb_scan_device_region_counts).  Computed as popc(H . H^T) of the (motif, sequence)
+ * bit matrix H, in word-range passes of at most 256 MB of H.  n_motifs / n_seqs must be the last scan's, which must
+ * have kept its sites (not MSB_SCAN_COUNTS, not compact): MSB_EINVAL otherwise.  MSB_T_PAIRS times it. */
+int msb_scan_device_pair_counts(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, int64_t *counts);
+/* Spacing histograms of the same sites around n_anchors (1..16) anchor motifs: for every ordered pair of distinct final
+ * sites in one sequence, the anchor (motif A = anchors[k], start sA, strand tA, length LA) and a partner (motif B, sB, tB,
+ * LB), the offset in the anchor's frame is d = sB - sA for a forward anchor and d = (sA + LA) - (sB + LB) for a reverse
+ * one; pairs with |d| <= max_offset (0..500) are counted in hist[((k * n_motifs + B) * 2 + (tA != tB)) * (2 max_offset +
+ * 1) + d + max_offset] (orientation 0 same strand, 1 opposite; overlapping windows included).  `motifs` gives the
+ * lengths and must have the last scan's motif count.  MSB_EINVAL for an anchor out of range, the ranges above or the
+ * last-scan states of msb_scan_device_pair_counts.  MSB_T_SPACING times it. */
+int msb_scan_device_spacing(msb_ctx *ctx, const msb_motifs *motifs, int32_t n_anchors, const int32_t *anchors,
+                            int32_t max_offset, int64_t *hist);
 /* Variant-effect scan.  Sequence i of `ref` is allele i's context on the reference genome, sequence i of `alt` the
  * same bases with the allele substituted (msb_seqs_extract / msb_seqs_extract_subst: equal lengths); the changed
  * bases are [core_start[i], core_start[i] + core_len[i]) of it.  Both sets are scanned (msb_scan_device without
@@ -363,6 +382,17 @@ int msb_write_haplotype_table(const char *path, const char *header, int64_t n, c
                               const double *alt_score, const int8_t *effect, int64_t n_clusters, const char *lead,
                               const int64_t *lead_off, int32_t n_motifs, const char *motif_text, const int64_t *motif_off,
                               const int32_t *motif_len, int32_t n_threads);
+/* motif_cooccurrence.xls written to `path`, formatted like msb_write_variant_table: `header` (may be NULL), then per row i,
+ * in the given order, motif_text[motif_off[m] .. motif_off[m + 1]) of motif_a[i] and of motif_b[i] ("id,name"), the
+ * region counts n_single[a], n_single[b] and n_both[i], then expected, ratio, p_cooccur, p_exclusive and q_cooccur
+ * (printed like Python's str()), then n_both_control, fold_change, p_enriched, p_depleted and p_corrected -- or five NA
+ * when n_both_control is NULL -- tab-separated, "\n". */
+int msb_write_cooccur_table(const char *path, const char *header, int64_t n, const int32_t *motif_a, const int32_t *motif_b,
+                            int32_t n_motifs, const char *motif_text, const int64_t *motif_off, const int64_t *n_single,
+                            const int64_t *n_both, const double *expected, const double *ratio, const double *p_cooccur,
+                            const double *p_exclusive, const double *q_cooccur, const int64_t *n_both_control,
+                            const double *fold_change, const double *p_enriched, const double *p_depleted,
+                            const double *p_corrected, int32_t n_threads);
 int msb_text_free(char *text);
 
 /* ---- score (replaces motif_score_thread + motif_score, cscore.c:174-302) -------------------- */

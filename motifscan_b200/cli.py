@@ -25,7 +25,14 @@ Same flags as the reference's subcommands (cli/main.py:407-430, 504-579) and the
     insertions and deletions too, as the VCF places them (normalise it first); `--haplotypes` reads the phased
     genotypes and scans the alleles each haplotype carries within a motif width of each other together;
 
+  * `scan --cooccur` (not in the reference) also writes motif_cooccurrence.xls: for every motif pair, the regions with
+    sites of both, tested for co-occurrence and mutual exclusion within the input and, unless --no-enrich, against the
+    control regions; `scan --spacing-anchor ID[,ID...] [--spacing-max D]` writes motif_spacing.xls: per anchor motif,
+    partner motif and orientation, the partner sites at offsets -D..D of the anchor's sites (default D = 50) and the
+    most enriched non-overlapping offset (motifscan_b200/cooccur.py).  Both are errors with --whole-genome;
+
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir
+    python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir --cooccur --spacing-anchor MA0099.3
     python -m motifscan_b200 scan --whole-genome -m <motif set> -g <genome> -o out_dir [--site]
     python -m motifscan_b200 motif --build <motif set> -g <genome>
     python -m motifscan_b200 variant -i calls.vcf.gz -m <motif set> -g <genome> -o out_dir [--indels]
@@ -39,6 +46,7 @@ from configparser import ConfigParser
 
 from . import io as msio
 from .builder import build_cutoffs
+from .cooccur import PairSpec, cooccur_table, spacing_rows
 from .genome import Genome
 from .motif import MotifPwms, PositionWeightMatrix, pfm_to_pwm, read_jaspar_pfms
 from .region import REGION_FORMATS, generate_control_regions, load_motifscan_regions
@@ -151,9 +159,11 @@ def run_scan(args):
         raise SystemExit("motifscan scan: error: give exactly one of -i and --whole-genome")
     if args.whole_genome:
         for flag, given in (("-c", args.control_file is not None), ("--cf", args.control_format_given),
-                            ("--loc", args.location is not None)):
+                            ("--loc", args.location is not None), ("--cooccur", args.cooccur),
+                            ("--spacing-anchor", args.spacing_anchor is not None)):
             if given:
-                raise SystemExit(f"motifscan scan: error: {flag} has no meaning with --whole-genome (no enrichment)")
+                raise SystemExit(f"motifscan scan: error: {flag} has no meaning with --whole-genome (no enrichment, and a "
+                                 "chromosome is not a region to co-occur in)")
         if args.plot_dist:
             raise SystemExit("motifscan scan: --plot needs matplotlib, which is out of scope here")
         return run_whole_genome(args)
@@ -164,6 +174,10 @@ def run_scan(args):
     logger.info("===== Loading data =====")
     genome = load_genome(args.genome)
     pwms = load_built_pwms(args.motif, genome.name)
+    anchors = resolve_anchors(pwms, args.spacing_anchor) if args.spacing_anchor is not None else []
+    pairs = None
+    if args.cooccur or anchors:
+        pairs = PairSpec(cooccur=args.cooccur, anchors=anchors, max_offset=args.spacing_max)
     regions = load_motifscan_regions(args.input_file, args.input_format)
     logger.info("===== Scanning motifs =====")
     devices = _devices(args.n_gpus)
@@ -171,11 +185,15 @@ def run_scan(args):
     source = packed_genome(genome, window_bp * (1 if args.no_enrich else 2), devices[0]) or genome
     common = dict(genome=source, window_size=args.window_size, strand=args.strand, p_value=args.p_value,
                   remove_dup=True, n_threads=args.n_threads, devices=devices)
-    sites = Scanner(regions=regions, **common).scan_motifs(pwms)
+    sites = Scanner(regions=regions, **common).scan_motifs(pwms, pairs=pairs)
     logger.info("Saving the result tables")
     msio.write_sites_table(args.output_dir, pwms, regions, sites)
     if args.report_site:
         msio.write_sites_bed(args.output_dir, pwms, regions, sites)
+    if anchors:
+        rows = spacing_rows(sites.pairs.spacing, anchors, [int(p.length) for p in pwms])
+        msio.write_spacing_table(args.output_dir, pwms, anchors, rows)
+    control_pairs = None
     if not args.no_enrich:
         logger.info("===== Motif Enrichment =====")
         if args.control_file:
@@ -185,8 +203,21 @@ def run_scan(args):
                 logger.warning("gene annotation found but unused: control regions are drawn from the whole "
                                "background, not matched by gene distance as the reference does (out of scope)")
             controls = generate_control_regions(args.n_random, regions, genome.chrom_sizes, random_seed=args.seed)
-        control_sites = Scanner(regions=controls, **common).scan_motifs(pwms)
+        control_sites = Scanner(regions=controls, **common).scan_motifs(
+            pwms, pairs=PairSpec(cooccur=True) if args.cooccur else None)
         msio.write_enrich_table(args.output_dir, motif_enrichment(pwms, sites, control_sites))
+        control_pairs = control_sites.pairs
+    if args.cooccur:
+        import time
+        logger.info("===== Motif Co-occurrence =====")
+        t0 = time.perf_counter()
+        table = cooccur_table(sites.pairs.counts, sites.pairs.n_regions,
+                              control_pairs.counts if control_pairs else None,
+                              control_pairs.n_regions if control_pairs else None, n_threads=COOCCUR_THREADS)
+        t1 = time.perf_counter()
+        msio.write_cooccur_table(args.output_dir, pwms, table)
+        logger.info(f"Co-occurrence of {len(table.a)} motif pairs: statistics {t1 - t0:.3f} s, "
+                    f"table {time.perf_counter() - t1:.3f} s")
     logger.info("===== MotifScan Finished =====")
     return 0
 
@@ -289,6 +320,28 @@ def run_motif(args):
     return 0
 
 
+COOCCUR_THREADS = min(os.cpu_count() or 1, 16)   # the scipy calls release the GIL: chunks run in parallel
+
+
+def resolve_anchors(pwms, text):
+    """`--spacing-anchor ID[,ID...]` -> motif indices: each item is a matrix_id or a unique motif name."""
+    out = []
+    for item in (x.strip() for x in text.split(",")):
+        if not item:
+            continue
+        hits = [i for i, p in enumerate(pwms) if p.matrix_id == item]
+        if not hits:
+            hits = [i for i, p in enumerate(pwms) if p.name == item]
+        if len(hits) != 1:
+            listed = ", ".join(f"{pwms[i].matrix_id},{pwms[i].name}" for i in hits)
+            what = "unknown" if not hits else f"ambiguous (matches {listed})"
+            raise SystemExit(f"motifscan scan: error: --spacing-anchor {item!r} is {what}")
+        out.append(hits[0])
+    if not 1 <= len(out) <= 16:
+        raise SystemExit("motifscan scan: error: --spacing-anchor takes 1 to 16 motifs")
+    return out
+
+
 def _devices(n_gpus):
     """`--gpus N`: the first N CUDA devices of this process (the reference's `-t` pool, cli/main.py:427-430,
     565-568, becomes one host thread per GPU); more than there are is an error, not a silent clamp."""
@@ -310,6 +363,13 @@ def _positive(text):
     value = int(text)
     if value <= 0:
         raise argparse.ArgumentTypeError(f"expect a positive integer, got {text!r}")
+    return value
+
+
+def _spacing_max(text):
+    value = int(text)
+    if not 0 <= value <= 500:
+        raise argparse.ArgumentTypeError(f"expect an integer in 0..500, got {text!r}")
     return value
 
 
@@ -342,6 +402,13 @@ def make_parser():
     scan.add_argument("-o", "--output-dir", dest="output_dir", required=True, metavar="DIR")
     scan.add_argument("--site", dest="report_site", action="store_true")
     scan.add_argument("--plot", dest="plot_dist", action="store_true")
+    scan.add_argument("--cooccur", action="store_true",
+                      help="write motif_cooccurrence.xls: regions with sites of both motifs, for every motif pair")
+    scan.add_argument("--spacing-anchor", dest="spacing_anchor", default=None, metavar="ID[,ID...]",
+                      help="write motif_spacing.xls: offsets of every motif's sites around these motifs' sites "
+                           "(matrix_id or unique name, up to 16)")
+    scan.add_argument("--spacing-max", dest="spacing_max", type=_spacing_max, default=50, metavar="D",
+                      help="largest |offset| of --spacing-anchor, 0..500 (default 50)")
     scan.add_argument("--verbose", action="store_true")
     scan.set_defaults(func=run_scan)
 

@@ -1052,4 +1052,138 @@ variant_gather_kernel(const uint64_t *__restrict__ key, const int32_t *__restric
     if (other_out) other_out[i] = other_in[j];
 }
 
+// ---------------------------------------------------------------------------------------------
+// Motif co-occurrence (msb_scan_device_pair_counts).  H is a bit matrix over (motif, sequence): row m holds the
+// words [w0, w0 + wp) of motif m's sequence bits, bit s % 32 of word s / 32 set when motif m has a site in
+// sequence s.  The final sites are sorted by (motif, sequence), so only the first site of a cell sets its bit.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+site_bits_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ seq_idx, int64_t n, int key_shift,
+                 int64_t w0, int64_t wp, uint32_t *__restrict__ H) {
+    const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t m = site_motif(key[i], key_shift);
+    const int32_t s = seq_idx[i];
+    if (i > 0 && site_motif(key[i - 1], key_shift) == m && seq_idx[i - 1] == s) return;
+    const int64_t w = (int64_t) (s >> 5) - w0;
+    if (w < 0 || w >= wp) return;
+    atomicOr(H + (int64_t) m * wp + w, 1u << (s & 31));
+}
+
+// C += popc(H . H^T) over the words of one pass: a bit-matrix SYRK on the CUDA cores, bound by POPC issue.  One CTA
+// per upper-triangular 128 x 128 tile of motifs (blockIdx.x, row-major over the triangle) and word split
+// (blockIdx.y).  32-word chunks of both row blocks are staged in shared memory (transposed, padded by one word so that
+// the staging stores do not conflict); each thread keeps an 8 x 8 register tile of uint32 counts (rows ty + 16 i,
+// columns tx + 16 j), whose inner loop is __popc(a & b), and adds it to C once.  A split covers at most 2^26 words, so
+// no count passes 2^31.  Only C[a][b] with a, b in an upper tile is written: the host mirrors the lower triangle.
+constexpr int kPairTile = 128, kPairK = 32;
+__global__ void __launch_bounds__(256, 2)
+pair_counts_kernel(const uint32_t *__restrict__ H, int32_t n_motifs, int64_t wp, int32_t n_tiles, int64_t k_split,
+                   unsigned long long *__restrict__ C) {
+    __shared__ uint32_t sa[kPairK][kPairTile + 1], sb[kPairK][kPairTile + 1];
+    int t = blockIdx.x, bi = 0;
+    while (t >= n_tiles - bi) { t -= n_tiles - bi; bi++; }
+    const int r0 = bi * kPairTile, c0 = (bi + t) * kPairTile;
+    const int64_t k0 = (int64_t) blockIdx.y * k_split, k1 = min(k0 + k_split, wp);
+    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    uint32_t acc[8][8];
+#pragma unroll
+    for (int i = 0; i < 8; i++)
+#pragma unroll
+        for (int j = 0; j < 8; j++) acc[i][j] = 0;
+    for (int64_t kc = k0; kc < k1; kc += kPairK) {
+        for (int idx = threadIdx.x; idx < kPairTile * kPairK; idx += blockDim.x) {
+            const int r = idx >> 5, k = idx & 31;
+            const int64_t kk = kc + k;
+            const int ra = r0 + r, rb = c0 + r;
+            sa[k][r] = (ra < n_motifs && kk < k1) ? __ldg(H + (int64_t) ra * wp + kk) : 0u;
+            sb[k][r] = (rb < n_motifs && kk < k1) ? __ldg(H + (int64_t) rb * wp + kk) : 0u;
+        }
+        __syncthreads();
+#pragma unroll 4
+        for (int k = 0; k < kPairK; k++) {
+            uint32_t a[8], b[8];
+#pragma unroll
+            for (int i = 0; i < 8; i++) { a[i] = sa[k][ty + 16 * i]; b[i] = sb[k][tx + 16 * i]; }
+#pragma unroll
+            for (int i = 0; i < 8; i++)
+#pragma unroll
+                for (int j = 0; j < 8; j++) acc[i][j] += __popc(a[i] & b[j]);
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < 8; i++)
+#pragma unroll
+        for (int j = 0; j < 8; j++) {
+            const int row = r0 + ty + 16 * i, col = c0 + tx + 16 * j;
+            if (row < n_motifs && col < n_motifs && acc[i][j])
+                atomicAdd(C + (int64_t) row * n_motifs + col, (unsigned long long) acc[i][j]);
+        }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Anchor spacing (msb_scan_device_spacing).  The final sites are re-keyed position-major, packed position <<
+// (motif_bits + 1) | motif << 1 | strand bit, and sorted with their sequence index as the value: all sites near a
+// position, of every motif, are then one contiguous run.  One warp per anchor site: it binary-searches the run's first
+// site and its lanes stride over the run; a partner in the same sequence at offset |d| <= D (in the anchor's frame)
+// is counted with a global atomic.  Within a sequence, differences of packed positions are differences of starts.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+position_keys_kernel(const uint64_t *__restrict__ key, int64_t n, int key_shift, int motif_bits, uint64_t *__restrict__ out) {
+    const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint64_t k = key[i];
+    out[i] = ((uint64_t) site_pos(k, key_shift) << (motif_bits + 1)) | ((uint64_t) site_motif(k, key_shift) << 1) | key_rev(k);
+}
+
+constexpr int kMaxSpacingAnchors = 16;
+struct SpacingAnchors {
+    int32_t n;
+    int32_t motif[kMaxSpacingAnchors];
+    int64_t seg[kMaxSpacingAnchors];            // first site of the anchor motif in the motif-major list
+    int64_t first[kMaxSpacingAnchors + 1];      // prefix sums of the anchors' site counts: warp w -> anchor
+};
+
+__global__ void __launch_bounds__(256)
+spacing_kernel(SpacingAnchors A, const uint64_t *__restrict__ key, const int32_t *__restrict__ seq_idx,
+               const uint64_t *__restrict__ pkey, const int32_t *__restrict__ pseq, int64_t n, int key_shift, int motif_bits,
+               const int32_t *__restrict__ mlen, int32_t lmax, int32_t n_motifs, int32_t D,
+               unsigned long long *__restrict__ hist) {
+    const int64_t w = ((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (w >= A.first[A.n]) return;
+    int a = 0;
+    while (w >= A.first[a + 1]) a++;
+    const int64_t i = A.seg[a] + (w - A.first[a]);
+    const uint64_t k = key[i];
+    const int64_t pA = site_pos(k, key_shift);
+    const uint32_t revA = key_rev(k);
+    const int32_t sq = seq_idx[i], mA = A.motif[a], LA = __ldg(mlen + mA);
+    // forward anchor: d = sB - sA; reverse: d = (sA + LA) - (sB + LB) with 1 <= LB <= lmax
+    const int64_t lo = revA ? pA + LA - lmax - D : pA - D;
+    const int64_t hi = revA ? pA + LA - 1 + D : pA + D;
+    const int sh = motif_bits + 1;
+    const uint64_t target = lo <= 0 ? 0ull : (uint64_t) lo << sh;
+    int64_t l = 0, h = n;
+    while (l < h) {
+        const int64_t mid = (l + h) >> 1;
+        if (__ldg(pkey + mid) < target) l = mid + 1; else h = mid;
+    }
+    const uint64_t self = ((uint64_t) pA << sh) | ((uint64_t) mA << 1) | revA;
+    const int64_t W = 2 * (int64_t) D + 1;
+    unsigned long long *ha = hist + (int64_t) a * n_motifs * 2 * W;
+    for (int64_t j = l + lane; j < n; j += 32) {
+        const uint64_t q = __ldg(pkey + j);
+        const int64_t pB = (int64_t) (q >> sh);
+        if (pB > hi) break;
+        if (q == self || __ldg(pseq + j) != sq) continue;
+        const int32_t mB = (int32_t) ((q >> 1) & ((1ull << motif_bits) - 1ull));
+        const uint32_t revB = (uint32_t) (q & 1ull);
+        const int64_t d = revA ? (pA + LA) - (pB + __ldg(mlen + mB)) : pB - pA;
+        if (d < -D || d > D) continue;
+        atomicAdd(ha + ((int64_t) mB * 2 + (revA != revB)) * W + (d + D), 1ull);
+    }
+}
+
 }  // namespace msb

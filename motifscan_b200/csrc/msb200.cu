@@ -128,6 +128,10 @@ struct msb_ctx {
     int opt_poison_pool = 0;         // tests: fill device buffers with 0xFF when they go back to the pool
     int opt_tc_interleave = 1;       // tensor-core prefilter: short and long motif tiles alternate (0: ascending by length)
     int opt_select_pilot = 1;        // msb_score_select: 0 = always score every sample for every motif (the plain form)
+    int opt_pair_pass_words = 0;     // tests: words per motif row in one pass of msb_scan_device_pair_counts (0 = 256 MB budget)
+    int opt_pair_split_words = 0;    // tests: words per CTA of pair_counts_kernel, rounded up to 32-word chunks (0 = sized to fill the SMs)
+    // msb_scan_device_pair_counts / msb_scan_device_spacing: bit matrix, counts / histogram, position-major sites
+    DevBuf pr_bits, pr_count, sp_key_in, sp_key, sp_seq;
 };
 
 // Tensor-core prefilter tables (prefilter_tc.cuh).
@@ -396,7 +400,8 @@ int msb_ctx_destroy(msb_ctx *ctx) {
                       &ctx->bnd_strand, &ctx->bnd_flags, &ctx->vr_key, &ctx->vr_idx, &ctx->vr_ref, &ctx->vr_alt,
                       &ctx->vr_eff, &ctx->vr_other, &ctx->vr_key_sorted, &ctx->vr_idx_sorted, &ctx->vr_core,
                       &ctx->vr_eoff, &ctx->vo_allele, &ctx->vo_motif, &ctx->vo_start, &ctx->vo_strand, &ctx->vo_ref,
-                      &ctx->vo_alt, &ctx->vo_eff, &ctx->vo_other})
+                      &ctx->vo_alt, &ctx->vo_eff, &ctx->vo_other, &ctx->pr_bits, &ctx->pr_count, &ctx->sp_key_in,
+                      &ctx->sp_key, &ctx->sp_seq})
         b->release();
     if (ctx->d2h_stream) cudaStreamSynchronize(ctx->d2h_stream);
     for (auto &f : ctx->fin) {
@@ -1689,6 +1694,8 @@ int msb_ctx_set_option(msb_ctx *ctx, const char *name, int value) {
     if (name && !std::strcmp(name, "poison_pool") && (value == 0 || value == 1)) { ctx->opt_poison_pool = value; return MSB_OK; }
     if (name && !std::strcmp(name, "tc_interleave") && (value == 0 || value == 1)) { ctx->opt_tc_interleave = value; return MSB_OK; }
     if (name && !std::strcmp(name, "select_pilot") && (value == 0 || value == 1)) { ctx->opt_select_pilot = value; return MSB_OK; }
+    if (name && !std::strcmp(name, "pair_pass_words") && value >= 0) { ctx->opt_pair_pass_words = value; return MSB_OK; }
+    if (name && !std::strcmp(name, "pair_split_words") && value >= 0) { ctx->opt_pair_split_words = value; return MSB_OK; }
     set_error("msb_ctx_set_option: unknown option or value");
     return MSB_EINVAL;
 }
@@ -1783,6 +1790,129 @@ int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, i
         const uint64_t k = keys[c], b = (k >> 63) ? (k & 0x7fffffffffffffffull) : ~k;   // order_key_inv
         std::memcpy(best + c, &b, 8);
     }
+    return MSB_OK;
+}
+
+// The last scan's final sites exist on the device in (motif, sequence, start) order (msb_scan_device_pair_counts /
+// msb_scan_device_spacing).
+static int check_final_sites(const msb_ctx *ctx, int32_t n_motifs, const char *what) {
+    if (n_motifs != ctx->last_n_motifs) { set_error(std::string(what) + ": no scan with that many motifs"); return MSB_EINVAL; }
+    if (ctx->last_counts_only) { set_error(std::string(what) + ": the last scan kept per-motif counts only (MSB_SCAN_COUNTS)"); return MSB_EINVAL; }
+    if (ctx->last_compact) { set_error(std::string(what) + ": the last scan kept compact sites (MSB_SCAN_COMPACT)"); return MSB_EINVAL; }
+    return MSB_OK;
+}
+
+static int motif_bits_of(int32_t n) {
+    int b = 1;
+    while ((1ll << b) < (int64_t) n) b++;
+    return b;
+}
+
+int msb_scan_device_pair_counts(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, int64_t *counts) {
+    if (!ctx || n_seqs < 0 || n_motifs < 0 || (!counts && n_motifs)) { set_error("msb_scan_device_pair_counts: null"); return MSB_EINVAL; }
+    MSB_TRY(check_final_sites(ctx, n_motifs, "msb_scan_device_pair_counts"));
+    if (n_seqs != ctx->last_n_seqs) { set_error("msb_scan_device_pair_counts: n_seqs differs from the scanned set"); return MSB_EINVAL; }
+    const size_t cells = (size_t) n_motifs * (size_t) n_motifs;
+    if (cells == 0) return MSB_OK;
+    std::fill(counts, counts + cells, (int64_t) 0);
+    ctx->t[MSB_T_PAIRS] = 0;
+    if (ctx->last_sites == 0 || n_seqs == 0) return MSB_OK;
+    MSB_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t W = (n_seqs + 31) / 32;
+    // word-range passes: at most 256 MB of H at a time, so n_seqs is bounded by int32 only
+    int64_t wp = std::max<int64_t>(1, ((int64_t) 1 << 26) / n_motifs);
+    if (ctx->opt_pair_pass_words > 0) wp = ctx->opt_pair_pass_words;
+    wp = std::min(wp, W);
+    MSB_TRY(ctx->pr_bits.ensure((size_t) n_motifs * (size_t) wp * 4));
+    MSB_TRY(ctx->pr_count.ensure(cells * 8));
+    MSB_CUDA(cudaEventRecord(ctx->ev[6], st));
+    MSB_CUDA(cudaMemsetAsync(ctx->pr_count.p, 0, cells * 8, st));
+    const int32_t n_tiles = (n_motifs + kPairTile - 1) / kPairTile;
+    const int64_t tiles = (int64_t) n_tiles * (n_tiles + 1) / 2;
+    if (tiles > 0x7fffffffll) { set_error("msb_scan_device_pair_counts: too many motifs"); return MSB_EINVAL; }
+    for (int64_t w0 = 0; w0 < W; w0 += wp) {
+        const int64_t wn = std::min(wp, W - w0);
+        MSB_CUDA(cudaMemsetAsync(ctx->pr_bits.p, 0, (size_t) n_motifs * (size_t) wn * 4, st));
+        site_bits_kernel<<<(unsigned) ((ctx->last_sites + 255) / 256), 256, 0, st>>>(
+            ctx->fin_key, ctx->fin_seq, ctx->last_sites, ctx->last_key_shift, w0, wn, ctx->pr_bits.as<uint32_t>());
+        MSB_CUDA(cudaGetLastError());
+        // split the words over enough CTAs to fill every SM twice, in whole 32-word chunks
+        const int64_t chunks = (wn + kPairK - 1) / kPairK;
+        const int64_t splits = std::min<int64_t>(chunks, std::max<int64_t>(1, (2 * (int64_t) ctx->sm_count + tiles - 1) / tiles));
+        int64_t k_split = (chunks + splits - 1) / splits * kPairK;
+        if (ctx->opt_pair_split_words > 0) k_split = ((int64_t) ctx->opt_pair_split_words + kPairK - 1) / kPairK * kPairK;
+        const dim3 grid((unsigned) tiles, (unsigned) ((wn + k_split - 1) / k_split));
+        pair_counts_kernel<<<grid, 256, 0, st>>>(ctx->pr_bits.as<uint32_t>(), n_motifs, wn, n_tiles, k_split,
+                                                 ctx->pr_count.as<unsigned long long>());
+        MSB_CUDA(cudaGetLastError());
+    }
+    MSB_CUDA(cudaEventRecord(ctx->ev[7], st));
+    MSB_CUDA(cudaMemcpyAsync(counts, ctx->pr_count.p, cells * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    ctx->t[MSB_T_PAIRS] = ev_ms(ctx->ev[6], ctx->ev[7]);
+    // the kernel fills the upper-triangular tiles: mirror them
+    for (int64_t a = 0; a < n_motifs; a++)
+        for (int64_t b = 0; b < a; b++) counts[a * n_motifs + b] = counts[b * n_motifs + a];
+    return MSB_OK;
+}
+
+int msb_scan_device_spacing(msb_ctx *ctx, const msb_motifs *M, int32_t n_anchors, const int32_t *anchors,
+                            int32_t max_offset, int64_t *hist) {
+    if (!ctx || !M || !anchors || !hist) { set_error("msb_scan_device_spacing: null"); return MSB_EINVAL; }
+    if (M->ctx != ctx) { set_error("msb_scan_device_spacing: motifs belong to another context"); return MSB_EINVAL; }
+    if (n_anchors < 1 || n_anchors > kMaxSpacingAnchors) { set_error("msb_scan_device_spacing: n_anchors must be 1..16"); return MSB_EINVAL; }
+    if (max_offset < 0 || max_offset > 500) { set_error("msb_scan_device_spacing: max_offset must be 0..500"); return MSB_EINVAL; }
+    MSB_TRY(check_final_sites(ctx, M->n, "msb_scan_device_spacing"));
+    for (int32_t k = 0; k < n_anchors; k++)
+        if (anchors[k] < 0 || anchors[k] >= M->n) { set_error("msb_scan_device_spacing: anchor index out of range"); return MSB_EINVAL; }
+    const int64_t W = 2 * (int64_t) max_offset + 1;
+    const size_t cells = (size_t) n_anchors * (size_t) M->n * 2 * (size_t) W;
+    std::fill(hist, hist + cells, (int64_t) 0);
+    ctx->t[MSB_T_SPACING] = 0;
+    if (ctx->last_sites == 0) return MSB_OK;
+    MSB_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t n = ctx->last_sites;
+    std::vector<int64_t> off((size_t) M->n + 1);
+    MSB_CUDA(cudaMemcpyAsync(off.data(), ctx->fin[ctx->fin_cur].offsets.p, off.size() * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    SpacingAnchors A;
+    A.n = n_anchors;
+    A.first[0] = 0;
+    for (int32_t k = 0; k < n_anchors; k++) {
+        A.motif[k] = anchors[k];
+        A.seg[k] = off[anchors[k]];
+        A.first[k + 1] = A.first[k] + (off[anchors[k] + 1] - off[anchors[k]]);
+    }
+    const int motif_bits = motif_bits_of(M->n);
+    const int end_bit = ctx->last_key_shift + motif_bits;
+    MSB_TRY(ctx->sp_key_in.ensure((size_t) n * 8));
+    MSB_TRY(ctx->sp_key.ensure((size_t) n * 8));
+    MSB_TRY(ctx->sp_seq.ensure((size_t) n * 4));
+    MSB_TRY(ctx->pr_count.ensure(cells * 8));
+    MSB_CUDA(cudaEventRecord(ctx->ev[6], st));
+    MSB_CUDA(cudaMemsetAsync(ctx->pr_count.p, 0, cells * 8, st));
+    if (A.first[n_anchors]) {
+        position_keys_kernel<<<(unsigned) ((n + 255) / 256), 256, 0, st>>>(ctx->fin_key, n, ctx->last_key_shift, motif_bits,
+                                                                           ctx->sp_key_in.as<uint64_t>());
+        MSB_CUDA(cudaGetLastError());
+        size_t tmp_bytes = 0;
+        MSB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, ctx->sp_key_in.as<uint64_t>(), ctx->sp_key.as<uint64_t>(),
+                                                 ctx->fin_seq, ctx->sp_seq.as<int32_t>(), n, 0, end_bit, st));
+        MSB_TRY(ctx->sort_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        MSB_CUDA(cub::DeviceRadixSort::SortPairs(ctx->sort_tmp.p, tmp_bytes, ctx->sp_key_in.as<uint64_t>(), ctx->sp_key.as<uint64_t>(),
+                                                 ctx->fin_seq, ctx->sp_seq.as<int32_t>(), n, 0, end_bit, st));
+        const int64_t threads = A.first[n_anchors] * 32;
+        spacing_kernel<<<(unsigned) ((threads + 255) / 256), 256, 0, st>>>(
+            A, ctx->fin_key, ctx->fin_seq, ctx->sp_key.as<uint64_t>(), ctx->sp_seq.as<int32_t>(), n, ctx->last_key_shift,
+            motif_bits, M->d_len.as<int32_t>(), M->lmax, M->n, max_offset, ctx->pr_count.as<unsigned long long>());
+        MSB_CUDA(cudaGetLastError());
+    }
+    MSB_CUDA(cudaEventRecord(ctx->ev[7], st));
+    MSB_CUDA(cudaMemcpyAsync(hist, ctx->pr_count.p, cells * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    ctx->t[MSB_T_SPACING] = ev_ms(ctx->ev[6], ctx->ev[7]);
     return MSB_OK;
 }
 
@@ -2807,6 +2937,57 @@ int msb_write_haplotype_table(const char *path, const char *header, int64_t n, c
     };
     return write_table_rows(path, header, n, lead_max + motif_max + 4 * 22 + kRowTailMax, n_threads, row,
                             "msb_write_haplotype_table");
+}
+
+int msb_write_cooccur_table(const char *path, const char *header, int64_t n, const int32_t *motif_a, const int32_t *motif_b,
+                            int32_t n_motifs, const char *motif_text, const int64_t *motif_off, const int64_t *n_single,
+                            const int64_t *n_both, const double *expected, const double *ratio, const double *p_cooccur,
+                            const double *p_exclusive, const double *q_cooccur, const int64_t *n_both_control,
+                            const double *fold_change, const double *p_enriched, const double *p_depleted,
+                            const double *p_corrected, int32_t n_threads) {
+    const bool control = n_both_control != nullptr;
+    if (!path || n < 0 || n_motifs < 0 || !motif_off || (n_motifs && !n_single) ||
+        (n && (!motif_a || !motif_b || !n_both || !expected || !ratio || !p_cooccur || !p_exclusive || !q_cooccur)) ||
+        (control && n && (!fold_change || !p_enriched || !p_depleted || !p_corrected))) {
+        set_error("msb_write_cooccur_table: bad argument");
+        return MSB_EINVAL;
+    }
+    size_t motif_max = 0;
+    for (int32_t m = 0; m < n_motifs; m++) motif_max = std::max<size_t>(motif_max, (size_t) (motif_off[m + 1] - motif_off[m]));
+    for (int64_t i = 0; i < n; i++)
+        if (motif_a[i] < 0 || motif_a[i] >= n_motifs || motif_b[i] < 0 || motif_b[i] >= n_motifs) {
+            set_error("msb_write_cooccur_table: row refers to an unknown motif");
+            return MSB_EINVAL;
+        }
+    auto num = [](double v, char *o) { *o++ = '\t'; return o + py_float_str(v, o); };
+    auto cnt = [](int64_t v, char *o) { *o++ = '\t'; return o + fmt_int(v, o); };
+    auto row = [&](int64_t i, char *o) {
+        const int32_t a = motif_a[i], b = motif_b[i];
+        const size_t an = (size_t) (motif_off[a + 1] - motif_off[a]), bn = (size_t) (motif_off[b + 1] - motif_off[b]);
+        std::memcpy(o, motif_text + motif_off[a], an); o += an;
+        *o++ = '\t';
+        std::memcpy(o, motif_text + motif_off[b], bn); o += bn;
+        o = cnt(n_single[a], o);
+        o = cnt(n_single[b], o);
+        o = cnt(n_both[i], o);
+        o = num(expected[i], o);
+        o = num(ratio[i], o);
+        o = num(p_cooccur[i], o);
+        o = num(p_exclusive[i], o);
+        o = num(q_cooccur[i], o);
+        if (control) {
+            o = cnt(n_both_control[i], o);
+            o = num(fold_change[i], o);
+            o = num(p_enriched[i], o);
+            o = num(p_depleted[i], o);
+            o = num(p_corrected[i], o);
+        } else {
+            std::memcpy(o, "\tNA\tNA\tNA\tNA\tNA", 15); o += 15;
+        }
+        *o++ = '\n';
+        return o;
+    };
+    return write_table_rows(path, header, n, 2 * motif_max + 4 * 22 + 9 * 26 + 8, n_threads, row, "msb_write_cooccur_table");
 }
 
 int msb_text_free(char *text) {

@@ -95,6 +95,28 @@ class Context:
                                                            ptr(best, ctypes.c_double)))
         return counts, best
 
+    def pair_counts(self, n_motifs, n_seqs):
+        """int64[n_motifs, n_motifs]: the number of sequences with a final site of both motifs in the last scan on this
+        context (the diagonal: with a site of the motif), from the (motif, sequence) bit matrix on the device
+        (msb_scan_device_pair_counts)."""
+        out = np.zeros((max(n_motifs, 1), max(n_motifs, 1)), dtype=np.int64)
+        with self._lock:
+            check(self._lib.msb_scan_device_pair_counts(self._h, int(n_motifs), int(n_seqs), ptr(out, ctypes.c_int64)))
+        return out[:n_motifs, :n_motifs]
+
+    def spacing(self, motifs, anchors, max_offset):
+        """int64[n_anchors, n_motifs, 2, 2 max_offset + 1]: partner sites around each anchor motif's sites in the last
+        scan on this context, by partner motif, orientation (0 same strand, 1 opposite) and offset -max_offset ..
+        max_offset in the anchor's frame (msb_scan_device_spacing)."""
+        a = np.ascontiguousarray(np.asarray(anchors, dtype=np.int32).reshape(-1))
+        d = int(max_offset)
+        ok = 1 <= len(a) <= 16 and 0 <= d <= 500
+        out = np.zeros((len(a), motifs.n, 2, 2 * d + 1) if ok else 1, dtype=np.int64)
+        with self._lock:
+            check(self._lib.msb_scan_device_spacing(self._h, motifs._h, len(a), ptr(a if len(a) else np.zeros(1, np.int32),
+                                                                                     ctypes.c_int32), d, ptr(out, ctypes.c_int64)))
+        return out
+
     def counters(self):
         a = np.zeros(len(_lib.C_NAMES), dtype=np.int64)
         check(self._lib.msb_ctx_counters(self._h, ptr(a, ctypes.c_int64), len(a)))

@@ -311,3 +311,62 @@ def write_enrich_table(output_dir, enrichment_results):
         for res in enrichment_results:
             out.write(f"{res.name}\t{res.n_input}\t{res.n_control}\t{res.fold_change}\t{res.p_enriched}\t"
                       f"{res.p_depleted}\t{res.p_corrected}\n")
+
+
+COOCCUR_HEADER = ("Motif_A\tMotif_B\tNum_A\tNum_B\tNum_both\tExpected\tRatio\tP_cooccur\tP_exclusive\tCorrected_P_value\t"
+                  "Num_both_control\tFold_change\tEnriched_P_value\tDepleted_P_value\tCorrected_enriched_P_value\n")
+SPACING_HEADER = "Anchor\tPartner\tOrientation\tPairs\tPeak_offset\tPeak_pairs\tExpected\tP_value\tCounts\n"
+
+
+def write_cooccur_table(output_dir, pwms, table):
+    """motif_cooccurrence.xls: one row per motif pair a < b (cooccur.cooccur_table), mutually exclusive pairs included,
+    ordered by (P_cooccur, -Ratio, a, b); motifs as `matrix_id,name`, numbers like Python's str(), the control columns
+    `NA` without controls.  Millions of rows are formatted by the library on host threads (msb_write_cooccur_table)."""
+    import ctypes
+    from . import _lib
+    from .cooccur import cooccur_order
+    lib = _lib.load()
+    os.makedirs(output_dir, exist_ok=True)
+    order = cooccur_order(table)
+    mtext = [name.encode() for name in _motif_names(pwms)]
+    motif_off = np.zeros(len(mtext) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in mtext], out=motif_off[1:])
+    single = np.zeros(max(len(pwms), 1), dtype=np.int64)
+    single[table.a] = table.n_a
+    single[table.b] = table.n_b
+    n = len(order)
+
+    def col(x, dtype, ct):
+        if x is None or n == 0:
+            return None, None
+        a = np.ascontiguousarray(np.asarray(x)[order], dtype=dtype)
+        return a, _lib.ptr(a, ct)
+    cols = [col(table.a, np.int32, ctypes.c_int32), col(table.b, np.int32, ctypes.c_int32)]
+    cols += [col(table.n_both, np.int64, ctypes.c_int64)]
+    cols += [col(getattr(table, f), np.float64, ctypes.c_double)
+             for f in ("expected", "ratio", "p_cooccur", "p_exclusive", "q_cooccur")]
+    cols += [col(table.n_both_control, np.int64, ctypes.c_int64)]
+    cols += [col(getattr(table, f), np.float64, ctypes.c_double)
+             for f in ("fold_change", "p_enriched", "p_depleted", "p_corrected")]
+    ptrs = [c[1] for c in cols]
+    _lib.check(lib.msb_write_cooccur_table(
+        os.path.join(output_dir, "motif_cooccurrence.xls").encode(), COOCCUR_HEADER.encode(), n, ptrs[0], ptrs[1], len(pwms),
+        b"".join(mtext), _lib.ptr(motif_off, ctypes.c_int64), _lib.ptr(single, ctypes.c_int64), *ptrs[2:],
+        min(os.cpu_count() or 1, 32)))
+
+
+def write_spacing_table(output_dir, pwms, anchors, rows):
+    """motif_spacing.xls: one row per (anchor, partner, orientation) with at least one pair (cooccur.spacing_rows):
+    the pairs at all offsets, the peak offset among the non-overlapping ones and its pairs, the pairs expected per
+    such offset, the peak's p-value (`NA` when every offset overlaps) and the counts from -D to D."""
+    os.makedirs(output_dir, exist_ok=True)
+    names = _motif_names(pwms)
+
+    def na(v):
+        return "NA" if v is None or (isinstance(v, float) and np.isnan(v)) else str(v)
+    with open(os.path.join(output_dir, "motif_spacing.xls"), "w") as out:
+        out.write(SPACING_HEADER)
+        for r in rows:
+            out.write(f"{names[anchors[r.anchor]]}\t{names[r.partner]}\t{'same' if r.orientation == 0 else 'opposite'}\t"
+                      f"{r.pairs}\t{na(r.peak_offset)}\t{na(r.peak_pairs)}\t{na(r.expected)}\t{na(r.p_value)}\t"
+                      f"{','.join(map(str, r.counts.tolist()))}\n")

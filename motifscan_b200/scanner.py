@@ -7,6 +7,7 @@ Same constructor arguments, attributes (`sequences`, `seq_starts`, `seq_ends`) a
 returns, so a (motif, region) cell costs nothing until it is looked at (the reference allocates
 one Python list per cell, scanner.py:140-143 -- 3.8e8 lists for configs[4]).
 """
+import contextlib
 import logging
 import os
 from collections import namedtuple
@@ -14,6 +15,7 @@ from collections import namedtuple
 import numpy as np
 
 from . import engine
+from .cooccur import PairResult
 
 logger = logging.getLogger(__name__)
 
@@ -99,9 +101,10 @@ class Scanner:
                 self._sequences = [c.decode("utf-8") for c in self._chunks]
         return self._sequences
 
-    def scan_motifs(self, pwms, ctx=None):
+    def scan_motifs(self, pwms, ctx=None, pairs=None):
         """Scan for motif occurrences; returns a `MotifSites` (nested-list view, (n_pwms,
-        n_regions, n_sites))."""
+        n_regions, n_sites)).  `pairs` (a cooccur.PairSpec): also reduce the final sites on the device to motif pair
+        counts and / or anchor spacing histograms, summed over the devices' blocks, as `MotifSites.pairs`."""
         cutoffs = []
         for pwm in pwms:
             try:
@@ -110,8 +113,13 @@ class Scanner:
                 raise ValueError(f"PWM has no motif score cutoff set for P-value {self.p_value!r}")
         matrices = [pwm.matrix for pwm in pwms]
         lengths = [pwm.length for pwm in pwms]
+        if pairs is not None and pairs.anchors and not all(0 <= int(a) < len(matrices) for a in pairs.anchors):
+            raise ValueError("spacing anchor index out of range")
         if not matrices:
-            return MotifSites(None, 0, self.seq_starts, lengths)
+            sites = MotifSites(None, 0, self.seq_starts, lengths)
+            if pairs is not None:
+                sites.pairs = PairResult(np.zeros((0, 0), dtype=np.int64) if pairs.cooccur else None, len(self.seq_starts), None)
+            return sites
         if self._resident is not None:
             ctxs = [self._resident.ctx]       # the windows live where the genome lives
         elif ctx is not None:
@@ -128,34 +136,55 @@ class Scanner:
         bounds = [n * k // len(ctxs) for k in range(len(ctxs) + 1)]    # contiguous blocks of regions
         strand = _STRAND_ARG[self.strand]
 
+        def reduce_pairs(c, motifs, n_block):
+            """The pair reductions of the scan just run on `c` (the caller holds c._lock)."""
+            counts = c.pair_counts(len(matrices), n_block) if pairs.cooccur else None
+            hist = c.spacing(motifs, list(pairs.anchors), pairs.max_offset) if pairs.anchors else None
+            return counts, hist
+
         def scan_block(k):
             c, a, b = ctxs[k], bounds[k], bounds[k + 1]
             motifs = engine.MotifSet(c, matrices, cutoffs)
             try:
-                if self._resident is not None or self._packed is not None:
-                    dg = self._resident if self._resident is not None else self._packed_on(c)
-                    sset = dg.extract(self._chroms[a:b], self.seq_starts[a:b], self.seq_ends[a:b])
-                    try:
-                        return engine.scan(c, motifs, sset, strand, remove_dup=self.remove_dup)
-                    finally:
-                        sset.close()
-                chunks = self._chunks[a:b]
-                off = np.zeros(len(chunks) + 1, dtype=np.int64)
-                if chunks:
-                    np.cumsum([len(x) for x in chunks], out=off[1:])
-                blob = np.frombuffer(b"".join(chunks), dtype=np.uint8)
-                return engine.scan_ascii(c, motifs, blob, off, strand, remove_dup=self.remove_dup)
+                # the reductions read the scan's sites on the device: no other scan on a shared context may come between
+                with c._lock if pairs is not None else contextlib.nullcontext():
+                    if self._resident is not None or self._packed is not None:
+                        dg = self._resident if self._resident is not None else self._packed_on(c)
+                        sset = dg.extract(self._chroms[a:b], self.seq_starts[a:b], self.seq_ends[a:b])
+                        try:
+                            res = engine.scan(c, motifs, sset, strand, remove_dup=self.remove_dup)
+                        finally:
+                            sset.close()
+                    else:
+                        chunks = self._chunks[a:b]
+                        off = np.zeros(len(chunks) + 1, dtype=np.int64)
+                        if chunks:
+                            np.cumsum([len(x) for x in chunks], out=off[1:])
+                        blob = np.frombuffer(b"".join(chunks), dtype=np.uint8)
+                        res = engine.scan_ascii(c, motifs, blob, off, strand, remove_dup=self.remove_dup)
+                    if pairs is None:
+                        return res, None
+                    return res, reduce_pairs(c, motifs, b - a)
             finally:
                 motifs.close()
 
         if len(ctxs) == 1:
-            res = scan_block(0).detach()
+            res, reduced = scan_block(0)
+            res = res.detach()
+            blocks = [reduced]
         else:
             import concurrent.futures
             with concurrent.futures.ThreadPoolExecutor(max_workers=len(ctxs)) as pool:
-                results = list(pool.map(scan_block, range(len(ctxs))))
-            res = _MergedResult(results, bounds[:-1], len(matrices), n)
-        return MotifSites(res, len(matrices), self.seq_starts, lengths)
+                out = list(pool.map(scan_block, range(len(ctxs))))
+            res = _MergedResult([r for r, _ in out], bounds[:-1], len(matrices), n)
+            blocks = [p for _, p in out]
+        sites = MotifSites(res, len(matrices), self.seq_starts, lengths)
+        if pairs is not None:
+            # the blocks hold disjoint regions: their counts and histograms add up
+            counts = sum(p[0] for p in blocks) if pairs.cooccur else None
+            hist = sum(p[1] for p in blocks) if pairs.anchors else None
+            sites.pairs = PairResult(counts, n, hist)
+        return sites
 
     def _packed_on(self, ctx):
         """The device-resident copy of a host PackedGenome on `ctx`'s GPU (made on first use, kept on the
@@ -212,6 +241,7 @@ class MotifSites:
         self.n_seqs = len(seq_starts)
         self.seq_starts = list(seq_starts)
         self.lengths = list(lengths)
+        self.pairs = None    # cooccur.PairResult when the scan was asked for pair reductions
         if res is None:
             self._off = np.zeros(n_pwms + 1, dtype=np.int64)
             self._seq_idx = np.zeros(0, dtype=np.int32)
