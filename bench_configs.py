@@ -378,14 +378,15 @@ def bench_enrich(args):
             "parity": {"regions_with_site_counts_identical_on_sample": bool(np.array_equal(got, want))}}
 
 
-def bench_cli(args, pair_flags=False):
+def bench_cli(args, pair_flags=False, extra_flags=None, window=0):
     """configs[4] through the command line: `python -m motifscan_b200 scan` on 200k target + 200k control 1 kb regions x
     1,900 motifs (20 of them 33-40 columns long), a synthetic genome directory with a packed-genome cache next to
     the FASTA; wall time and peak RSS of the whole process (region parsing, scans, both site tables -- 1,900 columns
     x 200,000 rows each -- and the enrichment table).  The first `--cpu-regions` rows of the tables are compared with
     the reference pipeline (its extension on the CPU, its regrouping, de-duplication and writers restated).
     `pair_flags`: the same command with `--cooccur --spacing-anchor <first --anchors motifs> --spacing-max D` is run
-    alternately with the plain one; its other output files must be byte-identical to the plain run's."""
+    alternately with the plain one; its other output files must be byte-identical to the plain run's.  `extra_flags`:
+    the same with these flags instead (e.g. `--centrality`), both commands at `-w window`."""
     import resource
     import shutil
     import subprocess
@@ -432,11 +433,12 @@ def bench_cli(args, pair_flags=False):
     setup_s = time.perf_counter() - t0
     out = os.path.join(root, "out")
     cmd = [sys.executable, "-m", "motifscan_b200", "scan", "-i", os.path.join(root, "targets.bed"), "-c", os.path.join(root, "controls.bed"),
-           "-m", mdir, "-g", gdir, "-o", out, "-w", "0", "-p", "1e-4", "--gpus", str(args.gpus)]
+           "-m", mdir, "-g", gdir, "-o", out, "-w", str(window), "-p", "1e-4", "--gpus", str(args.gpus)]
     runs = []
     pair_out = os.path.join(root, "out_pairs")
-    pair_cmd = cmd[:cmd.index("-o")] + ["-o", pair_out] + cmd[cmd.index("-o") + 2:] + [
-        "--cooccur", "--spacing-anchor", ",".join(ids[:args.anchors]), "--spacing-max", str(args.spacing_max)]
+    pair_cmd = cmd[:cmd.index("-o")] + ["-o", pair_out] + cmd[cmd.index("-o") + 2:] + (list(extra_flags) if extra_flags else [
+        "--cooccur", "--spacing-anchor", ",".join(ids[:args.anchors]), "--spacing-max", str(args.spacing_max)])
+    pair_flags = pair_flags or bool(extra_flags)
     pair_runs = []
     for _ in range(2):
         for c, o, into in ((cmd, out, runs),) + (((pair_cmd, pair_out, pair_runs),) if pair_flags else ()):
@@ -1158,10 +1160,127 @@ def bench_cooccur(args):
                        "cells_with_both": int((want_c > 0).sum())}}
 
 
+def bench_centrality(args):
+    """`scan --centrality` at the cooccur size: 1 kb regions (summit = midpoint, -w 1000: every window tested) scanned
+    in blocks, the two histograms reduced on the device after each block's scan and summed, then the host statistics
+    and the table writer.  The reduction is timed with shared-memory histograms and, on the same scan, with global
+    atomics only (the `centrality_shared` 0 A/B option).  Parity: the first --cpu-regions regions against the oracle,
+    as integers.  The CLI runs `scan -w 1000` with and without --centrality alternately."""
+    import subprocess
+    import tempfile
+    import oracle
+    from motifscan_b200 import engine, synth
+    from motifscan_b200 import io as msio
+    from motifscan_b200.centrality import CentralityResult, centrality_rows, half_bins
+    from motifscan_b200.motif import PositionWeightMatrix
+    ctx = engine.default_context(0)
+    _, pwms, ids = synth.motif_set(args.motifs, seed=2020, n_long=20)
+    motifs = engine.MotifSet(ctx, pwms)
+    lmax = max(p.shape[1] for p in pwms)
+    bblob, boff = synth.background_samples(100000, lmax, seed=1)
+    bg = engine.SequenceSet(ctx, blob=bblob, seq_off=boff)
+    cutoffs = np.around(engine.score_select(ctx, motifs, bg, 3, [int(100000 * 1e-4) - 1])[:, 0], 8)
+    bg.close()
+    motifs.set_cutoffs(cutoffs)
+    lengths = [p.shape[1] for p in pwms]
+    E, B = 500, args.centrality_bin
+    K = half_bins(E, B)
+    blob, off = synth.peak_set(args.regions, 2 * E, seed=200)
+    phases = ("prefilter", "exact", "order", "centrality")
+
+    def scan_centrality():
+        hist_all = np.zeros((args.motifs, 2 * K + 1), dtype=np.int64)
+        hist_best = np.zeros_like(hist_all)
+        ms = dict.fromkeys(phases + ("centrality_global_atomics",), 0.0)
+        same = True
+        for a in range(0, args.regions, args.region_block):
+            b = min(args.regions, a + args.region_block)
+            sset = engine.SequenceSet(ctx, blob=blob[off[a]:off[b]], seq_off=off[a:b + 1] - off[a])
+            engine.scan_device(ctx, motifs, sset, 3, remove_dup=True)
+            mid2 = np.full(b - a, 2 * E, dtype=np.int32)
+            ctx.set_option("centrality_shared", 0)
+            g_all, g_best = ctx.centrality(motifs, mid2, B, K)
+            ms["centrality_global_atomics"] += ctx.timings()["centrality"]
+            ctx.set_option("centrality_shared", 1)
+            h_all, h_best = ctx.centrality(motifs, mid2, B, K)
+            same &= bool(np.array_equal(g_all, h_all) and np.array_equal(g_best, h_best))
+            hist_all += h_all
+            hist_best += h_best
+            t = ctx.timings()
+            for k in phases:
+                ms[k] += t[k]
+            sset.close()
+        return hist_all, hist_best, ms, same
+
+    runs = []
+    for _ in range(args.steps + 1):
+        t0 = time.perf_counter()
+        out = scan_centrality()
+        runs.append((time.perf_counter() - t0,) + out)
+    scan_s, hist_all, hist_best, ms, ab_same = min(runs[1:], key=lambda r: r[0])
+    n_blocks = (args.regions + args.region_block - 1) // args.region_block
+    # A/B of the reduction alone on the last block's sites (still on the device): shared-memory histograms against
+    # global atomics, alternated
+    ab = {"shared": [], "global_atomics": []}
+    last = np.full(args.regions - (n_blocks - 1) * args.region_block, 2 * E, dtype=np.int32)
+    for _ in range(args.ab_reps):
+        for opt, k in ((1, "shared"), (0, "global_atomics")):
+            ctx.set_option("centrality_shared", opt)
+            ctx.centrality(motifs, last, B, K)
+            ab[k].append(ctx.timings()["centrality"])
+    ctx.set_option("centrality_shared", 1)
+    res = CentralityResult(hist_all, hist_best, args.regions, E, B)
+    t0 = time.perf_counter()
+    rows = centrality_rows(res, lengths)
+    stats_s = time.perf_counter() - t0
+    objs = [PositionWeightMatrix(p, name=f"TF{k}", matrix_id=ids[k]) for k, p in enumerate(pwms)]
+    with tempfile.TemporaryDirectory() as tmp:
+        t0 = time.perf_counter()
+        msio.write_centrality_tables(tmp, objs, res, rows)
+        write_s = time.perf_counter() - t0
+    # parity: the first cpu_regions regions, device vs oracle, as integers
+    n = args.cpu_regions
+    seqs = strs(blob, off, range(n))
+    sset = engine.SequenceSet(ctx, blob=blob[:off[n]], seq_off=off[:n + 1])
+    engine.scan_device(ctx, motifs, sset, 3, remove_dup=True)
+    got_all, got_best = ctx.centrality(motifs, np.full(n, 2 * E, dtype=np.int32), B, K)
+    sset.close()
+    flat = oracle.c_scan_motif([p.tolist() for p in pwms], cutoffs.tolist(), seqs, 3, os.cpu_count() or 1)
+    nested = oracle.deduplicate_motif_sites(oracle.make_motif_sites(flat, [0] * n), lengths)
+    want_all, want_best = np.zeros_like(got_all), np.zeros_like(got_best)
+    for m, per in enumerate(nested):
+        for cell in per:
+            if not cell:
+                continue
+            best = cell[0]
+            for site in cell:
+                want_all[m, (2 * site.start + lengths[m] - 2 * E + B) // (2 * B) + K] += 1
+                if site.score > best.score:
+                    best = site
+            want_best[m, (2 * best.start + lengths[m] - 2 * E + B) // (2 * B) + K] += 1
+    cli = bench_cli(args, extra_flags=["--centrality", "--centrality-bin", str(B)], window=2 * E)
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                          text=True).stdout.strip().splitlines()[0]
+    return {"config": f"centrality: {args.regions} 1 kb regions x {args.motifs} motifs (20 of 33-40 columns), blocks of "
+                      f"{args.region_block} regions, -w {2 * E} --centrality-bin {B} ({2 * K + 1} bins)",
+            "card": card,
+            "device_ms_per_block": {k: v / n_blocks for k, v in ms.items()},
+            "shared_and_global_histograms_equal": ab_same,
+            "reduction_ab_ms": {k: {"median": float(np.median(v)), "min": float(np.min(v)), "reps": len(v)}
+                                for k, v in ab.items()},
+            "scan_and_reduce_wall_s": scan_s, "sites": int(hist_all.sum()), "best_sites": int(hist_best.sum()),
+            "host_stats_s": stats_s, "writer_s": write_s,
+            "top_rows": [list(r)[:10] for r in rows[:3]],
+            "cli_wall_s": {"plain": min(cli["plain_runs_s"]), "with_centrality": cli["wall_s"], "runs": cli},
+            "parity": {"regions": n, "hist_all_equal": bool(np.array_equal(got_all, want_all)),
+                       "hist_best_equal": bool(np.array_equal(got_best, want_best)), "sites": int(want_all.sum()),
+                       "best_sites": int(want_best.sum())}}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("which", choices=["build", "genome", "enrich", "cli", "whole-genome", "variants", "haplotypes",
-                                          "cooccur"])
+                                          "cooccur", "centrality"])
     ap.add_argument("--alleles", type=int, default=None)
     ap.add_argument("--samples", type=int, default=16)
     ap.add_argument("--cpu-clusters", dest="cpu_clusters", type=int, default=500)
@@ -1183,14 +1302,16 @@ def main():
     ap.add_argument("--cpu-regions", dest="cpu_regions", type=int, default=None)
     ap.add_argument("--anchors", type=int, default=4)
     ap.add_argument("--spacing-max", dest="spacing_max", type=int, default=50)
+    ap.add_argument("--centrality-bin", dest="centrality_bin", type=int, default=10)
+    ap.add_argument("--ab-reps", dest="ab_reps", type=int, default=30)
     args = ap.parse_args()
     if args.motifs is None:
-        args.motifs = 1900 if args.which in ("enrich", "cli", "cooccur") else 750
+        args.motifs = 1900 if args.which in ("enrich", "cli", "cooccur", "centrality") else 750
     if args.cpu_regions is None:
-        args.cpu_regions = 2000 if args.which == "cooccur" else 4000
+        args.cpu_regions = 2000 if args.which in ("cooccur", "centrality") else 4000
     out = {"build": bench_build, "genome": bench_genome, "enrich": bench_enrich, "cli": bench_cli,
            "whole-genome": bench_whole_genome, "variants": bench_variants, "haplotypes": bench_haplotypes,
-           "cooccur": bench_cooccur}[args.which](args)
+           "cooccur": bench_cooccur, "centrality": bench_centrality}[args.which](args)
     if out is not None:
         print(json.dumps(out))
 

@@ -62,10 +62,10 @@ int msb_ctx_create(int device, void *stream, msb_ctx **ctx);
 int msb_ctx_destroy(msb_ctx *ctx);
 int msb_ctx_sync(msb_ctx *ctx);
 /* Per-phase device times (ms, CUDA events on the context's stream) of the last msb_scan /
- * msb_score / msb_seqs_from_ascii on this context.  Index by MSB_T_*.  MSB_T_PAIRS and MSB_T_SPACING hold the
- * last msb_scan_device_pair_counts / msb_scan_device_spacing. */
+ * msb_score / msb_seqs_from_ascii on this context.  Index by MSB_T_*.  MSB_T_PAIRS, MSB_T_SPACING and MSB_T_CENTRALITY
+ * hold the last msb_scan_device_pair_counts / msb_scan_device_spacing / msb_scan_device_centrality. */
 enum { MSB_T_H2D = 0, MSB_T_ENCODE, MSB_T_PREFILTER, MSB_T_EXACT, MSB_T_ORDER, MSB_T_D2H,
-       MSB_T_SCORE, MSB_T_SELECT, MSB_T_ROWS, MSB_T_ROW_SORT, MSB_T_PAIRS, MSB_T_SPACING, MSB_T_COUNT };
+       MSB_T_SCORE, MSB_T_SELECT, MSB_T_ROWS, MSB_T_ROW_SORT, MSB_T_PAIRS, MSB_T_SPACING, MSB_T_CENTRALITY, MSB_T_COUNT };
 int msb_ctx_timings(const msb_ctx *ctx, double *ms, int n);
 /* Counters of the last msb_scan: index by MSB_C_*. */
 enum { MSB_C_CANDIDATES = 0, MSB_C_DIRTY, MSB_C_HITS, MSB_C_LAUNCHES, MSB_C_RETRIES,
@@ -81,7 +81,8 @@ int msb_ctx_counters(const msb_ctx *ctx, int64_t *v, int n);
  * every sample for every motif instead of the pilot + scan scheme (A/B tests); "pair_pass_words" words of each motif's
  * sequence bits per pass of msb_scan_device_pair_counts (tests of the word-range passes; 0 = sized from a 256 MB
  * budget); "pair_split_words" words each CTA of the pair-count kernel covers, rounded up to whole 32-word chunks (tests
- * of CTAs that loop over several chunks; 0 = sized to fill every SM). */
+ * of CTAs that loop over several chunks; 0 = sized to fill every SM); "centrality_shared" 0 = msb_scan_device_centrality
+ * adds every site to the histograms in global memory instead of shared-memory histograms per CTA (A/B measurements). */
 int msb_ctx_set_option(msb_ctx *ctx, const char *name, int value);
 
 /* Pinned host memory for callers that want full-speed H2D (cudaHostAlloc / cudaFreeHost). */
@@ -260,6 +261,18 @@ int msb_scan_device_pair_counts(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, 
  * last-scan states of msb_scan_device_pair_counts.  MSB_T_SPACING times it. */
 int msb_scan_device_spacing(msb_ctx *ctx, const msb_motifs *motifs, int32_t n_anchors, const int32_t *anchors,
                             int32_t max_offset, int64_t *hist);
+/* Positional histograms of the same sites (`motifscan scan --centrality`): a final site of motif m (length L) at `start` in
+ * sequence s has the doubled offset d2 = 2 start + L - mid2[s] from twice the sequence's reference point mid2[s]
+ * (relative to the sequence's first base; mid2[s] < 0 leaves sequence s out) and lies in bin k = floor((d2 + bin) /
+ * (2 bin)), i.e. its centre is in [k bin - bin / 2, k bin + bin / 2) bases from the reference point.  Sites with k in
+ * -half_bins..half_bins are counted: hist_all[m * (2 half_bins + 1) + k + half_bins] counts every site, hist_best the
+ * best-scoring site of each (motif, sequence) cell with a site (ties: the first in (start, strand +) order) when that
+ * site's bin is in range.  `motifs` gives the lengths and must have the last scan's motif count, n_seqs its sequence
+ * count, with its sites kept (not MSB_SCAN_COUNTS, not compact).  MSB_EINVAL for those, a null pointer, bin < 1,
+ * half_bins < 0 or n_motifs * (2 half_bins + 1) > MSB_CENTRALITY_MAX_CELLS.  MSB_T_CENTRALITY times it. */
+#define MSB_CENTRALITY_MAX_CELLS (1ll << 26)
+int msb_scan_device_centrality(msb_ctx *ctx, const msb_motifs *motifs, int64_t n_seqs, const int32_t *mid2, int32_t bin,
+                               int32_t half_bins, int64_t *hist_all, int64_t *hist_best);
 /* Variant-effect scan.  Sequence i of `ref` is allele i's context on the reference genome, sequence i of `alt` the
  * same bases with the allele substituted (msb_seqs_extract / msb_seqs_extract_subst: equal lengths); the changed
  * bases are [core_start[i], core_start[i] + core_len[i]) of it.  Both sets are scanned (msb_scan_device without

@@ -18,7 +18,9 @@ MSB_SCAN_COUNTS = 2
 MSB_SCAN_ASYNC = 4
 MSB_SCAN_COMPACT = 8
 MSB_SEQS_ASYNC = 1
-T_NAMES = ("h2d", "encode", "prefilter", "exact", "order", "d2h", "score", "select", "rows", "row_sort", "pairs", "spacing")
+CENTRALITY_MAX_CELLS = 1 << 26    # MSB_CENTRALITY_MAX_CELLS
+T_NAMES = ("h2d", "encode", "prefilter", "exact", "order", "d2h", "score", "select", "rows", "row_sort", "pairs", "spacing",
+           "centrality")
 C_NAMES = ("candidates", "dirty", "hits", "launches", "retries", "prefilter_launches")
 
 c_i32p = ctypes.POINTER(ctypes.c_int32)
@@ -79,6 +81,8 @@ SIGNATURES = {
     "msb_scan_device_cell_stats": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int64, c_i64p, c_f64p]),
     "msb_scan_device_pair_counts": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int64, c_i64p]),
     "msb_scan_device_spacing": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int32, c_i32p, ctypes.c_int32, c_i64p]),
+    "msb_scan_device_centrality": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_i32p, ctypes.c_int32, ctypes.c_int32, c_i64p,
+                                                  c_i64p]),
     "msb_scan_variants": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
     "msb_scan_variants_ex": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_i32p, c_i32p, c_i32p, ctypes.c_int, c_i64p]),
     "msb_scan_device_variant_rows": (ctypes.c_int, [c_vp, ctypes.c_int64, c_i64p, c_i32p, c_i32p, c_i32p, c_i8p, c_f64p, c_f64p,

@@ -31,8 +31,16 @@ Same flags as the reference's subcommands (cli/main.py:407-430, 504-579) and the
     partner motif and orientation, the partner sites at offsets -D..D of the anchor's sites (default D = 50) and the
     most enriched non-overlapping offset (motifscan_b200/cooccur.py).  Both are errors with --whole-genome;
 
+  * `scan --centrality [--centrality-bin B]` (not in the reference) writes where each motif's sites fall around the
+    region summits: motif_site_distribution.xls, per motif the sites and the best site of each region in bins of B bases
+    (default 10) by their centre's offset from the summit, and motif_centrality.xls, a test of the best sites piling up
+    within +-(j + 1/2) B of the summit against a uniform position, at the most significant width
+    (motifscan_b200/centrality.py).  Only windows that no chromosome end clips are used; the control regions are not
+    (a random window has no summit).  An error with --whole-genome and with -w below 2;
+
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir
     python -m motifscan_b200 scan -i peaks.bed -m <motif set> -g <genome> -o out_dir --cooccur --spacing-anchor MA0099.3
+    python -m motifscan_b200 scan -i peaks.narrowPeak -f narrowpeak -m <motif set> -g <genome> -o out_dir --centrality
     python -m motifscan_b200 scan --whole-genome -m <motif set> -g <genome> -o out_dir [--site]
     python -m motifscan_b200 motif --build <motif set> -g <genome>
     python -m motifscan_b200 variant -i calls.vcf.gz -m <motif set> -g <genome> -o out_dir [--indels]
@@ -46,6 +54,7 @@ from configparser import ConfigParser
 
 from . import io as msio
 from .builder import build_cutoffs
+from .centrality import centrality_rows
 from .cooccur import PairSpec, cooccur_table, spacing_rows
 from .genome import Genome
 from .motif import MotifPwms, PositionWeightMatrix, pfm_to_pwm, read_jaspar_pfms
@@ -164,6 +173,9 @@ def run_scan(args):
             if given:
                 raise SystemExit(f"motifscan scan: error: {flag} has no meaning with --whole-genome (no enrichment, and a "
                                  "chromosome is not a region to co-occur in)")
+        if args.centrality:
+            raise SystemExit("motifscan scan: error: --centrality has no meaning with --whole-genome (a chromosome has no "
+                             "summit to be central to)")
         if args.plot_dist:
             raise SystemExit("motifscan scan: --plot needs matplotlib, which is out of scope here")
         return run_whole_genome(args)
@@ -171,6 +183,14 @@ def run_scan(args):
         raise SystemExit("motifscan scan: --loc needs the gene annotation layer, which is out of scope here")
     if args.plot_dist:
         raise SystemExit("motifscan scan: --plot needs matplotlib, which is out of scope here")
+    if args.centrality:
+        extend = args.window_size // 2
+        if extend < 1:
+            raise SystemExit("motifscan scan: error: --centrality needs windows centred on the summits (-w 2 or more): "
+                             "regions of their own lengths share no geometry to test positions against")
+        if args.centrality_bin > extend:
+            raise SystemExit(f"motifscan scan: error: --centrality-bin must be 1..{extend} (half of -w), "
+                             f"got {args.centrality_bin}")
     logger.info("===== Loading data =====")
     genome = load_genome(args.genome)
     pwms = load_built_pwms(args.motif, genome.name)
@@ -185,7 +205,8 @@ def run_scan(args):
     source = packed_genome(genome, window_bp * (1 if args.no_enrich else 2), devices[0]) or genome
     common = dict(genome=source, window_size=args.window_size, strand=args.strand, p_value=args.p_value,
                   remove_dup=True, n_threads=args.n_threads, devices=devices)
-    sites = Scanner(regions=regions, **common).scan_motifs(pwms, pairs=pairs)
+    sites = Scanner(regions=regions, **common).scan_motifs(pwms, pairs=pairs,
+                                                          centrality=args.centrality_bin if args.centrality else None)
     logger.info("Saving the result tables")
     msio.write_sites_table(args.output_dir, pwms, regions, sites)
     if args.report_site:
@@ -193,6 +214,14 @@ def run_scan(args):
     if anchors:
         rows = spacing_rows(sites.pairs.spacing, anchors, [int(p.length) for p in pwms])
         msio.write_spacing_table(args.output_dir, pwms, anchors, rows)
+    if args.centrality:
+        import time
+        t0 = time.perf_counter()
+        rows = centrality_rows(sites.centrality, [int(p.length) for p in pwms])
+        t1 = time.perf_counter()
+        msio.write_centrality_tables(args.output_dir, pwms, sites.centrality, rows)
+        logger.info(f"Centrality of {len(pwms)} motifs in {sites.centrality.n_tested} of {len(regions)} regions: "
+                    f"statistics {t1 - t0:.3f} s, tables {time.perf_counter() - t1:.3f} s")
     control_pairs = None
     if not args.no_enrich:
         logger.info("===== Motif Enrichment =====")
@@ -409,6 +438,11 @@ def make_parser():
                            "(matrix_id or unique name, up to 16)")
     scan.add_argument("--spacing-max", dest="spacing_max", type=_spacing_max, default=50, metavar="D",
                       help="largest |offset| of --spacing-anchor, 0..500 (default 50)")
+    scan.add_argument("--centrality", action="store_true",
+                      help="write motif_centrality.xls and motif_site_distribution.xls: where each motif's sites fall "
+                           "around the region summits, and a test of central enrichment")
+    scan.add_argument("--centrality-bin", dest="centrality_bin", type=_positive, default=10, metavar="B",
+                      help="bin width of --centrality in bases, 1..(-w)/2 (default 10)")
     scan.add_argument("--verbose", action="store_true")
     scan.set_defaults(func=run_scan)
 

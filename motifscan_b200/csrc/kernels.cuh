@@ -1186,4 +1186,72 @@ spacing_kernel(SpacingAnchors A, const uint64_t *__restrict__ key, const int32_t
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Positional centrality (msb_scan_device_centrality).  A site of motif m (length L) at `start` in sequence s has the
+// doubled offset d2 = 2 start + L - mid2[s] from the sequence's reference point and lies in bin
+// floor((d2 + B) / (2B)); sequences with mid2 < 0 and bins outside -H..H are not counted.  hist_all counts every final
+// site, hist_best one site per (motif, sequence) cell: the best score, ties to the first site in final order.
+//
+// One CTA per tile of kCentralityTile consecutive final sites, one thread per site.  A (motif, sequence) cell is a
+// contiguous run of the (motif, sequence, start, strand)-ordered sites, so the best site is a segmented arg-max: the
+// thread holding a run's first site walks the run (runs are a few sites; a walk may leave the tile) with a strict >,
+// which keeps the first of equal scores.  No dense (motif, sequence) array is needed.
+//
+// The sites are motif-major, so a tile touches a few consecutive motifs [m_lo, m_hi] -- at 1,900 motifs x 50,000
+// regions a motif has tens of thousands of sites, and every one of them would hit the same 2H + 1 global counters.
+// When both histograms of the tile's motifs fit in kCentralitySmemCells 32-bit cells they are privatised in shared
+// memory and flushed with one global atomic per non-empty cell (cell c of the tile's slice is global cell
+// m_lo (2H + 1) + c); otherwise, and with `privatise` 0 (A/B measurements), every site adds to global memory directly.
+// ---------------------------------------------------------------------------------------------
+constexpr int kCentralityTile = 2048, kCentralitySmemCells = 8192;
+
+__device__ __forceinline__ int64_t centrality_bin(int64_t d2, int32_t bin) {
+    const int64_t num = d2 + bin, den = 2 * (int64_t) bin;
+    return num >= 0 ? num / den : -((-num + den - 1) / den);
+}
+
+__global__ void __launch_bounds__(256)
+centrality_kernel(const uint64_t *__restrict__ key, const int32_t *__restrict__ seq_idx, const int32_t *__restrict__ start,
+                  const double *__restrict__ score, int64_t n, int key_shift, const int32_t *__restrict__ mlen,
+                  const int32_t *__restrict__ mid2, int32_t bin, int32_t half_bins, int privatise,
+                  unsigned long long *__restrict__ hist_all, unsigned long long *__restrict__ hist_best) {
+    __shared__ uint32_t sh[kCentralitySmemCells];
+    const int64_t i0 = (int64_t) blockIdx.x * kCentralityTile, i1 = min(i0 + kCentralityTile, n);
+    const int64_t nb = 2 * (int64_t) half_bins + 1;
+    const uint32_t m_lo = site_motif(key[i0], key_shift);
+    const int64_t span = ((int64_t) site_motif(key[i1 - 1], key_shift) - m_lo + 1) * nb;   // cells of one histogram
+    const bool priv = privatise && 2 * span <= kCentralitySmemCells;
+    if (priv) {
+        for (int c = threadIdx.x; c < 2 * span; c += blockDim.x) sh[c] = 0;
+        __syncthreads();
+    }
+    auto add = [&](int which, uint32_t m, int64_t d2) {
+        const int64_t b = centrality_bin(d2, bin);
+        if (b < -half_bins || b > half_bins) return;
+        const int64_t cell = (int64_t) (m - m_lo) * nb + b + half_bins;
+        if (priv) atomicAdd(sh + which * span + cell, 1u);
+        else atomicAdd((which ? hist_best : hist_all) + (int64_t) m_lo * nb + cell, 1ull);
+    };
+    for (int64_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        const uint32_t m = site_motif(key[i], key_shift);
+        const int32_t s = seq_idx[i];
+        const int32_t c = __ldg(mid2 + s);
+        if (c < 0) continue;
+        const int32_t L = __ldg(mlen + m);
+        add(0, m, 2 * (int64_t) start[i] + L - c);
+        if (i > 0 && site_motif(key[i - 1], key_shift) == m && seq_idx[i - 1] == s) continue;   // not the run's head
+        int64_t best = i;
+        double bs = score[i];
+        for (int64_t j = i + 1; j < n && site_motif(key[j], key_shift) == m && seq_idx[j] == s; j++)
+            if (score[j] > bs) bs = score[j], best = j;
+        add(1, m, 2 * (int64_t) start[best] + L - c);
+    }
+    if (priv) {
+        __syncthreads();
+        for (int c = threadIdx.x; c < 2 * span; c += blockDim.x)
+            if (sh[c]) atomicAdd((c < span ? hist_all : hist_best) + (int64_t) m_lo * nb + (c < span ? c : c - span),
+                                 (unsigned long long) sh[c]);
+    }
+}
+
 }  // namespace msb

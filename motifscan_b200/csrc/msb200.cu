@@ -130,8 +130,10 @@ struct msb_ctx {
     int opt_select_pilot = 1;        // msb_score_select: 0 = always score every sample for every motif (the plain form)
     int opt_pair_pass_words = 0;     // tests: words per motif row in one pass of msb_scan_device_pair_counts (0 = 256 MB budget)
     int opt_pair_split_words = 0;    // tests: words per CTA of pair_counts_kernel, rounded up to 32-word chunks (0 = sized to fill the SMs)
+    int opt_centrality_shared = 1;   // msb_scan_device_centrality: 0 = global atomics only, no shared-memory histograms (A/B)
     // msb_scan_device_pair_counts / msb_scan_device_spacing: bit matrix, counts / histogram, position-major sites
     DevBuf pr_bits, pr_count, sp_key_in, sp_key, sp_seq;
+    DevBuf ce_mid2;                  // msb_scan_device_centrality: the sequences' reference points
 };
 
 // Tensor-core prefilter tables (prefilter_tc.cuh).
@@ -401,7 +403,7 @@ int msb_ctx_destroy(msb_ctx *ctx) {
                       &ctx->vr_eff, &ctx->vr_other, &ctx->vr_key_sorted, &ctx->vr_idx_sorted, &ctx->vr_core,
                       &ctx->vr_eoff, &ctx->vo_allele, &ctx->vo_motif, &ctx->vo_start, &ctx->vo_strand, &ctx->vo_ref,
                       &ctx->vo_alt, &ctx->vo_eff, &ctx->vo_other, &ctx->pr_bits, &ctx->pr_count, &ctx->sp_key_in,
-                      &ctx->sp_key, &ctx->sp_seq})
+                      &ctx->sp_key, &ctx->sp_seq, &ctx->ce_mid2})
         b->release();
     if (ctx->d2h_stream) cudaStreamSynchronize(ctx->d2h_stream);
     for (auto &f : ctx->fin) {
@@ -1696,6 +1698,7 @@ int msb_ctx_set_option(msb_ctx *ctx, const char *name, int value) {
     if (name && !std::strcmp(name, "select_pilot") && (value == 0 || value == 1)) { ctx->opt_select_pilot = value; return MSB_OK; }
     if (name && !std::strcmp(name, "pair_pass_words") && value >= 0) { ctx->opt_pair_pass_words = value; return MSB_OK; }
     if (name && !std::strcmp(name, "pair_split_words") && value >= 0) { ctx->opt_pair_split_words = value; return MSB_OK; }
+    if (name && !std::strcmp(name, "centrality_shared") && (value == 0 || value == 1)) { ctx->opt_centrality_shared = value; return MSB_OK; }
     set_error("msb_ctx_set_option: unknown option or value");
     return MSB_EINVAL;
 }
@@ -1794,7 +1797,7 @@ int msb_scan_device_cell_stats(msb_ctx *ctx, int32_t n_motifs, int64_t n_seqs, i
 }
 
 // The last scan's final sites exist on the device in (motif, sequence, start) order (msb_scan_device_pair_counts /
-// msb_scan_device_spacing).
+// msb_scan_device_spacing / msb_scan_device_centrality).
 static int check_final_sites(const msb_ctx *ctx, int32_t n_motifs, const char *what) {
     if (n_motifs != ctx->last_n_motifs) { set_error(std::string(what) + ": no scan with that many motifs"); return MSB_EINVAL; }
     if (ctx->last_counts_only) { set_error(std::string(what) + ": the last scan kept per-motif counts only (MSB_SCAN_COUNTS)"); return MSB_EINVAL; }
@@ -1913,6 +1916,47 @@ int msb_scan_device_spacing(msb_ctx *ctx, const msb_motifs *M, int32_t n_anchors
     MSB_CUDA(cudaMemcpyAsync(hist, ctx->pr_count.p, cells * 8, cudaMemcpyDeviceToHost, st));
     MSB_CUDA(cudaStreamSynchronize(st));
     ctx->t[MSB_T_SPACING] = ev_ms(ctx->ev[6], ctx->ev[7]);
+    return MSB_OK;
+}
+
+int msb_scan_device_centrality(msb_ctx *ctx, const msb_motifs *M, int64_t n_seqs, const int32_t *mid2, int32_t bin,
+                               int32_t half_bins, int64_t *hist_all, int64_t *hist_best) {
+    if (!ctx || !M || n_seqs < 0 || (!mid2 && n_seqs) || !hist_all || !hist_best) {
+        set_error("msb_scan_device_centrality: null");
+        return MSB_EINVAL;
+    }
+    if (M->ctx != ctx) { set_error("msb_scan_device_centrality: motifs belong to another context"); return MSB_EINVAL; }
+    if (bin < 1) { set_error("msb_scan_device_centrality: bin must be >= 1"); return MSB_EINVAL; }
+    if (half_bins < 0) { set_error("msb_scan_device_centrality: half_bins must be >= 0"); return MSB_EINVAL; }
+    const int64_t nb = 2 * (int64_t) half_bins + 1, cells = (int64_t) M->n * nb;
+    if (cells > MSB_CENTRALITY_MAX_CELLS) {
+        set_error("msb_scan_device_centrality: n_motifs * (2 half_bins + 1) exceeds MSB_CENTRALITY_MAX_CELLS");
+        return MSB_EINVAL;
+    }
+    MSB_TRY(check_final_sites(ctx, M->n, "msb_scan_device_centrality"));
+    if (n_seqs != ctx->last_n_seqs) { set_error("msb_scan_device_centrality: n_seqs differs from the scanned set"); return MSB_EINVAL; }
+    std::fill(hist_all, hist_all + cells, (int64_t) 0);
+    std::fill(hist_best, hist_best + cells, (int64_t) 0);
+    ctx->t[MSB_T_CENTRALITY] = 0;
+    if (ctx->last_sites == 0 || cells == 0) return MSB_OK;
+    MSB_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t n = ctx->last_sites;
+    MSB_TRY(ctx->ce_mid2.ensure((size_t) n_seqs * 4));
+    MSB_TRY(ctx->pr_count.ensure((size_t) cells * 16));
+    unsigned long long *d_all = ctx->pr_count.as<unsigned long long>(), *d_best = d_all + cells;
+    MSB_CUDA(cudaMemcpyAsync(ctx->ce_mid2.p, mid2, (size_t) n_seqs * 4, cudaMemcpyHostToDevice, st));
+    MSB_CUDA(cudaEventRecord(ctx->ev[6], st));
+    MSB_CUDA(cudaMemsetAsync(d_all, 0, (size_t) cells * 16, st));
+    centrality_kernel<<<(unsigned) ((n + kCentralityTile - 1) / kCentralityTile), 256, 0, st>>>(
+        ctx->fin_key, ctx->fin_seq, ctx->fin_start, ctx->fin_score, n, ctx->last_key_shift, M->d_len.as<int32_t>(),
+        ctx->ce_mid2.as<int32_t>(), bin, half_bins, ctx->opt_centrality_shared, d_all, d_best);
+    MSB_CUDA(cudaGetLastError());
+    MSB_CUDA(cudaEventRecord(ctx->ev[7], st));
+    MSB_CUDA(cudaMemcpyAsync(hist_all, d_all, (size_t) cells * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaMemcpyAsync(hist_best, d_best, (size_t) cells * 8, cudaMemcpyDeviceToHost, st));
+    MSB_CUDA(cudaStreamSynchronize(st));
+    ctx->t[MSB_T_CENTRALITY] = ev_ms(ctx->ev[6], ctx->ev[7]);
     return MSB_OK;
 }
 

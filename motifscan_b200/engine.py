@@ -117,6 +117,22 @@ class Context:
                                                                                      ctypes.c_int32), d, ptr(out, ctypes.c_int64)))
         return out
 
+    def centrality(self, motifs, mid2, bin, half_bins):
+        """(hist_all, hist_best), int64[n_motifs, 2 half_bins + 1] each: the last scan's final sites on this context by
+        bin floor((d2 + bin) / (2 bin)), d2 = 2 start + L - mid2[s], for bins -half_bins..half_bins; hist_best counts
+        the best site of each (motif, sequence) cell.  mid2[s] < 0 leaves sequence s out; len(mid2) must be the
+        scanned set's sequence count (msb_scan_device_centrality)."""
+        m = np.ascontiguousarray(np.asarray(mid2, dtype=np.int32).reshape(-1))
+        h = int(half_bins)
+        ok = h >= 0 and motifs.n * (2 * h + 1) <= _lib.CENTRALITY_MAX_CELLS
+        hist_all = np.zeros((motifs.n, 2 * h + 1) if ok else 1, dtype=np.int64)
+        hist_best = np.zeros_like(hist_all)
+        with self._lock:
+            check(self._lib.msb_scan_device_centrality(self._h, motifs._h, len(m), ptr(m if len(m) else np.zeros(1, np.int32),
+                                                                                        ctypes.c_int32), int(bin), h,
+                                                       ptr(hist_all, ctypes.c_int64), ptr(hist_best, ctypes.c_int64)))
+        return hist_all, hist_best
+
     def counters(self):
         a = np.zeros(len(_lib.C_NAMES), dtype=np.int64)
         check(self._lib.msb_ctx_counters(self._h, ptr(a, ctypes.c_int64), len(a)))

@@ -6,6 +6,7 @@ columns and number formatting (`str()` of ints and Python floats), fed from the 
     motif_sites/<id>_<name>_sites.bed   chrom, site start, start + L, '.', score, strand
     motif_enrichment.xls     sorted by (enriched p-value, -fold change)
     motif_variant_sites.xls / motif_variant_summary.xls   `motifscan variant` (write_variant_tables)
+    motif_centrality.xls / motif_site_distribution.xls   `scan --centrality` (write_centrality_tables)
 """
 import os
 import re
@@ -370,3 +371,29 @@ def write_spacing_table(output_dir, pwms, anchors, rows):
             out.write(f"{names[anchors[r.anchor]]}\t{names[r.partner]}\t{'same' if r.orientation == 0 else 'opposite'}\t"
                       f"{r.pairs}\t{na(r.peak_offset)}\t{na(r.peak_pairs)}\t{na(r.expected)}\t{na(r.p_value)}\t"
                       f"{','.join(map(str, r.counts.tolist()))}\n")
+
+
+CENTRALITY_HEADER = ("Motif_ID\tMotif_name\tLength\tTested_regions\tRegions_with_site\tHalf_width\tCentral_best_sites\t"
+                     "Expected\tRatio\tP_value\tCorrected_P_value\n")
+
+
+def write_centrality_tables(output_dir, pwms, result, rows):
+    """motif_centrality.xls: one row per motif (centrality.centrality_rows, in its order), `NA` where the motif has no
+    site in a tested region or no width to test; motif_site_distribution.xls: per motif a row of all its sites and a row
+    of the regions' best sites, one column per bin headed by the bin centre k B (bases from the summit)."""
+    os.makedirs(output_dir, exist_ok=True)
+
+    def na(v):
+        return "NA" if v is None or (isinstance(v, float) and np.isnan(v)) else str(v)
+    with open(os.path.join(output_dir, "motif_centrality.xls"), "w") as out:
+        out.write(CENTRALITY_HEADER)
+        for r in rows:
+            p = pwms[r.motif]
+            out.write(f"{p.matrix_id}\t{p.name}\t{r.length}\t{r.n_tested}\t{r.n_regions}\t{na(r.half_width)}\t"
+                      f"{na(r.central)}\t{na(r.expected)}\t{na(r.ratio)}\t{na(r.p_value)}\t{na(r.p_corrected)}\n")
+    K = (result.hist_all.shape[1] - 1) // 2
+    with open(os.path.join(output_dir, "motif_site_distribution.xls"), "w") as out:
+        out.write("Motif_ID\tMotif_name\tSites\t" + "\t".join(str(k * int(result.bin)) for k in range(-K, K + 1)) + "\n")
+        for m, p in enumerate(pwms):
+            for what, hist in (("all", result.hist_all), ("best", result.hist_best)):
+                out.write(f"{p.matrix_id}\t{p.name}\t{what}\t" + "\t".join(map(str, hist[m].tolist())) + "\n")

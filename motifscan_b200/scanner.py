@@ -15,6 +15,7 @@ from collections import namedtuple
 import numpy as np
 
 from . import engine
+from .centrality import CentralityResult, half_bins
 from .cooccur import PairResult
 
 logger = logging.getLogger(__name__)
@@ -101,10 +102,13 @@ class Scanner:
                 self._sequences = [c.decode("utf-8") for c in self._chunks]
         return self._sequences
 
-    def scan_motifs(self, pwms, ctx=None, pairs=None):
+    def scan_motifs(self, pwms, ctx=None, pairs=None, centrality=None):
         """Scan for motif occurrences; returns a `MotifSites` (nested-list view, (n_pwms,
         n_regions, n_sites)).  `pairs` (a cooccur.PairSpec): also reduce the final sites on the device to motif pair
-        counts and / or anchor spacing histograms, summed over the devices' blocks, as `MotifSites.pairs`."""
+        counts and / or anchor spacing histograms, summed over the devices' blocks, as `MotifSites.pairs`.
+        `centrality` (a bin width B, 1 <= B <= window_size // 2): also reduce them to the histograms of the sites'
+        offsets from the summits in the windows that no chromosome end clips, summed likewise, as
+        `MotifSites.centrality` (a centrality.CentralityResult)."""
         cutoffs = []
         for pwm in pwms:
             try:
@@ -115,10 +119,28 @@ class Scanner:
         lengths = [pwm.length for pwm in pwms]
         if pairs is not None and pairs.anchors and not all(0 <= int(a) < len(matrices) for a in pairs.anchors):
             raise ValueError("spacing anchor index out of range")
+        mid2 = None
+        if centrality is not None:
+            E, B = self.extend, int(centrality)
+            if self.window_size == 0 or E < 1:
+                raise ValueError("centrality needs summit-centred windows (window_size >= 2)")
+            if not 1 <= B <= E:
+                raise ValueError(f"centrality bin width must be 1..{E} (window_size // 2), got {B}")
+            K = half_bins(E, B)
+            # twice the summit's offset in its window, or -1 for a window a chromosome end clipped
+            mid2 = np.where(np.asarray(self.seq_ends, dtype=np.int64) - np.asarray(self.seq_starts, dtype=np.int64) == 2 * E,
+                            2 * E, -1).astype(np.int32)
+            n_tested = int((mid2 >= 0).sum())
+            if n_tested < len(mid2):
+                logger.info(f"Centrality: {len(mid2) - n_tested} of {len(mid2)} regions have windows clipped by a "
+                            "chromosome end and are left out")
         if not matrices:
             sites = MotifSites(None, 0, self.seq_starts, lengths)
             if pairs is not None:
                 sites.pairs = PairResult(np.zeros((0, 0), dtype=np.int64) if pairs.cooccur else None, len(self.seq_starts), None)
+            if centrality is not None:
+                empty = np.zeros((0, 2 * K + 1), dtype=np.int64)
+                sites.centrality = CentralityResult(empty, empty.copy(), n_tested, E, B)
             return sites
         if self._resident is not None:
             ctxs = [self._resident.ctx]       # the windows live where the genome lives
@@ -142,12 +164,17 @@ class Scanner:
             hist = c.spacing(motifs, list(pairs.anchors), pairs.max_offset) if pairs.anchors else None
             return counts, hist
 
+        def reduce_block(c, motifs, a, b):
+            """The reductions of the scan of regions a..b just run on `c` (the caller holds c._lock)."""
+            return (reduce_pairs(c, motifs, b - a) if pairs is not None else None,
+                    c.centrality(motifs, mid2[a:b], B, K) if centrality is not None else None)
+
         def scan_block(k):
             c, a, b = ctxs[k], bounds[k], bounds[k + 1]
             motifs = engine.MotifSet(c, matrices, cutoffs)
             try:
                 # the reductions read the scan's sites on the device: no other scan on a shared context may come between
-                with c._lock if pairs is not None else contextlib.nullcontext():
+                with c._lock if pairs is not None or centrality is not None else contextlib.nullcontext():
                     if self._resident is not None or self._packed is not None:
                         dg = self._resident if self._resident is not None else self._packed_on(c)
                         sset = dg.extract(self._chroms[a:b], self.seq_starts[a:b], self.seq_ends[a:b])
@@ -162,9 +189,9 @@ class Scanner:
                             np.cumsum([len(x) for x in chunks], out=off[1:])
                         blob = np.frombuffer(b"".join(chunks), dtype=np.uint8)
                         res = engine.scan_ascii(c, motifs, blob, off, strand, remove_dup=self.remove_dup)
-                    if pairs is None:
+                    if pairs is None and centrality is None:
                         return res, None
-                    return res, reduce_pairs(c, motifs, b - a)
+                    return res, reduce_block(c, motifs, a, b)
             finally:
                 motifs.close()
 
@@ -179,11 +206,13 @@ class Scanner:
             res = _MergedResult([r for r, _ in out], bounds[:-1], len(matrices), n)
             blocks = [p for _, p in out]
         sites = MotifSites(res, len(matrices), self.seq_starts, lengths)
+        # the blocks hold disjoint regions: their counts and histograms add up
         if pairs is not None:
-            # the blocks hold disjoint regions: their counts and histograms add up
-            counts = sum(p[0] for p in blocks) if pairs.cooccur else None
-            hist = sum(p[1] for p in blocks) if pairs.anchors else None
+            counts = sum(p[0][0] for p in blocks) if pairs.cooccur else None
+            hist = sum(p[0][1] for p in blocks) if pairs.anchors else None
             sites.pairs = PairResult(counts, n, hist)
+        if centrality is not None:
+            sites.centrality = CentralityResult(sum(p[1][0] for p in blocks), sum(p[1][1] for p in blocks), n_tested, E, B)
         return sites
 
     def _packed_on(self, ctx):
@@ -242,6 +271,7 @@ class MotifSites:
         self.seq_starts = list(seq_starts)
         self.lengths = list(lengths)
         self.pairs = None    # cooccur.PairResult when the scan was asked for pair reductions
+        self.centrality = None    # centrality.CentralityResult when the scan was asked for the positional histograms
         if res is None:
             self._off = np.zeros(n_pwms + 1, dtype=np.int64)
             self._seq_idx = np.zeros(0, dtype=np.int32)
